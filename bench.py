@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the WeatherConverter hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c3|c2|c1|c5|ref] [--graph 0|1]
+                    [--dump-outputs DIR]
 
 Default workload (every N, weak scaling) = the configuration BASELINE.json's metric is quoted on:
   c3  SGG-guided translation at 256x512 (BASELINE.json configs[2]/[3]), batch 32 per GPU, N = 500 reverse steps,
@@ -108,6 +109,25 @@ class ClockSampler(threading.Thread):
         self.join(timeout=2)
         return {"sm_mhz": statistics.median(self.samples) if self.samples else None, "sm_max_mhz": self.max_mhz,
                 "reasons": sorted(self.reasons), "samples": len(self.samples)}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each array as <out_dir>/<name>.npy in float32.  An array over its share of DUMP_BYTES is written
+    as a fixed sample of its flattened elements (indices drawn with seed 0, ascending), so that two builds run with the same
+    arguments can be compared value for value."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > cap:
+            idx = torch.randint(0, t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def block_labels(gen, B, H, W, blk=8):
@@ -364,6 +384,8 @@ def run_train(args):
     launches = ops.launch_count() - l0
     ms_total = e0.elapsed_time(e1)
     loss_val = float(loss)
+    if args.dump_outputs and rank == 0:   # the last timed step's loss and the weights it left, before the e2e leg moves them
+        dump_outputs(args.dump_outputs, {"loss": loss, "params": trainer.flat_params[:trainer.used]})
     # e2e: batch from pinned host memory, loss read back each step (as the reference's loss.item(), train_ddpm.py:116)
     x_dev = torch.empty_like(imgs[0])
     barrier()
@@ -612,7 +634,11 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the short C5 (NCCL) record at N > 1")
     ap.add_argument("--resident-only", action="store_true", help="eager resident leg only (ncu launch lists)")
     ap.add_argument("--cpu-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last timed step as "
+                    "DIR/<name>.npy (float32, 64 MB at most; rank 0's shard at N > 1): x_prev, or loss and params for c5")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU arm's outputs")
     if args.impl == "reference":
         return run_reference(args)
     if WORKLOADS[args.workload]["kind"] == "train":
@@ -700,6 +726,8 @@ def main():
         sampler.start()
         ms_total = timed(lambda k: wl.graph_step(k, zs[k % 4]), K)
         clocks = sampler.finish()
+        if args.dump_outputs and rank == 0:   # x_{t-1} of the last timed step, before the e2e leg steps on from it
+            dump_outputs(args.dump_outputs, {"x_prev": wl.sg.xt})
         finite = finite and bool(torch.isfinite(wl.sg.xt).all())
         launches = wl.launches_per_step * K
         # ---------------- end-to-end leg: z from pinned host memory, x_{t-1} read back each step ----------------
@@ -713,6 +741,8 @@ def main():
         sampler.start()
         ms_total = timed(eager_step, K)
         clocks = sampler.finish()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"x_prev": state["xt"]})
         launches = eager_launches
         z_dev = torch.empty_like(x0)
 

@@ -4,7 +4,8 @@ Runs only where /root/reference exists (the build container):
     python tests/golden/make_golden.py
 Every tensor below is produced by the reference's own modules/functions (imported through
 ref_shim); the oracle is NOT involved.  Weights come from oracle.weights.synth_state_dict, a pure
-function of (name, shape, seed), loaded into the reference modules with load_state_dict.
+function of (name, shape, seed), loaded into the reference modules with load_state_dict.  The seeded
+inputs of the larger fixtures come from golden_inputs.py and are not stored (see there).
 """
 import os
 import sys
@@ -18,7 +19,10 @@ import ref_shim  # noqa: E402
 ref_shim.install()
 import io  # noqa: E402
 import contextlib  # noqa: E402
+import lzma  # noqa: E402
 import torch  # noqa: E402
+import golden_inputs  # noqa: E402
+from golden_inputs import block_labels  # noqa: E402
 from oracle.weights import synth_state_dict  # noqa: E402
 from oracle.unet import DEFAULT_MODEL_CONFIG  # noqa: E402
 
@@ -34,10 +38,29 @@ from sgg.sgg import apply_gsg  # noqa: E402
 torch.set_num_threads(os.cpu_count())
 
 
-def save(name, obj):
+def _drop_inputs(obj, inputs):
+    for k, v in inputs.items() if isinstance(inputs, dict) else enumerate(inputs):
+        if isinstance(v, torch.Tensor):
+            obj.pop(k, None)
+        else:
+            _drop_inputs(obj[k], v)
+
+
+def save(name, obj, inputs=None, xz=False):
+    """With `inputs` (drawn by golden_inputs.py) the fixture keeps their digest instead of the tensors; `xz` compresses it."""
+    if inputs is not None:
+        _drop_inputs(obj, inputs)
+        obj["inputs_sha256"] = golden_inputs.digest(inputs)
     path = os.path.join(HERE, name)
-    torch.save(obj, path)
-    print(f"{name}: {os.path.getsize(path) / 1024:.0f} KiB")
+    if xz:
+        buf = io.BytesIO()
+        torch.save(obj, buf)
+        path += ".xz"
+        with open(path, "wb") as f:
+            f.write(lzma.compress(buf.getvalue(), preset=9))
+    else:
+        torch.save(obj, path)
+    print(f"{os.path.basename(path)}: {os.path.getsize(path) / 1024:.0f} KiB")
 
 
 class InjectedRandn:
@@ -140,20 +163,12 @@ def seg_for(backbone, seed, output_stride=16):
     return m
 
 
-def block_labels(g, B, H, W, blk=8):
-    lab = torch.randint(0, 19, (B, H // blk, W // blk), generator=g)
-    ign = torch.rand(B, H // blk, W // blk, generator=g) < 0.05
-    lab[ign] = 255
-    return lab.repeat_interleave(blk, 1).repeat_interleave(blk, 2)
-
-
 def g_seg():
     out = {}
-    g = torch.Generator().manual_seed(31)
-    for backbone, (H, W) in (("resnet50", (64, 128)), ("resnet50", (128, 256)), ("resnet101", (64, 128))):
+    inputs = golden_inputs.seg_infer()
+    for backbone, (H, W) in golden_inputs.SEG_INFER_CASES:
         m = seg_for(backbone, 42)
-        x = torch.rand(1, 3, H, W, generator=g)
-        gt = block_labels(g, 1, H, W)
+        x, gt = inputs[f"{backbone}_{H}x{W}"]["x"], inputs[f"{backbone}_{H}x{W}"]["gt"]
         feats = {}
         hook = m.classifier.classifier.register_forward_hook(lambda mod, i, o: feats.__setitem__("low", o.detach()))
         with contextlib.redirect_stdout(io.StringIO()):
@@ -162,7 +177,7 @@ def g_seg():
         out[f"{backbone}_{H}x{W}"] = dict(seed=42, x=x, gt=gt, logits_lowres=feats["low"],
                                            pred=torch.from_numpy(pred).to(torch.uint8), grad=grad.detach().clone())
         print(backbone, H, W, float(grad.abs().max()))
-    save("seg_infer.pt", out)
+    save("seg_infer.pt", out, inputs)
     g_seg_os8()
 
 
@@ -188,22 +203,20 @@ def g_seg_conditioned():
     is multiplied by 0.2, i.e. residual branches are small corrections of the identity path as in a trained ResNet
     (zero_init_residual training recipes start them at 0).  The plain random-init net of seg_infer.pt is chaotic at bf16
     resolution (DESIGN.md section 4); this one is not, so the gradient tolerance can be tight."""
-    g = torch.Generator().manual_seed(131)
-    H, W = 128, 256
+    inputs = golden_inputs.seg_conditioned()
     m = network.modeling.deeplabv3plus_resnet50(num_classes=19, output_stride=16, pretrained_backbone=False).eval()
     sd = synth_state_dict(m.state_dict(), 42)
     for k in sd:
         if k.endswith("bn3.weight"):
             sd[k] = sd[k] * 0.2
     m.load_state_dict(sd)
-    x = torch.rand(2, 3, H, W, generator=g)
-    gt = block_labels(g, 2, H, W)
+    x, gt = inputs["x"], inputs["gt"]
     preds, grads = [], []
     for b in range(2):
         with contextlib.redirect_stdout(io.StringIO()):
             pred, grad, _ = seg_infer.infer(m, x[b:b + 1].clone(), gt[b:b + 1])
         preds.append(torch.from_numpy(pred).to(torch.uint8)); grads.append(grad.detach().clone())
-    save("seg_conditioned.pt", dict(seed=42, bn3_gain=0.2, x=x, gt=gt, pred=torch.stack(preds), grad=torch.cat(grads)))
+    save("seg_conditioned.pt", dict(seed=42, bn3_gain=0.2, x=x, gt=gt, pred=torch.stack(preds), grad=torch.cat(grads)), inputs)
 
 
 def g_srgan():
@@ -334,22 +347,21 @@ def g_train():
 
 def g_legacy():
     """Legacy old_modules.UNet (eval) forward, B=2, and 3 steps of the sample_integrated loop (sample_integrated.py:52-65)
-    with recorded noise."""
+    with recorded noise; each trajectory step is kept at the fixed element sample golden_inputs.legacy_unet()["traj_idx"]."""
     from diffusion_model.models.old_modules import UNet as LegacyUNet
     m = LegacyUNet().eval()
     sd = synth_state_dict(m.state_dict(), 21)
     m.load_state_dict(sd)
     sched = LinearNoiseScheduler(1000, 1e-4, 0.02)
-    g = torch.Generator().manual_seed(91)
-    x = torch.randn(2, 3, 128, 128, generator=g)
+    inputs = golden_inputs.legacy_unet()
+    x = inputs["x"]
     t_idx = torch.tensor([40, 900])
     out = dict(seed=21, x=x, t_idx=t_idx)
     with torch.no_grad():
         out["y"] = m(x, sched.one_minus_cum_prod[t_idx].view(-1, 1, 1, 1))
         T = 3
-        xt = torch.randn(2, 3, 128, 128, generator=g)
-        zs = [torch.randn(2, 3, 128, 128, generator=g) for _ in range(T)]
-        out["xT"], out["zs"], traj = xt.clone(), torch.stack(zs), []
+        xt, zs = inputs["xT"].clone(), inputs["zs"]
+        out["xT"], out["zs"], traj = xt.clone(), zs, []
         for i in reversed(range(T)):
             t = torch.full((xt.size(0),), i, dtype=torch.long)
             noise_pred = m(xt, sched.one_minus_cum_prod[t].view(-1, 1, 1, 1))
@@ -357,8 +369,8 @@ def g_legacy():
                 mean, sigma, _ = sched.sample_prev_timestep2(xt, noise_pred, t)
             xt = mean + sigma if i != 0 else mean
             traj.append(xt.clone())
-        out["traj"] = torch.stack(traj)
-    save("legacy_unet.pt", out)
+        out["traj"] = torch.stack(traj).flatten(1)[:, inputs["traj_idx"]].clone()
+    save("legacy_unet.pt", out, inputs)
 
 
 def g_io():
@@ -373,12 +385,10 @@ def g_io():
     from seg_model.datasets.acdc import ACDCDataset
     from seg_model.utils.ext_transforms import ExtCompose, ExtResize, ExtCenterCrop, ExtToTensor, ExtNormalize
     from diffusion_model.sample_integrated import postprocess
-    rng = np.random.default_rng(2024)
+    inputs = golden_inputs.image_io()
     out = {}
     # --- seg preprocessing (inference.py:75-82,103-104): label ids 0..33 in 16x16 blocks + a small image
-    lab = np.kron(rng.integers(0, 34, (68, 120), dtype=np.uint8), np.ones((16, 16), dtype=np.uint8))[:1080, :1920]
-    lab = (lab + (rng.random(lab.shape) < 0.02) * 1).clip(0, 33).astype(np.uint8)
-    img_small = rng.integers(0, 256, (96, 160, 3), dtype=np.uint8)
+    lab, img_small = inputs["label_ids"].numpy(), inputs["image_small"].numpy()
     val_transform = ExtCompose([ExtResize(size=(1080 // 2, 1920 // 2), interpolation=Image.BILINEAR, just_label=True),
                                 ExtCenterCrop(size=(512, 512), just_label=True), ExtToTensor(),
                                 ExtNormalize(mean=[0.485, 0.456, 0.406], std=[0.229, 0.224, 0.225])])
@@ -392,13 +402,11 @@ def g_io():
     tf = transforms.Compose([transforms.Resize(128, transforms.InterpolationMode.BILINEAR), transforms.CenterCrop(128),
                              transforms.ToTensor(), transforms.Lambda(lambd=lambda x: x * 2.0 - 1.0)])
     out["diffusion_inputs"] = []
-    for (h, w) in ((405, 720), (333, 500), (200, 150)):
-        im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-        im = np.clip(im // 3 + np.linspace(0, 160, w, dtype=np.int64)[None, :, None], 0, 255).astype(np.uint8)   # gradients + noise
+    for e in inputs["diffusion_inputs"]:
+        im = e["image"].numpy()
         out["diffusion_inputs"].append(dict(image=torch.from_numpy(im), tensor=tf(Image.fromarray(im)).unsqueeze(0)))
     # --- sample_ddpm.py:47-51
-    g = torch.Generator().manual_seed(8)
-    xt = torch.randn(5, 3, 24, 40, generator=g) * 0.8
+    xt = inputs["ddpm_xt"]
     ims = torch.clamp(xt, -1., 1.).detach().cpu()
     ims = (ims + 1) / 2
     grid = make_grid(ims, nrow=2)
@@ -407,9 +415,9 @@ def g_io():
     grid1 = make_grid(ims[:1], nrow=2)
     out["ddpm_grid_single"] = torch.from_numpy(np.array(torchvision.transforms.ToPILImage()(grid1)))
     # --- sample_integrated.postprocess
-    xl = torch.randn(2, 3, 16, 24, generator=g) * 2.0
+    xl = inputs["legacy_xt"]
     out["legacy_xt"], out["legacy_u8"] = xl, postprocess(xl)
-    save("image_io.pt", out)
+    save("image_io.pt", out, inputs, xz=True)
 
 
 if __name__ == "__main__":
