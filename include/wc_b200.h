@@ -227,7 +227,8 @@ int wc_unet_launches(const wc_unet* net);
  * gradient buffer (the host keeps them in flat buffers; see weatherconverter_b200/diffusion_model/train_ddpm.py).
  * bind builds the forward / backward launch plans for one [batch,3,H,W] shape in the given workspace.
  * forward: (repack != 0: rebuild the bf16 packed weights from the fp32 parameters first) pred = Unet(x, t) with
- * t int64 [batch]; loss[0] = mean((pred - target)^2) (nn.MSELoss, :107); pred_out may be NULL.
+ * t int64 [batch]; loss[0] = mean((pred - target)^2) (nn.MSELoss, :107); pred_out may be NULL.  target == NULL: no
+ * loss is computed (loss_out may be NULL, pred_out is required) and the backward must be the seeded one.
  * backward(op_begin, op_end): runs that slice of the backward plan (loss.backward(), :108); running all
  * [0, num_backward_ops) fills every gradient buffer (overwrite, like zero_grad + backward).  grad_ready_op(name) is
  * the op count after which that parameter's gradient is final, so the host can overlap bucketed all-reduces. */
@@ -241,6 +242,10 @@ int wc_unet_train_forward(wc_unet_train* net, const float* x, const int64_t* t, 
                           float* loss_out, float grad_scale, int repack, void* stream);
 int wc_unet_train_num_backward_ops(const wc_unet_train* net);
 int wc_unet_train_backward(wc_unet_train* net, int op_begin, int op_end, void* stream);
+/* Backward of the last wc_unet_train_forward seeded with dpred = dL/d(noise_pred), nchw fp32 [B,3,H,W].
+ * dx: nchw fp32 [B,3,H,W] receives dL/dx, or NULL.  param_grads == 0: skip every launch whose only product is a
+ * parameter gradient.  Parameter gradients (when computed) go to the grads pointers given at create, overwritten. */
+int wc_unet_train_backward_seeded(wc_unet_train* net, const float* dpred, float* dx, int param_grads, void* stream);
 int wc_unet_train_grad_ready_op(const wc_unet_train* net, const char* name);
 double wc_unet_train_flops(const wc_unet_train* net, int backward);
 

@@ -94,6 +94,7 @@ _SIGS = {
     "wc_unet_train_forward": (C.c_int, [c_ptr] * 6 + [C.c_float, C.c_int, c_ptr]),
     "wc_unet_train_num_backward_ops": (C.c_int, [c_ptr]),
     "wc_unet_train_backward": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr]),
+    "wc_unet_train_backward_seeded": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, c_ptr]),
     "wc_unet_train_grad_ready_op": (C.c_int, [c_ptr, C.c_char_p]),
     "wc_unet_train_flops": (C.c_double, [c_ptr, C.c_int]),
     "wc_legacy_unet_create": (C.c_int, [C.POINTER(c_ptr), C.c_int, C.POINTER(C.c_char_p), C.POINTER(c_ptr), C.POINTER(C.c_int64)]),

@@ -10,6 +10,10 @@
 // residual branches), so fan-in never needs a separate add kernel.  Weight-dependent device state (bf16 packed
 // weights of the forward and data-gradient GEMMs, folded biases, the concatenated t-embedding projection) is rebuilt
 // by `repack_ops` at the start of every step because the optimizer changes the fp32 master weights.
+//
+// The same backward also runs seeded with a caller's dL/dpred (wc_unet_train_backward_seeded: torch autograd of the
+// Unet module, diffusion_model/models/unet_base.py), optionally producing dL/dx and optionally skipping every op whose
+// only product is a parameter gradient.
 #include <map>
 
 #include "plan.cuh"
@@ -66,6 +70,7 @@ struct wc_unet_train {
   void* ws = nullptr;
   size_t ws_bytes = 0, ws_needed = 0;
   wc::OpList repack_ops, fwd_ops, bwd_ops;
+  std::vector<int> bwd_kind;  // per backward op: what it produces (kOpData / kOpParam / kOpInput)
   std::unordered_map<std::string, int> ready;  // parameter name -> number of backward ops after which its grad is final
   double flops_fwd = 0, flops_bwd = 0;
   // per-call pointers
@@ -75,10 +80,16 @@ struct wc_unet_train {
   float* pred_out = nullptr;
   float* loss_out = nullptr;
   float grad_scale = 1.f;
+  const float* dpred_seed = nullptr;  // upstream gradient of a seeded backward; NULL: the loss gradient of the forward
+  float* dx_out = nullptr;            // dL/dx of a seeded backward, or NULL
 };
 
 namespace wc {
 namespace {
+
+// What a backward op produces.  A seeded backward without parameter gradients skips every kOpParam op; a kOpInput op
+// launches only when the caller asked for dL/dx.
+enum { kOpData = 0, kOpParam = 1, kOpInput = 2 };
 
 struct TBuilder {
   wc_unet_train* net;
@@ -159,8 +170,9 @@ struct TBuilder {
     }
     return it->second;
   }
-  void push(std::function<int(cudaStream_t)> f) {
+  void push(std::function<int(cudaStream_t)> f, int kind = kOpData) {
     if (dry) return;
+    if (in_bwd) net->bwd_kind.push_back(kind);
     (in_bwd ? net->bwd_ops : net->fwd_ops).push_back(std::move(f));
   }
   void ready(const std::string& n) {
@@ -270,7 +282,7 @@ struct TBuilder {
                        : build_conv_wgrad(op.get(), x, dy, K, stride, pad, 1, dw, x2, dw2, wg_partial);
     if (e) { err = e; return; }
     net->flops_bwd += op->flops;
-    push([op](cudaStream_t s) { return op->run(s); });
+    push([op](cudaStream_t s) { return op->run(s); }, kOpParam);
     ready(wname + ".weight");
     if (x2) ready(w2name + ".weight");
   }
@@ -286,7 +298,7 @@ struct TBuilder {
       if (int e = colsum(dy.ptr, dy.B, dy.H * dy.W, C, dy.ld, rows, ldo, db, ws, s)) return e;
       if (db2) WC_CHECK_CUDA(cudaMemcpyAsync(db2, db, C * sizeof(float), cudaMemcpyDeviceToDevice, s));
       return 0;
-    });
+    }, kOpParam);
     ready(bname);
     if (db2) ready(bname2);
   }
@@ -395,7 +407,7 @@ struct TBuilder {
           auto wop = std::make_shared<WgradOp>();
           if (!err) {
             if (int e = build_conv_wgrad(wop.get(), a, dqkv, 1, 1, 0, 1, dw, nullptr, nullptr, wg_partial)) err = e;
-            else { net->flops_bwd += wop->flops; push([wop](cudaStream_t s) { return wop->run(s); }); }
+            else { net->flops_bwd += wop->flops; push([wop](cudaStream_t s) { return wop->run(s); }, kOpParam); }
           }
           ready(ap + ".in_proj_weight");
         }
@@ -450,12 +462,13 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
   void* mse_scratch = b.bump.take(8192);
   void* bw_scratch = b.bump.take(boundary_wgrad_scratch_bytes());
 
-  float *wcat = nullptr, *bcat = nullptr, *w_out_t = nullptr;
+  float *wcat = nullptr, *bcat = nullptr, *w_out_t = nullptr, *w_in_t = nullptr;
   if (!dry) {
     wcat = static_cast<float*>(b.arena->alloc(static_cast<size_t>(total) * T * 4));
     bcat = static_cast<float*>(b.arena->alloc(static_cast<size_t>(total) * 4));
     w_out_t = static_cast<float*>(b.arena->alloc(static_cast<size_t>(dc[0]) * c.im_channels * 9 * 4));
-    if (!wcat || !bcat || !w_out_t) return 1;
+    w_in_t = static_cast<float*>(b.arena->alloc(static_cast<size_t>(dc[0]) * c.im_channels * 9 * 4));
+    if (!wcat || !bcat || !w_out_t || !w_in_t) return 1;
     int off = 0;
     for (auto& e : tl) {
       const float *wsrc = b.P(e.first + ".weight"), *bsrc = b.P(e.first + ".bias");
@@ -500,15 +513,22 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
     });
     net->flops_fwd += 2.0 * B * H * W * 9.0 * cin * c0;
   }
-  b.tape.push_back([&b, skip0, net, B, H, W, bw_scratch]() {
+  b.tape.push_back([&b, skip0, net, B, H, W, bw_scratch, w_in_t]() {
     Act d = b.grad_written(skip0);
     if (b.dry) return;
+    const float* w = b.P("conv_in.weight");
     float *dw = b.G("conv_in.weight"), *db = b.G("conv_in.bias");
     if (b.err) return;
     wc_unet_train* n = net;
-    b.push([=](cudaStream_t s) { return boundary_wgrad(d.ptr, d.ld, n->x_in, B, H, W, +1, dw, db, bw_scratch, s); });
+    const int cin = net->cfg.im_channels, c0 = d.C;
+    b.push([=](cudaStream_t s) { return boundary_wgrad(d.ptr, d.ld, n->x_in, B, H, W, +1, dw, db, bw_scratch, s); }, kOpParam);
     b.ready("conv_in.weight");
     b.ready("conv_in.bias");
+    // dL/dx: the 64 -> 3 convolution of d(skip0) with the flipped, transposed conv_in weight (conv_out's forward kernel)
+    net->repack_ops.push_back([=](cudaStream_t s) { return flip_transpose_3x3(w, w_in_t, c0, cin, s); });
+    b.push([=](cudaStream_t s) {
+      return n->dx_out ? conv_small_cout(d.ptr, w_in_t, nullptr, n->dx_out, B, H, W, c0, cin, 3, d.ld, 0, s) : 0;
+    }, kOpInput);
   });
   Act cur = skip0;
 
@@ -608,6 +628,7 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
     b.push([=](cudaStream_t s) {
       float* pred = n->pred_out ? n->pred_out : pred_ws;
       if (int e = conv_small_cout(fin.ptr, w, bias, pred, B, H, W, cin, co, 3, fin.ld, 0, s)) return e;
+      if (!n->target) return 0;     // no loss: the backward is seeded with dL/dpred by the caller
       return mse_loss_grad(pred, n->target, dpred, numel, n->grad_scale, n->loss_out, mse_scratch, s);
     });
     net->flops_fwd += 2.0 * B * H * W * 9.0 * cin * co;
@@ -623,10 +644,15 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
       float *dw = b.G("conv_out.weight"), *db = b.G("conv_out.bias");
       if (b.err) return b.err;
       const int cin = dc[0], co = c.im_channels;
+      wc_unet_train* n = net;
       b.push([=](cudaStream_t s) {
-        if (int e = conv_small_cin(dpred, w_out_t, nullptr, nullptr, nullptr, dfin.ptr, B, co, H, W, cin, 3, 1, 1, dfin.ld, 0, s)) return e;
-        return boundary_wgrad(fin.ptr, fin.ld, dpred, B, H, W, -1, dw, db, bw_scratch, s);
+        const float* dp = n->dpred_seed ? n->dpred_seed : dpred;
+        return conv_small_cin(dp, w_out_t, nullptr, nullptr, nullptr, dfin.ptr, B, co, H, W, cin, 3, 1, 1, dfin.ld, 0, s);
       });
+      b.push([=](cudaStream_t s) {
+        const float* dp = n->dpred_seed ? n->dpred_seed : dpred;
+        return boundary_wgrad(fin.ptr, fin.ld, dp, B, H, W, -1, dw, db, bw_scratch, s);
+      }, kOpParam);
       net->flops_bwd += 4.0 * B * H * W * 9.0 * cin * co;
       b.ready("conv_out.weight");
       b.ready("conv_out.bias");
@@ -659,7 +685,7 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
     b.push([=](cudaStream_t s) {
       return temb_backward(dtp, total, B, T, wcat, w2, emb, h1, temb, temb_silu, nseg, segs_row0->data(), segs_rows->data(),
                            segs_dw->data(), segs_db->data(), dw1, db1, dw2, db2, temb_scratch, s);
-    });
+    }, kOpParam);
     for (auto& e : tl) { b.ready(e.first + ".weight"); b.ready(e.first + ".bias"); }
     b.ready("t_proj.0.weight"); b.ready("t_proj.0.bias"); b.ready("t_proj.2.weight"); b.ready("t_proj.2.bias");
   }
@@ -710,21 +736,21 @@ int wc_unet_train_bind(wc_unet_train* net, int batch, int H, int W, void* worksp
   int div = 1;
   for (int i = 0; i + 1 < net->cfg.n_down_channels; ++i) if (net->cfg.down_sample[i]) div *= 2;
   WC_REQUIRE(H % div == 0 && W % div == 0, "H and W must be divisible by the total down-sampling factor");
-  net->repack_ops.clear(); net->fwd_ops.clear(); net->bwd_ops.clear(); net->ready.clear();
+  net->repack_ops.clear(); net->fwd_ops.clear(); net->bwd_ops.clear(); net->bwd_kind.clear(); net->ready.clear();
   net->arena = std::make_unique<DeviceArena>();
   net->B = batch; net->H = H; net->W = W; net->ws = workspace; net->ws_bytes = workspace_bytes;
   net->flops_fwd = net->flops_bwd = 0;
   set_pack_recorder(&net->repack_ops);
   const int e = build(net, false, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
   set_pack_recorder(nullptr);
-  if (e) { net->B = 0; net->fwd_ops.clear(); net->bwd_ops.clear(); net->repack_ops.clear(); }
+  if (e) { net->B = 0; net->fwd_ops.clear(); net->bwd_ops.clear(); net->bwd_kind.clear(); net->repack_ops.clear(); }
   return e;
 }
 
 int wc_unet_train_forward(wc_unet_train* net, const float* x, const int64_t* t, const float* target, float* pred_out,
                           float* loss_out, float grad_scale, int repack, void* stream) {
   WC_REQUIRE(net && net->B > 0, "wc_unet_train_forward: not bound");
-  WC_REQUIRE(x && t && target && loss_out, "null argument");
+  WC_REQUIRE(x && t && (target ? loss_out != nullptr : pred_out != nullptr), "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   net->x_in = x; net->t_in = reinterpret_cast<const long long*>(t); net->target = target; net->pred_out = pred_out;
   net->loss_out = loss_out; net->grad_scale = grad_scale;
@@ -742,9 +768,25 @@ int wc_unet_train_backward(wc_unet_train* net, int op_begin, int op_end, void* s
   WC_REQUIRE(net && net->B > 0, "wc_unet_train_backward: not bound");
   WC_REQUIRE(op_begin >= 0 && op_end <= static_cast<int>(net->bwd_ops.size()) && op_begin <= op_end, "bad op range");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  net->dpred_seed = nullptr;
+  net->dx_out = nullptr;
   for (int i = op_begin; i < op_end; ++i)
     if (int e = net->bwd_ops[i](st)) return e;
   return 0;
+}
+
+int wc_unet_train_backward_seeded(wc_unet_train* net, const float* dpred, float* dx, int param_grads, void* stream) {
+  WC_REQUIRE(net && net->B > 0, "wc_unet_train_backward_seeded: not bound");
+  WC_REQUIRE(dpred, "null argument");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  net->dpred_seed = dpred;
+  net->dx_out = dx;
+  int err = 0;
+  for (size_t i = 0; i < net->bwd_ops.size() && !err; ++i)
+    if (param_grads || net->bwd_kind[i] != kOpParam) err = net->bwd_ops[i](st);
+  net->dpred_seed = nullptr;
+  net->dx_out = nullptr;
+  return err;
 }
 
 int wc_unet_train_grad_ready_op(const wc_unet_train* net, const char* name) {

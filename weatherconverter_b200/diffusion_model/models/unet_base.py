@@ -5,13 +5,24 @@
 names and shapes (382 tensors for config.yaml), so reference checkpoints load with ``load_state_dict``.
 
 The module only owns parameters and device buffers; the layer graph, weight re-packing (bf16, K-major) and all
-arithmetic live in the C library (csrc/unet.cu).  Inference only: outputs carry no autograd graph.
+arithmetic live in the C library (csrc/unet.cu).  By default outputs carry no autograd graph.
+
+Autograd (opt-in): with ``model.differentiable = True``, grad mode on and ``x`` or any parameter requiring grad,
+``forward`` runs the training plan (csrc/unet_train.cu) under a ``torch.autograd.Function`` whose inputs are ``x``,
+``t`` and every parameter, so ``loss.backward()`` with any loss, hooks, ``clip_grad_norm_``, gradient accumulation
+and any ``torch.optim`` optimizer work as on the reference module; ``x.grad`` is dL/dx.  The backward is
+``wc_unet_train_backward_seeded`` fed with dL/d(noise_pred); it skips the parameter-gradient launches when no
+parameter needs a gradient.  A graph holds one training plan (its saved activations) until its backward has run or
+it is freed; the plans live in a pool per (B, H, W).  A graph can be backpropagated once (no ``retain_graph``
+re-backward, no double backward).  The switch is off by default because the training plan keeps every activation
+and is slower than the inference plan, which sampling and translation call with grad mode on.
 """
 import ctypes as C
 import math
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from ..._lib import UnetConfigStruct, check, lib, ptr, stream_ptr
@@ -136,6 +147,9 @@ class Unet(nn.Module):
         self._workspaces = {}
         self._keepalive = None
         self._weights_epoch = 0      # bumped by DenoisingTrainer.optimizer_step (in-place kernel updates of the weights)
+        self.differentiable = False  # True: forward under grad mode builds an autograd graph (module docstring)
+        self._train_plans = {}       # (B, H, W) -> [_TrainPlan]: the autograd path's plan pool
+        self._train_key = None
 
     def _register(self, dotted, param):
         node = self
@@ -211,6 +225,26 @@ class Unet(nn.Module):
             self._workspaces[k] = ws
         return ws
 
+    def _lease_plan(self, B, H, W, device):
+        """A free training plan for (B, H, W), created when every plan of that shape is held by a live graph.  The pool is
+        rebuilt when a parameter's storage changes (.to(), load_state_dict with new tensors); in-place updates of the
+        weights need no rebuild because every differentiable forward re-packs them."""
+        named = list(self.named_parameters())
+        key = (str(device), tuple(p.data_ptr() for _, p in named))
+        if key != self._train_key:
+            for n, p in named:
+                if p.device != device or p.dtype != torch.float32 or not p.is_contiguous():
+                    raise RuntimeError(f"Unet parameter {n} must be a contiguous fp32 tensor on {device}; call .to(device)")
+            set_time_factor_table(self.t_emb_dim, device)
+            self._train_plans, self._train_key = {}, key
+        plans = self._train_plans.setdefault((B, H, W), [])
+        plan = next((p for p in plans if not p.busy), None)
+        if plan is None:
+            plan = _TrainPlan(self._config_struct(), named, B, H, W, device)
+            plans.append(plan)
+        plan.busy = True
+        return plan
+
     # ---- reference API ---------------------------------------------------------------------------------
     def forward(self, x, t, out=None):
         _lib.require_cuda(x)
@@ -221,6 +255,13 @@ class Unet(nn.Module):
         t = torch.as_tensor(t).long().to(x.device).reshape(-1)     # reference :461
         if t.numel() not in (1, B):
             raise RuntimeError("t must have 1 or batch entries")
+        if self.differentiable and torch.is_grad_enabled():
+            params = list(self.parameters())
+            if x.requires_grad or any(p.requires_grad for p in params):
+                if out is not None:
+                    raise RuntimeError("Unet.forward: out= cannot be combined with the autograd path "
+                                       "(differentiable = True under grad mode)")
+                return _UnetTrainFunction.apply(self, x, t.expand(B).contiguous(), *params)
         self._ensure_handle(x.device)
         ws = self._workspace(B, H, W, x.device)
         if out is None:
@@ -236,6 +277,95 @@ class Unet(nn.Module):
 
     def launches_per_forward(self) -> int:
         return int(lib().wc_unet_launches(self._handle)) if self._handle is not None else 0
+
+
+class _TrainPlan:
+    """One training plan of the C library bound to (B, H, W) with its own workspace and flat fp32 gradient buffer (every
+    tensor's slice 16-byte aligned, as in DenoisingTrainer).  Its parameter pointers are the module's parameters, kept
+    alive here because the backward reads GroupNorm and t-embedding weights in place."""
+
+    def __init__(self, cfg, named, B, H, W, device):
+        self.handle, self.busy = None, False
+        self.slices, off = [], 0
+        for _, p in named:
+            off = (off + 3) & ~3
+            self.slices.append((off, p.numel(), p.shape))
+            off += p.numel()
+        self.grads = torch.zeros(off, device=device, dtype=torch.float32)
+        self._params = [p.detach() for _, p in named]
+        n = len(named)
+        c_names = (C.c_char_p * n)(*[name.encode() for name, _ in named])
+        pp = (C.c_void_p * n)(*[p.data_ptr() for p in self._params])
+        gp = (C.c_void_p * n)(*[self.grads.data_ptr() + 4 * o for o, _, _ in self.slices])
+        L, handle = lib(), C.c_void_p()
+        check(L.wc_unet_train_create(C.byref(handle), C.byref(cfg), n, c_names, pp, gp))
+        self.handle = handle
+        nbytes = L.wc_unet_train_workspace_bytes(handle, B, H, W)
+        if nbytes == 0:
+            check(1)
+        self.ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        check(L.wc_unet_train_bind(handle, B, H, W, ptr(self.ws), self.ws.numel(), stream_ptr()))
+
+    def __del__(self):
+        try:
+            if self.handle is not None:
+                lib().wc_unet_train_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+
+class _Lease:
+    """A plan held by one autograd graph, with the forward's inputs (the backward reads x).  Released when the backward
+    has been enqueued, or when the graph is freed without one (the Function's ctx, which owns the lease, dies)."""
+
+    def __init__(self, plan, x, t):
+        self.plan, self.inputs = plan, (x, t)
+
+    def release(self):
+        if self.plan is not None:
+            self.plan.busy = False
+        self.plan, self.inputs = None, None
+
+    def __del__(self):
+        self.release()
+
+
+class _UnetTrainFunction(torch.autograd.Function):
+    """pred = Unet(x, t) on a leased training plan; backward seeded with dL/dpred.  Inputs: the module, x [B,3,H,W] fp32,
+    t int64 [B], then every parameter in ``named_parameters()`` order."""
+
+    @staticmethod
+    def forward(ctx, unet, x, t, *params):
+        B, _, H, W = x.shape
+        lease = _Lease(unet._lease_plan(B, H, W, x.device), x, t)
+        pred = torch.empty_like(x)
+        check(lib().wc_unet_train_forward(lease.plan.handle, ptr(x), ptr(t), None, ptr(pred), None, 1.0, 1, stream_ptr()))
+        ctx.lease = lease
+        return pred
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_pred):
+        lease = ctx.lease
+        plan = lease.plan
+        if plan is None:
+            raise RuntimeError("Unet autograd: this graph has already been backpropagated; its saved activations are gone "
+                               "(retain_graph=True re-backward is not supported: run the forward again)")
+        x = lease.inputs[0]
+        g = grad_pred.contiguous().float()
+        dx = torch.empty_like(x) if ctx.needs_input_grad[1] else None
+        need = ctx.needs_input_grad[3:]
+        param_grads = any(need)
+        check(lib().wc_unet_train_backward_seeded(plan.handle, ptr(g), ptr(dx), int(param_grads), stream_ptr()))
+        grads = [None] * len(need)
+        if param_grads:
+            # a fresh copy: AccumulateGrad may adopt these views as p.grad, and the plan's buffer is overwritten by the
+            # next backward
+            flat = plan.grads.clone()
+            grads = [flat[o:o + n].view(shape) if nd else None for (o, n, shape), nd in zip(plan.slices, need)]
+        lease.release()
+        return (None, dx, None, *grads)
 
 
 _FACTOR_SET = {}

@@ -10,6 +10,9 @@ Data parallelism (SURVEY 8e; the reference itself is single-GPU): one process pe
 its own mini-batch; gradients are summed with NCCL all-reduces issued per bucket as soon as the backward plan has
 finished the bucket's parameters (the flat gradient buffer is laid out in backward-completion order so that every
 bucket is one contiguous slice), then every rank applies the same fused Adam update with the 1/world scale folded in.
+
+``train()`` takes that fused path for the reference's own pair (``nn.MSELoss()`` + plain ``torch.optim.Adam``) and runs
+the reference's step body on the differentiable ``Unet`` (models/unet_base.py) for any other criterion and optimizer.
 """
 import ctypes as C
 
@@ -249,20 +252,75 @@ class DenoisingTrainer:
         return loss
 
 
+def fused_step_supported(criterion, optimizer) -> bool:
+    """True when (criterion, optimizer) is exactly what the fused step computes: mean-reduced nn.MSELoss and
+    torch.optim.Adam without weight decay, amsgrad or maximize (subclasses may change either, so the types must match)."""
+    if type(criterion) is not torch.nn.MSELoss or criterion.reduction != "mean":
+        return False
+    if type(optimizer) is not torch.optim.Adam:
+        return False
+    return all(not g.get("weight_decay", 0) and not g.get("amsgrad", False) and not g.get("maximize", False)
+               for g in optimizer.param_groups)
+
+
+def _train_generic(dataloader, model, optimizer, criterion, scheduler, epochs, log_interval, on_log, on_epoch_end, seed,
+                   process_group):
+    """The reference's step body (train_ddpm.py:95-114) verbatim on the differentiable Unet, with noise and t drawn as
+    DenoisingTrainer.step draws them."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(process_group) > 1:
+        raise RuntimeError("train(): data parallelism runs on the fused step only (nn.MSELoss() + torch.optim.Adam); "
+                           f"got {type(criterion).__name__} + {type(optimizer).__name__}")
+    dev = next(model.parameters()).device
+    if dev.type != "cuda":
+        raise RuntimeError("move the model to the GPU before training")
+    gen_cpu = gen_dev = None
+    if seed is not None:
+        gen_cpu = torch.Generator().manual_seed(int(seed))
+        gen_dev = torch.Generator(device=dev).manual_seed(int(seed))
+    was_differentiable = model.differentiable
+    model.differentiable = True
+    losses = []
+    try:
+        for epoch_idx in range(1, epochs + 1):
+            interval = 0.0
+            for batch_idx, images in enumerate(dataloader):
+                optimizer.zero_grad()
+                images = images.float().to(dev)
+                noise = torch.randn(images.shape, device=dev, generator=gen_dev)                # :99
+                t = torch.randint(0, scheduler.num_timesteps, (images.shape[0],), generator=gen_cpu).to(dev)   # :102
+                noisy = scheduler.add_noise(images, noise, t)                                   # :105
+                noise_pred = model(noisy, t)                                                    # :106-109
+                loss = criterion(noise_pred, noise)
+                loss.backward()
+                optimizer.step()                                                                # :113
+                interval += float(loss)
+                losses.append(float(loss))
+                if (batch_idx + 1) % log_interval == 0:
+                    if on_log is not None:
+                        on_log(epoch_idx, batch_idx + 1, interval / log_interval)
+                    interval = 0.0
+            if on_epoch_end is not None:
+                on_epoch_end(epoch_idx)
+    finally:
+        model.differentiable = was_differentiable
+    return losses
+
+
 def train(dataloader, model: Unet, optimizer, criterion, scheduler, epochs=1, log_interval=10, on_log=None, on_epoch_end=None,
           seed=None, process_group=None):
-    """Drop-in for the reference's ``train`` (train_ddpm.py:71-133): same arguments; the Adam hyper-parameters are read
-    from ``optimizer`` (built as ``Adam(model.parameters(), lr)`` at :151) and ``criterion`` must be ``nn.MSELoss()``.
-    Resume: an ``optimizer`` that already carries state (the reference's load_checkpoint, :63-68,81-84) has its moments and
-    step count imported, so Adam continues instead of restarting.  ``optimizer.state`` is re-pointed at the live moment buffers
-    before every ``on_log`` and ``on_epoch_end(epoch)`` call (the reference's per-epoch save_checkpoint, :135-141), so
-    ``optimizer.state_dict()`` taken inside those hooks is a valid checkpoint.  wandb / tqdm / file I/O of the reference are
-    host-side plumbing left to the two hooks."""
-    if not isinstance(criterion, torch.nn.MSELoss):
-        raise RuntimeError("the fused training step implements nn.MSELoss (train_ddpm.py:152)")
+    """Drop-in for the reference's ``train`` (train_ddpm.py:71-133): same arguments, same return value (the per-step
+    losses).  For ``nn.MSELoss()`` with ``torch.optim.Adam`` (no weight decay / amsgrad / maximize; the reference's pair,
+    :151-152) the step is the fused DenoisingTrainer step: the Adam hyper-parameters are read from ``optimizer``, and an
+    ``optimizer`` that already carries state (the reference's load_checkpoint, :63-68,81-84) has its moments and step count
+    imported, so Adam continues instead of restarting.  ``optimizer.state`` is re-pointed at the live moment buffers before
+    every ``on_log`` and ``on_epoch_end(epoch)`` call (the reference's per-epoch save_checkpoint, :135-141), so
+    ``optimizer.state_dict()`` taken inside those hooks is a valid checkpoint.  Any other criterion or optimizer runs the
+    reference's step body on the differentiable Unet (one GPU only), where ``optimizer.state`` is the real state.  wandb /
+    tqdm / file I/O of the reference are host-side plumbing left to the two hooks."""
+    if not fused_step_supported(criterion, optimizer):
+        return _train_generic(dataloader, model, optimizer, criterion, scheduler, epochs, log_interval, on_log,
+                              on_epoch_end, seed, process_group)
     g = optimizer.param_groups[0]
-    if g.get("weight_decay", 0) or g.get("amsgrad", False):
-        raise RuntimeError("the fused Adam implements torch.optim.Adam without weight decay / amsgrad (train_ddpm.py:151)")
     trainer = DenoisingTrainer(model, scheduler, lr=g["lr"], betas=g["betas"], eps=g["eps"], seed=seed,
                                process_group=process_group)
     trainer.import_optimizer_state(optimizer)
