@@ -287,6 +287,17 @@ int wc_seg_infer(wc_seg* net, const float* x, const int64_t* labels, int64_t* pr
 int wc_seg_infer_pooled(wc_seg* net, const float* x, const int64_t* labels, int64_t* pred, float* input_grad, float* loss,
                         float* logits, int batch, int H, int W, int grad_pool, void* workspace, size_t workspace_bytes,
                         void* stream);
+/* The plan of wc_seg_infer split at its loss head, so that a caller's own loss can drive the data gradient.
+ * wc_seg_forward: x nchw_f32 [B,3,H,W] -> logits nchw_f32 [B,19,H,W], bit-identical to wc_seg_infer's logits; no labels, no
+ * argmax, no loss.  save_for_backward = 1 binds the with-grad plan (workspace of wc_seg_workspace_bytes(..., with_grad = 1))
+ * and keeps the activations the backward reads in the workspace.
+ * wc_seg_backward_seeded: dlogits nchw_f32 [B,19,H,W] contiguous (d L / d logits of the saved forward) -> input_grad nchw_f32
+ * [B,3,H,W] = d L / d x.  No pixel is treated specially (ignore labels are the loss's business).  Fails unless the last call
+ * on this handle was wc_seg_forward(save_for_backward = 1); any infer or forward call in between discards the saved forward,
+ * and so does the backward itself. */
+int wc_seg_forward(wc_seg* net, const float* x, float* logits, int batch, int H, int W, int save_for_backward, void* workspace,
+                   size_t workspace_bytes, void* stream);
+int wc_seg_backward_seeded(wc_seg* net, const float* dlogits, float* input_grad, void* stream);
 double wc_seg_flops(const wc_seg* net, int backward);
 int wc_seg_launches(const wc_seg* net);
 

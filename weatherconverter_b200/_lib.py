@@ -110,6 +110,8 @@ _SIGS = {
     "wc_seg_workspace_bytes": (C.c_size_t, [c_ptr, C.c_int, C.c_int, C.c_int, C.c_int]),
     "wc_seg_infer": (C.c_int, [c_ptr] * 7 + [C.c_int] * 3 + [c_ptr, C.c_size_t, c_ptr]),
     "wc_seg_infer_pooled": (C.c_int, [c_ptr] * 7 + [C.c_int] * 4 + [c_ptr, C.c_size_t, c_ptr]),
+    "wc_seg_forward": (C.c_int, [c_ptr] * 3 + [C.c_int] * 4 + [c_ptr, C.c_size_t, c_ptr]),
+    "wc_seg_backward_seeded": (C.c_int, [c_ptr] * 4),
     "wc_seg_flops": (C.c_double, [c_ptr, C.c_int]),
     "wc_seg_launches": (C.c_int, [c_ptr]),
     "wc_srgan_create": (C.c_int, [C.POINTER(c_ptr), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_char_p), C.POINTER(c_ptr), c_ptr]),

@@ -5,6 +5,8 @@
 // gradient and throws it away); eval-mode BatchNorm is folded into the preceding convolution; ReLU derivatives
 // are applied as masks in the epilogue of the data-gradient convolution that produces each gradient.
 // Per-image semantics (SURVEY D6): the loss of image b is the mean over ITS valid pixels.
+// wc_seg_forward / wc_seg_backward_seeded split the same plan at the loss head so that any loss computed by the caller can
+// seed the data-gradient backward (torch autograd in seg_model/network/modeling.py).
 #include "plan.cuh"
 #include "../../include/wc_b200.h"
 
@@ -50,6 +52,12 @@ struct wc_seg {
   wc::OpList fwd_ops, bwd_ops;
   double flops_fwd = 0, flops_bwd = 0;
   size_t ws_needed = 0;
+  // seam between the network body and the loss head, for wc_seg_forward / wc_seg_backward_seeded: fwd_ops[0, n_body_ops)
+  // end at the low-resolution logits; the backward starts from dlo (NHWC bf16, 32 channels; with_grad plans only)
+  size_t n_body_ops = 0;
+  float* logits_lo = nullptr;
+  __nv_bfloat16* dlo = nullptr;
+  int saved_fwd = 0;   // the last call was wc_seg_forward(save_for_backward = 1) on the current binding
   // per-call pointers
   const float* x_in = nullptr;
   const long long* labels = nullptr;
@@ -286,6 +294,11 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   }
   Act dlo{};
   if (net->with_grad) dlo = b.act(H4, W4, NCP);
+  if (!dry) {
+    net->n_body_ops = net->fwd_ops.size();
+    net->logits_lo = logits_lo;
+    net->dlo = net->with_grad ? dlo.ptr : nullptr;
+  }
   {
     wc_seg* n = net;
     const bool with_grad = net->with_grad;
@@ -399,6 +412,24 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   return b.err;
 }
 
+// (Re)builds the plan when the geometry, the gradient mode or the workspace differ from the current binding.
+int bind_plan(wc_seg* net, int batch, int H, int W, int with_grad, int grad_pool, void* workspace, size_t workspace_bytes,
+              cudaStream_t st) {
+  if (net->B == batch && net->H == H && net->W == W && net->with_grad == with_grad && net->grad_pool == grad_pool && net->ws == workspace &&
+      net->ws_bytes == workspace_bytes)
+    return 0;
+  net->fwd_ops.clear(); net->bwd_ops.clear();
+  net->arena = std::make_unique<DeviceArena>();
+  net->B = batch; net->H = H; net->W = W; net->with_grad = with_grad; net->grad_pool = grad_pool; net->ws = workspace; net->ws_bytes = workspace_bytes;
+  net->flops_fwd = net->flops_bwd = 0;
+  if (int e = build(net, false, workspace, workspace_bytes, st)) {
+    net->B = 0;
+    net->fwd_ops.clear(); net->bwd_ops.clear();
+    return e;
+  }
+  return 0;
+}
+
 }  // namespace
 }  // namespace wc
 
@@ -425,6 +456,7 @@ int wc_seg_set_output_stride(wc_seg* net, int output_stride) {
   if (net->output_stride != output_stride) {
     net->output_stride = output_stride;
     net->B = net->H = net->W = 0;   // force a rebuild of the plan on the next call
+    net->saved_fwd = 0;
   }
   return 0;
 }
@@ -453,27 +485,50 @@ int wc_seg_infer(wc_seg* net, const float* x, const int64_t* labels, int64_t* pr
 int wc_seg_infer_pooled(wc_seg* net, const float* x, const int64_t* labels, int64_t* pred, float* input_grad, float* loss,
                         float* logits, int batch, int H, int W, int grad_pool, void* workspace, size_t workspace_bytes,
                         void* stream) {
+  if (net) net->saved_fwd = 0;
   WC_REQUIRE(grad_pool >= 1, "grad_pool must be >= 1");
   WC_REQUIRE(net && x && labels && workspace, "null argument");
   WC_REQUIRE(H % 32 == 0 && W % 32 == 0, "H and W must be multiples of 32 (output stride 16, stride-2 phase views)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int with_grad = input_grad != nullptr;
-  if (net->B != batch || net->H != H || net->W != W || net->with_grad != with_grad || net->grad_pool != grad_pool || net->ws != workspace ||
-      net->ws_bytes != workspace_bytes) {
-    net->fwd_ops.clear(); net->bwd_ops.clear();
-    net->arena = std::make_unique<DeviceArena>();
-    net->B = batch; net->H = H; net->W = W; net->with_grad = with_grad; net->grad_pool = grad_pool; net->ws = workspace; net->ws_bytes = workspace_bytes;
-    net->flops_fwd = net->flops_bwd = 0;
-    if (int e = build(net, false, workspace, workspace_bytes, st)) {
-      net->B = 0;
-      net->fwd_ops.clear(); net->bwd_ops.clear();
-      return e;
-    }
-  }
+  if (int e = bind_plan(net, batch, H, W, with_grad, grad_pool, workspace, workspace_bytes, st)) return e;
   net->x_in = x; net->labels = reinterpret_cast<const long long*>(labels);
   net->pred = reinterpret_cast<long long*>(pred); net->grad_out = input_grad; net->loss = loss; net->logits_hi = logits;
   for (auto& op : net->fwd_ops)
     if (int e = op(st)) return e;
+  for (auto& op : net->bwd_ops)
+    if (int e = op(st)) return e;
+  return 0;
+}
+
+int wc_seg_forward(wc_seg* net, const float* x, float* logits, int batch, int H, int W, int save_for_backward, void* workspace,
+                   size_t workspace_bytes, void* stream) {
+  if (net) net->saved_fwd = 0;
+  WC_REQUIRE(net && x && logits && workspace, "null argument");
+  WC_REQUIRE(H % 32 == 0 && W % 32 == 0, "H and W must be multiples of 32 (output stride 16, stride-2 phase views)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int e = bind_plan(net, batch, H, W, save_for_backward ? 1 : 0, 1, workspace, workspace_bytes, st)) return e;
+  net->x_in = x; net->labels = nullptr; net->pred = nullptr; net->grad_out = nullptr; net->loss = nullptr; net->logits_hi = logits;
+  for (size_t i = 0; i < net->n_body_ops; ++i)
+    if (int e = net->fwd_ops[i](st)) return e;
+  // the loss head's kernel without labels: only the up-sampled logits, the same bits wc_seg_infer writes
+  if (int e = seg_loss_grad(net->logits_lo, nullptr, nullptr, nullptr, nullptr, nullptr, logits, batch, H / 4, W / 4, H, W,
+                            net->num_classes, 255, st))
+    return e;
+  net->saved_fwd = save_for_backward ? 1 : 0;
+  return 0;
+}
+
+int wc_seg_backward_seeded(wc_seg* net, const float* dlogits, float* input_grad, void* stream) {
+  WC_REQUIRE(net && dlogits && input_grad, "null argument");
+  WC_REQUIRE(net->saved_fwd && net->dlo,
+             "wc_seg_backward_seeded: this handle holds no saved forward; the last call on it must be "
+             "wc_seg_forward(save_for_backward = 1) (an infer or another forward in between discards the saved activations)");
+  net->saved_fwd = 0;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = net->B, H = net->H, W = net->W;
+  net->grad_out = input_grad;
+  if (int e = logits_bilinear_bwd(dlogits, net->dlo, B, H / 4, W / 4, H, W, net->num_classes, 32, 32, st)) return e;
   for (auto& op : net->bwd_ops)
     if (int e = op(st)) return e;
   return 0;

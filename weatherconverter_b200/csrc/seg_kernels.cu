@@ -302,7 +302,8 @@ __global__ void count_valid_kernel(const long long* __restrict__ labels, int HW,
 
 // One thread per full-resolution pixel: bilinear logits (from low-res NCHW fp32 planes), argmax -> pred,
 // softmax-CE: dlogit = (softmax - onehot) / n_valid[b] (0 where ignored) written as fp32 class planes [B,NC,H,W];
-// per-image loss accumulated with one atomic per warp.
+// per-image loss accumulated with one atomic per warp.  labels == NULL (then pred, dlogit_hi and loss are NULL too): only the
+// up-sampled logits are written.
 template <int NC>
 __global__ void seg_loss_grad_kernel(const float* __restrict__ logits_lo, const long long* __restrict__ labels,
                                      const int* __restrict__ n_valid, long long* __restrict__ pred,
@@ -343,6 +344,7 @@ __global__ void seg_loss_grad_kernel(const float* __restrict__ logits_lo, const 
 #pragma unroll
         for (int c = 0; c < NC; ++c) logits_hi[(static_cast<size_t>(b) * NC + c) * pl_hi + static_cast<size_t>(oy) * W + ox] = v[c];
       }
+      if (!labels) continue;   // uniform across the grid: loss is NULL too, so no warp reduction is skipped
       const long long lab = labels[i];
       const size_t pl_hi2 = static_cast<size_t>(H) * W;
       float* d = dlogit_hi + static_cast<size_t>(b) * NC * pl_hi2 + static_cast<size_t>(oy) * W + ox;   // class planes
@@ -765,11 +767,14 @@ int bilinear_bwd(const __nv_bfloat16* dy, const __nv_bfloat16* mask, __nv_bfloat
 int seg_loss_grad(const float* logits_lo, const long long* labels, int* n_valid, long long* pred, float* dlogit_hi,
                   float* loss, float* logits_hi, int B, int h, int w, int H, int W, int nc, int ignore, cudaStream_t st) {
   WC_REQUIRE(nc == 19, "loss head is compiled for 19 classes (Cityscapes trainIds)");
+  WC_REQUIRE(labels || (!pred && !dlogit_hi && !loss), "seg_loss_grad without labels writes the up-sampled logits only");
   ProfScope prof(kProfOther, st, 0);
-  WC_CHECK_CUDA(cudaMemsetAsync(n_valid, 0, B * sizeof(int), st));
-  if (loss) WC_CHECK_CUDA(cudaMemsetAsync(loss, 0, B * sizeof(float), st));
-  launch_k(count_valid_kernel, dim3(std::min(64, (H * W + 255) / 256), B), 256, 0, st, labels, H * W, ignore, n_valid);
-  WC_LAUNCH_CHECK();
+  if (labels) {
+    WC_CHECK_CUDA(cudaMemsetAsync(n_valid, 0, B * sizeof(int), st));
+    if (loss) WC_CHECK_CUDA(cudaMemsetAsync(loss, 0, B * sizeof(float), st));
+    launch_k(count_valid_kernel, dim3(std::min(64, (H * W + 255) / 256), B), 256, 0, st, labels, H * W, ignore, n_valid);
+    WC_LAUNCH_CHECK();
+  }
   launch_k(seg_loss_grad_kernel<19>, grid_for(static_cast<size_t>(B) * H * W, 128), 128, 0, st, logits_lo, labels, n_valid, pred, dlogit_hi, loss, logits_hi, B, h, w, H, W, ignore);
   WC_LAUNCH_CHECK();
   return 0;

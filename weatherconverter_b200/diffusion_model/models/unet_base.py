@@ -26,6 +26,7 @@ from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from ..._lib import UnetConfigStruct, check, lib, ptr, stream_ptr
+from ..._plans import Lease, lease_plan
 
 
 def _cfg_get(cfg, k):
@@ -237,13 +238,7 @@ class Unet(nn.Module):
                     raise RuntimeError(f"Unet parameter {n} must be a contiguous fp32 tensor on {device}; call .to(device)")
             set_time_factor_table(self.t_emb_dim, device)
             self._train_plans, self._train_key = {}, key
-        plans = self._train_plans.setdefault((B, H, W), [])
-        plan = next((p for p in plans if not p.busy), None)
-        if plan is None:
-            plan = _TrainPlan(self._config_struct(), named, B, H, W, device)
-            plans.append(plan)
-        plan.busy = True
-        return plan
+        return lease_plan(self._train_plans, (B, H, W), lambda: _TrainPlan(self._config_struct(), named, B, H, W, device))
 
     # ---- reference API ---------------------------------------------------------------------------------
     def forward(self, x, t, out=None):
@@ -315,22 +310,6 @@ class _TrainPlan:
             pass
 
 
-class _Lease:
-    """A plan held by one autograd graph, with the forward's inputs (the backward reads x).  Released when the backward
-    has been enqueued, or when the graph is freed without one (the Function's ctx, which owns the lease, dies)."""
-
-    def __init__(self, plan, x, t):
-        self.plan, self.inputs = plan, (x, t)
-
-    def release(self):
-        if self.plan is not None:
-            self.plan.busy = False
-        self.plan, self.inputs = None, None
-
-    def __del__(self):
-        self.release()
-
-
 class _UnetTrainFunction(torch.autograd.Function):
     """pred = Unet(x, t) on a leased training plan; backward seeded with dL/dpred.  Inputs: the module, x [B,3,H,W] fp32,
     t int64 [B], then every parameter in ``named_parameters()`` order."""
@@ -338,7 +317,7 @@ class _UnetTrainFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, unet, x, t, *params):
         B, _, H, W = x.shape
-        lease = _Lease(unet._lease_plan(B, H, W, x.device), x, t)
+        lease = Lease(unet._lease_plan(B, H, W, x.device), x, t)
         pred = torch.empty_like(x)
         check(lib().wc_unet_train_forward(lease.plan.handle, ptr(x), ptr(t), None, ptr(pred), None, 1.0, 1, stream_ptr()))
         ctx.lease = lease

@@ -1,6 +1,13 @@
 """DeepLabV3+ factories with the reference's names and signatures (seg_model/network/modeling.py:182-202),
 backed by the C plan in csrc/seg.cu (forward, loss head and input gradient on libwc_b200.so).
 
+Autograd: with grad mode on and ``x.requires_grad``, ``forward(x)`` returns logits with a ``grad_fn``, so any loss on them
+backpropagates to ``x`` (``loss.backward()`` fills ``x.grad``; ``torch.autograd.grad(loss, x)`` works).  The graph is a
+function of ``x`` only: the parameters are constants, no weight gradient is computed and every ``p.grad`` stays ``None``
+(eval-mode BatchNorm is folded into the convolutions; segmentor training is not supported).  The backward is the plan's
+data-gradient pass seeded with dL/dlogits (``wc_seg_backward_seeded``).  A graph holds one plan (its saved activations)
+until its backward has run or it is freed; the plans live in a pool per (B, H, W).  A graph can be backpropagated once.
+
 Only the ResNet-50/101 DeepLabV3+ variants reachable from the reference's configured model name are provided
 (SURVEY.md section 2, rows 10-12); output_stride 16 (the reference's config, seg_model/config/config.yaml:66).
 The returned module's state_dict has the reference's keys/shapes/order (368 tensors for R50, 674 for R101).
@@ -10,10 +17,12 @@ import math
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from ..._lib import check, lib, ptr, stream_ptr
 from ..._params import register_dotted
+from ..._plans import Lease, lease_plan
 
 __all__ = ["deeplabv3plus_resnet50", "deeplabv3plus_resnet101", "DeepLabV3"]
 
@@ -89,6 +98,8 @@ class DeepLabV3(nn.Module):
         self._key = None
         self._ws = {}
         self._keep = None
+        self._grad_plans = {}        # (B, H, W) -> [_SegGradPlan]: the autograd path's plan pool
+        self._grad_key = None
 
     # ---- C handle --------------------------------------------------------------------------------------
     def _tensors(self):
@@ -111,12 +122,7 @@ class DeepLabV3(nn.Module):
         except Exception:
             pass
 
-    def _ensure(self, device):
-        ts = self._tensors()
-        key = (str(device), tuple((t.data_ptr(), t._version) for t in ts.values()))
-        if self._handle is not None and key == self._key:
-            return
-        self._destroy()
+    def _create_handle(self, ts, device):
         for n, t in ts.items():
             if t.device != device or not t.is_contiguous():
                 raise RuntimeError(f"seg parameter {n} must be contiguous on {device}; call .to(device)")
@@ -127,7 +133,26 @@ class DeepLabV3(nn.Module):
         h = C.c_void_p()
         check(lib().wc_seg_create(C.byref(h), layers, self.num_classes, n, names, ptrs, stream_ptr()))
         check(lib().wc_seg_set_output_stride(h, self.output_stride))
+        return h
+
+    def _ensure(self, device):
+        ts = self._tensors()
+        key = (str(device), tuple((t.data_ptr(), t._version) for t in ts.values()))
+        if self._handle is not None and key == self._key:
+            return
+        self._destroy()
+        h = self._create_handle(ts, device)
         self._handle, self._key, self._keep, self._ws = h, key, list(ts.values()), {}
+
+    def _lease_plan(self, B, H, W, device):
+        """A free autograd plan for (B, H, W), created when every plan of that shape is held by a live graph.  A plan packs
+        the weights once, when it is first bound, so the pool is rebuilt whenever a tensor's storage or version changes
+        (.to(), load_state_dict, any in-place update); a live graph keeps its own plan."""
+        ts = self._tensors()
+        key = (str(device), self.output_stride, tuple((t.data_ptr(), t._version) for t in ts.values()))
+        if key != self._grad_key:
+            self._grad_plans, self._grad_key = {}, key
+        return lease_plan(self._grad_plans, (B, H, W), lambda: _SegGradPlan(self, ts, B, H, W, device))
 
     def _workspace(self, B, H, W, with_grad, device):
         k = (B, H, W, with_grad)
@@ -167,15 +192,80 @@ class DeepLabV3(nn.Module):
         import copy
         r = copy.copy(self)          # shares _parameters / _buffers (no new tensors)
         r._handle, r._key, r._ws, r._keep = None, None, {}, None
+        r._grad_plans, r._grad_key = {}, None
         return r
 
     def forward(self, x):
+        """x [B,3,H,W] -> logits fp32 [B,num_classes,H,W].  With grad mode on and ``x.requires_grad`` the result carries an
+        autograd graph of ``x`` (the parameters are constants: no weight gradients, ``p.grad`` stays None)."""
+        _lib.require_cuda(x)
+        if self.training:
+            raise RuntimeError("the B200 DeepLabV3+ path implements eval-mode BatchNorm only; call .eval()")
+        if torch.is_grad_enabled() and x.requires_grad:
+            return _SegFunction.apply(self, x.contiguous().float())
+        x = x.contiguous().float()
         B, _, H, W = x.shape
-        dummy = torch.zeros(B, H, W, dtype=torch.long, device=x.device)
-        return self.infer(x, dummy, want_grad=False, want_logits=True)["logits"]
+        self._ensure(x.device)
+        ws = self._workspace(B, H, W, False, x.device)
+        logits = torch.empty(B, self.num_classes, H, W, device=x.device)
+        check(lib().wc_seg_forward(self._handle, ptr(x), ptr(logits), B, H, W, 0, ptr(ws), ws.numel(), stream_ptr()))
+        self._last = (x,)
+        return logits
 
     def flops(self):
         return (float(lib().wc_seg_flops(self._handle, 0)), float(lib().wc_seg_flops(self._handle, 1)))
+
+
+class _SegGradPlan:
+    """A C handle of its own with a with-grad workspace, bound to (B, H, W) by its first forward (which packs the weights).
+    Keeps the module's tensors alive: the handle reads them in place."""
+
+    def __init__(self, seg, ts, B, H, W, device):
+        self.handle, self.busy = None, False
+        self._keep = list(ts.values())
+        self.handle = seg._create_handle(ts, device)
+        nbytes = lib().wc_seg_workspace_bytes(self.handle, B, H, W, 1)
+        if nbytes == 0:
+            check(1)
+        self.ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+
+    def __del__(self):
+        try:
+            if self.handle is not None:
+                lib().wc_seg_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+
+class _SegFunction(torch.autograd.Function):
+    """logits = DeepLabV3(x) on a leased plan that saves its activations; backward seeded with dL/dlogits gives dL/dx.
+    Inputs: the module, x [B,3,H,W] fp32 contiguous."""
+
+    @staticmethod
+    def forward(ctx, seg, x):
+        B, _, H, W = x.shape
+        lease = Lease(seg._lease_plan(B, H, W, x.device), x)
+        plan = lease.plan
+        logits = torch.empty(B, seg.num_classes, H, W, device=x.device)
+        check(lib().wc_seg_forward(plan.handle, ptr(x), ptr(logits), B, H, W, 1, ptr(plan.ws), plan.ws.numel(), stream_ptr()))
+        ctx.lease = lease
+        return logits
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_logits):
+        lease = ctx.lease
+        plan = lease.plan
+        if plan is None:
+            raise RuntimeError("DeepLabV3 autograd: this graph has already been backpropagated; its saved activations are gone "
+                               "(retain_graph=True re-backward is not supported: run the forward again)")
+        x = lease.inputs[0]
+        g = grad_logits.contiguous().float()
+        dx = torch.empty_like(x)
+        check(lib().wc_seg_backward_seeded(plan.handle, ptr(g), ptr(dx), stream_ptr()))
+        lease.release()
+        return None, dx
 
 
 def _build(backbone, num_classes, output_stride, pretrained_backbone):

@@ -5,6 +5,10 @@
 ``mu + lambda*sigma*mag + sigma`` (csrc/elementwise.cu: sgg_update_kernel).  The reference returns float64
 (numpy promotion, SURVEY D7); this returns fp32 rounded from the same float64 arithmetic (the repaired driver casts
 back to fp32 anyway).  ``apply_lcg`` raises as shipped (SURVEY D3); here it runs with the documented repair of its final masked sum.
+
+``criterion``: GSG with any segmentation loss.  ``criterion(logits [B,19,H,W], gt [B,H,W]) -> [B]`` per-image losses; the
+gradient d(sum_b loss_b)/d sr_xt comes from torch autograd through the segmentor (DeepLabV3.forward), then goes through the
+same update kernel with its unfused average pooling.  ``None`` keeps the fused CE(ignore 255) plan.
 """
 import torch
 
@@ -13,12 +17,43 @@ from .._lib import check, lib, ptr, stream_ptr
 from ..seg_model.inference import infer_batch
 
 
-def apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, _lambda, pool=None, return_aux=False, fused_pool=True):
-    """Batched GSG: every image uses its own loss/gradient (vmap of the reference's B = 1 semantics)."""
+def _criterion_grad(seg_model, sr_xt, gt, criterion):
+    """d(sum_b criterion(seg_model(x), gt)_b)/dx at x = sr_xt by torch autograd through the segmentor."""
+    B = sr_xt.shape[0]
+    if gt.dim() == 4:
+        gt = gt.squeeze(1)
+    gt = gt.long()
+    with torch.enable_grad():
+        x = sr_xt.detach().contiguous().float().requires_grad_(True)
+        logits = seg_model(x)
+        loss = criterion(logits, gt)
+        if not torch.is_tensor(loss) or tuple(loss.shape) != (B,):
+            shape = tuple(loss.shape) if torch.is_tensor(loss) else type(loss).__name__
+            raise ValueError(f"criterion must return one loss per image, shape ({B},); got {shape} "
+                             "(a batch-mean scalar would scale every image's guidance by 1/B)")
+        grad, = torch.autograd.grad(loss.sum(), x)
+    return dict(grad=grad, loss=loss.detach(), logits=logits.detach())
+
+
+def apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, _lambda, pool=None, return_aux=False, fused_pool=True, criterion=None):
+    """Batched GSG: every image uses its own loss/gradient (vmap of the reference's B = 1 semantics).  ``criterion``
+    (optional): callable (logits [B,19,H,W], gt [B,H,W]) -> per-image losses [B] replacing the fused CE(ignore 255); image b
+    is guided by d loss_b / d sr_xt[b].  It runs torch autograd, so it cannot be captured in a CUDA graph."""
+    if criterion is not None and not callable(criterion):
+        raise TypeError("criterion must be a callable (logits, gt) -> per-image losses [B]")
     _lib.require_cuda(mu, sigma, sr_xt, gt)
     B, _, h, w = mu.shape
     if pool is None:
         pool = sr_xt.shape[-1] // w
+    if criterion is not None:
+        if torch.cuda.is_current_stream_capturing():
+            raise ValueError("apply_gsg_batch: a custom criterion runs torch autograd and cannot be captured in a CUDA graph")
+        out = _criterion_grad(seg_model, sr_xt, gt, criterion)
+        mu, sigma = mu.contiguous().float(), sigma.contiguous().float()
+        xt = torch.empty_like(mu)
+        check(lib().wc_sgg_update(ptr(out["grad"]), ptr(mu), ptr(sigma), ptr(xt), None, B, h, w, pool, float(_lambda),
+                                  stream_ptr()))
+        return (xt, out) if return_aux else xt
     # avg_pool2d(grad, pool) (sgg.py:18) is folded into the segmentor's stem data-gradient kernel when possible
     fused = fused_pool and pool in (2, 4, 6, 8)
     out = infer_batch(seg_model, sr_xt, gt, grad_pool=pool if fused else 1)
@@ -29,8 +64,8 @@ def apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, _lambda, pool=None, return_
     return (xt, out) if return_aux else xt
 
 
-def apply_gsg(seg_model, mu, sigma, sr_xt, gt, _lambda):
-    return apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, _lambda)
+def apply_gsg(seg_model, mu, sigma, sr_xt, gt, _lambda, criterion=None):
+    return apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, _lambda, criterion=criterion)
 
 
 def apply_lcg(seg_model, mu, sigma, sr_xt, gt, _lambda, num_classes=19, pool=None):

@@ -77,16 +77,25 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
 @torch.no_grad()
 def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srgan_model, *, n_steps=N_STEPS,
                     lam=LAMBDA, noise=None, t_forward=None, step_noise=None, device_noise=False, generator=None,
-                    guidance=True, mode="gsg", reference_quirks=False, record=None, record_base=None, use_graph=False):
+                    guidance=True, mode="gsg", reference_quirks=False, record=None, record_base=None, use_graph=False,
+                    criterion=None):
     """input_tensor [B,3,h,w] in [-1,1]; gt [B,4h,4w] int64 trainIds (255 = ignore).  Returns sr_x0 [B,3,4h,4w].
     Injection points for parity runs: ``t_forward`` [B] (reference :63 draws randint(0, N)), ``noise`` like the input
     (:64), ``step_noise`` [N, B,3,h,w] or callable i -> z (scheduler.py:110); ``record`` / ``record_base`` collect x_t and
     the unguided mu + sigma of every step.  ``mode``: "gsg" (global guidance on every
     step, the repaired default), "alternate" (reference :84-87: LCG when i is even, GSG when i is odd) or "lcg".
     ``use_graph=True`` captures the guided reverse step once per guidance kind as a CUDA graph (weatherconverter_b200/graphs.py)
-    and replays it: one cudaGraphLaunch per step instead of ~440 kernel launches, bit-identical to the eager loop."""
+    and replays it: one cudaGraphLaunch per step instead of ~440 kernel launches, bit-identical to the eager loop.
+    ``criterion``: callable (logits [B,19,H,W], gt [B,H,W]) -> per-image losses [B] that replaces the fused CE(ignore 255) of
+    every GSG step (sgg/sgg.py: apply_gsg_batch); eager loop and mode="gsg" only."""
     if mode not in ("gsg", "alternate", "lcg"):
         raise ValueError("mode must be 'gsg', 'alternate' or 'lcg'")
+    if criterion is not None:
+        if use_graph:
+            raise ValueError("criterion: a custom guidance loss runs torch autograd, which the step graph cannot capture; "
+                             "use use_graph=False")
+        if mode != "gsg":
+            raise ValueError("criterion applies to global guidance (mode='gsg') only; local class guidance uses the fused CE")
     x0 = input_tensor.to(device).float().contiguous()
     gt = gt.to(device)
     B = x0.shape[0]
@@ -118,7 +127,7 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
                 if mode == "lcg" or (mode == "alternate" and i % 2 == 0):
                     guided = apply_lcg(seg_model, mu, sigma, sr_xt, gt, lam)                # reference :84-85
                 else:
-                    guided = apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, lam)          # reference :86-87
+                    guided = apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, lam, criterion=criterion)  # reference :86-87
                 xt = (mu + sigma) if reference_quirks else guided                           # reference :90 (D1)
             else:
                 xt = mu + sigma
