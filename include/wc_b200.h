@@ -310,6 +310,16 @@ size_t wc_srgan_workspace_bytes(const wc_srgan* net, int batch, int h, int w);
 /* Generator.forward: x nchw_f32 [B,3,h,w] -> y nchw_f32 [B,3,upscale*h,upscale*w] in [0,1]. */
 int wc_srgan_forward(wc_srgan* net, const float* x, float* y, int batch, int h, int w, void* workspace,
                      size_t workspace_bytes, void* stream);
+/* The input gradient of the generator (the parameters are constants; no weight gradient).
+ * wc_srgan_forward_saved: the same ops as wc_srgan_forward, the same bits in y, on the with-grad plan (workspace of
+ * wc_srgan_grad_workspace_bytes), which also keeps what the backward reads: every PReLU's pre-activation and a copy of y.
+ * wc_srgan_backward_seeded: dy nchw_f32 [B,3,upscale*h,upscale*w] contiguous (d L / d y of the saved forward) -> dx nchw_f32
+ * [B,3,h,w] = d L / d x.  Fails unless the last call on this handle was wc_srgan_forward_saved; any forward in between
+ * discards the saved forward, and so does the backward itself. */
+size_t wc_srgan_grad_workspace_bytes(const wc_srgan* net, int batch, int h, int w);
+int wc_srgan_forward_saved(wc_srgan* net, const float* x, float* y, int batch, int h, int w, void* workspace,
+                           size_t workspace_bytes, void* stream);
+int wc_srgan_backward_seeded(wc_srgan* net, const float* dy, float* dx, void* stream);
 double wc_srgan_flops(const wc_srgan* net);
 int wc_srgan_launches(const wc_srgan* net);
 

@@ -118,6 +118,9 @@ _SIGS = {
     "wc_srgan_destroy": (None, [c_ptr]),
     "wc_srgan_workspace_bytes": (C.c_size_t, [c_ptr, C.c_int, C.c_int, C.c_int]),
     "wc_srgan_forward": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, C.c_size_t, c_ptr]),
+    "wc_srgan_grad_workspace_bytes": (C.c_size_t, [c_ptr, C.c_int, C.c_int, C.c_int]),
+    "wc_srgan_forward_saved": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, C.c_size_t, c_ptr]),
+    "wc_srgan_backward_seeded": (C.c_int, [c_ptr] * 4),
     "wc_srgan_flops": (C.c_double, [c_ptr]),
     "wc_srgan_launches": (C.c_int, [c_ptr]),
 }

@@ -1194,3 +1194,122 @@ int gather_stride(const float* src, float* dst, int n, int mul, int off, cudaStr
   return 0;
 }
 }  // namespace wc
+
+// =====================================================================================================================
+// SRGAN input-gradient backward (srgan.cu: wc_srgan_backward_seeded): the elementwise pieces between the data-gradient
+// convolutions.  PReLU derivatives read the pre-activation that the with-grad forward keeps (the PReLU output alone does
+// not determine the sign of the pre-activation when a slope is <= 0).
+namespace wc {
+namespace {
+
+// d(pre-tanh) of y = (tanh(z) + 1) / 2:  dz = dy * 2y(1 - y), fp32 NCHW
+__global__ void srgan_tanh_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ y, float* __restrict__ dz, size_t n) {
+  pdl_prologue();
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const float v = y[i];
+    dz[i] = dy[i] * (2.f * v * (1.f - v));
+  }
+}
+
+// wt[ci][co][KK-1-t] = w[co][ci][t]: the data gradient of a stride-1 'same' KxK convolution as a convolution of dy
+__global__ void flip_transpose_kk_kernel(const float* __restrict__ w, float* __restrict__ wt, int Co, int Ci, int KK) {
+  pdl_prologue();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= Co * Ci * KK) return;
+  const int t = i % KK, ci = (i / KK) % Ci, co = i / (KK * Ci);
+  wt[(static_cast<size_t>(ci) * Co + co) * KK + (KK - 1 - t)] = w[i];
+}
+
+// d := (d + add) * (pre > 0 ? 1 : slope[c]), NHWC bf16, 8 channels per thread (C % 8 == 0)
+__global__ void prelu_bwd_kernel(__nv_bfloat16* __restrict__ d, const __nv_bfloat16* __restrict__ add,
+                                 const __nv_bfloat16* __restrict__ pre, const float* __restrict__ slope, size_t npix, int C, int ldd,
+                                 int lda, int ldp) {
+  pdl_prologue();
+  const int c8n = C / 8;
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < npix * c8n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const size_t p = i / c8n;
+    const int c0 = static_cast<int>(i % c8n) * 8;
+    uint4* dp = reinterpret_cast<uint4*>(d + p * ldd + c0);
+    const uint4 u = *dp, m = *reinterpret_cast<const uint4*>(pre + p * ldp + c0);
+    const uint4 a = add ? *reinterpret_cast<const uint4*>(add + p * lda + c0) : make_uint4(0, 0, 0, 0);
+    const uint32_t uu[4] = {u.x, u.y, u.z, u.w}, mm[4] = {m.x, m.y, m.z, m.w}, aa[4] = {a.x, a.y, a.z, a.w};
+    uint32_t o[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const float2 g = unpack_bf16(uu[k]), s = unpack_bf16(mm[k]), q = unpack_bf16(aa[k]);
+      const float gx = g.x + q.x, gy = g.y + q.y;
+      o[k] = pack_bf16(s.x > 0.f ? gx : gx * slope[c0 + 2 * k], s.y > 0.f ? gy : gy * slope[c0 + 2 * k + 1]);
+    }
+    *dp = make_uint4(o[0], o[1], o[2], o[3]);
+  }
+}
+
+// PReLU(PixelShuffle(2)) backward: dconv[b][y][x][4c + 2i + j] = dup[b][2y+i][2x+j][c] * (pre > 0 ? 1 : slope[c]);
+// dup / pre: [B][2h][2w][C] (ld C), dconv: [B][h][w][4C].  One thread = 8 consecutive conv channels (two shuffled channels).
+__global__ void shuffle_prelu_bwd_kernel(const __nv_bfloat16* __restrict__ dup, const __nv_bfloat16* __restrict__ pre,
+                                         const float* __restrict__ slope, __nv_bfloat16* __restrict__ dconv, int B, int h, int w, int C) {
+  pdl_prologue();
+  const int k8 = C / 2;   // groups of 8 conv channels per pixel
+  const size_t total = static_cast<size_t>(B) * h * w * k8;
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    const int k = static_cast<int>(i % k8);
+    const size_t pix = i / k8;
+    const int x = static_cast<int>(pix % w), y = static_cast<int>((pix / w) % h), b = static_cast<int>(pix / (static_cast<size_t>(w) * h));
+    const int c = 2 * k;
+    const float s0 = slope[c], s1 = slope[c + 1];
+    float v[8];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const size_t off = ((static_cast<size_t>(b) * 2 * h + 2 * y + (q >> 1)) * 2 * w + 2 * x + (q & 1)) * C + c;
+      const float2 g = unpack_bf16(*reinterpret_cast<const uint32_t*>(dup + off));
+      const float2 m = unpack_bf16(*reinterpret_cast<const uint32_t*>(pre + off));
+      v[q] = m.x > 0.f ? g.x : g.x * s0;       // conv channel 4c + q
+      v[4 + q] = m.y > 0.f ? g.y : g.y * s1;   // conv channel 4(c+1) + q
+    }
+    uint4 o;
+    o.x = pack_bf16(v[0], v[1]); o.y = pack_bf16(v[2], v[3]); o.z = pack_bf16(v[4], v[5]); o.w = pack_bf16(v[6], v[7]);
+    *reinterpret_cast<uint4*>(dconv + pix * (4 * C) + 8 * k) = o;
+  }
+}
+
+__global__ void fill_f32_kernel(float* __restrict__ p, float v, int n) {
+  pdl_prologue();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) p[i] = v;
+}
+
+}  // namespace
+
+int srgan_tanh_bwd(const float* dy, const float* y, float* dz, size_t n, cudaStream_t st) {
+  ProfScope prof(kProfOther, st, 0);
+  launch_k(srgan_tanh_bwd_kernel, grid_for(n), 256, 0, st, dy, y, dz, n);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+int flip_transpose_kk(const float* w, float* wt, int Co, int Ci, int KK, cudaStream_t st) {
+  launch_k(flip_transpose_kk_kernel, (Co * Ci * KK + 255) / 256, 256, 0, st, w, wt, Co, Ci, KK);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+int prelu_bwd(__nv_bfloat16* d, const __nv_bfloat16* add, const __nv_bfloat16* pre, const float* slope, size_t npix, int C, int ldd,
+              int lda, int ldp, cudaStream_t st) {
+  WC_REQUIRE(C % 8 == 0 && ldd % 8 == 0 && lda % 8 == 0 && ldp % 8 == 0, "prelu_bwd: channels and pixel strides must be multiples of 8");
+  ProfScope prof(kProfOther, st, 0);
+  launch_k(prelu_bwd_kernel, grid_for(npix * (C / 8)), 256, 0, st, d, add, pre, slope, npix, C, ldd, lda, ldp);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+int shuffle_prelu_bwd(const __nv_bfloat16* dup, const __nv_bfloat16* pre, const float* slope, __nv_bfloat16* dconv, int B, int h, int w,
+                      int C, cudaStream_t st) {
+  WC_REQUIRE(C % 2 == 0, "shuffle_prelu_bwd: even channel count");
+  ProfScope prof(kProfOther, st, 0);
+  launch_k(shuffle_prelu_bwd_kernel, grid_for(static_cast<size_t>(B) * h * w * (C / 2)), 256, 0, st, dup, pre, slope, dconv, B, h, w, C);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+int fill_f32(float* p, float v, int n, cudaStream_t st) {
+  launch_k(fill_f32_kernel, (n + 255) / 256, 256, 0, st, p, v, n);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+}  // namespace wc

@@ -87,7 +87,7 @@ static inline const __nv_bfloat16* BF(const wc_bf16* p) { return reinterpret_cas
 extern "C" {
 
 const char* wc_last_error(void) { return last_error_cstr(); }
-int wc_abi_version(void) { return 4; }
+int wc_abi_version(void) { return 5; }
 long long wc_launch_count(void) { return launch_count(); }
 void wc_profile_begin(void) { prof_start(); }
 int wc_profile_detail(int cap, int* cls, double* ms, double* work, int* info) { return prof_detail(cap, cls, ms, work, info); }

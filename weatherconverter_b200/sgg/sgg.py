@@ -9,6 +9,10 @@ back to fp32 anyway).  ``apply_lcg`` raises as shipped (SURVEY D3); here it runs
 ``criterion``: GSG with any segmentation loss.  ``criterion(logits [B,19,H,W], gt [B,H,W]) -> [B]`` per-image losses; the
 gradient d(sum_b loss_b)/d sr_xt comes from torch autograd through the segmentor (DeepLabV3.forward), then goes through the
 same update kernel with its unfused average pooling.  ``None`` keeps the fused CE(ignore 255) plan.
+
+``apply_gsg_through_srgan``: GSG guided by the exact gradient d loss / d x_t through the SRGAN generator (chain rule through
+Generator.forward's autograd path) instead of the reference's stand-in avg_pool2d(d loss / d sr_xt, 4).  Its magnitude has a
+different scale from the pooled stand-in, so ``lambda`` may need retuning (DESIGN.md section 4).
 """
 import torch
 
@@ -89,3 +93,28 @@ def apply_lcg(seg_model, mu, sigma, sr_xt, gt, _lambda, num_classes=19, pool=Non
     check(lib().wc_lcg_combine(ptr(g4), ptr(gt), ptr(mu), ptr(sigma), ptr(xt), B, num_classes, h, w, pool, float(_lambda),
                                stream_ptr()))
     return xt
+
+
+def apply_gsg_through_srgan(seg_model, srgan_model, mu, sigma, xt, gt, _lambda, criterion=None, return_aux=False):
+    """GSG with image b guided by d loss_b / d x_t[b]: sr = srgan_model(x_t) (the bits of srgan_inference), g_sr = d(sum_b
+    loss_b)/d sr from the fused CE(ignore 255) plan (``criterion=None``) or from torch autograd through the segmentor, then
+    g_x = g_sr pulled back through the generator by autograd, and the update kernel without pooling (same de-normalise and
+    channel L2).  ``return_aux`` adds dict(sr, loss, grad = g_x).  Runs torch autograd: no CUDA-graph capture."""
+    if criterion is not None and not callable(criterion):
+        raise TypeError("criterion must be a callable (logits, gt) -> per-image losses [B]")
+    _lib.require_cuda(mu, sigma, xt, gt)
+    if torch.cuda.is_current_stream_capturing():
+        raise ValueError("apply_gsg_through_srgan runs torch autograd and cannot be captured in a CUDA graph")
+    B, _, h, w = mu.shape
+    with torch.enable_grad():
+        x = xt.detach().contiguous().float().requires_grad_(True)
+        sr = srgan_model(x)
+        if criterion is None:
+            out = infer_batch(seg_model, sr.detach(), gt, grad_pool=1)
+        else:
+            out = _criterion_grad(seg_model, sr.detach(), gt, criterion)
+        g_x, = torch.autograd.grad(sr, x, out["grad"])
+    mu, sigma = mu.contiguous().float(), sigma.contiguous().float()
+    new_xt = torch.empty_like(mu)
+    check(lib().wc_sgg_update(ptr(g_x), ptr(mu), ptr(sigma), ptr(new_xt), None, B, h, w, 1, float(_lambda), stream_ptr()))
+    return (new_xt, dict(sr=sr.detach(), loss=out["loss"], grad=g_x)) if return_aux else new_xt

@@ -12,7 +12,7 @@ Batches are independent chains: image b is guided by its own loss/gradient (vmap
 """
 import torch
 
-from .sgg.sgg import apply_gsg_batch, apply_lcg
+from .sgg.sgg import apply_gsg_batch, apply_gsg_through_srgan, apply_lcg
 from .srgan_model.inference import inference as srgan_inference
 
 device = torch.device('cuda' if torch.cuda.is_available() else 'cpu')
@@ -78,7 +78,7 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
 def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srgan_model, *, n_steps=N_STEPS,
                     lam=LAMBDA, noise=None, t_forward=None, step_noise=None, device_noise=False, generator=None,
                     guidance=True, mode="gsg", reference_quirks=False, record=None, record_base=None, use_graph=False,
-                    criterion=None):
+                    criterion=None, grad_through_srgan=False):
     """input_tensor [B,3,h,w] in [-1,1]; gt [B,4h,4w] int64 trainIds (255 = ignore).  Returns sr_x0 [B,3,4h,4w].
     Injection points for parity runs: ``t_forward`` [B] (reference :63 draws randint(0, N)), ``noise`` like the input
     (:64), ``step_noise`` [N, B,3,h,w] or callable i -> z (scheduler.py:110); ``record`` / ``record_base`` collect x_t and
@@ -87,7 +87,21 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
     ``use_graph=True`` captures the guided reverse step once per guidance kind as a CUDA graph (weatherconverter_b200/graphs.py)
     and replays it: one cudaGraphLaunch per step instead of ~440 kernel launches, bit-identical to the eager loop.
     ``criterion``: callable (logits [B,19,H,W], gt [B,H,W]) -> per-image losses [B] that replaces the fused CE(ignore 255) of
-    every GSG step (sgg/sgg.py: apply_gsg_batch); eager loop and mode="gsg" only."""
+    every GSG step (sgg/sgg.py: apply_gsg_batch); eager loop and mode="gsg" only.
+    ``grad_through_srgan=True``: every GSG step is guided by the exact d loss / d x_t through the SRGAN generator
+    (sgg/sgg.py: apply_gsg_through_srgan) instead of avg_pool2d(d loss / d sr_xt, 4); the SR image is computed once per step.
+    The guidance magnitude differs in scale from the pooled stand-in, so ``lam`` may need retuning.  Eager loop, mode="gsg"
+    and reference_quirks=False only."""
+    if not isinstance(grad_through_srgan, bool):
+        raise TypeError("grad_through_srgan must be a bool")
+    if grad_through_srgan:
+        if use_graph:
+            raise ValueError("grad_through_srgan: the step runs torch autograd through the generator, which the step graph "
+                             "cannot capture; use use_graph=False")
+        if mode != "gsg":
+            raise ValueError("grad_through_srgan applies to global guidance (mode='gsg') only")
+        if reference_quirks:
+            raise ValueError("grad_through_srgan has no reference counterpart; reference_quirks=True cannot be combined with it")
     if mode not in ("gsg", "alternate", "lcg"):
         raise ValueError("mode must be 'gsg', 'alternate' or 'lcg'")
     if criterion is not None:
@@ -122,7 +136,9 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
             mu, sigma, _ = diff_scheduler.sample_prev_timestep(xt, eps, i, z=z)             # reference :78
             if record_base is not None:
                 record_base.append(mu + sigma)       # the unguided update: x_t - this = the guidance term alone
-            if guidance:
+            if guidance and grad_through_srgan:
+                xt = apply_gsg_through_srgan(seg_model, srgan_model, mu, sigma, xt, gt, lam, criterion=criterion)
+            elif guidance:
                 sr_xt = srgan_inference(srgan_model, xt)                                    # reference :81
                 if mode == "lcg" or (mode == "alternate" and i % 2 == 0):
                     guided = apply_lcg(seg_model, mu, sigma, sr_xt, gt, lam)                # reference :84-85
