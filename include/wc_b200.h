@@ -57,6 +57,22 @@ int wc_ddpm_step_batched(const float* xt, const float* eps, const float* z, floa
 int wc_ddpm_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
                          size_t n_per_sample, int batch, const float* coef_tables, const int64_t* t_dev, int num_timesteps,
                          void* stream);
+/* DDIM reverse step from timestep tau to the previous timestep tau' of a strided schedule (Song et al., "Denoising Diffusion
+ * Implicit Models"; the reference has no DDIM).  Per element, each op rounded to fp32 in this order (no FMA contraction):
+ *   x0 = (xt - s_t*eps) / a_t ; mean = a_p*x0 + d*eps ; sigz = sigma*z ; out = mean + sigz
+ * with a_t = sqrt(acp_tau), s_t = sqrt(1 - acp_tau), a_prev = sqrt(acp_tau'),
+ * sigma = eta*sqrt((1 - acp_tau')/(1 - acp_tau)*(1 - acp_tau/acp_tau')), d = sqrt(max(0, 1 - acp_tau' - sigma^2)); on the
+ * final step of a schedule (to x0) a_prev = 1, d = 0, sigma = 0.  z == NULL or sigma == 0: out = mean, sigz_out = 0.
+ * n_per_sample % 4 == 0; out / mean_out / sigz_out may each be NULL. */
+int wc_ddim_step(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                 size_t n_per_sample, int batch, float a_t, float s_t, float a_prev, float d, float sigma, void* stream);
+/* wc_ddim_step with the timestep READ FROM DEVICE MEMORY (t_dev: one int64, clamped to [0, num_timesteps)) and the five
+ * coefficients gathered from coef_tables [5, num_timesteps] fp32 = rows {a_t, s_t, a_prev, d, sigma}, column tau holding
+ * the step that STARTS at tau (same values as the scalar path -> bit-identical results).  As wc_ddpm_step_indexed, ONE
+ * captured CUDA graph of a reverse step serves every step of any schedule. */
+int wc_ddim_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                         size_t n_per_sample, int batch, const float* coef_tables, const int64_t* t_dev, int num_timesteps,
+                         void* stream);
 /* :30-35 add_noise2 / :37-61 add_noise. */
 int wc_add_noise(const float* x0, const float* noise, float* out, size_t n_per_sample, int batch,
                  const float* sqrt_acp, const float* sqrt_one_minus_acp, const int64_t* t, int num_timesteps, void* stream);

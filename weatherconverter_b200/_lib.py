@@ -40,6 +40,8 @@ _SIGS = {
     "wc_ddpm_step": (C.c_int, [c_ptr] * 6 + [C.c_size_t, C.c_int] + [C.c_float] * 4 + [c_ptr]),
     "wc_ddpm_step_batched": (C.c_int, [c_ptr] * 6 + [C.c_size_t, C.c_int] + [c_ptr] * 4 + [C.c_int, c_ptr]),
     "wc_ddpm_step_indexed": (C.c_int, [c_ptr] * 6 + [C.c_size_t, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr]),
+    "wc_ddim_step": (C.c_int, [c_ptr] * 6 + [C.c_size_t, C.c_int] + [C.c_float] * 5 + [c_ptr]),
+    "wc_ddim_step_indexed": (C.c_int, [c_ptr] * 6 + [C.c_size_t, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr]),
     "wc_add_noise": (C.c_int, [c_ptr] * 3 + [C.c_size_t, C.c_int] + [c_ptr] * 3 + [C.c_int, c_ptr]),
     "wc_set_time_factor_table": (C.c_int, [C.POINTER(C.c_float), C.c_int]),
     "wc_time_embedding": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, c_ptr]),

@@ -71,6 +71,60 @@ ddpm_step_kernel(const float4* __restrict__ xt, const float4* __restrict__ eps, 
   }
 }
 
+// DDIM step tau -> tau' (Song et al., "Denoising Diffusion Implicit Models", eq. 12):
+//   x0 = (x - s_t*eps) / a_t ; mean = a_p*x0 + d*eps ; out = mean + sigma*z
+// a_t = sqrt(acp_tau), s_t = sqrt(1 - acp_tau), a_p = sqrt(acp_tau'), d = sqrt(1 - acp_tau' - sigma^2); the final step of a
+// schedule goes to x0 (a_p = 1, d = 0, sigma = 0).
+struct DdimCoef {
+  float a_t, s_t, a_p, d, sigma;
+};
+
+__device__ __forceinline__ float ddim_mean(float x, float e, const DdimCoef& c) {
+  const float x0 = __fdiv_rn(__fsub_rn(x, __fmul_rn(c.s_t, e)), c.a_t);
+  return __fadd_rn(__fmul_rn(c.a_p, x0), __fmul_rn(c.d, e));
+}
+
+// kMode 0: coefficients by value; 2: scalar tau READ FROM DEVICE MEMORY, coefficients gathered from a host-built [5][T] table
+// (rows {a_t, s_t, a_p, d, sigma}, column = the step's current tau), as ddpm_step_kernel<2>.  z == NULL or sigma == 0:
+// out = mean and sigz_out = 0.
+template <int kMode>
+__global__ void __launch_bounds__(256)
+ddim_step_kernel(const float4* __restrict__ xt, const float4* __restrict__ eps, const float4* __restrict__ z,
+                 float4* __restrict__ out, float4* __restrict__ mean_out, float4* __restrict__ sigz_out,
+                 size_t n4_per_sample, int B, DdimCoef c, const float* __restrict__ tables,
+                 const long long* __restrict__ t, int T) {
+  pdl_prologue();
+  const size_t total = n4_per_sample * B;
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    DdimCoef cc = c;
+    if (kMode == 2) {
+      const long long tb = clamp_t(t[0], T);
+      cc.a_t = tables[tb];
+      cc.s_t = tables[T + tb];
+      cc.a_p = tables[2 * T + tb];
+      cc.d = tables[3 * T + tb];
+      cc.sigma = tables[4 * T + tb];
+    }
+    const bool use_z = z != nullptr && cc.sigma != 0.f;
+    const float4 x = xt[i], e = eps[i];
+    float4 m;
+    m.x = ddim_mean(x.x, e.x, cc); m.y = ddim_mean(x.y, e.y, cc);
+    m.z = ddim_mean(x.z, e.z, cc); m.w = ddim_mean(x.w, e.w, cc);
+    if (mean_out) mean_out[i] = m;
+    if (!use_z && sigz_out) sigz_out[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (use_z) {
+      const float4 zz = z[i];
+      float4 s;
+      s.x = __fmul_rn(cc.sigma, zz.x); s.y = __fmul_rn(cc.sigma, zz.y);
+      s.z = __fmul_rn(cc.sigma, zz.z); s.w = __fmul_rn(cc.sigma, zz.w);
+      if (sigz_out) sigz_out[i] = s;
+      m.x = __fadd_rn(m.x, s.x); m.y = __fadd_rn(m.y, s.y); m.z = __fadd_rn(m.z, s.z); m.w = __fadd_rn(m.w, s.w);
+    }
+    if (out) out[i] = m;
+  }
+}
+
 // x_t = sqrt(acp[t_b]) * x0 + sqrt(1-acp[t_b]) * noise     (scheduler.py:30-35, 37-61)
 __global__ void __launch_bounds__(256)
 add_noise_kernel(const float4* __restrict__ x0, const float4* __restrict__ noise, float4* __restrict__ out,
@@ -217,6 +271,35 @@ int ddpm_step_indexed(const float* xt, const float* eps, const float* z, float* 
       reinterpret_cast<const float4*>(xt), reinterpret_cast<const float4*>(eps), reinterpret_cast<const float4*>(z),
       reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(mean_out), reinterpret_cast<float4*>(sigz_out), n4, B,
       c, coef_tables, nullptr, nullptr, t_dev, T);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+
+int ddim_step(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+              size_t n_per_sample, int B, float a_t, float s_t, float a_prev, float d, float sigma, cudaStream_t st) {
+  WC_REQUIRE(n_per_sample % 4 == 0, "elements per sample must be a multiple of 4");
+  DdimCoef c{a_t, s_t, a_prev, d, sigma};
+  const size_t n4 = n_per_sample / 4;
+  ProfScope prof(kProfScheduler, st, 4.0 * n_per_sample * B * (2 + (z ? 1 : 0) + (out ? 1 : 0) + (mean_out ? 1 : 0) + (sigz_out ? 1 : 0)));
+  launch_k(ddim_step_kernel<0>, grid_for(n4 * B), 256, 0, st,
+      reinterpret_cast<const float4*>(xt), reinterpret_cast<const float4*>(eps), reinterpret_cast<const float4*>(z),
+      reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(mean_out), reinterpret_cast<float4*>(sigz_out), n4, B,
+      c, nullptr, nullptr, 1);
+  WC_LAUNCH_CHECK();
+  return 0;
+}
+
+int ddim_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                      size_t n_per_sample, int B, const float* coef_tables, const long long* t_dev, int T, cudaStream_t st) {
+  WC_REQUIRE(n_per_sample % 4 == 0, "elements per sample must be a multiple of 4");
+  WC_REQUIRE(T >= 1 && coef_tables && t_dev, "ddim_step_indexed: tables and the device timestep are required");
+  DdimCoef c{1, 0, 1, 0, 0};
+  const size_t n4 = n_per_sample / 4;
+  ProfScope prof(kProfScheduler, st, 4.0 * n_per_sample * B * (2 + (z ? 1 : 0) + (out ? 1 : 0) + (mean_out ? 1 : 0) + (sigz_out ? 1 : 0)));
+  launch_k(ddim_step_kernel<2>, grid_for(n4 * B), 256, 0, st,
+      reinterpret_cast<const float4*>(xt), reinterpret_cast<const float4*>(eps), reinterpret_cast<const float4*>(z),
+      reinterpret_cast<float4*>(out), reinterpret_cast<float4*>(mean_out), reinterpret_cast<float4*>(sigz_out), n4, B,
+      c, coef_tables, t_dev, T);
   WC_LAUNCH_CHECK();
   return 0;
 }

@@ -12,6 +12,10 @@ int ddpm_step_batched(const float* xt, const float* eps, const float* z, float* 
                       const long long* t, int T, cudaStream_t st);
 int ddpm_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
                       size_t n_per_sample, int B, const float* coef_tables, const long long* t_dev, int T, cudaStream_t st);
+int ddim_step(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+              size_t n_per_sample, int B, float a_t, float s_t, float a_prev, float d, float sigma, cudaStream_t st);
+int ddim_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                      size_t n_per_sample, int B, const float* coef_tables, const long long* t_dev, int T, cudaStream_t st);
 int add_noise(const float* x0, const float* noise, float* out, size_t n_per_sample, int B, const float* sqrt_acp,
               const float* sqrt_1m_acp, const long long* t, int T, cudaStream_t st);
 int sgg_update(const float* grad, const float* mu, const float* sigz, float* out, float* mag_out, int B, int h, int w,
@@ -87,7 +91,7 @@ static inline const __nv_bfloat16* BF(const wc_bf16* p) { return reinterpret_cas
 extern "C" {
 
 const char* wc_last_error(void) { return last_error_cstr(); }
-int wc_abi_version(void) { return 5; }
+int wc_abi_version(void) { return 6; }
 long long wc_launch_count(void) { return launch_count(); }
 void wc_profile_begin(void) { prof_start(); }
 int wc_profile_detail(int cap, int* cls, double* ms, double* work, int* info) { return prof_detail(cap, cls, ms, work, info); }
@@ -111,6 +115,16 @@ int wc_ddpm_step_indexed(const float* xt, const float* eps, const float* z, floa
                          size_t n_per_sample, int batch, const float* coef_tables, const int64_t* t_dev, int num_timesteps,
                          void* stream) {
   return ddpm_step_indexed(xt, eps, z, out, mean_out, sigz_out, n_per_sample, batch, coef_tables,
+                           reinterpret_cast<const long long*>(t_dev), num_timesteps, S(stream));
+}
+int wc_ddim_step(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                 size_t n_per_sample, int batch, float a_t, float s_t, float a_prev, float d, float sigma, void* stream) {
+  return ddim_step(xt, eps, z, out, mean_out, sigz_out, n_per_sample, batch, a_t, s_t, a_prev, d, sigma, S(stream));
+}
+int wc_ddim_step_indexed(const float* xt, const float* eps, const float* z, float* out, float* mean_out, float* sigz_out,
+                         size_t n_per_sample, int batch, const float* coef_tables, const int64_t* t_dev, int num_timesteps,
+                         void* stream) {
+  return ddim_step_indexed(xt, eps, z, out, mean_out, sigz_out, n_per_sample, batch, coef_tables,
                            reinterpret_cast<const long long*>(t_dev), num_timesteps, S(stream));
 }
 int wc_add_noise(const float* x0, const float* noise, float* out, size_t n_per_sample, int batch,

@@ -24,27 +24,36 @@ def load_config(config_path: str) -> Config:
 
 @torch.no_grad()
 def sample_tensor(model, scheduler, shape=None, num_timesteps=None, xT=None, noise=None, device_noise=False,
-                  generator=None, record=None, use_graph=False):
+                  generator=None, record=None, use_graph=False, sampler=None):
     """Reverse loop of sample_ddpm.py:35-44.  noise: optional [T, *shape] tensor (or callable i -> tensor), noise[i]
     is the z drawn at step i.  device_noise=True draws z with the CUDA generator instead of the reference's CPU
-    generator (throughput runs).  Returns x_0 (un-clamped, as the loop leaves it)."""
+    generator (throughput runs).  sampler: a DDIMSchedule (``scheduler.ddim(...)``); the loop then walks
+    ``sampler.timesteps`` instead of every timestep, and noise[t] / noise(t) is the z of the step that starts at t.
+    ``record`` gets one entry per executed step.  Returns x_0 (un-clamped, as the loop leaves it)."""
     T = num_timesteps if num_timesteps is not None else scheduler.num_timesteps
+    steps = list(reversed(range(T))) if sampler is None else sampler.timesteps
+    if sampler is not None and max(steps) >= T:
+        raise ValueError(f"the DDIM schedule has timestep {max(steps)}, beyond this {T}-step chain")
+    sched = scheduler if sampler is None else sampler
+    noisy = sampler is None or sampler.eta > 0                     # eta == 0: DDIM draws no noise
     if xT is None:
         xT = torch.randn(shape).to(device)                         # reference :35 (CPU generator, then H2D)
     xt = xT.to(device).float().contiguous()
-    if use_graph and T > 1:
-        # every step i > 0 replays ONE captured CUDA graph (UNet forward + fused posterior update with the timestep read on
-        # the device): one cudaGraphLaunch per step instead of ~330 kernel launches; bit-identical to the eager loop below
+    if use_graph and len(steps) > 1:
+        # every step but the last replays ONE captured CUDA graph (UNet forward + fused posterior update with the timestep
+        # read on the device): one cudaGraphLaunch per step instead of ~330 kernel launches; bit-identical to the eager loop
         from ..graphs import StepGraph
 
         def step(x, t_dev, z):
-            return scheduler.step_indexed(x, model(x, t_dev), t_dev, z)
+            return sched.step_indexed(x, model(x, t_dev), t_dev, z)
         sg = StepGraph(step, xt.shape, xt.device)
         sg.load(xt)
         t_all = torch.arange(T, device=xt.device, dtype=torch.int64)
-        for i in reversed(range(1, T)):
+        for i in steps[:-1]:
             if noise is not None:
                 z = (noise(i) if callable(noise) else noise[i]).to(xt.device)
+            elif not noisy:
+                z = None
             elif device_noise:
                 z = torch.randn(xt.shape, device=xt.device, generator=generator)
             else:
@@ -52,24 +61,24 @@ def sample_tensor(model, scheduler, shape=None, num_timesteps=None, xT=None, noi
             sg.replay(t_all[i:i + 1], z)
             if record is not None:
                 record.append(sg.xt.clone())
-        xt = scheduler.step(sg.xt, model(sg.xt, t_all[0:1]), 0)
+        xt = sched.step(sg.xt, model(sg.xt, t_all[steps[-1]:steps[-1] + 1]), steps[-1])
         if record is not None:
             record.append(xt.clone())
         return xt
     eps = torch.empty_like(xt)
-    for i in reversed(range(T)):
+    for i in steps:
         t = torch.as_tensor(i).unsqueeze(0).to(xt.device)          # reference :39
         model(xt, t, out=eps)
-        if i == 0:
+        if i == steps[-1]:
             z = None
         elif noise is not None:
             z = noise(i) if callable(noise) else noise[i]
             z = z.to(xt.device)
-        elif device_noise:
+        elif device_noise and noisy:
             z = torch.randn(xt.shape, device=xt.device, generator=generator)
         else:
             z = None                                               # scheduler draws from the CPU generator (:110)
-        xt = scheduler.step(xt, eps, i, z=z)                       # fused mean + sigma*z (reference :42-44)
+        xt = sched.step(xt, eps, i, z=z)                           # fused mean + sigma*z (reference :42-44)
         if record is not None:
             record.append(xt.clone())
     return xt

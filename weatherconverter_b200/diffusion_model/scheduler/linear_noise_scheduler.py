@@ -155,6 +155,40 @@ class LinearNoiseScheduler:
                                  stream_ptr()))
         return mean, sigz, None
 
+    def ddim(self, num_steps=None, eta=0.0, num_timesteps=None, timesteps=None):
+        """DDIM sampler (Song et al., "Denoising Diffusion Implicit Models") on this scheduler's alpha_cum_prod: the same
+        trained eps-prediction model, sampled on a strided subsequence of the timesteps without retraining.
+        ``num_steps``: the timesteps are round(linspace(0, n - 1, num_steps)) (half to even), descending, n = ``num_timesteps``
+        or self.num_timesteps; they include n - 1 and 0.  ``timesteps``: an explicit strictly descending list of distinct ints
+        in [0, n) instead.  ``eta`` in [0, 1]: 0 is deterministic, 1 is DDPM-like noise.  The step from the last listed
+        timestep goes to x0 (at 0 it matches the DDPM loop's t == 0 step)."""
+        n = self.num_timesteps if num_timesteps is None else int(num_timesteps)
+        if not 1 <= n <= self.num_timesteps:
+            raise ValueError(f"num_timesteps must be in [1, {self.num_timesteps}], got {n}")
+        eta = float(eta)
+        if not 0.0 <= eta <= 1.0:
+            raise ValueError(f"eta must be in [0, 1], got {eta}")
+        if (num_steps is None) == (timesteps is None):
+            raise ValueError("give exactly one of num_steps and timesteps")
+        if timesteps is None:
+            num_steps = int(num_steps)
+            if not 1 <= num_steps <= n or (num_steps == 1 and n > 1):
+                raise ValueError(f"num_steps must be in [2, {n}] (1 only when num_timesteps == 1), got {num_steps}")
+            ts = torch.linspace(0, n - 1, num_steps, dtype=torch.float64).round().long().flip(0).tolist()
+        else:
+            ts = [int(t) for t in timesteps]
+            if any(a != b for a, b in zip(ts, timesteps)):
+                raise ValueError("timesteps must be integers")
+            if not ts:
+                raise ValueError("timesteps is empty")
+            if len(set(ts)) != len(ts):
+                raise ValueError("timesteps has duplicates")
+            if min(ts) < 0 or max(ts) >= n:
+                raise ValueError(f"timesteps must lie in [0, {n})")
+            if any(a <= b for a, b in zip(ts, ts[1:])):
+                raise ValueError("timesteps must be strictly descending")
+        return DDIMSchedule(self, ts, eta, n)
+
     def sample_prev_timestep2(self, xt, noise_pred, t, z=None):
         """Reference :63-77: batched t [B], sigma^2 = beta_t; (mean, None, None) only if ALL t == 0."""
         _lib.require_cuda(xt, noise_pred, z)
@@ -177,3 +211,102 @@ class LinearNoiseScheduler:
         check(lib().wc_ddpm_step_batched(ptr(xt), ptr(noise_pred), ptr(z), None, ptr(mean), ptr(sigz), xt[0].numel(),
                                          B, *tabs, ptr(t), self.num_timesteps, stream_ptr()))
         return mean, sigz, None
+
+
+class DDIMSchedule:
+    """A DDIM reverse process over ``timesteps`` (descending) of a LinearNoiseScheduler; built by
+    ``LinearNoiseScheduler.ddim``.  Same reverse-step methods and return conventions as the scheduler, so the sampling
+    drivers call either object the same way; the previous timestep of t is the next entry of ``timesteps``.
+
+    Coefficients per step (float64 from the scheduler's fp32 alpha_cum_prod, each rounded to fp32 once) live in a [5, n]
+    table, column t holding the step that starts at t: {a_t = sqrt(acp_t), s_t = sqrt(1 - acp_t), a_prev = sqrt(acp_t'),
+    d = sqrt(max(0, 1 - acp_t' - sigma^2)), sigma = eta * sqrt((1 - acp_t') / (1 - acp_t) * (1 - acp_t / acp_t'))}; the
+    final step goes to x0 (a_prev = 1, d = 0, sigma = 0).  Columns of timesteps outside the schedule hold the identity step
+    and are never read by the drivers.  Steps with sigma == 0 (eta == 0, and the final step) draw no noise."""
+
+    def __init__(self, scheduler, timesteps, eta, num_timesteps):
+        self.scheduler = scheduler
+        self.timesteps = list(timesteps)
+        self.eta = eta
+        self.num_timesteps = num_timesteps
+        acp = scheduler._host["alpha_cum_prod"].double()
+        tab = torch.zeros(5, num_timesteps, dtype=torch.float64)
+        tab[0] = 1.0
+        tab[2] = 1.0
+        for k, t in enumerate(self.timesteps):
+            a = acp[t]
+            tab[0, t], tab[1, t] = a.sqrt(), (1 - a).sqrt()
+            if k + 1 < len(self.timesteps):
+                ap = acp[self.timesteps[k + 1]]
+                sigma = eta * ((1 - ap) / (1 - a) * (1 - a / ap)).sqrt()
+                tab[2, t], tab[3, t], tab[4, t] = ap.sqrt(), (1 - ap - sigma * sigma).clamp(min=0).sqrt(), sigma
+        self.coef_table = tab.float()
+        self._coef = {t: self.coef_table[:, t].tolist() for t in self.timesteps}
+
+    def _check_t(self, t):
+        t = int(t)
+        if t not in self._coef:
+            raise IndexError(f"timestep {t} is not in this DDIM schedule")
+        return t
+
+    def _tables_on(self, dev):
+        key = str(dev)
+        cache = self.__dict__.setdefault("_coef_dev", {})
+        if key not in cache:
+            cache[key] = self.coef_table.to(dev).contiguous()
+        return cache[key]
+
+    def _launch(self, xt, noise_pred, t, z, out, mean, sigz):
+        check(lib().wc_ddim_step(ptr(xt), ptr(noise_pred), ptr(z), ptr(out), ptr(mean), ptr(sigz), xt[0].numel(),
+                                 xt.shape[0], *self._coef[t], stream_ptr()))
+
+    def _noise(self, xt, t, z):
+        """fp32 z for a step with sigma != 0 (drawn like the scheduler's when not given); None for a step without noise."""
+        if self._coef[t][4] == 0.0:
+            return None
+        return LinearNoiseScheduler._f32(xt, self.scheduler._draw(xt) if z is None else z)[1]
+
+    def step(self, xt, noise_pred, t, z=None):
+        """x_{t'} = mean + sigma * z in one launch (z ignored where sigma == 0)."""
+        _lib.require_cuda(xt, noise_pred, z)
+        t = self._check_t(t)
+        xt, noise_pred = LinearNoiseScheduler._f32(xt, noise_pred)
+        out = torch.empty_like(xt)
+        self._launch(xt, noise_pred, t, self._noise(xt, t, z), out, None, None)
+        return out
+
+    def sample_prev_timestep(self, xt, noise_pred, t, z=None):
+        """(mean, sigma * z, None); (mean, None, None) where sigma == 0."""
+        _lib.require_cuda(xt, noise_pred, z)
+        t = self._check_t(t)
+        xt, noise_pred = LinearNoiseScheduler._f32(xt, noise_pred)
+        z = self._noise(xt, t, z)
+        mean = torch.empty_like(xt)
+        sigz = None if z is None else torch.empty_like(xt)
+        self._launch(xt, noise_pred, t, z, None, mean, sigz)
+        return mean, sigz, None
+
+    def sample_prev_timestep_indexed(self, xt, noise_pred, t_dev, z, out=None):
+        """(mean, sigma*z[, x_{t'} into ``out``]) with t read on the device from ``t_dev`` (int64, one element): one captured
+        launch serves every step of the schedule.  sigma*z is zero where sigma == 0."""
+        _lib.require_cuda(xt, noise_pred, z, t_dev)
+        if t_dev.dtype != torch.int64 or t_dev.numel() != 1:
+            raise RuntimeError("t_dev must be a CUDA int64 tensor with one element")
+        xt, noise_pred, z = LinearNoiseScheduler._f32(xt, noise_pred, z)
+        mean, sigz = torch.empty_like(xt), torch.empty_like(xt)
+        check(lib().wc_ddim_step_indexed(ptr(xt), ptr(noise_pred), ptr(z), ptr(out), ptr(mean), ptr(sigz), xt[0].numel(),
+                                         xt.shape[0], ptr(self._tables_on(xt.device)), ptr(t_dev), self.num_timesteps,
+                                         stream_ptr()))
+        return mean, sigz, None
+
+    def step_indexed(self, xt, noise_pred, t_dev, z, out=None):
+        """x_{t'} = mean + sigma * z in one launch with the timestep read from device memory."""
+        _lib.require_cuda(xt, noise_pred, z, t_dev)
+        if t_dev.dtype != torch.int64 or t_dev.numel() != 1:
+            raise RuntimeError("t_dev must be a CUDA int64 tensor with one element")
+        xt, noise_pred, z = LinearNoiseScheduler._f32(xt, noise_pred, z)
+        if out is None:
+            out = torch.empty_like(xt)
+        check(lib().wc_ddim_step_indexed(ptr(xt), ptr(noise_pred), ptr(z), ptr(out), None, None, xt[0].numel(), xt.shape[0],
+                                         ptr(self._tables_on(xt.device)), ptr(t_dev), self.num_timesteps, stream_ptr()))
+        return out

@@ -31,10 +31,10 @@ def load_input_image(path: str, image_size: int = 128) -> torch.Tensor:
     return image_io.diffusion_input(img, image_size)
 
 
-def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srgan_model, n_steps, lam, step_noise, device_noise,
-                             generator, mode, record):
-    """The loop of sample_with_sgg with every guided step (i > 0) replayed from a captured CUDA graph.  One graph per
-    guidance kind in use (GSG and / or LCG); the timestep and the noise are fed through static device buffers."""
+def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, sched, steps, seg_model, gt, srgan_model, n_steps, lam,
+                             step_noise, device_noise, generator, mode, record):
+    """The loop of sample_with_sgg with every guided step (all but the last) replayed from a captured CUDA graph.  One graph
+    per guidance kind in use (GSG and / or LCG); the timestep and the noise are fed through static device buffers."""
     from .graphs import StepGraph
     dev = xt.device
     # GSG runs the segmentor on B images, LCG on 19 B masked images: two plan bindings that must both stay alive
@@ -43,7 +43,7 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
     def make(kind):
         def step(x, t_dev, z):
             eps = diff_model(x, t_dev)                                                      # reference :74
-            mu, sigma, _ = diff_scheduler.sample_prev_timestep_indexed(x, eps, t_dev, z)    # reference :78
+            mu, sigma, _ = sched.sample_prev_timestep_indexed(x, eps, t_dev, z)             # reference :78
             sr_xt = srgan_inference(srgan_model, x)                                         # reference :81
             if kind == "lcg":
                 return apply_lcg(seg_for["lcg"], mu, sigma, sr_xt, gt, lam)                 # reference :84-85
@@ -51,13 +51,14 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
         return StepGraph(step, xt.shape, dev)
 
     kinds = {"gsg": ("gsg",), "lcg": ("lcg",), "alternate": ("gsg", "lcg")}[mode]
-    graphs = {k: make(k) for k in kinds} if n_steps > 1 else {}
+    graphs = {k: make(k) for k in kinds} if len(steps) > 1 else {}
     t_all = torch.arange(n_steps, device=dev, dtype=torch.int64)
     cur = xt
-    for i in reversed(range(n_steps)):
-        if i == 0:
-            eps = diff_model(cur, t_all[0:1])
-            cur = diff_scheduler.step(cur, eps, 0)                                          # repair of D2: x_0 = mu
+    last = len(steps) - 1
+    for k, i in enumerate(steps):
+        if k == last:
+            eps = diff_model(cur, t_all[i:i + 1])
+            cur = sched.step(cur, eps, i)                                                   # repair of D2: x_0 = mu
         else:
             if step_noise is not None:
                 z = (step_noise(i) if callable(step_noise) else step_noise[i]).to(dev)
@@ -65,7 +66,7 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
                 z = torch.randn(cur.shape, device=dev, generator=generator)
             else:
                 z = diff_scheduler._draw(cur)                                               # reference scheduler.py:110
-            g = graphs["lcg" if (mode == "lcg" or (mode == "alternate" and i % 2 == 0)) else "gsg"]
+            g = graphs["lcg" if (mode == "lcg" or (mode == "alternate" and (last - k) % 2 == 0)) else "gsg"]
             if cur is not g.xt:
                 g.load(cur)
             cur = g.replay(t_all[i:i + 1], z)
@@ -78,7 +79,7 @@ def _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srga
 def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srgan_model, *, n_steps=N_STEPS,
                     lam=LAMBDA, noise=None, t_forward=None, step_noise=None, device_noise=False, generator=None,
                     guidance=True, mode="gsg", reference_quirks=False, record=None, record_base=None, use_graph=False,
-                    criterion=None, grad_through_srgan=False):
+                    criterion=None, grad_through_srgan=False, sampler=None):
     """input_tensor [B,3,h,w] in [-1,1]; gt [B,4h,4w] int64 trainIds (255 = ignore).  Returns sr_x0 [B,3,4h,4w].
     Injection points for parity runs: ``t_forward`` [B] (reference :63 draws randint(0, N)), ``noise`` like the input
     (:64), ``step_noise`` [N, B,3,h,w] or callable i -> z (scheduler.py:110); ``record`` / ``record_base`` collect x_t and
@@ -91,7 +92,11 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
     ``grad_through_srgan=True``: every GSG step is guided by the exact d loss / d x_t through the SRGAN generator
     (sgg/sgg.py: apply_gsg_through_srgan) instead of avg_pool2d(d loss / d sr_xt, 4); the SR image is computed once per step.
     The guidance magnitude differs in scale from the pooled stand-in, so ``lam`` may need retuning.  Eager loop, mode="gsg"
-    and reference_quirks=False only."""
+    and reference_quirks=False only.
+    ``sampler``: a DDIMSchedule (``diff_scheduler.ddim(..., num_timesteps=n_steps)``); the loop walks ``sampler.timesteps``
+    instead of all n_steps timesteps, guidance runs on every step but the last with mu = the DDIM mean and sigma = its
+    sigma * z, and "alternate" runs LCG on the steps whose position from the end is even.  Choosing ``lam`` for a strided
+    schedule is the caller's job: a DDIM step's sigma is larger than a DDPM step's, and nothing is rescaled."""
     if not isinstance(grad_through_srgan, bool):
         raise TypeError("grad_through_srgan must be a bool")
     if grad_through_srgan:
@@ -110,6 +115,17 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
                              "use use_graph=False")
         if mode != "gsg":
             raise ValueError("criterion applies to global guidance (mode='gsg') only; local class guidance uses the fused CE")
+    if sampler is not None:
+        if max(sampler.timesteps) >= n_steps:
+            raise ValueError(f"the DDIM schedule has timestep {max(sampler.timesteps)}, beyond this {n_steps}-step chain")
+        if reference_quirks:
+            raise ValueError("the reference has no DDIM sampler; reference_quirks=True cannot be combined with sampler")
+        if guidance and sampler.eta == 0:
+            raise ValueError("guidance scales its term by the step's sigma * z, which is 0 for a DDIM schedule with eta == 0: "
+                             "guidance would silently do nothing; use eta > 0 or guidance=False")
+    sched = diff_scheduler if sampler is None else sampler
+    steps = list(reversed(range(n_steps))) if sampler is None else sampler.timesteps
+    noisy = sampler is None or sampler.eta > 0                                             # eta == 0: DDIM draws no noise
     x0 = input_tensor.to(device).float().contiguous()
     gt = gt.to(device)
     B = x0.shape[0]
@@ -117,36 +133,37 @@ def sample_with_sgg(input_tensor, diff_model, diff_scheduler, seg_model, gt, srg
     noise = noise if noise is not None else torch.randn_like(x0)                            # reference :64
     xt = diff_scheduler.add_noise2(x0, noise.to(device), t.to(device))                      # reference :65
     if use_graph and guidance and not reference_quirks and record_base is None:
-        return _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, seg_model, gt, srgan_model, n_steps, lam, step_noise,
-                                        device_noise, generator, mode, record)
+        return _sample_with_sgg_graphed(xt, diff_model, diff_scheduler, sched, steps, seg_model, gt, srgan_model, n_steps,
+                                        lam, step_noise, device_noise, generator, mode, record)
     eps = torch.empty_like(xt)
-    for i in reversed(range(n_steps)):                                                      # reference :70
+    last = len(steps) - 1
+    for k, i in enumerate(steps):                                                           # reference :70
         diff_model(xt, torch.as_tensor(i).unsqueeze(0).to(device), out=eps)                # reference :74
-        if i == 0:
-            xt = diff_scheduler.step(xt, eps, 0)                                            # repair of D2: x_0 = mu
+        if k == last:
+            xt = sched.step(xt, eps, i)                                                     # repair of D2: x_0 = mu
             if record_base is not None:
                 record_base.append(xt.clone())
         else:
             if step_noise is not None:
                 z = (step_noise(i) if callable(step_noise) else step_noise[i]).to(device)
-            elif device_noise:
+            elif device_noise and noisy:
                 z = torch.randn(xt.shape, device=xt.device, generator=generator)
             else:
                 z = None
-            mu, sigma, _ = diff_scheduler.sample_prev_timestep(xt, eps, i, z=z)             # reference :78
-            if record_base is not None:
-                record_base.append(mu + sigma)       # the unguided update: x_t - this = the guidance term alone
+            mu, sigma, _ = sched.sample_prev_timestep(xt, eps, i, z=z)                      # reference :78
+            if record_base is not None:              # the unguided update: x_t - this = the guidance term alone
+                record_base.append(mu if sigma is None else mu + sigma)                     # sigma None: DDIM, eta == 0
             if guidance and grad_through_srgan:
                 xt = apply_gsg_through_srgan(seg_model, srgan_model, mu, sigma, xt, gt, lam, criterion=criterion)
             elif guidance:
                 sr_xt = srgan_inference(srgan_model, xt)                                    # reference :81
-                if mode == "lcg" or (mode == "alternate" and i % 2 == 0):
+                if mode == "lcg" or (mode == "alternate" and (last - k) % 2 == 0):
                     guided = apply_lcg(seg_model, mu, sigma, sr_xt, gt, lam)                # reference :84-85
                 else:
                     guided = apply_gsg_batch(seg_model, mu, sigma, sr_xt, gt, lam, criterion=criterion)  # reference :86-87
                 xt = (mu + sigma) if reference_quirks else guided                           # reference :90 (D1)
             else:
-                xt = mu + sigma
+                xt = mu if sigma is None else mu + sigma
         if record is not None:
             record.append(xt.clone())
     return srgan_inference(srgan_model, xt)                                                 # reference :95-97
