@@ -50,6 +50,18 @@ def test_no_oracle_in_product():
     assert not bad, bad
 
 
+def test_no_environment_switches():
+    """The library reads no environment variables: every tuning choice is fixed in the code (DESIGN.md section 8)."""
+    bad = []
+    for dp, _, fns in os.walk(os.path.join(ROOT, "weatherconverter_b200")):
+        for fn in fns:
+            if fn.endswith((".py", ".cu", ".cuh", ".h")):
+                src = open(os.path.join(dp, fn)).read()
+                if re.search(r"\bgetenv\s*\(|\bos\.environ\b|\bos\.getenv\b", src):
+                    bad.append(os.path.join(dp, fn))
+    assert not bad, bad
+
+
 def test_unet_state_dict_matches_oracle_spec():
     from oracle.unet import DEFAULT_MODEL_CONFIG, unet_param_spec
     from weatherconverter_b200.diffusion_model.models.unet_base import Unet, param_spec

@@ -18,4 +18,4 @@ for (B, h, N, hd) in shapes:
     e0.record()
     for _ in range(5): ops.attention(q, k, vt, scale=-1.0)
     e1.record(); torch.cuda.synchronize()
-    print(f"B{B} h{h} N{N} hd{hd} poly={os.environ.get('WC_ATTN_SMALL4_POLY')} hd32four={os.environ.get('WC_ATTN_SMALL4_HD32')}: {e0.elapsed_time(e1)/5:.3f} ms", flush=True)
+    print(f"B{B} h{h} N{N} hd{hd}: {e0.elapsed_time(e1)/5:.3f} ms", flush=True)

@@ -8,14 +8,13 @@
 //   warps 4-7   softmax for query tile 0 (one thread per query row; no shuffles needed)
 //   warps 8-11  softmax for query tile 1 (NQ == 2): while one group exponentiates, the tensor core works for
 //               the other group, so MUFU and tcgen05 overlap.
-// S and O live in TMEM (per query tile: BKV + hd fp32 columns); P is written as bf16 into shared memory in the
-// canonical K-major 128-byte-swizzled UMMA layout; V is consumed as V^T[hd][keys] (K-major B operand), which the
-// QKV projection epilogue writes directly.  Online softmax with lazy rescaling (only when the running max grows
+// S, O and P live in TMEM (per query tile: BKV + hd fp32 columns, then BKV / 2 columns of bf16 pairs): the softmax threads write P
+// with tcgen05.st (lane = query row) and the PV tcgen05.mma reads it as its A operand; V is consumed as V^T[hd][keys] (K-major B
+// operand), which the QKV projection epilogue writes directly.  Head_dim 16 / 32 run on attention_small*.cu instead.  Online softmax with lazy rescaling (only when the running max grows
 // by more than 2^8), accumulation in fp32.
 #include "wc_host.h"
 #include "wc_ptx.cuh"
 
-#include <cstdlib>
 #include <type_traits>
 
 namespace wc {
@@ -33,9 +32,7 @@ struct AttnMaps {
   CUtensorMap q, k, vt;
 };
 
-// TP: P lives in TENSOR MEMORY (written by the softmax threads with tcgen05.st, read by the PV tcgen05.mma as its A operand:
-// lane = query row, two bf16 per 32-bit column) instead of shared memory.
-template <int HD, int BKV, int NQ, bool TP = false>
+template <int HD, int BKV, int NQ>
 struct AttnCfg {
   static constexpr int kKBlocks = HD >= 64 ? HD / 64 : 1;          // 64-wide K blocks of the QK^T contraction
   static constexpr int kSwz = HD >= 64 ? 128 : HD * 2;             // swizzle span of Q/K rows (bytes)
@@ -44,27 +41,26 @@ struct AttnCfg {
   static constexpr uint32_t kQTile = 128 * HD * 2;
   static constexpr uint32_t kKTile = BKV * HD * 2;
   static constexpr uint32_t kVTile = HD * BKV * 2;
-  static constexpr uint32_t kPTile = 128 * BKV * 2;
   static constexpr int kStages = 2;
-  static constexpr uint32_t kSmem = NQ * kQTile + kStages * (kKTile + kVTile) + (TP ? 0 : NQ * kPTile) + 1024 + 256;
+  static constexpr uint32_t kSmem = NQ * kQTile + kStages * (kKTile + kVTile) + 1024 + 256;
   static constexpr int kThreads = 128 + 128 * NQ;
-  static constexpr int kColsPerQ = BKV + HD + (TP ? BKV / 2 : 0);
+  static constexpr int kColsPerQ = BKV + HD + BKV / 2;   // S, O, P (two bf16 per 32-bit column)
   static_assert(NQ * kColsPerQ <= 512, "TMEM budget");
   static constexpr uint32_t kTmemCols = NQ * kColsPerQ <= 256 ? 256 : 512;
 };
 
-// POLY: of every 32 exponentials, this many run on the FMA pipe (even)
-template <int HD, int BKV, int NQ, int POLY, bool TP>
-__global__ void __launch_bounds__(AttnCfg<HD, BKV, NQ, TP>::kThreads, 1)
+constexpr int kAttnPoly = 14;   // of every 32 exponentials, this many run on the FMA pipe (even)
+
+template <int HD, int BKV, int NQ>
+__global__ void __launch_bounds__(AttnCfg<HD, BKV, NQ>::kThreads, 1)
 attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ AttnArgs p) {
-  using Cfg = AttnCfg<HD, BKV, NQ, TP>;
+  using Cfg = AttnCfg<HD, BKV, NQ>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t q_smem = base;
   const uint32_t k_smem = q_smem + NQ * Cfg::kQTile;
   const uint32_t v_smem = k_smem + Cfg::kStages * Cfg::kKTile;
-  const uint32_t p_smem = v_smem + Cfg::kStages * Cfg::kVTile;
-  const uint32_t bars = p_smem + (TP ? 0u : NQ * Cfg::kPTile);
+  const uint32_t bars = v_smem + Cfg::kStages * Cfg::kVTile;
   // barrier map (8 bytes each)
   const uint32_t q_full = bars;
   auto k_full = [&](int s) { return bars + 8u * (1 + s); };
@@ -142,10 +138,10 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
       // Descriptors: constant high words, low words advanced with 32-bit adds (the issuing lane's integer work is
       // exposed latency between MMAs).
       const uint64_t dq = umma_smem_desc(q_smem, Cfg::kSwz, 8 * Cfg::kRowBytes);
-      const uint64_t dp = umma_smem_desc(p_smem, 128, 1024);
-      const uint32_t hi_qk = umma_desc_hi(dq), hi_pv = umma_desc_hi(dp);
+      const uint64_t dv = umma_smem_desc(v_smem, 128, 1024);
+      const uint32_t hi_qk = umma_desc_hi(dq), hi_pv = umma_desc_hi(dv);
       const uint32_t q_lo0 = umma_desc_lo(dq), k_lo0 = q_lo0 + ((k_smem - q_smem) >> 4);
-      const uint32_t p_lo0 = umma_desc_lo(dp), v_lo0 = p_lo0 - ((p_smem - v_smem) >> 4);
+      const uint32_t v_lo0 = umma_desc_lo(dv);
       auto issue_s = [&](int q, int j) {
         const uint32_t d = tmem_base + q * Cfg::kColsPerQ;
         const uint32_t q_lo = q_lo0 + q * (Cfg::kQTile >> 4), k_lo = k_lo0 + (j & 1) * (Cfg::kKTile >> 4);
@@ -160,17 +156,13 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
       };
       auto issue_pv = [&](int q, int j) {
         const uint32_t d = tmem_base + q * Cfg::kColsPerQ + BKV;
-        const uint32_t p_lo = p_lo0 + q * (Cfg::kPTile >> 4), v_lo = v_lo0 + (j & 1) * (Cfg::kVTile >> 4);
+        const uint32_t v_lo = v_lo0 + (j & 1) * (Cfg::kVTile >> 4);
 #pragma unroll
         for (int vb = 0; vb < BKV / 64; ++vb) {
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            if (TP)
-              umma_bf16_ts(d, d + HD + 8u * (vb * 4 + k), umma_desc_join(v_lo + vb * ((HD * 128) >> 4) + 2u * k, hi_pv), idesc_o,
-                           (j | vb | k) != 0 ? 1u : 0u);
-            else
-              umma_bf16(d, umma_desc_join(p_lo + vb * ((128 * 128) >> 4) + 2u * k, hi_pv),
-                        umma_desc_join(v_lo + vb * ((HD * 128) >> 4) + 2u * k, hi_pv), idesc_o, (j | vb | k) != 0 ? 1u : 0u);
+            umma_bf16_ts(d, d + HD + 8u * (vb * 4 + k), umma_desc_join(v_lo + vb * ((HD * 128) >> 4) + 2u * k, hi_pv), idesc_o,
+                         (j | vb | k) != 0 ? 1u : 0u);
         }
         umma_commit(pv_done(q));
       };
@@ -213,7 +205,6 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
     const uint32_t lane_off = static_cast<uint32_t>(quad * 32) << 16;
     const uint32_t s_tmem = tmem_base + q * Cfg::kColsPerQ + lane_off;
     const uint32_t o_tmem = s_tmem + BKV;
-    const uint32_t p_row = p_smem + q * Cfg::kPTile + row * 128;
     const float sl2 = p.scale_log2;
     float m = -INFINITY;
     float2 lsum[2] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
@@ -273,7 +264,7 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
           tmem_wait_st();
         }
       }
-      // ---- pass 2: p = 2^(s*sl2 - m*sl2), row sum, bf16 P in the swizzled K-major layout
+      // ---- pass 2: p = 2^(s*sl2 - m*sl2), row sum, bf16 P into tensor memory behind O
       const float mneg = -m * sl2;
 #pragma unroll
       for (int c = 0; c < NCH; ++c) {
@@ -286,7 +277,7 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
         for (int i = 0; i < 32; i += 2) {
           const float2 xs = ffma2(make_float2(__uint_as_float(cur[i]), __uint_as_float(cur[i + 1])), sl2v, mnegv);
           float2 v;
-          if (i < POLY) {
+          if (i < kAttnPoly) {
             v = exp2_poly2(xs);
           } else {
             v.x = ex2_approx(xs.x);
@@ -299,25 +290,12 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
           pv[i] = v.x; pv[i + 1] = v.y;
           lsum[(i >> 1) & 1] = fadd2(lsum[(i >> 1) & 1], v);
         }
-        if (TP) {
-          uint32_t w[16];
+        uint32_t w[16];
 #pragma unroll
-          for (int i = 0; i < 16; ++i) w[i] = pack_bf16(pv[2 * i], pv[2 * i + 1]);
-          tmem_st16(o_tmem + HD + 16 * c, w);
-          continue;
-        }
-        const uint32_t blk = p_row + ((32 * c) >> 6) * (128 * 128);
-#pragma unroll
-        for (int ch = 0; ch < 4; ++ch) {
-          const int chunk = (((32 * c) & 63) >> 3) + ch;
-          const uint32_t addr = blk + (static_cast<uint32_t>(chunk ^ (row & 7)) << 4);
-          const uint32_t w0 = pack_bf16(pv[8 * ch + 0], pv[8 * ch + 1]), w1 = pack_bf16(pv[8 * ch + 2], pv[8 * ch + 3]);
-          const uint32_t w2 = pack_bf16(pv[8 * ch + 4], pv[8 * ch + 5]), w3 = pack_bf16(pv[8 * ch + 6], pv[8 * ch + 7]);
-          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(w0), "r"(w1), "r"(w2), "r"(w3) : "memory");
-        }
+        for (int i = 0; i < 16; ++i) w[i] = pack_bf16(pv[2 * i], pv[2 * i + 1]);
+        tmem_st16(o_tmem + HD + 16 * c, w);
       }
-      if (TP) tmem_wait_st();
-      else fence_proxy_async_smem();
+      tmem_wait_st();
       tc_fence_before();
       mbar_arrive(p_full(q));
     };
@@ -364,10 +342,10 @@ attention_kernel(const __grid_constant__ AttnMaps maps, const __grid_constant__ 
   }
 }
 
-template <int HD, int BKV, int NQ, int POLY, bool TP>
-int launch_attention_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
+template <int HD, int BKV, int NQ>
+int launch_attention(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
                      int heads, int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
-  using Cfg = AttnCfg<HD, BKV, NQ, TP>;
+  using Cfg = AttnCfg<HD, BKV, NQ>;
   AttnMaps maps;
   const int BH = B * heads;
   const uint32_t inner = HD >= 64 ? 64 : HD;
@@ -390,32 +368,16 @@ int launch_attention_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __n
   args.scale_log2 = attn_scale_log2(scale, HD);
   static bool attr_set = false;
   if (!attr_set) {
-    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<HD, BKV, NQ, POLY, TP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel<HD, BKV, NQ>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        Cfg::kSmem));
     attr_set = true;
   }
   dim3 grid((ntok + 128 * NQ - 1) / (128 * NQ), BH);
   ProfScope prof(kProfAttention, st, 4.0 * BH * static_cast<double>(ntok) * ntok * HD);
   prof.note(BH, ntok, HD);
-  launch_k<1>(attention_kernel<HD, BKV, NQ, POLY, TP>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, args);
+  launch_k<1>(attention_kernel<HD, BKV, NQ>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, args);
   WC_LAUNCH_CHECK();
   return 0;
-}
-
-template <int HD, int BKV, int NQ, bool TP = false>
-int launch_attention(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
-                     int heads, int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("WC_ATTN_POLY");
-    poly = e ? atoi(e) : 14;
-  }
-  switch (poly) {   // tuning knob; 14 is the shipped setting
-    case 0: return launch_attention_p<HD, BKV, NQ, 0, TP>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 8: return launch_attention_p<HD, BKV, NQ, 8, TP>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 20: return launch_attention_p<HD, BKV, NQ, 20, TP>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    default: return launch_attention_p<HD, BKV, NQ, 14, TP>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-  }
 }
 
 }  // namespace
@@ -430,46 +392,13 @@ int attention_forward(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv
                       int heads, int ntok, int hd, int ldo, cudaStream_t st, float* lse, float scale) {
   WC_REQUIRE(ntok % 8 == 0, "token count must be a multiple of 8");
   WC_REQUIRE(ldo % 8 == 0, "output row stride must be a multiple of 8");
-  static int small = -1;   // WC_ATTN_SMALL=0: general kernel for head_dim 16 / 32 too (previous design)
-  if (small < 0) {
-    const char* e = getenv("WC_ATTN_SMALL");
-    small = e ? atoi(e) : 1;
-  }
-  if (small && (hd == 16 || hd == 32)) {
-    static int four = -1;   // WC_ATTN_SMALL4=0: three softmax groups with a double-buffered S (attention_small.cu, round 1)
-    if (four < 0) {
-      const char* e = getenv("WC_ATTN_SMALL4");
-      four = e ? atoi(e) : 1;
-    }
-    // Measured on B200 (batch 32, N 8192): head_dim 16 2.42 -> 2.24 ms with four groups; head_dim 32 2.35 (three groups, P' in
-    // tensor memory) vs 2.41 (four groups, P' through shared memory) -> head_dim 32 keeps the 3-group kernel.  Four groups per
-    // CTA cover 512 queries: shorter sequences keep the 3-group kernel too.
-    static int four32 = -1;   // WC_ATTN_SMALL4_HD32: head_dim 32 through the four-group kernel as well (row sums on the tensor core there too)
-    if (four32 < 0) {
-      const char* e = getenv("WC_ATTN_SMALL4_HD32");
-      four32 = e ? atoi(e) : 1;
-    }
-    if (four && (hd == 16 || (hd == 32 && four32)) && ntok >= 2048) return attention_small4_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
+  // Measured on B200 (batch 32, N 8192): head_dim 16 2.42 -> 2.24 ms with four softmax groups per CTA (attention_small4.cu) instead of
+  // three with a double-buffered S (attention_small.cu).  Four groups cover 512 queries: shorter sequences keep the 3-group kernel.
+  if (hd == 16 || hd == 32) {
+    if (ntok >= 2048) return attention_small4_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
     return attention_small_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
   }
-  static int tp = -1;   // WC_ATTN_TP=0: P through shared memory (previous design); default: P in tensor memory
-  if (tp < 0) {
-    const char* e = getenv("WC_ATTN_TP");
-    tp = e ? atoi(e) : 1;
-  }
-  if (tp) {
-    switch (hd) {
-      // head_dim <= 32 keeps P in shared memory: three query tiles per CTA (which no longer fit in TMEM with P there)
-      // matter more than the saved stores (measured: 3.15 vs 2.84 T exp/s at head_dim 16)
-      case 64: return launch_attention<64, 128, 2, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      case 128: return launch_attention<128, 64, 2, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      case 192: return launch_attention<192, 64, 1, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      default: break;
-    }
-  }
   switch (hd) {
-    case 16: return launch_attention<16, 128, 3>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 32: return launch_attention<32, 128, 3>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
     case 64: return launch_attention<64, 128, 2>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
     case 128: return launch_attention<128, 64, 2>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
     case 192: return launch_attention<192, 64, 1>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);

@@ -13,7 +13,6 @@
 // D_i = rowsum(dO_i o O_i) is precomputed (attn_rowdot).  Accumulators (S, dP, dV/dK or dQ) live in TMEM.
 // Outputs are written as bf16 into one [B, N, 3C] buffer (dQ | dK | dV per token), which is exactly the dY operand
 // of the in-projection's data / weight gradients.
-#include <cstdlib>
 
 #include "wc_host.h"
 #include "wc_ptx.cuh"
@@ -39,9 +38,9 @@ constexpr int kPoly = 12;             // of every 32 exponentials, this many run
 // NSW = number of softmax warpgroups.  NSW == 2: one CTA per SM, two warps per TMEM lane quadrant interleave the
 // 32-column chunks.  NSW == 1 (head_dim <= 64, BT = 64): the CTA needs <= 256 TMEM columns and <= 113 KB of shared
 // memory, so TWO CTAs share an SM and one CTA's exp / dS phase overlaps the other's MMA phase.
-// TA: the P'/dS' operands of the accumulating MMAs live in TENSOR MEMORY (written by the softmax threads with
-// tcgen05.st, read by tcgen05.mma as its A operand) instead of shared memory.
-template <int HD, int BT, int STAGES, bool KV, int NSW, bool TA = false>
+// The dQ pass (!KV) keeps its dS' operand in TENSOR MEMORY (written by the softmax threads with tcgen05.st, read by tcgen05.mma as
+// its A operand); the KV pass keeps P' and dS' in shared memory.
+template <int HD, int BT, int STAGES, bool KV, int NSW>
 struct BwdCfg {
   static constexpr int kKBlocks = HD >= 64 ? HD / 64 : 1;
   static constexpr int kRowBytes = HD >= 64 ? 128 : HD * 2;
@@ -58,13 +57,13 @@ struct BwdCfg {
   static constexpr uint32_t kSmemLimit = NSW == 1 ? 115712 : 232448;
   static constexpr int kColsBase = 2 * BT + (KV ? 2 : 1) * HD;
   static constexpr int kTmemBudget = 512 / kCtasPerSm;
-  static constexpr int kPB = TA ? ((kColsBase + 2 * kNP * (BT / 2) <= kTmemBudget) ? 2 : 1)
-                                : ((kFixed + 2 * kNP * kPTile <= kSmemLimit) ? 2 : 1);
-  static constexpr uint32_t kSmem = kFixed + (TA ? 0 : kPB * kNP * kPTile);
-  static constexpr int kPCol = kColsBase;   // TA: buffer b at kPCol + b*kNP*(BT/2): dS' first, then (KV) P' 
+  static constexpr int kPB = !KV ? ((kColsBase + 2 * kNP * (BT / 2) <= kTmemBudget) ? 2 : 1)
+                                 : ((kFixed + 2 * kNP * kPTile <= kSmemLimit) ? 2 : 1);
+  static constexpr uint32_t kSmem = kFixed + (KV ? kPB * kNP * kPTile : 0);
+  static constexpr int kPCol = kColsBase;   // dQ pass: dS' buffer b at kPCol + b*(BT/2)
   static constexpr int kSoftmaxThreads = 128 * NSW;
   static constexpr int kThreads = 128 + kSoftmaxThreads;  // warp 0 TMA, warp 1 MMA, warp 2 TMEM alloc, warps 4.. softmax / epilogue
-  static constexpr int kCols = kColsBase + (TA ? kPB * kNP * (BT / 2) : 0);
+  static constexpr int kCols = kColsBase + (KV ? 0 : kPB * kNP * (BT / 2));
   static constexpr uint32_t kTmemCols = kCols <= 128 ? 128 : (kCols <= 256 ? 256 : 512);
   static constexpr int kAcc0 = 2 * BT;                  // KV: dV ; Q: dQ
   static constexpr int kAcc1 = 2 * BT + (KV ? HD : 0);  // KV: dK
@@ -72,10 +71,10 @@ struct BwdCfg {
   static_assert(kSmem <= kSmemLimit, "shared memory budget");
 };
 
-template <int HD, int BT, int STAGES, bool KV, int NSW, bool TA>
+template <int HD, int BT, int STAGES, bool KV, int NSW>
 __global__ void __launch_bounds__(128 + 128 * NSW, NSW == 1 ? 2 : 1)
 attention_bwd_kernel(const __grid_constant__ AttnBwdMaps maps, const __grid_constant__ AttnBwdArgs p) {
-  using Cfg = BwdCfg<HD, BT, STAGES, KV, NSW, TA>;
+  using Cfg = BwdCfg<HD, BT, STAGES, KV, NSW>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_u32 = smem_u32(smem_raw);
   const uint32_t base = (raw_u32 + 1023u) & ~1023u;
@@ -83,7 +82,7 @@ attention_bwd_kernel(const __grid_constant__ AttnBwdMaps maps, const __grid_cons
   const uint32_t r2_smem = r1_smem + Cfg::kRTile;
   const uint32_t t_smem = r2_smem + Cfg::kRTile;                  // stage s: T1 at t_smem + s*2*kTTile, T2 right after
   const uint32_t p_smem = t_smem + STAGES * 2 * Cfg::kTTile;      // dS' first, then (KV) P'
-  const uint32_t vec_smem = p_smem + (TA ? 0u : Cfg::kPB * Cfg::kNP * Cfg::kPTile);
+  const uint32_t vec_smem = p_smem + (KV ? Cfg::kPB * Cfg::kNP * Cfg::kPTile : 0u);
   const uint32_t bars = vec_smem + Cfg::kVecBytes;
   const uint32_t r_full = bars;
   auto t_full = [&](int s) { return bars + 8u * (1 + s); };
@@ -186,15 +185,12 @@ attention_bwd_kernel(const __grid_constant__ AttnBwdMaps maps, const __grid_cons
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             const int kk = cb * 4 + k;
-            if (TA) {
+            if (!KV) {
               const uint32_t pa = tmem_base + Cfg::kPCol + (i % Cfg::kPB) * (Cfg::kNP * (BT / 2)) + 8u * kk;
-              if (KV)
-                umma_bf16_ts(tmem_base + Cfg::kAcc0, pa + BT / 2, umma_desc_join(t2_mn + kk * kstep16, hi_k), idesc_acc, (i | kk) != 0 ? 1u : 0u);
               umma_bf16_ts(tmem_base + Cfg::kAcc1, pa, umma_desc_join(t1_mn + kk * kstep16, hi_k), idesc_acc, (i | kk) != 0 ? 1u : 0u);
             } else {
-              if (KV)
-                umma_bf16(tmem_base + Cfg::kAcc0, umma_desc_join(p_lo + (Cfg::kPTile >> 4) + cb * ((128 * 128) >> 4) + 2u * k, hi_p),
-                          umma_desc_join(t2_mn + kk * kstep16, hi_k), idesc_acc, (i | kk) != 0 ? 1u : 0u);
+              umma_bf16(tmem_base + Cfg::kAcc0, umma_desc_join(p_lo + (Cfg::kPTile >> 4) + cb * ((128 * 128) >> 4) + 2u * k, hi_p),
+                        umma_desc_join(t2_mn + kk * kstep16, hi_k), idesc_acc, (i | kk) != 0 ? 1u : 0u);
               umma_bf16(tmem_base + Cfg::kAcc1, umma_desc_join(p_lo + cb * ((128 * 128) >> 4) + 2u * k, hi_p),
                         umma_desc_join(t1_mn + kk * kstep16, hi_k), idesc_acc, (i | kk) != 0 ? 1u : 0u);
             }
@@ -298,10 +294,8 @@ attention_bwd_kernel(const __grid_constant__ AttnBwdMaps maps, const __grid_cons
           mbar_wait(acc_done(i % Cfg::kPB), ((i / Cfg::kPB) - 1) & 1u);
           p_free = true;
         }
-        if (TA) {
-          const uint32_t pt = s_tmem + Cfg::kPCol + (i % Cfg::kPB) * (Cfg::kNP * (BT / 2)) + 16 * c;
-          tmem_st16(pt, wd);
-          if (KV) tmem_st16(pt + BT / 2, wp);
+        if (!KV) {
+          tmem_st16(s_tmem + Cfg::kPCol + (i % Cfg::kPB) * (Cfg::kNP * (BT / 2)) + 16 * c, wd);
           continue;
         }
         const uint32_t blk_off = ((32 * c) >> 6) * (128 * 128);
@@ -311,13 +305,12 @@ attention_bwd_kernel(const __grid_constant__ AttnBwdMaps maps, const __grid_cons
           const uint32_t sw = static_cast<uint32_t>(chunk ^ (row & 7)) << 4;
           asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(ds_row + blk_off + sw), "r"(wd[4 * ch]), "r"(wd[4 * ch + 1]),
                        "r"(wd[4 * ch + 2]), "r"(wd[4 * ch + 3]) : "memory");
-          if (KV)
-            asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(pp_row + blk_off + sw), "r"(wp[4 * ch]), "r"(wp[4 * ch + 1]),
-                         "r"(wp[4 * ch + 2]), "r"(wp[4 * ch + 3]) : "memory");
+          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(pp_row + blk_off + sw), "r"(wp[4 * ch]), "r"(wp[4 * ch + 1]),
+                       "r"(wp[4 * ch + 2]), "r"(wp[4 * ch + 3]) : "memory");
         }
       }
-      if (TA) tmem_wait_st();
-      else fence_proxy_async_smem();
+      if (KV) fence_proxy_async_smem();
+      else tmem_wait_st();
       tc_fence_before();
       mbar_arrive(p_full);
     }
@@ -378,10 +371,10 @@ int make_head_map(CUtensorMap* m, const __nv_bfloat16* ptr, int hd, int ntok, in
   return encode_tmap_bf16(m, ptr, 4, dims, strides, box, hd >= 64 ? 128 : hd * 2);
 }
 
-template <int HD, int BT, int STAGES, bool KV, int NSW, bool TA = false>
+template <int HD, int BT, int STAGES, bool KV, int NSW>
 int launch_bwd(const BwdTensors& t, const float* lse, const float* D, __nv_bfloat16* dqkv, int ld3, int B, int heads, int ntok,
                cudaStream_t st) {
-  using Cfg = BwdCfg<HD, BT, STAGES, KV, NSW, TA>;
+  using Cfg = BwdCfg<HD, BT, STAGES, KV, NSW>;
   AttnBwdMaps maps;
   const uint64_t sh = static_cast<uint64_t>(ntok) * HD, sb = sh * heads;
   const uint64_t dsb = static_cast<uint64_t>(ntok) * t.ldd;
@@ -403,41 +396,22 @@ int launch_bwd(const BwdTensors& t, const float* lse, const float* D, __nv_bfloa
   a.lse = lse; a.D = D; a.dqkv = dqkv;
   static bool attr_set = false;
   if (!attr_set) {
-    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_bwd_kernel<HD, BT, STAGES, KV, NSW, TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
+    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_bwd_kernel<HD, BT, STAGES, KV, NSW>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
     attr_set = true;
   }
   dim3 grid((ntok + 127) / 128, B * heads);
   const double flops = (KV ? 8.0 : 6.0) * B * heads * static_cast<double>(ntok) * ntok * HD;
   ProfScope prof(kProfAttention, st, flops);
-  launch_k<1>(attention_bwd_kernel<HD, BT, STAGES, KV, NSW, TA>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, a);
+  launch_k<1>(attention_bwd_kernel<HD, BT, STAGES, KV, NSW>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, a);
   WC_LAUNCH_CHECK();
   return 0;
-}
-
-bool tmem_a() {  // dQ pass: dS operand in tensor memory (default on; WC_ATTN_BWD_TA=0 selects the shared-memory variant)
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("WC_ATTN_BWD_TA");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 
 template <int HD, int BT, int SKV, int SQ, int NSW>
 int launch_both(const BwdTensors& t, const float* lse, const float* D, __nv_bfloat16* dqkv, int ld3, int B, int heads, int ntok,
                 cudaStream_t st) {
   if (int e = launch_bwd<HD, BT, SKV, true, NSW>(t, lse, D, dqkv, ld3, B, heads, ntok, st)) return e;
-  if (tmem_a()) return launch_bwd<HD, BT, SQ, false, NSW, true>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
   return launch_bwd<HD, BT, SQ, false, NSW>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
-}
-
-bool two_cta() {  // WC_ATTN_BWD_2CTA=0 selects the one-CTA-per-SM variant for head_dim <= 64 (tuning knob)
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("WC_ATTN_BWD_2CTA");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
 }
 
 }  // namespace
@@ -450,12 +424,10 @@ int attention_backward(const __nv_bfloat16* q, const __nv_bfloat16* k, const __n
   WC_REQUIRE(ntok % 8 == 0 && ldd % 8 == 0 && ld3 % 8 == 0, "attention backward: strides / token count must be multiples of 8");
   BwdTensors t{q, k, v, d_o, ldd};
   switch (hd) {
-    case 16: return two_cta() ? launch_both<16, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st)
-                              : launch_both<16, 128, 2, 2, 2>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
-    case 32: return two_cta() ? launch_both<32, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st)
-                              : launch_both<32, 128, 2, 2, 2>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
-    case 64: return two_cta() ? launch_both<64, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st)
-                              : launch_both<64, 128, 2, 2, 2>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
+    // head_dim <= 64: two CTAs per SM (NSW == 1, BT = 64)
+    case 16: return launch_both<16, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
+    case 32: return launch_both<32, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
+    case 64: return launch_both<64, 64, 2, 2, 1>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
     case 128: return launch_both<128, 128, 1, 1, 2>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
     case 192: return launch_both<192, 64, 1, 2, 2>(t, lse, D, dqkv, ld3, B, heads, ntok, st);
     default: return fail("attention backward: unsupported head_dim " + std::to_string(hd));

@@ -29,7 +29,6 @@
 #include "wc_host.h"
 #include "wc_ptx.cuh"
 
-#include <cstdlib>
 #include <type_traits>
 
 namespace wc {
@@ -695,34 +694,12 @@ int launch_small_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bf
 template <int HD>
 int launch_small(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B, int heads,
                  int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("WC_ATTN_SMALL_POLY");
-    poly = e ? atoi(e) : (HD == 16 ? 12 : 8);   // measured best on B200 (N 8192, batch 32): 2.46 ms (hd 16), 2.55 ms (hd 32)
-  }
-  // P in tensor memory (aliased on the consumed S buffer) instead of shared memory.  Measured on B200 (batch 32, N 8192):
+  // POLY (how many of every 32 exponentials run on the FMA pipe), measured best on B200 (N 8192, batch 32): 12 for head_dim 16
+  // (2.46 ms), 8 for head_dim 32 (2.55 ms).
+  // TP: P in tensor memory (aliased on the consumed S buffer) instead of shared memory.  Measured on B200 (batch 32, N 8192):
   // head_dim 32: 2.52 -> 2.40 ms; head_dim 16: 2.43 -> 2.48 ms (the whole S tile held in registers spills at 128 registers,
-  // which costs more than the saved stores when there are no row-sum FADDs to begin with) -> default on for head_dim 32 only.
-  static int tp = -1;
-  if (tp < 0) {
-    const char* e = getenv("WC_ATTN_SMALL_TP");
-    tp = e ? atoi(e) : (HD == 32 ? 1 : 0);
-  }
-  if (tp) {
-    switch (poly) {
-      case 0: return launch_small_p<HD, 0, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      case 12: return launch_small_p<HD, 12, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      case 16: return launch_small_p<HD, 16, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      default: return launch_small_p<HD, 8, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    }
-  }
-  switch (poly) {   // tuning knob: how many of every 32 exponentials run on the FMA pipe
-    case 0: return launch_small_p<HD, 0, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 4: return launch_small_p<HD, 4, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 12: return launch_small_p<HD, 12, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 16: return launch_small_p<HD, 16, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    default: return launch_small_p<HD, 8, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-  }
+  // which costs more than the saved stores when there are no row-sum FADDs to begin with) -> head_dim 32 only.
+  return launch_small_p<HD, HD == 16 ? 12 : 8, HD == 32>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
 }
 
 }  // namespace

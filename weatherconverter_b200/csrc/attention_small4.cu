@@ -19,7 +19,6 @@
 #include "wc_host.h"
 #include "wc_ptx.cuh"
 
-#include <cstdlib>
 #include <type_traits>
 
 namespace wc {
@@ -109,7 +108,11 @@ __device__ __forceinline__ float2 exp2_poly2_scaled(float2 x, float2 c, float lo
   return o;
 }
 
-template <int HD, int POLY, bool UNIT>   // UNIT: the softmax scale is exactly 1 in the log2 domain (Q prescaled by the QKV projection)
+// Of every 32 exponentials, this many run on the FMA pipe.  Measured on B200 (batch 32, N 8192, head_dim 16): 8: 2.245 ms, 12: 2.262,
+// 16: 2.427.
+constexpr int kSmall4Poly = 8;
+
+template <int HD, bool UNIT>   // UNIT: the softmax scale is exactly 1 in the log2 domain (Q prescaled by the QKV projection)
 __global__ void __launch_bounds__(Cfg4<HD>::kThreads, 1)
 attention_small4_kernel(const __grid_constant__ Small4Maps maps, const __grid_constant__ Small4Args p) {
   using Cfg = Cfg4<HD>;
@@ -345,7 +348,7 @@ attention_small4_kernel(const __grid_constant__ Small4Maps maps, const __grid_co
           for (int i = 0; i < 32; i += 2) {
             const float2 xs = make_float2(__uint_as_float(cur[i]), __uint_as_float(cur[i + 1]));
             float2 v;
-            if (i < POLY) {
+            if (i < kSmall4Poly) {
               v = exp2_poly2_scaled(xs, cv, lo);
             } else {
               const float2 y = UNIT ? xs : fmul2(xs, cv);
@@ -483,7 +486,7 @@ attention_small4_kernel(const __grid_constant__ Small4Maps maps, const __grid_co
   }
 }
 
-template <int HD, int POLY, bool UNIT>
+template <int HD, bool UNIT>
 int launch_small4_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B, int heads,
                     int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
   using Cfg = Cfg4<HD>;
@@ -514,14 +517,14 @@ int launch_small4_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_b
   }
   static bool attr_set = false;
   if (!attr_set) {
-    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_small4_kernel<HD, POLY, UNIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
+    WC_CHECK_CUDA(cudaFuncSetAttribute(attention_small4_kernel<HD, UNIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
     attr_set = true;
   }
   const int nqb = (ntok + 128 * kNQ - 1) / (128 * kNQ);
   dim3 grid(HD == 16 ? BH : nqb, HD == 16 ? nqb : BH);
   ProfScope prof(kProfAttention, st, 4.0 * BH * static_cast<double>(ntok) * ntok * HD);
   prof.note(BH, ntok, HD);
-  launch_k<1>(attention_small4_kernel<HD, POLY, UNIT>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, args);
+  launch_k<1>(attention_small4_kernel<HD, UNIT>, grid, Cfg::kThreads, Cfg::kSmem, st, maps, args);
   WC_LAUNCH_CHECK();
   return 0;
 }
@@ -529,26 +532,9 @@ int launch_small4_p(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_b
 template <int HD>
 int launch_small4(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B, int heads,
                   int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
-  static int poly = -1;
-  if (poly < 0) {
-    const char* e = getenv("WC_ATTN_SMALL4_POLY");
-    poly = e ? atoi(e) : 8;   // measured best on B200 (batch 32, N 8192): 8: 2.245 ms, 12: 2.262, 16: 2.427 (head_dim 16)
-  }
-  const bool unit = attn_scale_log2(scale, HD) == 1.f;
-  {
-    if (unit) {
-      switch (poly) {
-        case 8: return launch_small4_p<HD, 8, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-        case 16: return launch_small4_p<HD, 16, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-        default: return launch_small4_p<HD, 12, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-      }
-    }
-  }
-  switch (poly) {   // how many of every 32 exponentials run on the FMA pipe
-    case 8: return launch_small4_p<HD, 8, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    case 16: return launch_small4_p<HD, 16, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-    default: return launch_small4_p<HD, 12, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
-  }
+  // inference runs Q prescaled by the QKV projection (unit scale), the training plan unscaled Q
+  if (attn_scale_log2(scale, HD) == 1.f) return launch_small4_p<HD, true>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
+  return launch_small4_p<HD, false>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
 }
 
 }  // namespace

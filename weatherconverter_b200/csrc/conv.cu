@@ -1,12 +1,11 @@
 #include "conv.cuh"
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace wc {
 
 int pack_tap(__nv_bfloat16* dst, int ldk, int koff, const float* src, int Nn, int Cc, int Cpad, int KH, int KW, int ky,
-             int kx, int transpose, const float* scale, int row_mul, int row_off, cudaStream_t st);
+             int kx, int transpose, const float* scale, cudaStream_t st);
 int pack_taps(__nv_bfloat16* dst, int ldk, int ntaps, const float* const* src, const float* const* scale, const int* params,
               cudaStream_t st);
 
@@ -32,77 +31,29 @@ void set_pack_recorder(std::vector<std::function<int(cudaStream_t)>>* recorder) 
 
 namespace {
 
-int row3_mode() {  // 1: descriptors rely on address-based swizzling; 2 (WC_ROW3=2): explicit base_offset
-  const char* e = getenv("WC_ROW3");
-  return (e && e[0] == '2') ? 2 : 1;
-}
-
-bool row3_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("WC_ROW3");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-
-bool lean_enabled() {   // WC_IGEMM_LEAN=0: previous epilogue everywhere
-  static int lean = -1;
-  if (lean < 0) {
-    const char* e = getenv("WC_IGEMM_LEAN");
-    lean = e ? atoi(e) : 1;
-  }
-  return lean != 0;
-}
-
-bool lean_mask_enabled() {   // WC_IGEMM_LEAN_MASK=1: layers with a ReLU-mask input (segmentor data gradients) use the lean epilogue
-  static int v = -1;          // too.  Default off: measured neutral (C3 igemm 10.96 vs 10.99 ms) - those layers are bound by the mask rows
-  if (v < 0) {
-    const char* e = getenv("WC_IGEMM_LEAN_MASK");
-    v = e ? atoi(e) : 0;
-  }
-  return v != 0;
-}
-
 // Residual stream epilogue (igemm.cu, LEAN == 3) for layers with a residual input and a short main loop: K <= 768, plain mode, no
-// ReLU mask, no PReLU / GELU, full N tiles that are multiples of 64.  WC_IGEMM_RES_DEEP = load buffers per warp (2..4, default 3; 0: off).
+// ReLU mask, no PReLU / GELU, full N tiles that are multiples of 64.  Layers with a ReLU-mask input (segmentor data gradients) stream
+// the mask rows the same way.
+constexpr int kStreamLoadSlots = 3;   // load buffers per epilogue warp (fewer when the ring would get too short)
+constexpr int kStreamMaxKb = 12;      // longest main loop (in 64-channel blocks) that still takes the stream epilogue (12 / 16 / 40 /
+                                      // unlimited measured equal on C3: 21.30 - 21.32 ms)
+constexpr int kStreamMinStages = 2;   // these layers are epilogue-bound: a short ring suffices
 void apply_res_deep(IgemmPlan* plan, int N, bool res_candidate) {
-  static int deep = -1;
-  if (deep < 0) {
-    const char* e = getenv("WC_IGEMM_RES_DEEP");
-    deep = e ? atoi(e) : 3;
-    if (deep > 4) deep = 4;
-  }
-  static int deep_mask = -1;   // WC_IGEMM_STREAM_MASK=0: layers with a ReLU-mask input keep the generic epilogue
-  if (deep_mask < 0) {
-    const char* e = getenv("WC_IGEMM_STREAM_MASK");
-    deep_mask = e ? atoi(e) : 1;
-  }
   IgemmArgs& a = plan->args;
   a.res_deep = 0;
   const bool mask_candidate = a.stream_mask == 2;
   a.stream_mask = 0;
   a.stream_res = 0;
-  static int max_kb = -1;   // WC_IGEMM_STREAM_MAX_KB: longest main loop (in 64-channel blocks) that still takes the stream epilogue
-  if (max_kb < 0) {
-    const char* e = getenv("WC_IGEMM_STREAM_MAX_KB");
-    max_kb = e ? atoi(e) : 12;
-  }
-  if (deep < 2 || !lean_enabled() || !a.tma_store || a.row3 || a.wres || a.prelu || a.act == 3 || a.phase_n ||
-      a.total_kb > max_kb || a.BN % 64 != 0 || N % a.BN != 0 || a.out_mode != kOutNHWC)
+  if (!a.tma_store || a.row3 || a.prelu || a.act == 3 || a.phase_n || a.total_kb > kStreamMaxKb || a.BN % 64 != 0 ||
+      N % a.BN != 0 || a.out_mode != kOutNHWC)
     return;
   if (a.res && !res_candidate) return;             // a residual that cannot go through TMA
-  if (a.mask && !(mask_candidate && deep_mask)) return;
+  if (a.mask && !mask_candidate) return;
   const int nbox = (a.res ? 1 : 0) + (a.mask ? 1 : 0);
   if (nbox == 0) return;
-  for (int nl = deep; nl >= 2; --nl) {
+  for (int nl = kStreamLoadSlots; nl >= 2; --nl) {
     const int ns = igemm_res_deep_stages(a.BN, nl * nbox);
-    static int min_stages = -1;   // WC_IGEMM_STREAM_MIN_STAGES (default 2): these layers are epilogue-bound, a short ring suffices
-    if (min_stages < 0) {
-      const char* e = getenv("WC_IGEMM_STREAM_MIN_STAGES");
-      min_stages = e ? atoi(e) : 2;
-    }
-    if (ns >= 2 && ns >= (a.total_kb < min_stages ? a.total_kb + 1 : min_stages)) {
+    if (ns >= 2 && ns >= (a.total_kb < kStreamMinStages ? a.total_kb + 1 : kStreamMinStages)) {
       a.res_deep = nl;
       a.stream_res = a.res ? 1 : 0;
       a.stream_mask = a.mask ? 1 : 0;
@@ -122,7 +73,7 @@ struct TapDef {
   int C;  // true input channels of this tap
 };
 
-int out_channels_of(const WeightSrc& w) { return w.n_out > 0 ? w.n_out : (w.transpose ? w.d1 : w.d0); }
+int out_channels_of(const WeightSrc& w) { return w.transpose ? w.d1 : w.d0; }
 int in_channels_of(const WeightSrc& w) { return w.transpose ? w.d0 : w.d1; }
 
 // Pack weights for a tap list and fill everything of the plan except the A tensor maps.
@@ -168,10 +119,10 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
     WC_REQUIRE(n_src <= N, "weight has more output channels than N");
     const int cpad = (t.C + kIgemmBK - 1) / kIgemmBK * kIgemmBK;
     const int ky = w.flip ? w.KH - 1 - t.ky : t.ky, kx = w.flip ? w.KW - 1 - t.kx : t.kx;
-    if (int e = pack_tap(wp, ktotal, koff, w.w, n_src, t.C, cpad, w.KH, w.KW, ky, kx, w.transpose, w.scale, w.row_mul, w.row_off, st)) return e;
+    if (int e = pack_tap(wp, ktotal, koff, w.w, n_src, t.C, cpad, w.KH, w.KW, ky, kx, w.transpose, w.scale, st)) return e;
     rec_src->push_back(w.w);
     rec_scale->push_back(w.scale);
-    for (int v : {koff, n_src, t.C, cpad, w.KH, w.KW, ky, kx, w.transpose, w.row_mul, w.row_off}) rec_par->push_back(v);
+    for (int v : {koff, n_src, t.C, cpad, w.KH, w.KW, ky, kx, w.transpose}) rec_par->push_back(v);
     koff += cpad;
     macs_per_pixel += static_cast<double>(t.C) * n_src;
   }
@@ -209,7 +160,7 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
   if (out.mode == kOutNHWC && out.phases == 4) {
     // four phase blocks of N/4 channels, one strided output map per phase; lean epilogue only (igemm.cu)
     const int pn = N / 4;
-    WC_REQUIRE(sy == 2 && sx == 2 && N % 128 == 0 && a.BN % 32 == 0 && lean_enabled(), "phase-block output needs up == 2, N % 128 == 0 and the lean epilogue");
+    WC_REQUIRE(sy == 2 && sx == 2 && N % 128 == 0 && a.BN % 32 == 0, "phase-block output needs up == 2 and N % 128 == 0");
     WC_REQUIRE(out.out.ptr && out.out.B == B && out.out.H == a.Ho && out.out.W == a.Wo && out.out.ld % 8 == 0 && !ep.res && !ep.mask, "phase-block output grid mismatch");
     a.out = out.out.ptr; a.ldc = out.out.ld;
     a.qw = tw < 32 ? tw : 32;
@@ -227,18 +178,9 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
     WC_REQUIRE(out.out.ptr && out.out.B == B && out.out.H == a.Ho && out.out.W == a.Wo, "output grid mismatch");
     WC_REQUIRE(out.out.ld % 8 == 0, "output pixel stride must be a multiple of 8");
     a.out = out.out.ptr; a.ldc = out.out.ld;
-    static int tma_store = -1;   // WC_IGEMM_TMA_STORE=0: row-per-lane global stores (previous epilogue)
-    if (tma_store < 0) {
-      const char* e = getenv("WC_IGEMM_TMA_STORE");
-      tma_store = e ? atoi(e) : 1;
-    }
-    static int tma_strided = -1;   // WC_IGEMM_TMA_STRIDED=0: up-sampling phases (sy = sx = 2) keep the row-per-lane stores
-    if (tma_strided < 0) {
-      const char* e = getenv("WC_IGEMM_TMA_STRIDED");
-      tma_strided = e ? atoi(e) : 1;
-    }
+    // TMA-store epilogue where the box fits the tile; otherwise row-per-lane global stores (epilogue_tile)
     const bool unit = (sy == 1 && sx == 1);
-    if (tma_store && (unit || (tma_strided && out.out.H == H * sy && out.out.W == W * sx && (out.out.ld * sx * 2) % 16 == 0))) {
+    if (unit || (out.out.H == H * sy && out.out.W == W * sx && (out.out.ld * sx * 2) % 16 == 0)) {
       const int nc = (a.BN % 32 == 0 && N % 32 == 0) ? 32 : 16;   // the epilogue's chunk width (see igemm_kernel)
       a.qw = tw < 32 ? tw : 32;
       a.qh = th < 32 / a.qw ? th : 32 / a.qw;
@@ -246,12 +188,7 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
       if (a.qb <= tb) {
         if (int e = igemm_make_cmap(&plan->maps.c, out.out, N, nc, a.qw, a.qh, a.qb, sy, sx, py, px)) return e;
         a.tma_store = 1;
-        static int tma_res = -1;   // WC_IGEMM_TMA_RES=0: residual rows through per-lane global loads
-        if (tma_res < 0) {
-          const char* e2 = getenv("WC_IGEMM_TMA_RES");
-          tma_res = e2 ? atoi(e2) : 1;
-        }
-        if (tma_res && ep.res && ep.res->ld % 8 == 0) {
+        if (ep.res && ep.res->ld % 8 == 0) {
           if (int e = igemm_make_cmap(&plan->maps.r, *ep.res, N, nc, a.qw, a.qh, a.qb, sy, sx, py, px)) return e;
           a.tma_res = 2;   // candidate: confirmed by the caller once the ring depth is known
         }
@@ -264,13 +201,8 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
   } else if (out.mode == kOutNCHWf32) {
     a.out_f32 = out.out_f32; a.n_store = out.n_store;
     // lean epilogue with bulk-tensor stores of [16 planes][32 pixels] fp32 boxes (igemm.cu) when a TMEM lane quadrant is 32 consecutive
-    // pixels of one image row; the map addresses the fp32 planes as bf16 pairs.  WC_IGEMM_F32_TMA=0: per-lane stores.
-    static int f32_tma = -1;
-    if (f32_tma < 0) {
-      const char* e = getenv("WC_IGEMM_F32_TMA");
-      f32_tma = e ? atoi(e) : 1;
-    }
-    if (f32_tma && lean_enabled() && sy == 1 && sx == 1 && tw >= 32 && W % 32 == 0 && (W * 2) % 8 == 0 && !ep.res && !ep.mask) {
+    // pixels of one image row; the map addresses the fp32 planes as bf16 pairs.  Otherwise per-lane stores (epilogue_tile).
+    if (sy == 1 && sx == 1 && tw >= 32 && W % 32 == 0 && (W * 2) % 8 == 0 && !ep.res && !ep.mask) {
       uint64_t dims[4] = {static_cast<uint64_t>(2 * W), static_cast<uint64_t>(H), static_cast<uint64_t>(out.n_store), static_cast<uint64_t>(B)};
       uint64_t strides[4] = {1, static_cast<uint64_t>(2 * W), static_cast<uint64_t>(2 * W) * H, static_cast<uint64_t>(2 * W) * H * out.n_store};
       uint32_t box[4] = {64, 1, 16, 1};
@@ -284,16 +216,11 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
     WC_REQUIRE(N == 3 * a.C, "QKV epilogue needs N == 3*C");
     WC_REQUIRE((H * W) % 8 == 0, "token count must be a multiple of 8");
     // Lean epilogue with bulk-tensor stores (igemm.cu: the kOutQKV branch of epilogue_tile_lean) when a TMEM lane quadrant is 32
-    // consecutive tokens of one image and a 32-channel chunk stays inside q / k / v and inside whole heads.  WC_IGEMM_QKV_TMA=0: the
-    // per-lane scatter stores of round 1.
-    static int qkv_tma = -1;
-    if (qkv_tma < 0) {
-      const char* e = getenv("WC_IGEMM_QKV_TMA");
-      qkv_tma = e ? atoi(e) : 1;
-    }
+    // consecutive tokens of one image and a 32-channel chunk stays inside q / k / v and inside whole heads.  Otherwise (V stored as
+    // well for the training plan, tokens not contiguous) the per-lane scatter stores of epilogue_tile.
     const int qw = tw < 32 ? tw : 32, qh = th < 32 / qw ? th : 32 / qw, qb = 32 / (qw * qh);
     const bool tokens_contiguous = qb == 1 && ((qh == 1 && W % qw == 0) || qw == W);
-    if (qkv_tma && lean_enabled() && !out.v && tokens_contiguous && a.C % 32 == 0 && a.BN % 32 == 0 && (out.hd == 16 || out.hd % 32 == 0)) {
+    if (!out.v && tokens_contiguous && a.C % 32 == 0 && a.BN % 32 == 0 && (out.hd == 16 || out.hd % 32 == 0)) {
       const int hd = out.hd, heads = out.heads, ntok = H * W;
       const uint32_t inner = hd == 16 ? 16u : 32u;
       uint64_t dqk[4] = {static_cast<uint64_t>(hd), static_cast<uint64_t>(ntok), static_cast<uint64_t>(heads), static_cast<uint64_t>(B)};
@@ -346,7 +273,7 @@ int build_conv(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w,
     }
     for (int i = nmaps; i < kMaxMaps; ++i) plan.maps.a[i] = plan.maps.a[0];
     // Row-segment mode: 3x3 / dilation 1 on maps at least 128 pixels wide with narrow N (the L2->SM bound layers)
-    if (g.K == 3 && g.dil == 1 && tw == 128 && th == 1 && tb == 1 && (N <= 128 || (out.bn_max > 0 && out.bn_max <= 128)) && row3_enabled()) {
+    if (g.K == 3 && g.dil == 1 && tw == 128 && th == 1 && tb == 1 && (N <= 128 || (out.bn_max > 0 && out.bn_max <= 128))) {
       if (int e = igemm_make_rowseg_map(&plan.maps.a[2], x)) return e;
       want_row3 = true;
     }
@@ -367,34 +294,16 @@ int build_conv(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w,
       }
   }
   if (int e = finish_plan(&plan, arena, taps, B, H, W, tb, th, tw, N, ep, out, out.up, out.up, out.py, out.px, st)) return e;
-  plan.args.row3 = (want_row3 && plan.args.BN <= 128) ? row3_mode() : 0;
+  plan.args.row3 = (want_row3 && plan.args.BN <= 128) ? 1 : 0;
   plan.args.row_nky = plan.args.row_nkx = 3;
-  int wres_bytes = 0;
-  {
-    // resident weights: one N tile, the packed matrix fits next to a useful ring, and every CTA processes several tiles
-    // WC_IGEMM_WRES=1 enables it.  Default OFF: measured on B200 (batch 32, 64 x 128) it does not pay - 3x3 64->64 (row-segment
-    // mode) 34.7 -> 40.9 us, 1x1 256->64 37.2 -> 35.9 us, 1x1 64->256 unchanged - although it cuts the L2->SM traffic of the 3x3
-    // layer 2.4x: that traffic is not what bounds these layers (same finding as in round 1, before the TMA epilogue).
-    static int wres = -1;
-    if (wres < 0) {
-      const char* e = getenv("WC_IGEMM_WRES");
-      wres = e ? atoi(e) : 0;
-    }
-    const long wb = static_cast<long>(plan.args.BN) * plan.args.total_kb * kIgemmBK * 2;
-    const long m_tiles = (static_cast<long>(B) * H * W + kIgemmBM - 1) / kIgemmBM;
-    if (wres && plan.args.BN >= N && wb <= kIgemmWresMaxBytes && m_tiles >= 2 * num_sms()) {
-      plan.args.wres = 1;
-      wres_bytes = static_cast<int>(wb);
-    }
-  }
-  plan.args.nstages = igemm_stages_for(plan.args.BN, plan.args.row3, wres_bytes);
-  plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, plan.args.row3, plan.args.nstages, wres_bytes) ? 1 : 0;
+  // (resident weights do not pay here: measured on B200 (batch 32, 64 x 128) 3x3 64->64 in row-segment mode 34.7 -> 40.9 us, 1x1
+  // 256->64 37.2 -> 35.9 us, 1x1 64->256 unchanged, although they cut the L2->SM traffic of the 3x3 layer 2.4x)
+  plan.args.nstages = igemm_stages_for(plan.args.BN, plan.args.row3);
+  plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, plan.args.row3, plan.args.nstages) ? 1 : 0;
   const bool res_candidate = plan.args.tma_res == 2;
   plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-  plan.args.lean = (lean_enabled() && plan.args.tma_store && (!plan.args.mask || lean_mask_enabled()) && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
+  plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
   apply_res_deep(&plan, N, res_candidate);
-  { const char* e = getenv("WC_IGEMM_DBG"); plan.args.dbg = e ? atoi(e) : 0; }
-  { const char* e = getenv("WC_IGEMM_TRACE"); plan.args.trace = e ? reinterpret_cast<long long*>(strtoull(e, nullptr, 0)) : nullptr; }
   op->flops = plan.flops;
   return 0;
 }
@@ -432,7 +341,7 @@ int build_conv_stem7s2(ConvOp* op, DeviceArena* arena, const __nv_bfloat16* xp, 
   plan.args.nstages = igemm_stages_for(plan.args.BN, 0);
   plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, 0, plan.args.nstages) ? 1 : 0;
   plan.args.tma_res = 0;
-  plan.args.lean = (lean_enabled() && plan.args.tma_store && !plan.args.mask && !plan.args.res) ? 1 : 0;
+  plan.args.lean = (plan.args.tma_store && !plan.args.mask && !plan.args.res) ? 1 : 0;
   plan.flops = 2.0 * 147.0 * N * static_cast<double>(B) * Ho * Wo;   // algorithmic (the reference's 7x7x3 taps), not the padded K
   op->flops = plan.flops;
   return 0;
@@ -456,31 +365,21 @@ int build_conv_hrow(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSr
   std::vector<TapDef> taps;
   for (int kx = 0; kx < w.KW; ++kx) taps.push_back({0, 0, kx - w.KW / 2, &w, 0, kx, x.C});
   if (int e = finish_plan(&plan, arena, taps, x.B, x.H, x.W, tb, th, tw, N, ep, out, 1, 1, 0, 0, st)) return e;
-  // Row-segment mode with all KW taps in one stage (WC_HROW_SEG=0: one stage per tap): one box of 128 + KW - 1 pixels per tile instead
-  // of KW boxes of 128, one barrier hand-over per tile instead of KW
-  static int hseg = -1;
-  if (hseg < 0) {
-    const char* e = getenv("WC_HROW_SEG");
-    hseg = e ? atoi(e) : 1;
-  }
+  // Row-segment mode with all KW taps in one stage: one box of 128 + KW - 1 pixels per tile instead of KW boxes of 128, one barrier
+  // hand-over per tile instead of KW
   plan.args.row3 = 0;
   plan.args.row_nky = 1; plan.args.row_nkx = w.KW;
   // (the kernel is instantiated for 3 x 3 and 1 x 9 windows: other widths keep one stage per tap)
-  if (hseg && w.KW == 9 && row3_enabled() && tw == 128 && th == 1 && tb == 1 && plan.args.BN <= 128 && igemm_stages_for(plan.args.BN, 1, 0, w.KW) >= 2) {
+  if (w.KW == 9 && tw == 128 && th == 1 && tb == 1 && plan.args.BN <= 128 && igemm_stages_for(plan.args.BN, 1, 0, w.KW) >= 2) {
     if (int e = igemm_make_rowseg_map(&plan.maps.a[2], x, w.KW)) return e;
-    plan.args.row3 = row3_mode();
+    plan.args.row3 = 1;
   }
   // the packed weights of all taps (KW x BN x 64 bf16) are the same for every tile: keep them resident (one load per CTA) when this
   // is a single N tile - the ring then carries activations only
   int wres_bytes = 0;
   {
-    static int hres = -1;
-    if (hres < 0) {
-      const char* e = getenv("WC_HROW_WRES");
-      hres = e ? atoi(e) : 1;
-    }
     const long wb = static_cast<long>(plan.args.BN) * plan.args.total_kb * kIgemmBK * 2;
-    if (hres && plan.args.row3 && plan.args.BN >= N && wb <= kIgemmWresMaxBytes) {
+    if (plan.args.row3 && plan.args.BN >= N && wb <= kIgemmWresMaxBytes) {
       plan.args.wres = 1;
       wres_bytes = static_cast<int>(wb);
     }
@@ -488,7 +387,7 @@ int build_conv_hrow(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSr
   plan.args.nstages = igemm_stages_for(plan.args.BN, plan.args.row3, wres_bytes, w.KW);
   plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, plan.args.row3, plan.args.nstages, wres_bytes, w.KW) ? 1 : 0;
   plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-  plan.args.lean = (lean_enabled() && plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
+  plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
   op->flops = plan.flops;
   return 0;
 }
@@ -516,7 +415,7 @@ int build_conv_transposed_s2(ConvOp* op, DeviceArena* arena, const Act& x, const
       plan.args.nstages = igemm_stages_for(plan.args.BN, 0);
       plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, 0, plan.args.nstages) ? 1 : 0;
       plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-      plan.args.lean = (lean_enabled() && plan.args.tma_store && (!plan.args.mask || lean_mask_enabled()) && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
+      plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
       op->flops += plan.flops;
     }
   return 0;

@@ -32,8 +32,6 @@ struct WeightSrc {
   int transpose = 0;            // 0: out-channel = dim0 (Conv2d fwd); 1: out-channel = dim1 (ConvTranspose2d / dgrad)
   int flip = 0;                 // use tap (KH-1-ky, KW-1-kx): stride-1 data gradient
   const float* scale = nullptr;  // optional per-dim0 scale (folded BatchNorm)
-  int n_out = 0;                 // >0: number of output rows to take (row n reads source row n*row_mul + row_off)
-  int row_mul = 1, row_off = 0;  // PixelShuffle phases: conv output channel 4c+q feeds phase q
 };
 
 struct ConvGeom {

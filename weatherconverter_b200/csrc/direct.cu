@@ -259,7 +259,7 @@ __global__ void linear_rows_kernel(const float* __restrict__ in, int dim, const 
 // (ConvTranspose2d weight, or a dgrad view of a Conv2d weight).  scale (optional) is indexed by the src dim-0.
 __global__ void pack_tap_kernel(__nv_bfloat16* __restrict__ dst, int ldk, int koff, const float* __restrict__ src,
                                 int Nn, int Cc, int Cpad, int KH, int KW, int ky, int kx, int transpose,
-                                const float* __restrict__ scale, int row_mul, int row_off, int D0, int D1src) {
+                                const float* __restrict__ scale, int D0, int D1src) {
   pdl_prologue();
   const size_t total = static_cast<size_t>(Nn) * Cpad;
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < total;
@@ -267,7 +267,7 @@ __global__ void pack_tap_kernel(__nv_bfloat16* __restrict__ dst, int ldk, int ko
     const int c = static_cast<int>(i % Cpad), n = static_cast<int>(i / Cpad);
     float v = 0.f;
     if (c < Cc) {
-      const size_t d0 = transpose ? c : static_cast<size_t>(n) * row_mul + row_off, d1 = transpose ? n : c;
+      const size_t d0 = transpose ? c : n, d1 = transpose ? n : c;
       const size_t D1 = D1src;
       v = src[((d0 * D1 + d1) * KH + ky) * KW + kx];
       if (scale) v *= scale[d0];
@@ -280,7 +280,7 @@ __global__ void pack_tap_kernel(__nv_bfloat16* __restrict__ dst, int ldk, int ko
 struct PackTapDesc {
   const float* src;
   const float* scale;
-  int koff, Nn, Cc, Cpad, KH, KW, ky, kx, transpose, row_mul, row_off, D1;
+  int koff, Nn, Cc, Cpad, KH, KW, ky, kx, transpose, D1;
 };
 constexpr int kPackMaxTaps = 20;
 struct PackTapsArgs {
@@ -297,7 +297,7 @@ __global__ void pack_taps_kernel(const __grid_constant__ PackTapsArgs a) {
     const int c = static_cast<int>(i % t.Cpad), n = static_cast<int>(i / t.Cpad);
     float v = 0.f;
     if (c < t.Cc) {
-      const size_t d0 = t.transpose ? c : static_cast<size_t>(n) * t.row_mul + t.row_off, d1 = t.transpose ? n : c;
+      const size_t d0 = t.transpose ? c : n, d1 = t.transpose ? n : c;
       v = t.src[((d0 * t.D1 + d1) * t.KH + t.ky) * t.KW + t.kx];
       if (t.scale) v *= t.scale[d0];
     }
@@ -448,28 +448,28 @@ int linear_rows(const float* in, int Bt, int dim, const float* w, const float* b
 }
 
 int pack_tap(__nv_bfloat16* dst, int ldk, int koff, const float* src, int Nn, int Cc, int Cpad, int KH, int KW, int ky,
-             int kx, int transpose, const float* scale, int row_mul, int row_off, cudaStream_t st) {
+             int kx, int transpose, const float* scale, cudaStream_t st) {
   // source dim-1 extent: transposed sources are [Cc][Nn], plain sources [rows][Cc]
   launch_k(pack_tap_kernel, grid_for(static_cast<size_t>(Nn) * Cpad), 256, 0, st, dst, ldk, koff, src, Nn, Cc, Cpad, KH, KW,
-                                                                           ky, kx, transpose, scale, row_mul, row_off, 0,
+                                                                           ky, kx, transpose, scale, 0,
                                                                            transpose ? Nn : Cc);
   WC_LAUNCH_CHECK();
   return 0;
 }
 
-// One launch for up to 20 taps; taps[i] = {src, scale, koff, Nn, Cc, Cpad, KH, KW, ky, kx, transpose, row_mul, row_off}
-int pack_taps(__nv_bfloat16* dst, int ldk, int ntaps, const float* const* src, const float* const* scale, const int* params /*[ntaps][11]*/,
+// One launch for up to 20 taps; taps[i] = {src, scale, koff, Nn, Cc, Cpad, KH, KW, ky, kx, transpose}
+int pack_taps(__nv_bfloat16* dst, int ldk, int ntaps, const float* const* src, const float* const* scale, const int* params /*[ntaps][9]*/,
               cudaStream_t st) {
   WC_REQUIRE(ntaps >= 1 && ntaps <= kPackMaxTaps, "pack_taps: tap count out of range");
   PackTapsArgs a;
   a.dst = dst; a.ldk = ldk; a.ntaps = ntaps;
   size_t max_total = 0;
   for (int i = 0; i < ntaps; ++i) {
-    const int* p = params + i * 11;
+    const int* p = params + i * 9;
     PackTapDesc& t = a.t[i];
     t.src = src[i]; t.scale = scale[i];
     t.koff = p[0]; t.Nn = p[1]; t.Cc = p[2]; t.Cpad = p[3]; t.KH = p[4]; t.KW = p[5]; t.ky = p[6]; t.kx = p[7];
-    t.transpose = p[8]; t.row_mul = p[9]; t.row_off = p[10];
+    t.transpose = p[8];
     t.D1 = t.transpose ? t.Nn : t.Cc;
     max_total = std::max(max_total, static_cast<size_t>(t.Nn) * t.Cpad);
   }

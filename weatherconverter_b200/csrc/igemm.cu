@@ -72,7 +72,6 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
   if (grp * NC < p.BN) prefetch(n0 + grp * NC);   // issued BEFORE waiting for the accumulator: overlaps the main loop's tail
   mbar_wait(tfull_addr, tfull_parity);
   tc_fence_after();
-  if (p.dbg & 16) return;   // experiment: no TMEM reads / math / stores
   for (int c0 = grp * NC; c0 < p.BN; c0 += 2 * NC) {
     const int nb = n0 + c0;
     if (nb >= p.N) break;  // warp-uniform
@@ -164,7 +163,6 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
         if (!(f3.y > 0.f)) v[8 * j + 7] = 0.f;
       }
     }
-    if (p.dbg & 1) continue;
     if constexpr (tma_out) {
       // the previous chunk's store must have finished READING the staging buffer
       if (lane == 0) tma_store_wait_read0();
@@ -252,8 +250,8 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
 // chunk by chunk (ectr counts this warp's chunks across tiles): the TMA store of chunk i reads buffer i & 1 while chunk i + 1 is
 // staged in the other one.  With a residual the box of chunk i is loaded by TMA INTO the buffer chunk i will be stored from; each
 // lane reads its row, adds, and writes the bf16 result back in place.
-template <int NC, bool RES, bool MASK>
-__device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t tacc, int n0, int b, int y, int x, bool valid, int grp,
+template <int NC, bool RES>
+__device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t tacc, int n0, int b, int grp,
                                                    const float* s_bias,
                                                    const float* s_prelu, uint32_t tfull_addr, uint32_t tfull_parity,
                                                    const CUtensorMap* cmap, const CUtensorMap* rmap, uint32_t buf0, uint32_t buf1,
@@ -273,17 +271,6 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
   };
   const int c_first = grp * NC;
   if (RES && c_first < p.BN && n0 + c_first < p.N) request(ectr, n0 + c_first);   // before the accumulator is ready: overlaps the main loop
-  // ReLU-derivative mask rows (segmentor data gradients): per-lane global loads of this pixel's row, one chunk ahead
-  const uint4* mask_row = nullptr;
-  uint4 mk[NV];
-  if (MASK) {
-    const int oy = y * p.sy + p.py, ox = x * p.sx + p.px;
-    mask_row = reinterpret_cast<const uint4*>(p.mask + ((static_cast<size_t>(b) * p.Ho + oy) * p.Wo + ox) * p.ldm);
-    if (valid && c_first < p.BN && n0 + c_first < p.N) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) mk[j] = __ldg(mask_row + ((n0 + c_first) >> 3) + j);
-    }
-  }
   mbar_wait(tfull_addr, tfull_parity);
   tc_fence_after();
   const float* rb = p.rowbias ? p.rowbias + static_cast<size_t>(b < p.B ? b : p.B - 1) * p.ldrb : nullptr;
@@ -303,15 +290,6 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
                      : "r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
       // the next box goes into the OTHER buffer (last touched, through the generic proxy, one chunk ago and fenced then)
       if (c0 + 2 * NC < p.BN && nb + 2 * NC < p.N) request(ectr + 1, nb + 2 * NC);
-    }
-    uint4 mcur[NV];
-    if (MASK) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) mcur[j] = mk[j];
-      if (valid && c0 + 2 * NC < p.BN && nb + 2 * NC < p.N) {
-#pragma unroll
-        for (int j = 0; j < NV; ++j) mk[j] = __ldg(mask_row + ((nb + 2 * NC) >> 3) + j);
-      }
     }
     tmem_wait_ld();
     float v[NC];
@@ -365,21 +343,6 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
         v[j + 2] = v[j + 2] > 0.f ? v[j + 2] : v[j + 2] * sv.z; v[j + 3] = v[j + 3] > 0.f ? v[j + 3] : v[j + 3] * sv.w;
       }
     }
-    if (MASK) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) {
-        const uint4 u = mcur[j];
-        const float2 f0 = unpack_bf16(u.x), f1 = unpack_bf16(u.y), f2 = unpack_bf16(u.z), f3 = unpack_bf16(u.w);
-        if (!(f0.x > 0.f)) v[8 * j + 0] = 0.f;
-        if (!(f0.y > 0.f)) v[8 * j + 1] = 0.f;
-        if (!(f1.x > 0.f)) v[8 * j + 2] = 0.f;
-        if (!(f1.y > 0.f)) v[8 * j + 3] = 0.f;
-        if (!(f2.x > 0.f)) v[8 * j + 4] = 0.f;
-        if (!(f2.y > 0.f)) v[8 * j + 5] = 0.f;
-        if (!(f3.x > 0.f)) v[8 * j + 6] = 0.f;
-        if (!(f3.y > 0.f)) v[8 * j + 7] = 0.f;
-      }
-    }
     if (!RES) {   // the store that last read this buffer (two chunks ago with two buffers, the previous one otherwise)
       if (lane == 0) {
         if (nbuf == 2) tma_store_wait_read<1>();
@@ -387,7 +350,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
       }
       __syncwarp();
     }
-    if (NC == 16 && !RES && !MASK && p.out_mode == kOutNCHWf32) {
+    if (NC == 16 && !RES && p.out_mode == kOutNCHWf32) {
       // ---- fp32 planes [B, n_store, H, W] through a bulk-tensor store: the staging block is [16 planes][32 pixels] fp32 (2 KiB), the
       // tensor map sees the planes as bf16 pairs (a pure byte mover); planes beyond n_store are clipped by the TMA
       const uint32_t blk = buf_of(ectr);
@@ -403,7 +366,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
       ++ectr;
       continue;
     }
-    if (NC == 32 && !RES && !MASK && p.out_mode == kOutQKV) {
+    if (NC == 32 && !RES && p.out_mode == kOutQKV) {
       // ---- QKV projection: the quadrant's 32 pixels are 32 consecutive tokens of image qb0 (host-checked); a 32-channel chunk lies
       // inside q, k or v and covers two heads of 16, one head of 32 or part of a wider head.  Q / K [B,heads,N,hd]: rows of the
       // staging block are tokens (two 1 KiB blocks of 32-byte rows for head_dim 16, else one block of 64-byte rows, as for NHWC);
@@ -499,8 +462,7 @@ struct ResStream {
 
 // ROWK: 0 plain taps; 3: row-segment mode for a 3 x 3 window; 9: for a 1 x 9 window (compile-time so that the tap loops of the producer and
 // of the MMA issuer unroll - with run-time tap counts the 3 x 3 layers lost 8 %)
-template <int ROWK, bool TMA_OUT, bool TMA_RES, int LEAN = 0>   // LEAN: 0 generic epilogue, 1 lean, 2 lean with a ReLU-mask input,
-                                                                  // 3 lean with the residual stream
+template <int ROWK, bool TMA_OUT, bool TMA_RES, int LEAN = 0>   // LEAN: 0 generic epilogue, 1 lean, 3 lean with the residual stream
 __global__ void __launch_bounds__(kThreads, 1)
 igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ IgemmArgs p) {
   extern __shared__ uint8_t smem_raw[];
@@ -573,15 +535,6 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
-  // debug trace: role r in {0 producer, 1 mma, 2 epilogue warp 2 lane 0} appends (event id, clock) pairs
-  int trace_n = 0;
-  auto trace = [&](int role, int ev) {
-    if (p.trace && blockIdx.x == 0 && trace_n < 2000) {
-      p.trace[(role * 2000 + trace_n) * 2] = ev;
-      p.trace[(role * 2000 + trace_n) * 2 + 1] = clock64();
-      ++trace_n;
-    }
-  };
 
   auto decode = [&](int tile, int& n0, int& b0, int& y0, int& x0) {
     const int nt = tile % n_tiles, mt = tile / n_tiles;
@@ -624,13 +577,11 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
             for (int kb = 0; kb < nkb; ++kb) {
               mbar_wait(empty_bar(stage), phase ^ 1u);
               if (elect_one_sync()) {
-                trace(0, 1);
                 const uint32_t sa = smem_base + stage * kStageSz;
-                mbar_arrive_expect_tx(full_bar(stage), ((p.dbg & 8) ? 0u : a_bytes) + (((p.dbg & 4) || p.wres) ? 0u : static_cast<uint32_t>(nkx) * b_bytes));
-                if (!(p.dbg & 8)) tma_load_4d(sa, &maps.a[2], full_bar(stage), kb * kIgemmBK, x0 - nkx / 2, y0 + ky - nky / 2, b0);
-                for (int kx = 0; kx < nkx && !(p.dbg & 4) && !p.wres; ++kx)
+                mbar_arrive_expect_tx(full_bar(stage), a_bytes + (p.wres ? 0u : static_cast<uint32_t>(nkx) * b_bytes));
+                tma_load_4d(sa, &maps.a[2], full_bar(stage), kb * kIgemmBK, x0 - nkx / 2, y0 + ky - nky / 2, b0);
+                for (int kx = 0; kx < nkx && !p.wres; ++kx)
                   tma_load_2d(sa + kAOff + kx * b_bytes, &maps.b, full_bar(stage), ((ky * nkx + kx) * nkb + kb) * kIgemmBK, n0);
-                trace(0, 2);
               }
               __syncwarp();
               if (++stage == kStages) { stage = 0; phase ^= 1u; }
@@ -683,7 +634,6 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
             mbar_wait(full_bar(stage), phase);
             tc_fence_after();
             if (elect_one_sync()) {
-              trace(1, 11);
               // stage sg = (ky, kb): its three B tiles are k-blocks (ky*3 + kx) * nkb + kb of the packed weights
               const int nkb3 = p.taps[0].nkb, ky3 = sg / nkb3, kb3 = sg - ky3 * nkb3;
               const uint32_t a_lo = a_lo0 + stage * stage16;
@@ -695,12 +645,10 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
                 // UMMA swizzle is a function of the absolute shared-memory address, so the shifted start needs no fix-up
 #pragma unroll
                 for (int k = 0; k < kIgemmBK / 16; ++k)
-                  if (!(p.dbg & 32))
-                    umma_bf16(d_tmem, umma_desc_join(a_lo + 8u * kx + 2u * k, dhi), umma_desc_join(b_lo + kx * bkx16 + 2u * k, dhi), idesc,
-                              (sg | kx | k) != 0 ? 1u : 0u);
+                  umma_bf16(d_tmem, umma_desc_join(a_lo + 8u * kx + 2u * k, dhi), umma_desc_join(b_lo + kx * bkx16 + 2u * k, dhi), idesc,
+                            (sg | kx | k) != 0 ? 1u : 0u);
               }
               umma_commit(empty_bar(stage));
-              trace(1, 12);
             }
             __syncwarp();
             if (++stage == kStages) { stage = 0; phase ^= 1u; }
@@ -721,10 +669,7 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
           __syncwarp();
           if (++stage == kStages) { stage = 0; phase ^= 1u; }
         }
-        if (elect_one_sync()) {
-          umma_commit(tfull_bar(a));
-          trace(1, 13);
-        }
+        if (elect_one_sync()) umma_commit(tfull_bar(a));
         __syncwarp();
       }
     }
@@ -791,7 +736,6 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
       const int b = b0 + bb, y = y0 + yy, x = x0 + xx;
       const bool valid = (b < p.B) && (y < p.H) && (x < p.W);
       const uint32_t tacc = tmem_base + static_cast<uint32_t>(a) * 256u + (static_cast<uint32_t>(quad * 32) << 16);
-      if (warp == 2 && lane == 0) trace(2, 20);
       if (LEAN == 3) {
         // ---- residual stream: chunks grp*32 + k*64 of this tile; residual rows come from the load ring, results go out through two
         // alternating store buffers
@@ -898,10 +842,10 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
         }
       } else if (LEAN) {
         if ((p.BN % 32 == 0) && (p.N % 32 == 0) && p.out_mode != kOutNCHWf32)
-          epilogue_tile_lean<32, TMA_RES, LEAN == 2>(p, tacc, n0, b, y, x, valid, grp, s_bias, s_prelu, tfull_bar(a), aphase, &maps.c, &maps.r, out_stage, res_stage,
+          epilogue_tile_lean<32, TMA_RES>(p, tacc, n0, b, grp, s_bias, s_prelu, tfull_bar(a), aphase, &maps.c, &maps.r, out_stage, res_stage,
                                           p.stage2 ? 2 : 1, x0 + qx0, y0 + qy0, b0 + qb0, res_bar, res_phase, ectr, maps.qkv);
         else
-          epilogue_tile_lean<16, TMA_RES, LEAN == 2>(p, tacc, n0, b, y, x, valid, grp, s_bias, s_prelu, tfull_bar(a), aphase, &maps.c, &maps.r, out_stage, res_stage,
+          epilogue_tile_lean<16, TMA_RES>(p, tacc, n0, b, grp, s_bias, s_prelu, tfull_bar(a), aphase, &maps.c, &maps.r, out_stage, res_stage,
                                           p.stage2 ? 2 : 1, x0 + qx0, y0 + qy0, b0 + qb0, res_bar, res_phase, ectr);
       } else if (p.out_mode != kOutQKV && (p.BN % 32 == 0) && (p.N % 32 == 0) && !(p.out_mode == kOutNCHWf32 && p.BN == 32))
         // (fp32 planes with a single 32-column N tile: 16-column chunks keep BOTH epilogue groups busy)
@@ -912,7 +856,6 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
                           y0 + qy0, b0 + qb0, &maps.r, res_stage, res_bar, res_phase);
       tc_fence_before();
       mbar_arrive(tempty_bar(a));
-      if (warp == 2 && lane == 0) trace(2, 22);
     }
     if (TMA_OUT && lane == 0) tma_store_wait_read0();   // shared memory must outlive the last bulk store's read
   }
@@ -973,9 +916,6 @@ int igemm_launch(const IgemmPlan& plan, cudaStream_t stream) {
     e = plan.args.lean ? launch_variant<9, true, false, 1>(plan, stream) : launch_variant<9, false, false>(plan, stream);
   } else if (plan.args.lean == 3) {
     e = launch_variant<0, true, true, 3>(plan, stream);
-  } else if (plan.args.lean && plan.args.mask) {
-    if (plan.args.row3) e = plan.args.tma_res ? launch_variant<3, true, true, 2>(plan, stream) : launch_variant<3, true, false, 2>(plan, stream);
-    else e = plan.args.tma_res ? launch_variant<0, true, true, 2>(plan, stream) : launch_variant<0, true, false, 2>(plan, stream);
   } else if (plan.args.lean) {
     if (plan.args.row3) e = plan.args.tma_res ? launch_variant<3, true, true, 1>(plan, stream) : launch_variant<3, true, false, 1>(plan, stream);
     else e = plan.args.tma_res ? launch_variant<0, true, true, 1>(plan, stream) : launch_variant<0, true, false, 1>(plan, stream);

@@ -37,8 +37,6 @@ struct IgemmArgs {
   int tb, th, tw;  // tile shape, tb*th*tw == 128
   int N, BN;       // true output channels (multiple of 16) and N tile
   int ntaps, total_kb;
-  long long* trace;  // debug: CTA 0 writes (event, clock) pairs here (WC_IGEMM_TRACE), else nullptr
-  int dbg;      // debug/experiment bits (WC_IGEMM_DBG): 1 skip epilogue global stores, 2 skip MMA issue, 4 skip B loads
   int nstages;  // depth of the TMA ring (set by igemm_stages_for)
   int row3;  // 1: taps 0..8 form a 3x3 stride-1 window executed in row-segment mode (see igemm.cu)
   IgemmTap taps[kMaxTaps];

@@ -2,7 +2,6 @@
 // Reference ops: nn.GroupNorm(8, C) [+ nn.SiLU] at unet_base.py:89-90,101-102,107,155-156,483-484.
 // Two bandwidth-bound passes: (1) per-(sample, slab) partial sums, (2) deterministic combine + normalise.
 // Statistics are identical for the 4-D [B,C,H,W] and 3-D [B,C,HW] uses (biased variance over C/8 x HW).
-#include <cstdlib>
 #include "wc_host.h"
 #include "wc_ptx.cuh"
 
@@ -388,131 +387,6 @@ __global__ void colsum_finish_kernel(const float* __restrict__ part, int B, int 
 }
 
 
-// ---- single-launch GroupNorm for maps of at most 2048 pixels: one thread-block CLUSTER per sample --------------------------------
-// 52 of the 65 GroupNorms of a C3 step (61 of 61 below the first level at batch 1) normalise tensors of 2 - 8 MB: the two-pass
-// pair above takes 6 + 9 us of almost pure launch / ramp latency for them.  Here the nsplit (1, 2, 4 or 8) CTAs of a sample
-// form a cluster: each loads its slab ONCE (kept in registers when it is at most 16 vectors per thread), reduces its partial
-// sums exactly like gn_stats_kernel, publishes them in its own shared memory, and after one cluster barrier every CTA combines
-// all partials of the sample in rank order through distributed shared memory (deterministic, independent of the batch) and
-// applies the normalisation.  Partials are also written to the global workspace in the layout the backward pass expects.
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ float2 ld_cluster_f2(uint32_t local_smem_addr, uint32_t rank) {
-  uint32_t remote;
-  float2 v;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(local_smem_addr), "r"(rank));
-  asm volatile("ld.shared::cluster.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(remote) : "memory");
-  return v;
-}
-
-constexpr int kGnFusedMaxVec = 16;
-
-__global__ void gn_fused_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y, int HW, int C, int ld, int ldy,
-                                int nsplit, float2* __restrict__ partial, const float* __restrict__ gamma,
-                                const float* __restrict__ beta, float eps, int silu) {
-  pdl_prologue();
-  extern __shared__ float2 stash[];                     // [blockDim.x] per-thread partial sums
-  __shared__ float2 s_part[kGroups];                    // this CTA's partial sums (read by the whole cluster)
-  __shared__ float s_mean[kGroups], s_rstd[kGroups];
-  const int vpp = C / 8, gv = (C / kGroups) / 8, cpg = C / kGroups;
-  const int rows = blockDim.x / vpp;
-  const int v = threadIdx.x % vpp, r = threadIdx.x / vpp;
-  const int b = blockIdx.y, split = blockIdx.x;         // split == rank in the cluster (cluster dims = (nsplit, 1, 1))
-  const int p0 = static_cast<int>(static_cast<long long>(HW) * split / nsplit);
-  const int p1 = static_cast<int>(static_cast<long long>(HW) * (split + 1) / nsplit);
-  const int nvec = (p1 - p0 - r + rows - 1) / rows;     // pixels p0 + r + k * rows, k < nvec
-  const bool in_regs = (p1 - p0 + rows - 1) / rows <= kGnFusedMaxVec;   // block-uniform
-  const __nv_bfloat16* xb = x + static_cast<size_t>(b) * HW * ld + v * 8;
-  uint4 keep[kGnFusedMaxVec];
-  float s = 0.f, ss = 0.f;
-  auto acc = [&](const uint4& u) {
-    const float2 a = unpack_bf16(u.x), bq = unpack_bf16(u.y), c = unpack_bf16(u.z), d = unpack_bf16(u.w);
-    s += (a.x + a.y) + (bq.x + bq.y) + (c.x + c.y) + (d.x + d.y);
-    ss += (a.x * a.x + a.y * a.y) + (bq.x * bq.x + bq.y * bq.y) + (c.x * c.x + c.y * c.y) + (d.x * d.x + d.y * d.y);
-  };
-  if (in_regs) {
-#pragma unroll
-    for (int k = 0; k < kGnFusedMaxVec; ++k)
-      if (k < nvec) keep[k] = __ldg(reinterpret_cast<const uint4*>(xb + static_cast<size_t>(p0 + r + k * rows) * ld));
-#pragma unroll
-    for (int k = 0; k < kGnFusedMaxVec; ++k)
-      if (k < nvec) acc(keep[k]);
-  } else {
-    for (int p = p0 + r; p < p1; p += rows) acc(__ldg(reinterpret_cast<const uint4*>(xb + static_cast<size_t>(p) * ld)));
-  }
-  stash[threadIdx.x] = make_float2(s, ss);
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-  for (int g = warp; g < kGroups; g += nwarps) {        // same fixed-order reduction as gn_stats_kernel
-    const int cnt = rows * gv;
-    float as = 0.f, ass = 0.f;
-    for (int i = lane; i < cnt; i += 32) {
-      const float2 t = stash[(i / gv) * vpp + g * gv + (i % gv)];
-      as += t.x; ass += t.y;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      as += __shfl_xor_sync(0xffffffffu, as, o);
-      ass += __shfl_xor_sync(0xffffffffu, ass, o);
-    }
-    if (lane == 0) {
-      s_part[g] = make_float2(as, ass);
-      partial[(static_cast<size_t>(b) * nsplit + split) * kGroups + g] = make_float2(as, ass);
-    }
-  }
-  cluster_sync_all();                                   // every CTA of the sample has published its partials
-  if (threadIdx.x < kGroups) {
-    double ds = 0.0, dss = 0.0;
-    const uint32_t mine = smem_u32(&s_part[threadIdx.x]);
-    for (int i = 0; i < nsplit; ++i) {
-      const float2 t = ld_cluster_f2(mine, static_cast<uint32_t>(i));
-      ds += t.x; dss += t.y;
-    }
-    const double n = static_cast<double>(HW) * cpg;
-    const double mean = ds / n;
-    double var = dss / n - mean * mean;
-    if (var < 0.0) var = 0.0;
-    s_mean[threadIdx.x] = static_cast<float>(mean);
-    s_rstd[threadIdx.x] = static_cast<float>(1.0 / sqrt(var + static_cast<double>(eps)));
-  }
-  __syncthreads();
-  const int g = (v * 8) / cpg;
-  const float mean = s_mean[g], rstd = s_rstd[g];
-  float ga[8], be[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    ga[j] = gamma[v * 8 + j] * rstd;
-    be[j] = beta[v * 8 + j] - mean * ga[j];
-  }
-  __nv_bfloat16* yb = y + static_cast<size_t>(b) * HW * ldy + v * 8;
-  auto one = [&](const uint4& u, int p) {
-    float f[8];
-    float2 t;
-    t = unpack_bf16(u.x); f[0] = t.x; f[1] = t.y;
-    t = unpack_bf16(u.y); f[2] = t.x; f[3] = t.y;
-    t = unpack_bf16(u.z); f[4] = t.x; f[5] = t.y;
-    t = unpack_bf16(u.w); f[6] = t.x; f[7] = t.y;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      float o = fmaf(f[j], ga[j], be[j]);
-      if (silu) o = silu_fast(o);
-      f[j] = o;
-    }
-    uint4 w;
-    w.x = pack_bf16(f[0], f[1]); w.y = pack_bf16(f[2], f[3]); w.z = pack_bf16(f[4], f[5]); w.w = pack_bf16(f[6], f[7]);
-    *reinterpret_cast<uint4*>(yb + static_cast<size_t>(p) * ldy) = w;
-  };
-  if (in_regs) {
-#pragma unroll
-    for (int k = 0; k < kGnFusedMaxVec; ++k)
-      if (k < nvec) one(keep[k], p0 + r + k * rows);
-  } else {
-    for (int p = p0 + r; p < p1; p += rows) one(__ldg(reinterpret_cast<const uint4*>(xb + static_cast<size_t>(p) * ld)), p);
-  }
-  cluster_sync_all();                                   // no CTA leaves while a peer may still read its s_part
-}
-
 }  // namespace
 
 size_t groupnorm_workspace_bytes(int B) { return static_cast<size_t>(B) * 64 * kGroups * sizeof(float2); }
@@ -525,7 +399,7 @@ size_t groupnorm_workspace_bytes(int B) { return static_cast<size_t>(B) * 64 * k
 int groupnorm_stats_splits(int B, int HW) {
   (void)B;
   int nsplit = (HW + 127) / 128;     // >= 128 pixels per block (a block of 2048 got 1.5x slower with 32-pixel slabs)
-  if (HW <= 2048) {                  // single-launch cluster kernel: 1, 2, 4 or 8 CTAs per sample (portable cluster size)
+  if (HW <= 2048) {                  // 1, 2, 4 or 8 slabs per sample: this rule fixes the summation order, and with it the bits
     int c = 1;
     while (c * 2 <= nsplit && c < 8) c *= 2;
     return c;
@@ -545,42 +419,14 @@ int groupnorm_silu(const __nv_bfloat16* x, __nv_bfloat16* y, int B, int HW, int 
   const int nsplit = groupnorm_stats_splits(B, HW);
   const int max_split = (HW + 31) / 32;
   float2* partial = reinterpret_cast<float2*>(workspace);
-  // Single-launch cluster kernel, for tensors of at most WC_GN_FUSED_MAX_BYTES bytes.  Default 0 = OFF: measured on B200 it loses
-  // in both regimes - batch 32 (all maps of <= 2048 pixels): GroupNorm 1.55 -> 2.13 ms per C3 step (8 CTAs per sample cannot fill
-  // the chip on 25 - 67 MB tensors); batch 1 (reference geometry, tensors <= 4 MiB): 0.94 -> 1.61 ms per step (a cluster launch
-  // plus two cluster barriers cost more than the second small launch they replace).  Both paths partition and order the sums
-  // identically and give bit-identical results.
-  static long fused_max = -1;
-  if (fused_max < 0) {
-    const char* e = getenv("WC_GN_FUSED_MAX_BYTES");
-    fused_max = e ? atol(e) : 0;
-  }
-  if (HW <= 2048 && 2l * B * HW * C <= fused_max) {
-    ProfScope prof(kProfGroupNorm, st, 4.0 * B * static_cast<double>(HW) * C);  // algorithmic bytes: 1 read + 1 write, bf16
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(nsplit, B);
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = threads * sizeof(float2);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = nsplit; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    WC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gn_fused_kernel, x, y, HW, C, ld, ldy, nsplit, partial, gamma, beta, eps, silu));
-    WC_LAUNCH_CHECK();
-    return 0;
-  }
+  // Two passes, statistics then apply.  A single-launch variant with one thread-block cluster per sample was measured slower on B200
+  // in both regimes: batch 32, GroupNorm 1.55 -> 2.13 ms per C3 step (8 CTAs per sample cannot fill the chip on 25 - 67 MB tensors);
+  // batch 1, 0.94 -> 1.61 ms per step (a cluster launch plus two cluster barriers cost more than the second small launch).
   ProfScope prof(kProfGroupNorm, st, 6.0 * B * static_cast<double>(HW) * C);  // algorithmic bytes: 2 reads + 1 write, bf16
   launch_k(gn_stats_kernel, dim3(nsplit, B), threads, threads * sizeof(float2), st, x, HW, C, ld, nsplit, partial);
   WC_LAUNCH_CHECK();
-  static int per_sm = -1;   // WC_GN_APPLY_BLOCKS_PER_SM: blocks of the apply pass per SM (the result does not depend on it)
-  if (per_sm < 0) {
-    const char* e = getenv("WC_GN_APPLY_BLOCKS_PER_SM");
-    per_sm = e ? atoi(e) : 8;
-    if (per_sm < 1) per_sm = 1;
-  }
-  int asplit = (per_sm * num_sms() + B - 1) / B;
+  constexpr int kApplyBlocksPerSm = 8;   // 2 .. 8 measured within 3 % of each other, 16 is 9 % slower; the result does not depend on it
+  int asplit = (kApplyBlocksPerSm * num_sms() + B - 1) / B;
   if (asplit > max_split) asplit = max_split;
   if (asplit < 1) asplit = 1;
   launch_k(gn_apply_kernel, dim3(asplit, B), threads, 0, st, x, y, HW, C, ld, ldy, nsplit, asplit, partial, gamma, beta, eps,

@@ -153,17 +153,11 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   const int B = net->B, H = net->H, W = net->W, NC = net->num_classes;
   SegBuilder b{net, dry ? Bump::dry() : Bump(ws, ws_bytes), net->arena.get(), st, dry, B};
   const int H2 = H / 2, W2 = W / 2, H4 = H / 4, W4 = W / 4;
-  // ---------------- stem: conv1 7x7 s2 + bn1 + relu (direct, from NCHW fp32), maxpool 3x3 s2
+  // ---------------- stem: conv1 7x7 s2 + bn1 + relu (tensor core, from NCHW fp32), maxpool 3x3 s2
   Act c1 = b.act(H2, W2, 64);
   Act p1 = b.act(H4, W4, 64);
   uint8_t* pool_idx = static_cast<uint8_t*>(b.bump.take(p1.pixels() * 64));
-  static int stem_tc = -1;   // WC_SEG_STEM_TC=0: direct fp32 CUDA-core stem (round-1 kernel: 0.85 ms at 32 x 256 x 512)
-  if (stem_tc < 0) {
-    const char* e = getenv("WC_SEG_STEM_TC");
-    stem_tc = e ? atoi(e) : 1;
-  }
-  const bool tc_stem = stem_tc && H % 2 == 0 && W % 2 == 0;
-  __nv_bfloat16* xpad = tc_stem ? static_cast<__nv_bfloat16*>(b.bump.take(static_cast<size_t>(B) * H * (W + 8) * 8 * sizeof(__nv_bfloat16))) : nullptr;
+  __nv_bfloat16* xpad = static_cast<__nv_bfloat16*>(b.bump.take(static_cast<size_t>(B) * H * (W + 8) * 8 * sizeof(__nv_bfloat16)));
   std::pair<float*, float*> bn1{nullptr, nullptr};
   const float* w_conv1 = nullptr;
   if (!dry) {
@@ -172,26 +166,19 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     if (b.err) return b.err;
     wc_seg* n = net;
     const float *sc = bn1.first, *sh = bn1.second;
-    if (tc_stem) {
-      // tensor-core stem: image -> padded NHWC-8 bf16, then an implicit GEMM with overlapping TMA boxes (conv.cu)
-      float* wprime = static_cast<float*>(b.arena->alloc(64 * 64 * 7 * sizeof(float)));
-      if (!wprime) return 1;
-      if (int e = stem_weights(w_conv1, wprime, 64, st)) return e;
-      Epilogue ep; ep.bias = sh; ep.relu = 1;
-      OutSpec os; os.mode = kOutNHWC; os.out = c1;
-      auto op = std::make_shared<ConvOp>();
-      if (int e = build_conv_stem7s2(op.get(), b.arena, xpad, B, H, W, wprime, sc, 64, ep, os, st)) return e;
-      b.push([=](cudaStream_t s) {
-        if (int e = stem_prepare(n->x_in, xpad, B, H, W, s)) return e;
-        if (int e = op->run(s)) return e;
-        return maxpool_fwd(c1.ptr, p1.ptr, pool_idx, B, H2, W2, 64, s);
-      });
-    } else {
-      b.push([=](cudaStream_t s) {
-        if (int e = conv_small_cin(n->x_in, w_conv1, nullptr, sc, sh, c1.ptr, B, 3, H, W, 64, 7, 2, 3, 64, 1, s)) return e;
-        return maxpool_fwd(c1.ptr, p1.ptr, pool_idx, B, H2, W2, 64, s);
-      });
-    }
+    // image -> padded NHWC-8 bf16, then an implicit GEMM with overlapping TMA boxes (conv.cu)
+    float* wprime = static_cast<float*>(b.arena->alloc(64 * 64 * 7 * sizeof(float)));
+    if (!wprime) return 1;
+    if (int e = stem_weights(w_conv1, wprime, 64, st)) return e;
+    Epilogue ep; ep.bias = sh; ep.relu = 1;
+    OutSpec os; os.mode = kOutNHWC; os.out = c1;
+    auto op = std::make_shared<ConvOp>();
+    if (int e = build_conv_stem7s2(op.get(), b.arena, xpad, B, H, W, wprime, sc, 64, ep, os, st)) return e;
+    b.push([=](cudaStream_t s) {
+      if (int e = stem_prepare(n->x_in, xpad, B, H, W, s)) return e;
+      if (int e = op->run(s)) return e;
+      return maxpool_fwd(c1.ptr, p1.ptr, pool_idx, B, H2, W2, 64, s);
+    });
     net->flops_fwd += 2.0 * B * H2 * W2 * 147.0 * 64;
   }
   // ---------------- residual layers
@@ -285,13 +272,9 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   // ---------------- loss head: bilinear to the input size, argmax, softmax-CE gradient (inference.py:135-141)
   float* dlogit_hi = static_cast<float*>(b.bump.take(static_cast<size_t>(B) * H * W * NC * sizeof(float)));
   int* n_valid = static_cast<int*>(b.bump.take(B * sizeof(int)));
-  // WC_SEG_LOSS_FUSED (default 1): with the input gradient requested, pred / loss / low-resolution d-logits come from ONE kernel and the
-  // 19-plane full-resolution d-logit tensor is never written (seg_kernels.cu: seg_loss_head_fused_kernel)
-  static int loss_fused = -1;
-  if (loss_fused < 0) {
-    const char* e = getenv("WC_SEG_LOSS_FUSED");
-    loss_fused = e ? atoi(e) : 1;
-  }
+  // With the input gradient requested, pred / loss / low-resolution d-logits come from ONE kernel and the 19-plane full-resolution
+  // d-logit tensor is never written (seg_kernels.cu: seg_loss_head_fused_kernel); geometries it does not take, and requests for the
+  // full-resolution logits, go through the two-pass head below.
   Act dlo{};
   if (net->with_grad) dlo = b.act(H4, W4, NCP);
   if (!dry) {
@@ -302,9 +285,8 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   {
     wc_seg* n = net;
     const bool with_grad = net->with_grad;
-    const int fused = loss_fused;
     b.push([=](cudaStream_t s) {
-      if (with_grad && fused && !n->logits_hi) {
+      if (with_grad && !n->logits_hi) {
         const int e = seg_loss_head_fused(logits_lo, n->labels, n_valid, n->pred, n->loss, dlo.ptr, B, H4, W4, H, W, NC, NCP, NCP, 255, s);
         if (e != -1) return e;
       }

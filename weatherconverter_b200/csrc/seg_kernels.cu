@@ -862,7 +862,7 @@ int compose_sep(const float* dw, const float* pw, const float* dwb, const float*
 // =====================================================================================================================
 // SRGAN final layer (srgan_model/models.py:85,92): depthwise 9x9 (64 ch, bias) -> pointwise 64->3 (bias) -> (tanh+1)/2,
 // NHWC bf16 in, NCHW fp32 out.  One CTA = an 8 x 64 output tile; the (8+8) x (64+8) x 64-channel halo tile is staged
-// in shared memory as 32 channel-pair planes (conflict-free row reads); each thread owns 4 adjacent pixels and half
+// in shared memory as 32 channel-pair planes of half2 (conflict-free row reads); each thread owns 4 adjacent pixels and half
 // of the channel pairs, sliding a 12-wide register window over every kernel row.
 namespace wc {
 namespace {
@@ -870,28 +870,22 @@ namespace {
 constexpr int kFT_H = 8, kFT_W = 64, kFHalo = 4, kFPlaneW = kFT_W + 2 * kFHalo /*72*/, kFPlaneH = kFT_H + 2 * kFHalo /*16*/;
 constexpr int kFPlane = kFPlaneW * kFPlaneH + 1;  // +1 word: de-phase the planes across banks for the staging writes
 
-template <bool HALF>
 __global__ void __launch_bounds__(512, 1)
 srgan_final_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ dw /*[64][81]*/,
                    const float* __restrict__ dwb, const float* __restrict__ pw /*[3][64]*/, const float* __restrict__ pwb,
                    float* __restrict__ y, int B, int H, int W, int ldx) {
   pdl_prologue();
   extern __shared__ uint32_t sm[];
-  uint32_t* tile = sm;                                            // [32][kFPlane] bf16x2
-  float* wsm = reinterpret_cast<float*>(sm + 32 * kFPlane);       // [32][81][2] fp32, or (HALF) [32][81] half2 in the first half
+  uint32_t* tile = sm;                                            // [32][kFPlane] half2
+  float* wsm = reinterpret_cast<float*>(sm + 32 * kFPlane);       // [32][81] half2 in the first half of [32][81][2] words
   float* red = wsm + 32 * 81 * 2;                                 // [3 groups][128 threads][12]
   const int tiles_x = (W + kFT_W - 1) / kFT_W, tiles_y = (H + kFT_H - 1) / kFT_H;
   const int tid = threadIdx.x;
-  if (HALF) {
+  {
     __half2* wh = reinterpret_cast<__half2*>(wsm);
     for (int i = tid; i < 32 * 81; i += 512) {
       const int tap = i % 81, c2 = i / 81;
       wh[i] = __floats2half2_rn(dw[(c2 * 2) * 81 + tap], dw[(c2 * 2 + 1) * 81 + tap]);
-    }
-  } else {
-    for (int i = tid; i < 32 * 81 * 2; i += 512) {
-      const int j = i & 1, tap = (i >> 1) % 81, c2 = (i >> 1) / 81;
-      wsm[i] = dw[(c2 * 2 + j) * 81 + tap];
     }
   }
   // thread -> column tx (lanes sweep x: conflict-free shared-memory reads) and 4 vertically adjacent output rows
@@ -907,13 +901,12 @@ srgan_final_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict_
       if (gy >= 0 && gy < H && gx >= 0 && gx < W)
         u = __ldg(reinterpret_cast<const uint4*>(x + ((static_cast<size_t>(b) * H + gy) * W + gx) * ldx + c8 * 8));
       uint32_t* dst = tile + (c8 * 4) * kFPlane + py * kFPlaneW + px;
-      if (HALF) {   // channel pairs as half2 (11-bit mantissa: exact for bf16 values inside the fp16 range)
-        auto h2 = [](uint32_t w) {
-          const __half2 h = __floats2half2_rn(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
-          return *reinterpret_cast<const uint32_t*>(&h);
-        };
-        u.x = h2(u.x); u.y = h2(u.y); u.z = h2(u.z); u.w = h2(u.w);
-      }
+      // channel pairs as half2 (11-bit mantissa: exact for bf16 values inside the fp16 range)
+      auto h2 = [](uint32_t w) {
+        const __half2 h = __floats2half2_rn(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
+        return *reinterpret_cast<const uint32_t*>(&h);
+      };
+      u.x = h2(u.x); u.y = h2(u.y); u.z = h2(u.z); u.w = h2(u.w);
       dst[0] = u.x; dst[kFPlane] = u.y; dst[2 * kFPlane] = u.z; dst[3 * kFPlane] = u.w;
     }
     __syncthreads();
@@ -928,48 +921,30 @@ srgan_final_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict_
 #pragma unroll
       for (int p = 0; p < 4; ++p) acc2[p] = make_float2(b0, b1);
       const uint32_t* pl = tile + c2 * kFPlane + ty * kFPlaneW + tx;
-      const float2* wp = reinterpret_cast<const float2*>(wsm) + c2 * 81;
-      if (HALF) {
-        // packed fp16 FMAs (HFMA2: two channels per instruction, no bf16 unpacking) over the nine rows of one kernel column,
-        // folded into the fp32 accumulators after every column: 9 fp16 roundings per partial sum instead of 81
-        const __half2* wh = reinterpret_cast<const __half2*>(wsm) + c2 * 81;
-#pragma unroll
-        for (int kx = 0; kx < 9; ++kx) {
-          __half2 v[12];
-#pragma unroll
-          for (int i = 0; i < 12; ++i) {
-            const uint32_t u = pl[i * kFPlaneW + kx];
-            v[i] = *reinterpret_cast<const __half2*>(&u);
-          }
-          __half2 part[4];
-#pragma unroll
-          for (int p = 0; p < 4; ++p) part[p] = __hmul2(v[p], wh[kx]);
-#pragma unroll
-          for (int ky = 1; ky < 9; ++ky) {
-            const __half2 wv = wh[ky * 9 + kx];
-#pragma unroll
-            for (int p = 0; p < 4; ++p) part[p] = __hfma2(v[p + ky], wv, part[p]);
-          }
-#pragma unroll
-          for (int p = 0; p < 4; ++p) {
-            const float2 f = __half22float2(part[p]);
-            acc2[p].x += f.x; acc2[p].y += f.y;
-          }
-        }
-      } else
+      // packed fp16 FMAs (HFMA2: two channels per instruction, no bf16 unpacking) over the nine rows of one kernel column,
+      // folded into the fp32 accumulators after every column: 9 fp16 roundings per partial sum instead of 81
+      const __half2* wh = reinterpret_cast<const __half2*>(wsm) + c2 * 81;
 #pragma unroll
       for (int kx = 0; kx < 9; ++kx) {
-        float2 v[12];   // 12-row register window of column tx + kx (rows ty .. ty+11 of the halo tile)
+        __half2 v[12];   // 12-row register window of column tx + kx (rows ty .. ty+11 of the halo tile)
 #pragma unroll
         for (int i = 0; i < 12; ++i) {
           const uint32_t u = pl[i * kFPlaneW + kx];
-          v[i] = make_float2(__uint_as_float(u << 16), __uint_as_float(u & 0xffff0000u));
+          v[i] = *reinterpret_cast<const __half2*>(&u);
+        }
+        __half2 part[4];
+#pragma unroll
+        for (int p = 0; p < 4; ++p) part[p] = __hmul2(v[p], wh[kx]);
+#pragma unroll
+        for (int ky = 1; ky < 9; ++ky) {
+          const __half2 wv = wh[ky * 9 + kx];
+#pragma unroll
+          for (int p = 0; p < 4; ++p) part[p] = __hfma2(v[p + ky], wv, part[p]);
         }
 #pragma unroll
-        for (int ky = 0; ky < 9; ++ky) {
-          const float2 wv = wp[ky * 9 + kx];
-#pragma unroll
-          for (int p = 0; p < 4; ++p) acc2[p] = ffma2(v[p + ky], wv, acc2[p]);
+        for (int p = 0; p < 4; ++p) {
+          const float2 f = __half22float2(part[p]);
+          acc2[p].x += f.x; acc2[p].y += f.y;
         }
       }
 #pragma unroll
@@ -1076,12 +1051,6 @@ __global__ void phase_major_rows_kernel(const float* __restrict__ src, float* __
   dst[i] = src[static_cast<size_t>(rep_src ? c : c * 4 + q) * len + e];
 }
 
-__global__ void gather_stride_kernel(const float* src, float* dst, int n, int mul, int off) {
-  pdl_prologue();
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) dst[i] = src[i * mul + off];
-}
-
 }  // namespace
 
 int srgan_final(const __nv_bfloat16* x, const float* dw, const float* dwb, const float* pw, const float* pwb, float* y, int B,
@@ -1089,19 +1058,12 @@ int srgan_final(const __nv_bfloat16* x, const float* dw, const float* dwb, const
   const size_t smem = (32 * kFPlane) * 4 + 32 * 81 * 2 * 4 + 3 * 128 * 12 * 4;
   static bool attr = false;
   if (!attr) {
-    WC_CHECK_CUDA(cudaFuncSetAttribute(srgan_final_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    WC_CHECK_CUDA(cudaFuncSetAttribute(srgan_final_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    WC_CHECK_CUDA(cudaFuncSetAttribute(srgan_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     attr = true;
-  }
-  static int half = -1;   // WC_SRGAN_FINAL_F16=0: fp32 FFMA2 inner loop (round 1)
-  if (half < 0) {
-    const char* e = getenv("WC_SRGAN_FINAL_F16");
-    half = e ? atoi(e) : 1;
   }
   const int tiles = B * ((W + kFT_W - 1) / kFT_W) * ((H + kFT_H - 1) / kFT_H);
   ProfScope prof(kProfBoundaryConv, st, static_cast<double>(B) * H * W * (128.0 + 12.0));
-  if (half) launch_k(srgan_final_kernel<true>, std::min(tiles, num_sms()), 512, smem, st, x, dw, dwb, pw, pwb, y, B, H, W, ldx);
-  else launch_k(srgan_final_kernel<false>, std::min(tiles, num_sms()), 512, smem, st, x, dw, dwb, pw, pwb, y, B, H, W, ldx);
+  launch_k(srgan_final_kernel, std::min(tiles, num_sms()), 512, smem, st, x, dw, dwb, pw, pwb, y, B, H, W, ldx);
   WC_LAUNCH_CHECK();
   return 0;
 }
@@ -1185,11 +1147,6 @@ int srgan_initial(const float* x, const float* dw, const float* dwb, const float
 int phase_major_rows(const float* src, float* dst, int cb, int len, int rep_src, cudaStream_t st) {
   const size_t total = static_cast<size_t>(4) * cb * len;
   launch_k(phase_major_rows_kernel, static_cast<int>((total + 255) / 256), 256, 0, st, src, dst, cb, len, rep_src);
-  WC_LAUNCH_CHECK();
-  return 0;
-}
-int gather_stride(const float* src, float* dst, int n, int mul, int off, cudaStream_t st) {
-  launch_k(gather_stride_kernel, (n + 255) / 256, 256, 0, st, src, dst, n, mul, off);
   WC_LAUNCH_CHECK();
   return 0;
 }

@@ -22,7 +22,6 @@ int srgan_initial(const float* x, const float* dw, const float* dwb, const float
                   __nv_bfloat16* y, int B, int H, int W, int ldy, cudaStream_t st);
 int srgan_final(const __nv_bfloat16* x, const float* dw, const float* dwb, const float* pw, const float* pwb, float* y, int B,
                 int H, int W, int ldx, cudaStream_t st);
-int gather_stride(const float* src, float* dst, int n, int mul, int off, cudaStream_t st);
 int phase_major_rows(const float* src, float* dst, int cb, int len, int rep_src, cudaStream_t st);
 int srgan_final_compose(const float* dw, const float* dwb, const float* pw, const float* pwb, float* wq, float* bias3, cudaStream_t st);
 int srgan_final_combine(const float* t, const float* bias3, float* y, int B, int H, int W, cudaStream_t st);
@@ -187,46 +186,24 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       const float* slope = P(p + ".act.weight");
       if (err) return err;
       ups[u].c = c; ups[u].slope = slope;
-      static int merged = -1;   // WC_SRGAN_UP_MERGED=0: one launch per PixelShuffle phase (round 1)
-      if (merged < 0) {
-        const char* e = getenv("WC_SRGAN_UP_MERGED");
-        merged = e ? atoi(e) : 1;
-      }
-      if (merged && NCH % 32 == 0) {
-        // ONE launch for the four phases: weight rows, bias and PReLU slopes re-ordered phase-major (row q*64 + c = conv channel 4c + q),
-        // N tile 128 so that the row-segment mode applies; every 32-channel chunk is stored through the strided map of its phase
-        float* wpm = fa(static_cast<size_t>(NCH) * 4 * NCH * 9);
-        float* bpm = fa(NCH * 4);
-        float* spm = fa(NCH * 4);
-        if (!wpm || !bpm || !spm) return 1;
-        if (int e = phase_major_rows(c.w, wpm, NCH, NCH * 9, 0, st)) return e;
-        if (int e = phase_major_rows(c.bias, bpm, NCH, 1, 0, st)) return e;
-        if (int e = phase_major_rows(slope, spm, NCH, 1, 1, st)) return e;
-        for (int pass = 0; pass < (grad ? 2 : 1); ++pass) {   // pass 1 (with-grad plans): the pre-activation, without the PReLU
-          WeightSrc ws_; ws_.w = wpm; ws_.d0 = NCH * 4; ws_.d1 = NCH; ws_.KH = ws_.KW = 3;
-          ConvGeom g; g.K = 3; g.pad = 1;
-          Epilogue ep; ep.bias = bpm; ep.prelu = pass ? nullptr : spm;
-          OutSpec os; os.mode = kOutNHWC; os.out = pass ? ups[u].pre : up; os.up = 2; os.phases = 4; os.bn_max = 128;
-          auto op = std::make_shared<ConvOp>();
-          if (int e = build_conv(op.get(), arena, cur, ws_, g, NCH * 4, nullptr, nullptr, ep, os, st)) return e;
-          op->flops = 2.0 * cur.pixels() * (9.0 * NCH + static_cast<double>(NCH) * NCH * 4);
-          for (auto& pl : op->plans) pl.flops = op->flops / op->plans.size();
-          net->flops += op->flops;
-          net->ops.push_back([op](cudaStream_t s) { return op->run(s); });
-        }
-      } else
-      for (int pass = 0; pass < (grad ? 2 : 1); ++pass)
-      for (int q = 0; q < 4; ++q) {   // PixelShuffle: out[c, 2y+i, 2x+j] = conv[4c + 2i + j, y, x]
-        float* bq = fa(NCH);
-        if (!bq) return 1;
-        if (int e = gather_stride(c.bias, bq, NCH, 4, q, st)) return e;
-        WeightSrc ws_; ws_.w = c.w; ws_.d0 = NCH * 4; ws_.d1 = NCH; ws_.KH = ws_.KW = 3; ws_.n_out = NCH; ws_.row_mul = 4; ws_.row_off = q;
+      // ONE launch for the four PixelShuffle phases (out[c, 2y+i, 2x+j] = conv[4c + 2i + j, y, x]): weight rows, bias and PReLU
+      // slopes re-ordered phase-major (row q*64 + c = conv channel 4c + q), N tile 128 so that the row-segment mode applies; every
+      // 32-channel chunk is stored through the strided map of its phase
+      float* wpm = fa(static_cast<size_t>(NCH) * 4 * NCH * 9);
+      float* bpm = fa(NCH * 4);
+      float* spm = fa(NCH * 4);
+      if (!wpm || !bpm || !spm) return 1;
+      if (int e = phase_major_rows(c.w, wpm, NCH, NCH * 9, 0, st)) return e;
+      if (int e = phase_major_rows(c.bias, bpm, NCH, 1, 0, st)) return e;
+      if (int e = phase_major_rows(slope, spm, NCH, 1, 1, st)) return e;
+      for (int pass = 0; pass < (grad ? 2 : 1); ++pass) {   // pass 1 (with-grad plans): the pre-activation, without the PReLU
+        WeightSrc ws_; ws_.w = wpm; ws_.d0 = NCH * 4; ws_.d1 = NCH; ws_.KH = ws_.KW = 3;
         ConvGeom g; g.K = 3; g.pad = 1;
-        Epilogue ep; ep.bias = bq; ep.prelu = pass ? nullptr : slope;
-        OutSpec os; os.mode = kOutNHWC; os.out = pass ? ups[u].pre : up; os.up = 2; os.py = q / 2; os.px = q % 2;
+        Epilogue ep; ep.bias = bpm; ep.prelu = pass ? nullptr : spm;
+        OutSpec os; os.mode = kOutNHWC; os.out = pass ? ups[u].pre : up; os.up = 2; os.phases = 4; os.bn_max = 128;
         auto op = std::make_shared<ConvOp>();
-        if (int e = build_conv(op.get(), arena, cur, ws_, g, NCH, nullptr, nullptr, ep, os, st)) return e;
-        op->flops = 2.0 * cur.pixels() * (9.0 * NCH / 4.0 + static_cast<double>(NCH) * NCH);   // this phase's share
+        if (int e = build_conv(op.get(), arena, cur, ws_, g, NCH * 4, nullptr, nullptr, ep, os, st)) return e;
+        op->flops = 2.0 * cur.pixels() * (9.0 * NCH + static_cast<double>(NCH) * NCH * 4);
         for (auto& pl : op->plans) pl.flops = op->flops / op->plans.size();
         net->flops += op->flops;
         net->ops.push_back([op](cudaStream_t s) { return op->run(s); });
@@ -235,14 +212,10 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     cur = up; h *= 2; w *= 2;
   }
   // ---- final: depthwise 9x9 + pointwise 64->3 + (tanh + 1)/2, NCHW fp32 out
-  // WC_SRGAN_FINAL_TC (default 1): on the tensor core - a 1x9 horizontal convolution with N = (kernel row, output) = 27 columns
-  // into fp32 planes (igemm), then the vertical shift-add + bias + tanh (seg_kernels.cu: srgan_final_combine); 0: CUDA-core kernel
-  static int final_tc = -1;
-  if (final_tc < 0) {
-    const char* e = getenv("WC_SRGAN_FINAL_TC");
-    final_tc = e ? atoi(e) : 1;
-  }
-  const bool tc = final_tc && NCH == 64 && w % 4 == 0;
+  // On the tensor core where the output width is a multiple of 4: a 1x9 horizontal convolution with N = (kernel row, output) = 27
+  // columns into fp32 planes (igemm), then the vertical shift-add + bias + tanh (seg_kernels.cu: srgan_final_combine).  Otherwise
+  // (upscale 2 with an odd latent width) the CUDA-core kernel srgan_final.
+  const bool tc = NCH == 64 && w % 4 == 0;
   float* tplanes = tc ? static_cast<float*>(bump.take(static_cast<size_t>(B) * 27 * h * w * sizeof(float))) : nullptr;
   if (!dry) {
     const float *dw = P("final_conv.depthwise.weight"), *dwb = Popt("final_conv.depthwise.bias");

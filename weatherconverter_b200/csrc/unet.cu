@@ -35,16 +35,6 @@ int linear_rows(const float* in, int Bt, int dim, const float* w, const float* b
 
 namespace {
 
-// WC_ATTN_QPRESCALE (default 1): the QKV projection stores Q * log2(e)/sqrt(hd) and the attention kernels run with a unit scale
-bool q_prescale() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("WC_ATTN_QPRESCALE");
-    v = e ? (atoi(e) != 0) : 1;
-  }
-  return v != 0;
-}
-
 __global__ void add_vec_kernel(const float* a, const float* b, float* o, int n) {
   pdl_prologue();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -208,7 +198,7 @@ struct Builder {
       ConvGeom g; g.K = 1; g.stride = 1; g.pad = 0; g.dil = 1;
       Epilogue ep; ep.bias = P(ap + ".in_proj_bias");
       OutSpec os; os.mode = kOutQKV; os.q = q; os.k = k; os.vt = vt; os.heads = heads; os.hd = hd;
-      if (q_prescale()) os.q_scale = 1.4426950408889634f / sqrtf(static_cast<float>(hd));
+      os.q_scale = 1.4426950408889634f / sqrtf(static_cast<float>(hd));   // attention then runs with a unit log2-domain scale
       if (err) return out;
       auto op = std::make_shared<ConvOp>();
       if (int e = build_conv(op.get(), arena, a, w, g, 3 * C, nullptr, nullptr, ep, os, st)) { err = e; return out; }
@@ -218,7 +208,7 @@ struct Builder {
     {
       const int Bc = B;
       net->flops += attention_flops(B, heads, ntok, hd);
-      push([=](cudaStream_t s) { return attention_forward(q, k, vt, o.ptr, Bc, heads, ntok, hd, o.ld, s, nullptr, q_prescale() ? kAttnScalePrescaled : 0.f); });
+      push([=](cudaStream_t s) { return attention_forward(q, k, vt, o.ptr, Bc, heads, ntok, hd, o.ld, s, nullptr, kAttnScalePrescaled); });
     }
     conv(o, ap + ".out_proj", C, 1, 1, 0, P(ap + ".out_proj.bias"), nullptr, 0, &x, nullptr, "", out);
     return out;

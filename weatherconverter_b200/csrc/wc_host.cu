@@ -76,19 +76,6 @@ int prof_stop(double* ms, long long* count, double* work) {
   return 0;
 }
 
-bool pdl_enabled(int klass) {
-  // WC_PDL bit 0: light kernels, bit 1: tcgen05 kernels.  Default 2, measured on B200 (C3, batch 32, graph replay, ms/step):
-  // off 25.66, tcgen05 kernels only 25.38, light kernels only 25.97, both 26.04 - parked blocks of early-launched light kernels
-  // next to a running one-CTA-per-SM kernel cost more than the hidden launch gap; a tcgen05 kernel parked next to a light
-  // kernel hides its mbarrier / TMEM set-up.  At batch 1 (launch-bound) both bits help the eager loop: 6.53 -> 5.54 ms/step.
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("WC_PDL");
-    mode = e ? atoi(e) : 2;
-  }
-  return (mode >> klass) & 1;
-}
-
 int num_sms() {
   static int sms = 0;
   if (sms == 0) {

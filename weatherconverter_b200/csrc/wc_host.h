@@ -66,13 +66,16 @@ struct ProfScope {
 int num_sms();
 
 // ---- programmatic dependent launch (PDL) -----------------------------------------------------------------------------------
-// Every kernel of the library is launched through launch_k with cudaLaunchAttributeProgrammaticStreamSerialization set (unless
-// WC_PDL=0): the kernel may then be scheduled while its predecessor in the stream is still draining, and its set-up (block
-// scheduling, shared-memory carve-up, mbarrier init, TMEM allocation, tensor-map prefetch) overlaps the predecessor's tail.
+// Every kernel of the library is launched through launch_k.  Launches of tcgen05 kernels (KLASS 1) set
+// cudaLaunchAttributeProgrammaticStreamSerialization: the kernel may then be scheduled while its predecessor in the stream is still
+// draining, and its set-up (block scheduling, shared-memory carve-up, mbarrier init, TMEM allocation, tensor-map prefetch) overlaps
+// the predecessor's tail.  Light kernels (KLASS 0) are launched without it.  Measured on B200 (C3, batch 32, graph replay, ms/step):
+// no PDL 25.66, tcgen05 kernels only 25.38, light kernels only 25.97, both 26.04 - parked blocks of early-launched light kernels
+// next to a running one-CTA-per-SM kernel cost more than the hidden launch gap; a tcgen05 kernel parked next to a light kernel
+// hides its mbarrier / TMEM set-up.  (At batch 1, launch-bound, PDL on both classes helped the eager loop: 6.53 -> 5.54 ms/step.)
 // Contract: a kernel launched this way executes pdl_prologue() / pdl_wait() (griddepcontrol.wait) BEFORE its first access to
 // global memory that any earlier kernel may write or still read; griddepcontrol.launch_dependents lets its own successor in.
 // A step is ~440 back-to-back launches (~520 at batch 1), so the per-launch gap is what the small-batch regime is made of.
-bool pdl_enabled(int klass = 0);   // klass 0: light kernels (no TMEM / full-SM shared memory); 1: tcgen05 kernels (one CTA per SM)
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -80,7 +83,7 @@ __device__ __forceinline__ void pdl_prologue() {
   pdl_launch_dependents();
   pdl_wait();
 }
-template <int KLASS = 0, typename... KArgs, typename... Args>
+template <int KLASS = 0, typename... KArgs, typename... Args>   // KLASS 0: light kernels; 1: tcgen05 kernels (one CTA per SM)
 inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
@@ -91,7 +94,7 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled(KLASS) ? 1 : 0;
+  cfg.numAttrs = KLASS == 1 ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 #endif
