@@ -149,7 +149,7 @@ def main():
         "gsg_step_peak_extra_gib": {k: v / 2 ** 30 for k, v in step_peak.items()},
         "peak_note": "torch allocator peak during one call above what was allocated before it (plan workspaces allocated "
                      "during warm-up are not included); library launches count kernels of libwc_b200 only, not torch's CE",
-        "seg_fused_workspace_gib": sum(w.numel() for w in seg._ws.values()) / 2 ** 30,
+        "seg_fused_workspace_gib": seg._infer.plan.ws.numel() / 2 ** 30,
         "seg_autograd_workspace_gib": sum(p.ws.numel() for ps in seg._grad_plans.values() for p in ps) / 2 ** 30,
         "hbm_gib_resident_end": torch.cuda.memory_allocated() / 2 ** 30,
         "ms_all": {k: v for k, v in {**seg_ms, **step_ms}.items()},

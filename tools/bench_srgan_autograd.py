@@ -85,7 +85,7 @@ def main():
     y = torch.empty(B, 3, 4 * h, 4 * w, device=dev)
     dy = torch.randn(B, 3, 4 * h, 4 * w, generator=torch.Generator().manual_seed(1235)).to(dev) * 1e-3
     dx = torch.empty_like(x)
-    plan = G._lease_plan(B, h, w, x.device)
+    plan = G._grad_plan(B, h, w, x.device)
 
     def timed(fn):
         torch.cuda.synchronize()
@@ -181,7 +181,7 @@ def main():
         "gsg_step_pooled_ms": med["gsg_step_pooled"], "gsg_step_through_srgan_ms": med["gsg_step_through_srgan"],
         "gsg_step_through_over_pooled": med["gsg_step_through_srgan"] / med["gsg_step_pooled"],
         "gsg_step_library_launches": step_launches,
-        "nograd_workspace_gib": sum(t.numel() for t in G._ws.values()) / 2 ** 30,
+        "nograd_workspace_gib": G._infer.plan.ws.numel() / 2 ** 30,
         "grad_plan_workspace_gib": grad_ws / 2 ** 30,
         "grad_plans": sum(len(ps) for ps in G._grad_plans.values()),
         "hbm_gib_resident_end": torch.cuda.memory_allocated() / 2 ** 30,

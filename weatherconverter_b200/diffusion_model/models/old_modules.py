@@ -4,9 +4,8 @@
 sample_integrated.py:60 passes) and returns the predicted noise [B,3,128,128].  ``state_dict()`` has the reference's key
 names, shapes and buffers (BatchNorm running statistics), so reference checkpoints load with ``load_state_dict``.
 Inference only (eval-mode BatchNorm, as load_model at sample_integrated.py:70-75 sets up); the layer graph and all
-arithmetic live in csrc/legacy.cu.
+arithmetic live in csrc/legacy.cu, and the C handle and its workspace are held through ``_plans.py``.
 """
-import ctypes as C
 import math
 
 import torch
@@ -14,6 +13,7 @@ import torch.nn as nn
 
 from ... import _lib
 from ..._lib import check, lib, ptr, stream_ptr
+from ..._plans import PlanHandle, PlanPool, c_tensor_args
 from .unet_base import _Node
 
 DEPTH = 3
@@ -106,7 +106,7 @@ class UNet(nn.Module):
                 self._register(name, t, buffer=True)
             else:
                 self._register(name, nn.Parameter(t))
-        self._handle, self._handle_key, self._keep, self._ws = None, None, None, {}
+        self._infer = PlanPool()
 
     def _register(self, dotted, tensor, buffer=False):
         node = self
@@ -140,40 +140,20 @@ class UNet(nn.Module):
         wop[:, :, :hd] = wo.view(Cc, heads, hd)
         return wp.reshape(3 * heads * hdp, Cc).contiguous(), bp.reshape(-1).contiguous(), wop.reshape(Cc, heads * hdp).contiguous()
 
-    def _destroy(self):
-        if self._handle is not None:
-            lib().wc_legacy_unet_destroy(self._handle)
-            self._handle = None
-
-    def __del__(self):
-        try:
-            self._destroy()
-        except Exception:
-            pass
-
-    def _ensure_handle(self, device):
+    def _inference_plan(self, device):
         sd = {k: v for k, v in self.state_dict().items() if v.dtype == torch.float32}
         key = (str(device), tuple((v.data_ptr(), v._version) for v in sd.values()))
-        if self._handle is not None and key == self._handle_key:
-            return
-        self._destroy()
-        tensors = {}
-        for k, v in sd.items():
-            if v.device != device:
-                raise RuntimeError(f"UNet tensor {k} is on {v.device}, expected {device}; call .to(device)")
-            tensors[k] = v.detach().contiguous()
+        return self._infer.one(key, lambda: self._make_inference_plan(sd, device))
+
+    def _make_inference_plan(self, sd, device):
+        tensors = {k: v.detach().contiguous() for k, v in sd.items()}
         for prefix, Cc in (("attn_down3", 64), ("attn_down4", 96), ("attn_bottleneck", 256), ("attn_up1", 128), ("attn_up2", 96)):
             w, b, wo = self._pad_attention(tensors, prefix, Cc)
             tensors[prefix + ".mha.in_proj_weight"], tensors[prefix + ".mha.in_proj_bias"] = w, b
             tensors[prefix + ".mha.out_proj.weight"] = wo
-        names = list(tensors)
-        n = len(names)
-        c_names = (C.c_char_p * n)(*[s.encode() for s in names])
-        c_ptrs = (C.c_void_p * n)(*[tensors[s].data_ptr() for s in names])
-        c_numels = (C.c_int64 * n)(*[tensors[s].numel() for s in names])
-        handle = C.c_void_p()
-        check(lib().wc_legacy_unet_create(C.byref(handle), n, c_names, c_ptrs, c_numels))
-        self._handle, self._handle_key, self._keep, self._ws = handle, key, tensors, {}
+        names, ptrs, numels = c_tensor_args(tensors, device, "UNet")
+        L = lib()
+        return PlanHandle(L.wc_legacy_unet_create, L.wc_legacy_unet_destroy, len(tensors), names, ptrs, numels, keep=tensors)
 
     def forward(self, x, t, out=None):
         _lib.require_cuda(x)
@@ -186,22 +166,18 @@ class UNet(nn.Module):
             t = t.expand(B).contiguous()
         if t.numel() != B:
             raise RuntimeError("t must have one entry per sample")
-        self._ensure_handle(x.device)
-        ws = self._ws.get(B)
-        if ws is None:
-            nbytes = lib().wc_legacy_unet_workspace_bytes(self._handle, B, H)
-            if nbytes == 0:
-                check(1)
-            self._ws = {B: torch.empty(nbytes, dtype=torch.uint8, device=x.device)}
-            ws = self._ws[B]
+        plan = self._inference_plan(x.device)
+        ws = plan.workspace(B, lambda: lib().wc_legacy_unet_workspace_bytes(plan.handle, B, H), x.device)
         if out is None:
             out = torch.empty_like(x)
-        check(lib().wc_legacy_unet_forward(self._handle, ptr(x), ptr(t), ptr(out), B, H, ptr(ws), ws.numel(), stream_ptr()))
+        check(lib().wc_legacy_unet_forward(plan.handle, ptr(x), ptr(t), ptr(out), B, H, ptr(ws), ws.numel(), stream_ptr()))
         self._last_io = (x, t)
         return out
 
     def flops_per_forward(self):
-        return float(lib().wc_legacy_unet_flops(self._handle)) if self._handle is not None else 0.0
+        plan = self._infer.plan
+        return float(lib().wc_legacy_unet_flops(plan.handle)) if plan is not None else 0.0
 
     def launches_per_forward(self):
-        return int(lib().wc_legacy_unet_launches(self._handle)) if self._handle is not None else 0
+        plan = self._infer.plan
+        return int(lib().wc_legacy_unet_launches(plan.handle)) if plan is not None else 0

@@ -5,10 +5,11 @@
 names and shapes (382 tensors for config.yaml), so reference checkpoints load with ``load_state_dict``.
 
 The module only owns parameters and device buffers; the layer graph, weight re-packing (bf16, K-major) and all
-arithmetic live in the C library (csrc/unet.cu).  By default outputs carry no autograd graph.
+arithmetic live in the C library (csrc/unet.cu), and the C handles, their workspaces and the plan pool are held through
+``_plans.py``.  By default outputs carry no autograd graph.
 
 Autograd (opt-in): with ``model.differentiable = True``, grad mode on and ``x`` or any parameter requiring grad,
-``forward`` runs the training plan (csrc/unet_train.cu) under a ``torch.autograd.Function`` whose inputs are ``x``,
+``forward`` runs the training plan (csrc/unet_train.cu) under ``_plans.PlanFunction`` whose inputs are ``x``,
 ``t`` and every parameter, so ``loss.backward()`` with any loss, hooks, ``clip_grad_norm_``, gradient accumulation
 and any ``torch.optim`` optimizer work as on the reference module; ``x.grad`` is dL/dx.  The backward is
 ``wc_unet_train_backward_seeded`` fed with dL/d(noise_pred); it skips the parameter-gradient launches when no
@@ -22,11 +23,10 @@ import math
 
 import torch
 import torch.nn as nn
-from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from ..._lib import UnetConfigStruct, check, lib, ptr, stream_ptr
-from ..._plans import Lease, lease_plan
+from ..._plans import PlanFunction, PlanHandle, PlanPool, c_tensor_args
 
 
 def _cfg_get(cfg, k):
@@ -143,14 +143,10 @@ class Unet(nn.Module):
                     fan_in *= s
                 init = torch.empty(shape).uniform_(-1.0 / math.sqrt(fan_in), 1.0 / math.sqrt(fan_in))
             self._register(name, nn.Parameter(init))
-        self._handle = None
-        self._handle_key = None
-        self._workspaces = {}
-        self._keepalive = None
+        self._infer = PlanPool()      # the inference plan
         self._weights_epoch = 0      # bumped by DenoisingTrainer.optimizer_step (in-place kernel updates of the weights)
         self.differentiable = False  # True: forward under grad mode builds an autograd graph (module docstring)
-        self._train_plans = {}       # (B, H, W) -> [_TrainPlan]: the autograd path's plan pool
-        self._train_key = None
+        self._train_plans = PlanPool()   # (B, H, W) -> training plans: the autograd path's plan pool
 
     def _register(self, dotted, param):
         node = self
@@ -180,65 +176,47 @@ class Unet(nn.Module):
             c.attn_resolutions[i] = v
         return c
 
-    def _destroy(self):
-        if self._handle is not None:
-            lib().wc_unet_destroy(self._handle)
-            self._handle = None
-
-    def __del__(self):
-        try:
-            self._destroy()
-        except Exception:
-            pass
-
-    def _ensure_handle(self, device):
+    def _inference_plan(self, device):
         params = dict(self.named_parameters())
         key = (str(device), self._weights_epoch, tuple((p.data_ptr(), p._version) for p in params.values()))
-        if self._handle is not None and key == self._handle_key:
-            return
-        self._destroy()
-        names, tensors = [], []
-        for n, p in params.items():
-            if p.device != device or p.dtype != torch.float32 or not p.is_contiguous():
-                raise RuntimeError(f"Unet parameter {n} must be a contiguous fp32 tensor on {device}; call .to(device)")
-            names.append(n.encode())
-            tensors.append(p.detach())
-        n = len(names)
-        c_names = (C.c_char_p * n)(*names)
-        c_ptrs = (C.c_void_p * n)(*[t.data_ptr() for t in tensors])
-        c_numels = (C.c_int64 * n)(*[t.numel() for t in tensors])
-        handle = C.c_void_p()
+        return self._infer.one(key, lambda: self._make_inference_plan(params, device))
+
+    def _make_inference_plan(self, params, device):
+        tensors = {n: p.detach() for n, p in params.items()}
+        names, ptrs, numels = c_tensor_args(tensors, device, "Unet", torch.float32)
         cfg = self._config_struct()
         set_time_factor_table(self.t_emb_dim, device)
-        check(lib().wc_unet_create(C.byref(handle), C.byref(cfg), n, c_names, c_ptrs, c_numels, stream_ptr()))
-        self._handle, self._handle_key, self._keepalive = handle, key, tensors
-        self._workspaces = {}
+        L = lib()
+        return PlanHandle(L.wc_unet_create, L.wc_unet_destroy, C.byref(cfg), len(tensors), names, ptrs, numels, stream_ptr(),
+                          keep=tensors)
 
-    def _workspace(self, B, H, W, device):
-        k = (B, H, W)
-        ws = self._workspaces.get(k)
-        if ws is None:
-            nbytes = lib().wc_unet_workspace_bytes(self._handle, B, H, W)
-            if nbytes == 0:
-                check(1)
-            self._workspaces = {}        # one live binding at a time: the C plan is bound to one workspace
-            ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
-            self._workspaces[k] = ws
-        return ws
-
-    def _lease_plan(self, B, H, W, device):
-        """A free training plan for (B, H, W), created when every plan of that shape is held by a live graph.  The pool is
-        rebuilt when a parameter's storage changes (.to(), load_state_dict with new tensors); in-place updates of the
-        weights need no rebuild because every differentiable forward re-packs them."""
+    def _grad_plan(self, B, H, W, device):
+        """A free training plan for (B, H, W), created when every plan of that shape is held by a live graph.  Each plan has
+        its own workspace and flat fp32 gradient buffer (every tensor's slice 16-byte aligned, as in DenoisingTrainer); it
+        reads the module's parameters in place (the backward reads GroupNorm and t-embedding weights)."""
         named = list(self.named_parameters())
         key = (str(device), tuple(p.data_ptr() for _, p in named))
-        if key != self._train_key:
-            for n, p in named:
-                if p.device != device or p.dtype != torch.float32 or not p.is_contiguous():
-                    raise RuntimeError(f"Unet parameter {n} must be a contiguous fp32 tensor on {device}; call .to(device)")
-            set_time_factor_table(self.t_emb_dim, device)
-            self._train_plans, self._train_key = {}, key
-        return lease_plan(self._train_plans, (B, H, W), lambda: _TrainPlan(self._config_struct(), named, B, H, W, device))
+        return self._train_plans.lease(key, (B, H, W), lambda: self._make_train_plan(named, B, H, W, device))
+
+    def _make_train_plan(self, named, B, H, W, device):
+        params = {n: p.detach() for n, p in named}
+        names, pp, _ = c_tensor_args(params, device, "Unet", torch.float32)
+        set_time_factor_table(self.t_emb_dim, device)
+        slices, off = [], 0
+        for p in params.values():
+            off = (off + 3) & ~3
+            slices.append((off, p.numel(), p.shape))
+            off += p.numel()
+        grads = torch.zeros(off, device=device, dtype=torch.float32)
+        _, gp, _ = c_tensor_args({n: grads[o:o + k] for n, (o, k, _) in zip(params, slices)}, device, "Unet gradient")
+        cfg = self._config_struct()
+        L = lib()
+        plan = PlanHandle(L.wc_unet_train_create, L.wc_unet_train_destroy, C.byref(cfg), len(params), names, pp, gp,
+                          keep=(params, grads))
+        plan.grads, plan.slices = grads, slices
+        ws = plan.workspace((B, H, W), lambda: L.wc_unet_train_workspace_bytes(plan.handle, B, H, W), device)
+        check(L.wc_unet_train_bind(plan.handle, B, H, W, ptr(ws), ws.numel(), stream_ptr()))
+        return plan
 
     # ---- reference API ---------------------------------------------------------------------------------
     def forward(self, x, t, out=None):
@@ -256,85 +234,35 @@ class Unet(nn.Module):
                 if out is not None:
                     raise RuntimeError("Unet.forward: out= cannot be combined with the autograd path "
                                        "(differentiable = True under grad mode)")
-                return _UnetTrainFunction.apply(self, x, t.expand(B).contiguous(), *params)
-        self._ensure_handle(x.device)
-        ws = self._workspace(B, H, W, x.device)
+                return PlanFunction.apply(self, x, t.expand(B).contiguous(), *params)
+        plan = self._inference_plan(x.device)
+        ws = plan.workspace((B, H, W), lambda: lib().wc_unet_workspace_bytes(plan.handle, B, H, W), x.device)
         if out is None:
             out = torch.empty_like(x)
-        check(lib().wc_unet_forward(self._handle, ptr(x), ptr(t), t.numel(), ptr(out), B, H, W, ptr(ws), ws.numel(),
+        check(lib().wc_unet_forward(plan.handle, ptr(x), ptr(t), t.numel(), ptr(out), B, H, W, ptr(ws), ws.numel(),
                                     stream_ptr()))
         self._last_io = (x, t)   # keep inputs alive until the stream has consumed them
         return out
 
     def flops_per_forward(self) -> float:
         """Algorithmic FLOPs (2*MAC) of the last bound forward."""
-        return float(lib().wc_unet_flops(self._handle)) if self._handle is not None else 0.0
+        plan = self._infer.plan
+        return float(lib().wc_unet_flops(plan.handle)) if plan is not None else 0.0
 
     def launches_per_forward(self) -> int:
-        return int(lib().wc_unet_launches(self._handle)) if self._handle is not None else 0
+        plan = self._infer.plan
+        return int(lib().wc_unet_launches(plan.handle)) if plan is not None else 0
 
-
-class _TrainPlan:
-    """One training plan of the C library bound to (B, H, W) with its own workspace and flat fp32 gradient buffer (every
-    tensor's slice 16-byte aligned, as in DenoisingTrainer).  Its parameter pointers are the module's parameters, kept
-    alive here because the backward reads GroupNorm and t-embedding weights in place."""
-
-    def __init__(self, cfg, named, B, H, W, device):
-        self.handle, self.busy = None, False
-        self.slices, off = [], 0
-        for _, p in named:
-            off = (off + 3) & ~3
-            self.slices.append((off, p.numel(), p.shape))
-            off += p.numel()
-        self.grads = torch.zeros(off, device=device, dtype=torch.float32)
-        self._params = [p.detach() for _, p in named]
-        n = len(named)
-        c_names = (C.c_char_p * n)(*[name.encode() for name, _ in named])
-        pp = (C.c_void_p * n)(*[p.data_ptr() for p in self._params])
-        gp = (C.c_void_p * n)(*[self.grads.data_ptr() + 4 * o for o, _, _ in self.slices])
-        L, handle = lib(), C.c_void_p()
-        check(L.wc_unet_train_create(C.byref(handle), C.byref(cfg), n, c_names, pp, gp))
-        self.handle = handle
-        nbytes = L.wc_unet_train_workspace_bytes(handle, B, H, W)
-        if nbytes == 0:
-            check(1)
-        self.ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
-        check(L.wc_unet_train_bind(handle, B, H, W, ptr(self.ws), self.ws.numel(), stream_ptr()))
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                lib().wc_unet_train_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
-
-
-class _UnetTrainFunction(torch.autograd.Function):
-    """pred = Unet(x, t) on a leased training plan; backward seeded with dL/dpred.  Inputs: the module, x [B,3,H,W] fp32,
-    t int64 [B], then every parameter in ``named_parameters()`` order."""
-
-    @staticmethod
-    def forward(ctx, unet, x, t, *params):
-        B, _, H, W = x.shape
-        lease = Lease(unet._lease_plan(B, H, W, x.device), x, t)
+    # ---- the autograd path (PlanFunction): inputs x [B,3,H,W] fp32, t int64 [B], then every parameter in
+    # named_parameters() order
+    def _grad_forward(self, plan, x, t, *params):
         pred = torch.empty_like(x)
-        check(lib().wc_unet_train_forward(lease.plan.handle, ptr(x), ptr(t), None, ptr(pred), None, 1.0, 1, stream_ptr()))
-        ctx.lease = lease
+        check(lib().wc_unet_train_forward(plan.handle, ptr(x), ptr(t), None, ptr(pred), None, 1.0, 1, stream_ptr()))
         return pred
 
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_pred):
-        lease = ctx.lease
-        plan = lease.plan
-        if plan is None:
-            raise RuntimeError("Unet autograd: this graph has already been backpropagated; its saved activations are gone "
-                               "(retain_graph=True re-backward is not supported: run the forward again)")
-        x = lease.inputs[0]
-        g = grad_pred.contiguous().float()
-        dx = torch.empty_like(x) if ctx.needs_input_grad[1] else None
-        need = ctx.needs_input_grad[3:]
+    def _grad_backward(self, plan, g, needs_input_grad, x, t, *params):
+        dx = torch.empty_like(x) if needs_input_grad[0] else None
+        need = needs_input_grad[2:]
         param_grads = any(need)
         check(lib().wc_unet_train_backward_seeded(plan.handle, ptr(g), ptr(dx), int(param_grads), stream_ptr()))
         grads = [None] * len(need)
@@ -343,8 +271,7 @@ class _UnetTrainFunction(torch.autograd.Function):
             # next backward
             flat = plan.grads.clone()
             grads = [flat[o:o + n].view(shape) if nd else None for (o, n, shape), nd in zip(plan.slices, need)]
-        lease.release()
-        return (None, dx, None, *grads)
+        return (dx, None, *grads)
 
 
 _FACTOR_SET = {}

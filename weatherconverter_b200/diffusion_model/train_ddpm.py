@@ -21,6 +21,7 @@ import torch.distributed as dist
 
 from .. import _lib
 from .._lib import check, lib, ptr, stream_ptr
+from .._plans import PlanHandle, c_tensor_args
 from .models.unet_base import Unet
 
 device = torch.device("cuda" if torch.cuda.is_available() else "cpu")
@@ -82,7 +83,7 @@ def backward_with_buckets(run_ops, n_ops, flat_grads, buckets, world, group=None
 
 class DenoisingTrainer:
     """Owns flat fp32 parameter / gradient / Adam-moment buffers (the model's parameters become views into the flat
-    parameter buffer) and the C training plan bound to one (batch, H, W)."""
+    parameter buffer) and the C training plan bound to one (batch, H, W), held as a ``_plans.PlanHandle``."""
 
     def __init__(self, model: Unet, scheduler, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, process_group=None,
                  bucket_bytes=64 << 20, seed=None, data_parallel=True):
@@ -125,9 +126,8 @@ class DenoisingTrainer:
             off += n
         self.used = off
         self.names = [named[i][0] for i in order]
-        self._handle = None
+        self._plan = None            # PlanHandle of the training plan, made by the first _bind
         self._bound = None
-        self._ws = None
         self._buckets = []
         self._keep = None
         self.loss = torch.zeros(1, device=dev, dtype=torch.float32)
@@ -175,36 +175,25 @@ class DenoisingTrainer:
             self.step_count = steps.pop()
         return restored
 
-    def __del__(self):
-        try:
-            if self._handle is not None:
-                lib().wc_unet_train_destroy(self._handle)
-        except Exception:
-            pass
-
     def _bind(self, B, H, W):
         if self._bound == (B, H, W):
             return
-        L = lib()
-        if self._handle is None:
-            n = len(self.names)
-            c_names = (C.c_char_p * n)(*[s.encode() for s in self.names])
-            pp = (C.c_void_p * n)(*[self.flat_params.data_ptr() + 4 * self.slices[s][0] for s in self.names])
-            gp = (C.c_void_p * n)(*[self.flat_grads.data_ptr() + 4 * self.slices[s][0] for s in self.names])
-            handle = C.c_void_p()
+        L, dev = lib(), self.flat_params.device
+        if self._plan is None:
+            params = {s: self.flat_params[o:o + n] for s, (o, n) in self.slices.items()}     # in self.names order
+            grads = {s: self.flat_grads[o:o + n] for s, (o, n) in self.slices.items()}
+            c_names, pp, _ = c_tensor_args(params, dev, "DenoisingTrainer")
+            _, gp, _ = c_tensor_args(grads, dev, "DenoisingTrainer")
             cfg = self.model._config_struct()
-            check(L.wc_unet_train_create(C.byref(handle), C.byref(cfg), n, c_names, pp, gp))
-            self._handle = handle
-        nbytes = L.wc_unet_train_workspace_bytes(self._handle, B, H, W)
-        if nbytes == 0:
-            check(1)
-        self._ws = None
-        self._ws = torch.empty(nbytes, dtype=torch.uint8, device=self.flat_params.device)
-        check(L.wc_unet_train_bind(self._handle, B, H, W, ptr(self._ws), self._ws.numel(), stream_ptr()))
+            self._plan = PlanHandle(L.wc_unet_train_create, L.wc_unet_train_destroy, C.byref(cfg), len(self.names), c_names,
+                                    pp, gp, keep=(self.flat_params, self.flat_grads))
+        handle = self._plan.handle
+        ws = self._plan.workspace((B, H, W), lambda: L.wc_unet_train_workspace_bytes(handle, B, H, W), dev)
+        check(L.wc_unet_train_bind(handle, B, H, W, ptr(ws), ws.numel(), stream_ptr()))
         self._bound = (B, H, W)
         # ---- gradient buckets: contiguous slices of the flat buffer, closed when the backward plan is done with them
-        n_ops = L.wc_unet_train_num_backward_ops(self._handle)
-        ready = [L.wc_unet_train_grad_ready_op(self._handle, s.encode()) for s in self.names]
+        n_ops = L.wc_unet_train_num_backward_ops(handle)
+        ready = [L.wc_unet_train_grad_ready_op(handle, s.encode()) for s in self.names]
         if min(ready) < 0:
             raise RuntimeError("internal: a parameter has no gradient producer: " + self.names[ready.index(min(ready))])
         self._buckets = make_buckets(self.names, self.slices, self.groups, ready, n_ops, self.used, self.bucket_bytes)
@@ -212,8 +201,8 @@ class DenoisingTrainer:
 
     @property
     def flops_per_step(self):
-        L = lib()
-        return float(L.wc_unet_train_flops(self._handle, 0) + L.wc_unet_train_flops(self._handle, 1)) if self._handle else 0.0
+        L, plan = lib(), self._plan
+        return float(L.wc_unet_train_flops(plan.handle, 0) + L.wc_unet_train_flops(plan.handle, 1)) if plan else 0.0
 
     def forward_backward(self, noisy, t, target, pred_out=None):
         """loss (device scalar) and all gradients for pred = model(noisy, t), loss = MSE(pred, target)."""
@@ -224,9 +213,9 @@ class DenoisingTrainer:
         if t.numel() != B:
             raise RuntimeError("training needs one timestep per sample")
         self._bind(B, H, W)
-        L, st = lib(), stream_ptr()
-        check(L.wc_unet_train_forward(self._handle, ptr(noisy), ptr(t), ptr(target), ptr(pred_out), ptr(self.loss), 1.0, 1, st))
-        backward_with_buckets(lambda a, b: check(L.wc_unet_train_backward(self._handle, a, b, st)), self._n_bwd_ops,
+        L, st, handle = lib(), stream_ptr(), self._plan.handle
+        check(L.wc_unet_train_forward(handle, ptr(noisy), ptr(t), ptr(target), ptr(pred_out), ptr(self.loss), 1.0, 1, st))
+        backward_with_buckets(lambda a, b: check(L.wc_unet_train_backward(handle, a, b, st)), self._n_bwd_ops,
                               self.flat_grads, self._buckets, self.world, self.group)
         self._keep = (noisy, t, target, pred_out)
         return self.loss

@@ -7,6 +7,7 @@ function of ``x`` only: the parameters are constants, no weight gradient is comp
 (eval-mode BatchNorm is folded into the convolutions; segmentor training is not supported).  The backward is the plan's
 data-gradient pass seeded with dL/dlogits (``wc_seg_backward_seeded``).  A graph holds one plan (its saved activations)
 until its backward has run or it is freed; the plans live in a pool per (B, H, W).  A graph can be backpropagated once.
+The handles, workspaces, pool and autograd Function are those of ``_plans.py``.
 
 Only the ResNet-50/101 DeepLabV3+ variants reachable from the reference's configured model name are provided
 (SURVEY.md section 2, rows 10-12); output_stride 16 (the reference's config, seg_model/config/config.yaml:66).
@@ -17,12 +18,11 @@ import math
 
 import torch
 import torch.nn as nn
-from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from ..._lib import check, lib, ptr, stream_ptr
 from ..._params import register_dotted
-from ..._plans import Lease, lease_plan
+from ..._plans import PlanFunction, PlanHandle, PlanPool, c_tensor_args
 
 __all__ = ["deeplabv3plus_resnet50", "deeplabv3plus_resnet101", "DeepLabV3"]
 
@@ -94,12 +94,8 @@ class DeepLabV3(nn.Module):
                 register_dotted(self, name, torch.ones(shape), buffer=True)
             else:
                 register_dotted(self, name, torch.zeros(shape, dtype=torch.long), buffer=True)
-        self._handle = None
-        self._key = None
-        self._ws = {}
-        self._keep = None
-        self._grad_plans = {}        # (B, H, W) -> [_SegGradPlan]: the autograd path's plan pool
-        self._grad_key = None
+        self._infer = PlanPool()
+        self._grad_plans = PlanPool()    # (B, H, W) -> plans with a with-grad workspace: the autograd path's plan pool
 
     # ---- C handle --------------------------------------------------------------------------------------
     def _tensors(self):
@@ -111,57 +107,35 @@ class DeepLabV3(nn.Module):
                 sd[n] = b
         return sd
 
-    def _destroy(self):
-        if self._handle is not None:
-            lib().wc_seg_destroy(self._handle)
-            self._handle = None
-
-    def __del__(self):
-        try:
-            self._destroy()
-        except Exception:
-            pass
-
-    def _create_handle(self, ts, device):
-        for n, t in ts.items():
-            if t.device != device or not t.is_contiguous():
-                raise RuntimeError(f"seg parameter {n} must be contiguous on {device}; call .to(device)")
-        n = len(ts)
-        names = (C.c_char_p * n)(*[k.encode() for k in ts])
-        ptrs = (C.c_void_p * n)(*[t.data_ptr() for t in ts.values()])
+    def _make_plan(self, ts, device):
+        names, ptrs, _ = c_tensor_args(ts, device, "seg")
         layers = (C.c_int * 4)(*_LAYERS[self.backbone_name])
-        h = C.c_void_p()
-        check(lib().wc_seg_create(C.byref(h), layers, self.num_classes, n, names, ptrs, stream_ptr()))
-        check(lib().wc_seg_set_output_stride(h, self.output_stride))
-        return h
+        L = lib()
+        plan = PlanHandle(L.wc_seg_create, L.wc_seg_destroy, layers, self.num_classes, len(ts), names, ptrs, stream_ptr(),
+                          keep=list(ts.values()))
+        check(L.wc_seg_set_output_stride(plan.handle, self.output_stride))
+        return plan
 
-    def _ensure(self, device):
+    def _inference_plan(self, device):
         ts = self._tensors()
         key = (str(device), tuple((t.data_ptr(), t._version) for t in ts.values()))
-        if self._handle is not None and key == self._key:
-            return
-        self._destroy()
-        h = self._create_handle(ts, device)
-        self._handle, self._key, self._keep, self._ws = h, key, list(ts.values()), {}
+        return self._infer.one(key, lambda: self._make_plan(ts, device))
 
-    def _lease_plan(self, B, H, W, device):
-        """A free autograd plan for (B, H, W), created when every plan of that shape is held by a live graph.  A plan packs
-        the weights once, when it is first bound, so the pool is rebuilt whenever a tensor's storage or version changes
-        (.to(), load_state_dict, any in-place update); a live graph keeps its own plan."""
+    def _grad_plan(self, B, H, W, device):
+        """A free autograd plan for (B, H, W) with a with-grad workspace, created when every plan of that shape is held by a
+        live graph.  Its first forward binds it and packs the weights."""
         ts = self._tensors()
         key = (str(device), self.output_stride, tuple((t.data_ptr(), t._version) for t in ts.values()))
-        if key != self._grad_key:
-            self._grad_plans, self._grad_key = {}, key
-        return lease_plan(self._grad_plans, (B, H, W), lambda: _SegGradPlan(self, ts, B, H, W, device))
 
-    def _workspace(self, B, H, W, with_grad, device):
-        k = (B, H, W, with_grad)
-        if k not in self._ws:
-            nbytes = lib().wc_seg_workspace_bytes(self._handle, B, H, W, 1 if with_grad else 0)
-            if nbytes == 0:
-                check(1)
-            self._ws = {k: torch.empty(nbytes, dtype=torch.uint8, device=device)}
-        return self._ws[k]
+        def make():
+            plan = self._make_plan(ts, device)
+            plan.workspace((B, H, W), lambda: lib().wc_seg_workspace_bytes(plan.handle, B, H, W, 1), device)
+            return plan
+        return self._grad_plans.lease(key, (B, H, W), make)
+
+    def _workspace(self, plan, B, H, W, with_grad, device):
+        return plan.workspace((B, H, W, with_grad),
+                              lambda: lib().wc_seg_workspace_bytes(plan.handle, B, H, W, 1 if with_grad else 0), device)
 
     def infer(self, x, labels, want_grad=True, want_logits=False, grad_pool=1):
         """Forward + argmax + per-image CE(ignore 255) + input gradient in one stream-ordered plan.
@@ -173,13 +147,13 @@ class DeepLabV3(nn.Module):
         x = x.contiguous().float()
         labels = labels.contiguous().long()
         B, _, H, W = x.shape
-        self._ensure(x.device)
-        ws = self._workspace(B, H, W, want_grad, x.device)
+        plan = self._inference_plan(x.device)
+        ws = self._workspace(plan, B, H, W, want_grad, x.device)
         pred = torch.empty(B, H, W, dtype=torch.long, device=x.device)
         grad = torch.empty(B, 3, H // grad_pool, W // grad_pool, device=x.device) if want_grad else None
         loss = torch.empty(B, dtype=torch.float32, device=x.device)
         logits = torch.empty(B, self.num_classes, H, W, device=x.device) if want_logits else None
-        check(lib().wc_seg_infer_pooled(self._handle, ptr(x), ptr(labels), ptr(pred), ptr(grad), ptr(loss), ptr(logits), B, H, W,
+        check(lib().wc_seg_infer_pooled(plan.handle, ptr(x), ptr(labels), ptr(pred), ptr(grad), ptr(loss), ptr(logits), B, H, W,
                                         int(grad_pool), ptr(ws), ws.numel(), stream_ptr()))
         self._last = (x, labels)
         return dict(pred=pred, grad=grad, loss=loss, logits=logits)
@@ -191,8 +165,7 @@ class DeepLabV3(nn.Module):
         replica."""
         import copy
         r = copy.copy(self)          # shares _parameters / _buffers (no new tensors)
-        r._handle, r._key, r._ws, r._keep = None, None, {}, None
-        r._grad_plans, r._grad_key = {}, None
+        r._infer, r._grad_plans = PlanPool(), PlanPool()
         return r
 
     def forward(self, x):
@@ -202,70 +175,32 @@ class DeepLabV3(nn.Module):
         if self.training:
             raise RuntimeError("the B200 DeepLabV3+ path implements eval-mode BatchNorm only; call .eval()")
         if torch.is_grad_enabled() and x.requires_grad:
-            return _SegFunction.apply(self, x.contiguous().float())
+            return PlanFunction.apply(self, x.contiguous().float())
         x = x.contiguous().float()
         B, _, H, W = x.shape
-        self._ensure(x.device)
-        ws = self._workspace(B, H, W, False, x.device)
+        plan = self._inference_plan(x.device)
+        ws = self._workspace(plan, B, H, W, False, x.device)
         logits = torch.empty(B, self.num_classes, H, W, device=x.device)
-        check(lib().wc_seg_forward(self._handle, ptr(x), ptr(logits), B, H, W, 0, ptr(ws), ws.numel(), stream_ptr()))
+        check(lib().wc_seg_forward(plan.handle, ptr(x), ptr(logits), B, H, W, 0, ptr(ws), ws.numel(), stream_ptr()))
         self._last = (x,)
         return logits
 
     def flops(self):
-        return (float(lib().wc_seg_flops(self._handle, 0)), float(lib().wc_seg_flops(self._handle, 1)))
+        plan = self._infer.plan
+        handle = plan.handle if plan is not None else None
+        return (float(lib().wc_seg_flops(handle, 0)), float(lib().wc_seg_flops(handle, 1)))
 
-
-class _SegGradPlan:
-    """A C handle of its own with a with-grad workspace, bound to (B, H, W) by its first forward (which packs the weights).
-    Keeps the module's tensors alive: the handle reads them in place."""
-
-    def __init__(self, seg, ts, B, H, W, device):
-        self.handle, self.busy = None, False
-        self._keep = list(ts.values())
-        self.handle = seg._create_handle(ts, device)
-        nbytes = lib().wc_seg_workspace_bytes(self.handle, B, H, W, 1)
-        if nbytes == 0:
-            check(1)
-        self.ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
-
-    def __del__(self):
-        try:
-            if self.handle is not None:
-                lib().wc_seg_destroy(self.handle)
-                self.handle = None
-        except Exception:
-            pass
-
-
-class _SegFunction(torch.autograd.Function):
-    """logits = DeepLabV3(x) on a leased plan that saves its activations; backward seeded with dL/dlogits gives dL/dx.
-    Inputs: the module, x [B,3,H,W] fp32 contiguous."""
-
-    @staticmethod
-    def forward(ctx, seg, x):
+    # ---- the autograd path (PlanFunction): the plan saves its activations; the backward seeded with dL/dlogits gives dL/dx
+    def _grad_forward(self, plan, x):
         B, _, H, W = x.shape
-        lease = Lease(seg._lease_plan(B, H, W, x.device), x)
-        plan = lease.plan
-        logits = torch.empty(B, seg.num_classes, H, W, device=x.device)
+        logits = torch.empty(B, self.num_classes, H, W, device=x.device)
         check(lib().wc_seg_forward(plan.handle, ptr(x), ptr(logits), B, H, W, 1, ptr(plan.ws), plan.ws.numel(), stream_ptr()))
-        ctx.lease = lease
         return logits
 
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, grad_logits):
-        lease = ctx.lease
-        plan = lease.plan
-        if plan is None:
-            raise RuntimeError("DeepLabV3 autograd: this graph has already been backpropagated; its saved activations are gone "
-                               "(retain_graph=True re-backward is not supported: run the forward again)")
-        x = lease.inputs[0]
-        g = grad_logits.contiguous().float()
+    def _grad_backward(self, plan, g, needs_input_grad, x):
         dx = torch.empty_like(x)
         check(lib().wc_seg_backward_seeded(plan.handle, ptr(g), ptr(dx), stream_ptr()))
-        lease.release()
-        return None, dx
+        return (dx,)
 
 
 def _build(backbone, num_classes, output_stride, pretrained_backbone):
