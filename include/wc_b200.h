@@ -223,7 +223,8 @@ typedef struct {
   int n_attn_resolutions;
   int attn_resolutions[8];
 } wc_unet_config;
-/* names/ptrs: the reference state_dict (382 fp32 device tensors for config.yaml), read once and re-packed. */
+/* names/ptrs: the reference state_dict (382 fp32 device tensors for config.yaml), read when a binding
+   is built and re-packed. */
 int wc_unet_create(wc_unet** out, const wc_unet_config* cfg, int n_params, const char* const* names,
                    const float* const* ptrs, const int64_t* numels, void* stream);
 void wc_unet_destroy(wc_unet* net);

@@ -421,4 +421,13 @@ int build_conv_transposed_s2(ConvOp* op, DeviceArena* arena, const Act& x, const
   return 0;
 }
 
+int build_conv_dgrad(ConvOp* op, DeviceArena* arena, const Act& dy, const WeightSrc& w, const ConvGeom& g, const Epilogue& ep,
+                     const OutSpec& out, cudaStream_t st) {
+  WeightSrc wt = w;
+  wt.transpose = 1;
+  if (g.stride != 1) return build_conv_transposed_s2(op, arena, dy, wt, g.K, g.pad, w.d1, ep, out, st);
+  wt.flip = 1;
+  return build_conv(op, arena, dy, wt, g, w.d1, nullptr, nullptr, ep, out, st);
+}
+
 }  // namespace wc

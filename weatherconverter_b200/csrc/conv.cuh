@@ -71,6 +71,11 @@ struct OutSpec {
 struct ConvOp {
   std::vector<IgemmPlan> plans;
   double flops = 0;
+  // Reports f algorithmic FLOPs (e.g. a separable layer run as a composed dense one), spread evenly over the launches.
+  void set_flops(double f) {
+    flops = f;
+    for (auto& p : plans) p.flops = f / plans.size();
+  }
   int run(cudaStream_t st) const {
     for (const auto& p : plans)
       if (int e = igemm_launch(p, st)) return e;
@@ -99,5 +104,10 @@ int build_conv_hrow(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSr
 // Weight source must have transpose = 1 semantics (out-channel = dim1).
 int build_conv_transposed_s2(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w, int K, int pad, int N,
                              const Epilogue& ep, const OutSpec& out, cudaStream_t st);
+
+// Data gradient dx (w.d1 channels) of y = conv(x, W, g) with W as stored (d0 = out-channels, d1 = in-channels): for stride 1
+// the convolution of dy with the flipped, transposed weight at padding g.pad, for stride 2 the transposed convolution.
+int build_conv_dgrad(ConvOp* op, DeviceArena* arena, const Act& dy, const WeightSrc& w, const ConvGeom& g, const Epilogue& ep,
+                     const OutSpec& out, cudaStream_t st);
 
 }  // namespace wc

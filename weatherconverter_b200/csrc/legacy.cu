@@ -167,11 +167,15 @@ struct wc_legacy_unet {
   wc::ParamTable params;
   std::unordered_map<std::string, int64_t> numels;
   std::unique_ptr<wc::DeviceArena> arena;
-  int B = 0, S = 0;
+  struct Geom {
+    int B, S;
+    bool operator==(const Geom& o) const { return B == o.B && S == o.S; }
+  } geom{};
   void* ws = nullptr;
-  size_t ws_bytes = 0, ws_needed = 0;
+  size_t ws_bytes = 0;
   wc::OpList ops;
   double flops = 0;
+  void reset_plan() { ops.clear(); flops = 0; }
   const float* x_in = nullptr;
   const float* t_in = nullptr;
   float* y_out = nullptr;
@@ -180,17 +184,9 @@ struct wc_legacy_unet {
 namespace wc {
 namespace {
 
-struct LBuilder {
-  wc_legacy_unet* net;
-  Bump bump;
-  DeviceArena* arena;
-  cudaStream_t st;
-  bool dry;
-  int B;
-  int err = 0;
+struct LBuilder : PlanBuilder<wc_legacy_unet> {
+  using PlanBuilder::PlanBuilder;
 
-  const float* P(const std::string& n) { return dry ? nullptr : net->params.get(n, &err); }
-  Act act(int H, int W, int C) { return make_act(bump, B, H, W, C); }
   void push(std::function<int(cudaStream_t)> f) {
     if (!dry) net->ops.push_back(std::move(f));
   }
@@ -280,9 +276,10 @@ struct LBuilder {
   }
 };
 
-int build(wc_legacy_unet* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const int B = net->B, S = net->S;
-  LBuilder b{net, dry ? Bump::dry() : Bump(ws, ws_bytes), net->arena.get(), st, dry, B};
+int build(const wc_legacy_unet&, const wc_legacy_unet::Geom& geo, wc_legacy_unet* net, cudaStream_t st, size_t* need) {
+  const int B = geo.B, S = geo.S;
+  LBuilder b(net, B, st);
+  const bool dry = b.dry;
   const int depth = 3;
   struct Level { const char* down; const char* up; int cin_d, cout_d, cin_u, cout_u; };
   // DownBlock(cin_d, cout_d) at size S >> l pairs with UpBlock(cin_u, cout_u, skip = cout_d)  (old_modules.py:252-275)
@@ -360,10 +357,7 @@ int build(wc_legacy_unet* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t
     b.push([=](cudaStream_t s) { return conv_small_cout(fin.ptr, w, nullptr, n->y_out, B, S, S, fin.C, 3, 3, fin.ld, 0, s); });
     net->flops += 2.0 * B * S * S * 9.0 * 32 * 3;
   }
-  if (b.err) return b.err;
-  if (dry) net->ws_needed = b.bump.used() + 4096;
-  else if (b.bump.overflow()) return fail("legacy UNet workspace too small");
-  return 0;
+  return b.finish("legacy UNet", need);
 }
 
 }  // namespace
@@ -387,12 +381,7 @@ int wc_legacy_unet_create(wc_legacy_unet** out, int n_params, const char* const*
 void wc_legacy_unet_destroy(wc_legacy_unet* net) { delete net; }
 
 size_t wc_legacy_unet_workspace_bytes(wc_legacy_unet* net, int batch, int size) {
-  const int sB = net->B, sS = net->S;
-  net->B = batch; net->S = size;
-  size_t need = 0;
-  if (build(net, true, nullptr, 0, nullptr) == 0) need = net->ws_needed;
-  net->B = sB; net->S = sS;
-  return need;
+  return plan_workspace_bytes(*net, {batch, size}, build);
 }
 
 int wc_legacy_unet_forward(wc_legacy_unet* net, const float* x, const float* t, float* out, int batch, int size, void* workspace,
@@ -400,21 +389,9 @@ int wc_legacy_unet_forward(wc_legacy_unet* net, const float* x, const float* t, 
   WC_REQUIRE(net && x && t && out && workspace, "null argument");
   WC_REQUIRE(size == 128, "the legacy UNet's attention blocks are built for 128 x 128 inputs (old_modules.py:256-270)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (net->B != batch || net->S != size || net->ws != workspace || net->ws_bytes != workspace_bytes) {
-    net->ops.clear();
-    net->arena = std::make_unique<DeviceArena>();
-    net->B = batch; net->S = size; net->ws = workspace; net->ws_bytes = workspace_bytes;
-    net->flops = 0;
-    if (int e = build(net, false, workspace, workspace_bytes, st)) {
-      net->B = 0;
-      net->ops.clear();
-      return e;
-    }
-  }
+  if (int e = bind(net, {batch, size}, workspace, workspace_bytes, st, build)) return e;
   net->x_in = x; net->t_in = t; net->y_out = out;
-  for (auto& op : net->ops)
-    if (int e = op(st)) return e;
-  return 0;
+  return run_ops(net->ops, st);
 }
 double wc_legacy_unet_flops(const wc_legacy_unet* net) { return net ? net->flops : 0.0; }
 int wc_legacy_unet_launches(const wc_legacy_unet* net) { return net ? static_cast<int>(net->ops.size()) : 0; }

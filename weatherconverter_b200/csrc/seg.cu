@@ -46,12 +46,17 @@ struct wc_seg {
   int output_stride = 16;   // 16: layer4 dilated, ASPP rates 6/12/18; 8: layers 3-4 dilated, rates 12/24/36 (modeling.py:34-39)
   wc::ParamTable params;
   std::unique_ptr<wc::DeviceArena> arena;
-  int B = 0, H = 0, W = 0, with_grad = 0, grad_pool = 1;
+  struct Geom {
+    int B, H, W, with_grad, grad_pool;
+    bool operator==(const Geom& o) const {
+      return B == o.B && H == o.H && W == o.W && with_grad == o.with_grad && grad_pool == o.grad_pool;
+    }
+  } geom{};
   void* ws = nullptr;
   size_t ws_bytes = 0;
   wc::OpList fwd_ops, bwd_ops;
   double flops_fwd = 0, flops_bwd = 0;
-  size_t ws_needed = 0;
+  void reset_plan() { fwd_ops.clear(); bwd_ops.clear(); flops_fwd = flops_bwd = 0; }
   // seam between the network body and the loss head, for wc_seg_forward / wc_seg_backward_seeded: fwd_ops[0, n_body_ops)
   // end at the low-resolution logits; the backward starts from dlo (NHWC bf16, 32 channels; with_grad plans only)
   size_t n_body_ops = 0;
@@ -77,23 +82,22 @@ struct BlockRec {
   Act x_in, y1, y2, out;
 };
 
-struct SegBuilder {
-  wc_seg* net;
-  Bump bump;
-  DeviceArena* arena;
-  cudaStream_t st;
-  bool dry;
-  int B;
-  int err = 0;
+// Forward geometry of a ResNet / ASPP convolution: 'same' padding at stride 1, Ho = H / 2 at stride 2.
+ConvGeom conv_geom(int K, int stride, int dil) {
+  ConvGeom g; g.K = K; g.stride = stride; g.dil = dil;
+  g.pad = (stride == 1) ? dil * (K - 1) / 2 : (K == 3 ? 1 : 0);
+  return g;
+}
+
+struct SegBuilder : PlanBuilder<wc_seg> {
+  using PlanBuilder::PlanBuilder;
   bool in_bwd = false;
   std::unordered_map<std::string, std::pair<float*, float*>> bn;  // prefix -> (scale, shift)
 
-  const float* P(const std::string& n) { return net->params.get(n, &err); }
   void push(std::function<int(cudaStream_t)> f) {
     if (dry) return;
     (in_bwd ? net->bwd_ops : net->fwd_ops).push_back(std::move(f));
   }
-  Act act(int H, int W, int C) { return make_act(bump, B, H, W, C); }
 
   std::pair<float*, float*> bnfold(const std::string& prefix, int C) {
     auto it = bn.find(prefix);
@@ -115,12 +119,10 @@ struct SegBuilder {
     auto sb = bnfold(bnname, cout);
     WeightSrc w; w.w = P(wname + ".weight"); w.d0 = cout; w.d1 = cin; w.KH = w.KW = K; w.scale = sb.first;
     if (err) return;
-    ConvGeom g; g.K = K; g.stride = stride; g.dil = dil;
-    g.pad = (stride == 1) ? dil * (K - 1) / 2 : (K == 3 ? 1 : 0);
     Epilogue ep; ep.bias = sb.second; ep.res = res; ep.relu = relu;
     OutSpec os; os.mode = kOutNHWC; os.out = out;
     auto op = std::make_shared<ConvOp>();
-    if (int e = build_conv(op.get(), arena, x, w, g, cout, nullptr, nullptr, ep, os, st)) { err = e; return; }
+    if (int e = build_conv(op.get(), arena, x, w, conv_geom(K, stride, dil), cout, nullptr, nullptr, ep, os, st)) { err = e; return; }
     net->flops_fwd += op->flops;
     push([op](cudaStream_t s) { return op->run(s); });
   }
@@ -130,28 +132,21 @@ struct SegBuilder {
              int dil, const Act* res, const Act* mask, const Act& dx, const float* scale_override = nullptr, bool no_bn = false) {
     if (dry) return;
     const float* sc = no_bn ? scale_override : bnfold(bnname, cout).first;
-    WeightSrc w; w.w = P(wname + ".weight"); w.d0 = cout; w.d1 = cin; w.KH = w.KW = K; w.transpose = 1; w.scale = sc;
+    WeightSrc w; w.w = P(wname + ".weight"); w.d0 = cout; w.d1 = cin; w.KH = w.KW = K; w.scale = sc;
     if (err) return;
     Epilogue ep; ep.res = res; ep.mask = mask;
     OutSpec os; os.mode = kOutNHWC; os.out = dx;
     auto op = std::make_shared<ConvOp>();
-    int e;
-    if (stride == 1) {
-      w.flip = 1;
-      ConvGeom g; g.K = K; g.stride = 1; g.dil = dil; g.pad = dil * (K - 1) / 2;
-      e = build_conv(op.get(), arena, dz, w, g, cin, nullptr, nullptr, ep, os, st);
-    } else {
-      e = build_conv_transposed_s2(op.get(), arena, dz, w, K, K == 3 ? 1 : 0, cin, ep, os, st);
-    }
-    if (e) { err = e; return; }
+    if (int e = build_conv_dgrad(op.get(), arena, dz, w, conv_geom(K, stride, dil), ep, os, st)) { err = e; return; }
     net->flops_bwd += op->flops;
     push([op](cudaStream_t s) { return op->run(s); });
   }
 };
 
-int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const int B = net->B, H = net->H, W = net->W, NC = net->num_classes;
-  SegBuilder b{net, dry ? Bump::dry() : Bump(ws, ws_bytes), net->arena.get(), st, dry, B};
+int build(const wc_seg& cfg, const wc_seg::Geom& geo, wc_seg* net, cudaStream_t st, size_t* need) {
+  const int B = geo.B, H = geo.H, W = geo.W, NC = cfg.num_classes;
+  SegBuilder b(net, B, st);
+  const bool dry = b.dry;
   const int H2 = H / 2, W2 = W / 2, H4 = H / 4, W4 = W / 4;
   // ---------------- stem: conv1 7x7 s2 + bn1 + relu (tensor core, from NCHW fp32), maxpool 3x3 s2
   Act c1 = b.act(H2, W2, 64);
@@ -186,13 +181,13 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   {
     int inplanes = 64, dilation = 1;
     const int planes_l[4] = {64, 128, 256, 512}, stride_l[4] = {1, 2, 2, 2};
-    const bool os8 = net->output_stride == 8;
+    const bool os8 = cfg.output_stride == 8;
     const bool dilate_l[4] = {false, false, os8, true};  // replace_stride_with_dilation: os 16 [F,F,T], os 8 [F,T,T] (modeling.py:34-39)
     for (int li = 0; li < 4; ++li) {
       const int prev = dilation;
       int stride = stride_l[li];
       if (dilate_l[li]) { dilation *= stride; stride = 1; }
-      for (int bi = 0; bi < net->layers[li]; ++bi) {
+      for (int bi = 0; bi < cfg.layers[li]; ++bi) {
         BlockRec r;
         r.p = "backbone.layer" + std::to_string(li + 1) + "." + std::to_string(bi);
         r.inplanes = inplanes; r.planes = planes_l[li];
@@ -222,7 +217,7 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     r.out = b.act(Ho, Wo, r.planes * 4);
     b.conv_bn(r.y2, r.p + ".conv3", r.p + ".bn3", r.planes, r.planes * 4, 1, 1, 1, &idt, 1, r.out);
     cur = r.out;
-    if (static_cast<int>(i) + 1 == net->layers[0]) low = cur;
+    if (static_cast<int>(i) + 1 == cfg.layers[0]) low = cur;
     if (b.err) return b.err;
   }
   const Act feat = cur;  // [B, H/16, W/16, 2048]
@@ -231,7 +226,7 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   const std::string c = "classifier";
   Act cat5 = b.act(h, w, 1280);
   b.conv_bn(feat, c + ".aspp.convs.0.0", c + ".aspp.convs.0.1", 2048, 256, 1, 1, 1, nullptr, 1, slice_act(cat5, 0, 256));
-  const int rmul = net->output_stride == 8 ? 2 : 1;
+  const int rmul = cfg.output_stride == 8 ? 2 : 1;
   const int rates[3] = {6 * rmul, 12 * rmul, 18 * rmul};   // ASPP dilations (modeling.py:35,38)
   for (int k = 0; k < 3; ++k)
     b.conv_bn(feat, c + ".aspp.convs." + std::to_string(k + 1) + ".0", c + ".aspp.convs." + std::to_string(k + 1) + ".1", 2048,
@@ -276,15 +271,15 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   // d-logit tensor is never written (seg_kernels.cu: seg_loss_head_fused_kernel); geometries it does not take, and requests for the
   // full-resolution logits, go through the two-pass head below.
   Act dlo{};
-  if (net->with_grad) dlo = b.act(H4, W4, NCP);
+  const bool with_grad = geo.with_grad;
+  if (with_grad) dlo = b.act(H4, W4, NCP);
   if (!dry) {
     net->n_body_ops = net->fwd_ops.size();
     net->logits_lo = logits_lo;
-    net->dlo = net->with_grad ? dlo.ptr : nullptr;
+    net->dlo = with_grad ? dlo.ptr : nullptr;
   }
   {
     wc_seg* n = net;
-    const bool with_grad = net->with_grad;
     b.push([=](cudaStream_t s) {
       if (with_grad && !n->logits_hi) {
         const int e = seg_loss_head_fused(logits_lo, n->labels, n_valid, n->pred, n->loss, dlo.ptr, B, H4, W4, H, W, NC, NCP, NCP, 255, s);
@@ -294,11 +289,7 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       return with_grad ? logits_bilinear_bwd(dlogit_hi, dlo.ptr, B, H4, W4, H, W, NC, NCP, NCP, s) : 0;
     });
   }
-  if (!net->with_grad) {
-    if (dry) net->ws_needed = b.bump.used() + 4096;
-    else if (b.bump.overflow()) return fail("seg workspace too small");
-    return b.err;
-  }
+  if (!with_grad) return b.finish("seg", need);
   // =================================================== backward (data gradients only)
   b.in_bwd = true;
   Act dlo19 = dlo; dlo19.C = NC;
@@ -339,7 +330,7 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   for (int i = static_cast<int>(blocks.size()) - 1; i >= 0; --i) {
     const BlockRec& r = blocks[i];
     const bool first_block = (i == 0);
-    const bool feeds_low = (i == net->layers[0]);  // this block's input is layer1's output (the low-level feature)
+    const bool feeds_low = (i == cfg.layers[0]);  // this block's input is layer1's output (the low-level feature)
     Act d2 = b.act(g.H, g.W, r.planes);
     b.dgrad(g, r.p + ".conv3", r.p + ".bn3", r.planes, r.planes * 4, 1, 1, 1, nullptr, &r.y2, d2);
     Act d1 = b.act(r.x_in.H, r.x_in.W, r.planes);
@@ -374,7 +365,7 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     wc_seg* n = net;
     const Act gp = g;
     const float* sc = bn1.first;
-    const int P = net->grad_pool;
+    const int P = geo.grad_pool;
     float* weff = nullptr;
     if (!dry && P > 1) {
       const int R = P / 2 + 3;
@@ -387,29 +378,9 @@ int build(wc_seg* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       if (P > 1) return conv1_dgrad_pooled(dc1.ptr, weff, n->grad_out, B, H, W, P, s);
       return conv1_dgrad(dc1.ptr, w_conv1, sc, n->grad_out, B, H, W, 64, s);
     });
-    net->flops_bwd += 2.0 * B * H2 * W2 * 147.0 * 64;
+    if (!dry) net->flops_bwd += 2.0 * B * H2 * W2 * 147.0 * 64;
   }
-  if (dry) net->ws_needed = b.bump.used() + 4096;
-  else if (b.bump.overflow()) return fail("seg workspace too small: need " + std::to_string(b.bump.used()) + " bytes");
-  return b.err;
-}
-
-// (Re)builds the plan when the geometry, the gradient mode or the workspace differ from the current binding.
-int bind_plan(wc_seg* net, int batch, int H, int W, int with_grad, int grad_pool, void* workspace, size_t workspace_bytes,
-              cudaStream_t st) {
-  if (net->B == batch && net->H == H && net->W == W && net->with_grad == with_grad && net->grad_pool == grad_pool && net->ws == workspace &&
-      net->ws_bytes == workspace_bytes)
-    return 0;
-  net->fwd_ops.clear(); net->bwd_ops.clear();
-  net->arena = std::make_unique<DeviceArena>();
-  net->B = batch; net->H = H; net->W = W; net->with_grad = with_grad; net->grad_pool = grad_pool; net->ws = workspace; net->ws_bytes = workspace_bytes;
-  net->flops_fwd = net->flops_bwd = 0;
-  if (int e = build(net, false, workspace, workspace_bytes, st)) {
-    net->B = 0;
-    net->fwd_ops.clear(); net->bwd_ops.clear();
-    return e;
-  }
-  return 0;
+  return b.finish("seg", need);
 }
 
 }  // namespace
@@ -437,7 +408,7 @@ int wc_seg_set_output_stride(wc_seg* net, int output_stride) {
   WC_REQUIRE(output_stride == 8 || output_stride == 16, "output_stride must be 8 or 16 (modeling.py:34-39)");
   if (net->output_stride != output_stride) {
     net->output_stride = output_stride;
-    net->B = net->H = net->W = 0;   // force a rebuild of the plan on the next call
+    net->geom = {};   // the next call rebuilds the plan
     net->saved_fwd = 0;
   }
   return 0;
@@ -445,14 +416,8 @@ int wc_seg_set_output_stride(wc_seg* net, int output_stride) {
 
 void wc_seg_destroy(wc_seg* net) { delete net; }
 
-size_t wc_seg_workspace_bytes(const wc_seg* net_c, int batch, int H, int W, int with_grad) {
-  wc_seg* net = const_cast<wc_seg*>(net_c);
-  const int sB = net->B, sH = net->H, sW = net->W, sg = net->with_grad;
-  net->B = batch; net->H = H; net->W = W; net->with_grad = with_grad;
-  size_t need = 0;
-  if (build(net, true, nullptr, 0, nullptr) == 0) need = net->ws_needed;
-  net->B = sB; net->H = sH; net->W = sW; net->with_grad = sg;
-  return need;
+size_t wc_seg_workspace_bytes(const wc_seg* net, int batch, int H, int W, int with_grad) {
+  return plan_workspace_bytes(*net, {batch, H, W, with_grad, 1}, build);
 }
 
 int wc_seg_infer_pooled(wc_seg* net, const float* x, const int64_t* labels, int64_t* pred, float* input_grad, float* loss,
@@ -473,14 +438,11 @@ int wc_seg_infer_pooled(wc_seg* net, const float* x, const int64_t* labels, int6
   WC_REQUIRE(H % 32 == 0 && W % 32 == 0, "H and W must be multiples of 32 (output stride 16, stride-2 phase views)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int with_grad = input_grad != nullptr;
-  if (int e = bind_plan(net, batch, H, W, with_grad, grad_pool, workspace, workspace_bytes, st)) return e;
+  if (int e = bind(net, {batch, H, W, with_grad, grad_pool}, workspace, workspace_bytes, st, build)) return e;
   net->x_in = x; net->labels = reinterpret_cast<const long long*>(labels);
   net->pred = reinterpret_cast<long long*>(pred); net->grad_out = input_grad; net->loss = loss; net->logits_hi = logits;
-  for (auto& op : net->fwd_ops)
-    if (int e = op(st)) return e;
-  for (auto& op : net->bwd_ops)
-    if (int e = op(st)) return e;
-  return 0;
+  if (int e = run_ops(net->fwd_ops, st)) return e;
+  return run_ops(net->bwd_ops, st);
 }
 
 int wc_seg_forward(wc_seg* net, const float* x, float* logits, int batch, int H, int W, int save_for_backward, void* workspace,
@@ -489,7 +451,7 @@ int wc_seg_forward(wc_seg* net, const float* x, float* logits, int batch, int H,
   WC_REQUIRE(net && x && logits && workspace, "null argument");
   WC_REQUIRE(H % 32 == 0 && W % 32 == 0, "H and W must be multiples of 32 (output stride 16, stride-2 phase views)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int e = bind_plan(net, batch, H, W, save_for_backward ? 1 : 0, 1, workspace, workspace_bytes, st)) return e;
+  if (int e = bind(net, {batch, H, W, save_for_backward ? 1 : 0, 1}, workspace, workspace_bytes, st, build)) return e;
   net->x_in = x; net->labels = nullptr; net->pred = nullptr; net->grad_out = nullptr; net->loss = nullptr; net->logits_hi = logits;
   for (size_t i = 0; i < net->n_body_ops; ++i)
     if (int e = net->fwd_ops[i](st)) return e;
@@ -508,12 +470,10 @@ int wc_seg_backward_seeded(wc_seg* net, const float* dlogits, float* input_grad,
              "wc_seg_forward(save_for_backward = 1) (an infer or another forward in between discards the saved activations)");
   net->saved_fwd = 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = net->B, H = net->H, W = net->W;
+  const int B = net->geom.B, H = net->geom.H, W = net->geom.W;
   net->grad_out = input_grad;
   if (int e = logits_bilinear_bwd(dlogits, net->dlo, B, H / 4, W / 4, H, W, net->num_classes, 32, 32, st)) return e;
-  for (auto& op : net->bwd_ops)
-    if (int e = op(st)) return e;
-  return 0;
+  return run_ops(net->bwd_ops, st);
 }
 
 double wc_seg_flops(const wc_seg* net, int backward) { return net ? (backward ? net->flops_bwd : net->flops_fwd) : 0.0; }

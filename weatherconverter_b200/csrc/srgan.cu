@@ -40,12 +40,15 @@ struct wc_srgan {
   int num_blocks = 16, upscale = 4, nc = 64;
   wc::ParamTable params;
   std::unique_ptr<wc::DeviceArena> arena;
-  int B = 0, H = 0, W = 0, with_grad = 0;
+  struct Geom {
+    int B, H, W, with_grad;
+    bool operator==(const Geom& o) const { return B == o.B && H == o.H && W == o.W && with_grad == o.with_grad; }
+  } geom{};
   void* ws = nullptr;
   size_t ws_bytes = 0;
   wc::OpList ops, bwd_ops;   // bwd_ops: with-grad plans only
   double flops = 0;
-  size_t ws_needed = 0;
+  void reset_plan() { ops.clear(); bwd_ops.clear(); flops = 0; }
   int saved_fwd = 0;   // the last call on this handle was wc_srgan_forward_saved
   const float* x_in = nullptr;
   float* y_out = nullptr;
@@ -56,19 +59,21 @@ struct wc_srgan {
 namespace wc {
 namespace {
 
-int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const int B = net->B, H = net->H, W = net->W, NCH = net->nc;
-  Bump bump = dry ? Bump::dry() : Bump(ws, ws_bytes);
-  DeviceArena* arena = net->arena.get();
-  int err = 0;
-  auto P = [&](const std::string& n) { return net->params.get(n, &err); };
+int build(const wc_srgan& cfg, const wc_srgan::Geom& geo, wc_srgan* net, cudaStream_t st, size_t* need) {
+  const int B = geo.B, H = geo.H, W = geo.W, NCH = cfg.nc;
+  PlanBuilder<wc_srgan> b(net, B, st);
+  const bool dry = b.dry;
+  Bump& bump = b.bump;
+  DeviceArena* arena = b.arena;
+  int& err = b.err;
+  auto P = [&](const std::string& n) { return b.P(n); };
   auto Popt = [&](const std::string& n) -> const float* {
     auto it = net->params.ptr.find(n);
     return it == net->params.ptr.end() ? nullptr : it->second;
   };
   auto push = [&](std::function<int(cudaStream_t)> f) { if (!dry) net->ops.push_back(std::move(f)); };
   auto pushb = [&](std::function<int(cudaStream_t)> f) { if (!dry) net->bwd_ops.push_back(std::move(f)); };
-  const bool grad = net->with_grad;
+  const bool grad = geo.with_grad;
   auto fa = [&](size_t n) { return static_cast<float*>(arena->alloc(n * sizeof(float))); };
 
   // composed dense weights of a SeperableConv2d (+ optional folded BN): returns (weights, bias/shift, scale)
@@ -100,20 +105,19 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     auto op = std::make_shared<ConvOp>();
     if (int e = build_conv(op.get(), arena, x, w, g, co, nullptr, nullptr, ep, os, st)) { err = e; return; }
     // algorithmic FLOPs = the reference's separable form (depthwise 3x3 + pointwise), not the composed dense conv
-    op->flops = 2.0 * x.pixels() * (9.0 * x.C + static_cast<double>(x.C) * co);
-    for (auto& pl : op->plans) pl.flops = op->flops / op->plans.size();
+    op->set_flops(2.0 * x.pixels() * (9.0 * x.C + static_cast<double>(x.C) * co));
     net->flops += op->flops;
     net->ops.push_back([op](cudaStream_t s) { return op->run(s); });
   };
   // data gradient of conv3 (stride 1, 'same'): dx = conv(dz, flipped W^T) (+ res), the folded BN scale applied to W's rows
   auto dgrad3 = [&](const Act& dz, const Composed& c, int ci, const Act* res, const Act& dx) {
     if (dry || err) return;
-    WeightSrc w; w.w = c.w; w.d0 = dz.C; w.d1 = ci; w.KH = w.KW = 3; w.transpose = 1; w.flip = 1; w.scale = c.scale;
+    WeightSrc w; w.w = c.w; w.d0 = dz.C; w.d1 = ci; w.KH = w.KW = 3; w.scale = c.scale;
     ConvGeom g; g.K = 3; g.pad = 1;
     Epilogue ep; ep.res = res;
     OutSpec os; os.mode = kOutNHWC; os.out = dx;
     auto op = std::make_shared<ConvOp>();
-    if (int e = build_conv(op.get(), arena, dz, w, g, ci, nullptr, nullptr, ep, os, st)) { err = e; return; }
+    if (int e = build_conv_dgrad(op.get(), arena, dz, w, g, ep, os, st)) { err = e; return; }
     net->bwd_ops.push_back([op](cudaStream_t s) { return op->run(s); });
   };
 
@@ -147,9 +151,9 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   }
   // ---- residual trunk
   struct BlockRec { Composed c1, c2; const float* slope; Act pre1; };
-  std::vector<BlockRec> blocks(net->num_blocks);
+  std::vector<BlockRec> blocks(cfg.num_blocks);
   Act cur = initial;
-  for (int i = 0; i < net->num_blocks; ++i) {
+  for (int i = 0; i < cfg.num_blocks; ++i) {
     const std::string p = "residual." + std::to_string(i);
     Act t1 = make_act(bump, B, H, W, NCH), out = make_act(bump, B, H, W, NCH);
     if (grad) blocks[i].pre1 = make_act(bump, B, H, W, NCH);
@@ -175,9 +179,9 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
   cur = trunk;
   // ---- upsamplers: SeperableConv2d(64->256, k3) + PixelShuffle(2) + PReLU(64)
   struct UpRec { Composed c; const float* slope; Act pre; };
-  std::vector<UpRec> ups(net->upscale / 2);
+  std::vector<UpRec> ups(cfg.upscale / 2);
   int h = H, w = W;
-  for (int u = 0; u < net->upscale / 2; ++u) {
+  for (int u = 0; u < cfg.upscale / 2; ++u) {
     const std::string p = "upsampler." + std::to_string(u);
     Act up = make_act(bump, B, 2 * h, 2 * w, NCH);
     if (grad) ups[u].pre = make_act(bump, B, 2 * h, 2 * w, NCH);
@@ -203,8 +207,7 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
         OutSpec os; os.mode = kOutNHWC; os.out = pass ? ups[u].pre : up; os.up = 2; os.phases = 4; os.bn_max = 128;
         auto op = std::make_shared<ConvOp>();
         if (int e = build_conv(op.get(), arena, cur, ws_, g, NCH * 4, nullptr, nullptr, ep, os, st)) return e;
-        op->flops = 2.0 * cur.pixels() * (9.0 * NCH + static_cast<double>(NCH) * NCH * 4);
-        for (auto& pl : op->plans) pl.flops = op->flops / op->plans.size();
+        op->set_flops(2.0 * cur.pixels() * (9.0 * NCH + static_cast<double>(NCH) * NCH * 4));
         net->flops += op->flops;
         net->ops.push_back([op](cudaStream_t s) { return op->run(s); });
       }
@@ -235,8 +238,7 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       OutSpec os; os.mode = kOutNCHWf32; os.out_f32 = tplanes; os.n_store = 27;
       auto op = std::make_shared<ConvOp>();
       if (int e = build_conv_hrow(op.get(), arena, last, ws_, 32, ep, os, st)) return e;
-      op->flops = fl;
-      for (auto& pl : op->plans) pl.flops = fl / op->plans.size();
+      op->set_flops(fl);
       net->ops.push_back([op](cudaStream_t s) { return op->run(s); });
       push([=](cudaStream_t s) { return srgan_final_combine(tplanes, bias3, n->y_out, B, hh, ww, s); });
     } else {
@@ -270,7 +272,7 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       });
     }
     // up-samplers: PReLU + PixelShuffle backward into the conv's 256 channels (4c + q), then the 64 -> 256 conv's data gradient
-    for (int u = net->upscale / 2 - 1; u >= 0; --u) {
+    for (int u = cfg.upscale / 2 - 1; u >= 0; --u) {
       const int hu = h / 2, wu = w / 2;
       Act dconv = make_act(bump, B, hu, wu, 4 * NCH), dx = make_act(bump, B, hu, wu, NCH);
       if (!dry) {
@@ -287,7 +289,7 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
     Act dt = make_act(bump, B, H, W, NCH);
     int gi = 0;
     dgrad3(dtrunk, c_convblock, NCH, nullptr, gbuf[gi]);
-    for (int i = net->num_blocks - 1; i >= 0; --i) {
+    for (int i = cfg.num_blocks - 1; i >= 0; --i) {
       const Act g = gbuf[gi], gn = gbuf[gi ^ 1], pre = blocks[i].pre1;
       dgrad3(g, blocks[i].c2, NCH, nullptr, dt);
       if (!dry) {
@@ -308,35 +310,7 @@ int build(wc_srgan* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
       });
     }
   }
-  if (dry) net->ws_needed = bump.used() + 4096;
-  else if (bump.overflow()) return fail("SRGAN workspace too small");
-  return err;
-}
-
-// (Re)builds the plan when the geometry, the gradient mode or the workspace differ from the current binding.
-int bind_plan(wc_srgan* net, int batch, int h, int w, int with_grad, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (net->B == batch && net->H == h && net->W == w && net->with_grad == with_grad && net->ws == workspace &&
-      net->ws_bytes == workspace_bytes)
-    return 0;
-  net->ops.clear(); net->bwd_ops.clear();
-  net->arena = std::make_unique<DeviceArena>();
-  net->B = batch; net->H = h; net->W = w; net->with_grad = with_grad; net->ws = workspace; net->ws_bytes = workspace_bytes;
-  net->flops = 0;
-  if (int e = build(net, false, workspace, workspace_bytes, st)) {
-    net->B = 0;
-    net->ops.clear(); net->bwd_ops.clear();
-    return e;
-  }
-  return 0;
-}
-
-size_t workspace_bytes(wc_srgan* net, int batch, int h, int w, int with_grad) {
-  const int sB = net->B, sH = net->H, sW = net->W, sg = net->with_grad;
-  net->B = batch; net->H = h; net->W = w; net->with_grad = with_grad;
-  size_t need = 0;
-  if (build(net, true, nullptr, 0, nullptr) == 0) need = net->ws_needed;
-  net->B = sB; net->H = sH; net->W = sW; net->with_grad = sg;
-  return need;
+  return b.finish("SRGAN", need);
 }
 
 }  // namespace
@@ -359,45 +333,40 @@ int wc_srgan_create(wc_srgan** out, int num_blocks, int upscale, int n_params, c
 }
 void wc_srgan_destroy(wc_srgan* net) { delete net; }
 size_t wc_srgan_workspace_bytes(const wc_srgan* net, int batch, int h, int w) {
-  return workspace_bytes(const_cast<wc_srgan*>(net), batch, h, w, 0);
+  return plan_workspace_bytes(*net, {batch, h, w, 0}, build);
 }
 size_t wc_srgan_grad_workspace_bytes(const wc_srgan* net, int batch, int h, int w) {
-  return workspace_bytes(const_cast<wc_srgan*>(net), batch, h, w, 1);
+  return plan_workspace_bytes(*net, {batch, h, w, 1}, build);
 }
 int wc_srgan_forward(wc_srgan* net, const float* x, float* y, int batch, int h, int w, void* workspace,
                      size_t workspace_bytes, void* stream) {
   if (net) net->saved_fwd = 0;
   WC_REQUIRE(net && x && y && workspace, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int e = bind_plan(net, batch, h, w, 0, workspace, workspace_bytes, st)) return e;
+  if (int e = bind(net, {batch, h, w, 0}, workspace, workspace_bytes, st, build)) return e;
   net->x_in = x; net->y_out = y;
-  for (auto& op : net->ops)
-    if (int e = op(st)) return e;
-  return 0;
+  return run_ops(net->ops, st);
 }
 int wc_srgan_forward_saved(wc_srgan* net, const float* x, float* y, int batch, int h, int w, void* workspace,
                            size_t workspace_bytes, void* stream) {
   if (net) net->saved_fwd = 0;
   WC_REQUIRE(net && x && y && workspace, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (int e = bind_plan(net, batch, h, w, 1, workspace, workspace_bytes, st)) return e;
+  if (int e = bind(net, {batch, h, w, 1}, workspace, workspace_bytes, st, build)) return e;
   net->x_in = x; net->y_out = y;
-  for (auto& op : net->ops)
-    if (int e = op(st)) return e;
+  if (int e = run_ops(net->ops, st)) return e;
   net->saved_fwd = 1;
   return 0;
 }
 int wc_srgan_backward_seeded(wc_srgan* net, const float* dy, float* dx, void* stream) {
   WC_REQUIRE(net && dy && dx, "null argument");
-  WC_REQUIRE(net->saved_fwd && net->with_grad,
+  WC_REQUIRE(net->saved_fwd && net->geom.with_grad,
              "wc_srgan_backward_seeded: this handle holds no saved forward; the last call on it must be wc_srgan_forward_saved "
              "(any forward in between discards the saved activations, and so does the backward itself)");
   net->saved_fwd = 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   net->dy_in = dy; net->dx_out = dx;
-  for (auto& op : net->bwd_ops)
-    if (int e = op(st)) return e;
-  return 0;
+  return run_ops(net->bwd_ops, st);
 }
 double wc_srgan_flops(const wc_srgan* net) { return net ? net->flops : 0.0; }
 int wc_srgan_launches(const wc_srgan* net) { return net ? static_cast<int>(net->ops.size()) : 0; }

@@ -14,11 +14,8 @@
 // The same backward also runs seeded with a caller's dL/dpred (wc_unet_train_backward_seeded: torch autograd of the
 // Unet module, diffusion_model/models/unet_base.py), optionally producing dL/dx and optionally skipping every op whose
 // only product is a parameter gradient.
-#include <map>
-
-#include "plan.cuh"
+#include "unet_plan.cuh"
 #include "wgrad.cuh"
-#include "../../include/wc_b200.h"
 
 namespace wc {
 int groupnorm_silu(const __nv_bfloat16* x, __nv_bfloat16* y, int B, int HW, int C, int ld, int ldy, const float* gamma,
@@ -66,13 +63,20 @@ struct wc_unet_train {
   wc::ParamTable params;
   std::unordered_map<std::string, float*> grads;
   std::unique_ptr<wc::DeviceArena> arena;
-  int B = 0, H = 0, W = 0;
+  struct Geom {
+    int B, H, W;
+    bool operator==(const Geom& o) const { return B == o.B && H == o.H && W == o.W; }
+  } geom{};
   void* ws = nullptr;
-  size_t ws_bytes = 0, ws_needed = 0;
+  size_t ws_bytes = 0;
   wc::OpList repack_ops, fwd_ops, bwd_ops;
   std::vector<int> bwd_kind;  // per backward op: what it produces (kOpData / kOpParam / kOpInput)
   std::unordered_map<std::string, int> ready;  // parameter name -> number of backward ops after which its grad is final
   double flops_fwd = 0, flops_bwd = 0;
+  void reset_plan() {
+    repack_ops.clear(); fwd_ops.clear(); bwd_ops.clear(); bwd_kind.clear(); ready.clear();
+    flops_fwd = flops_bwd = 0;
+  }
   // per-call pointers
   const float* x_in = nullptr;
   const float* target = nullptr;
@@ -91,20 +95,16 @@ namespace {
 // launches only when the caller asked for dL/dx.
 enum { kOpData = 0, kOpParam = 1, kOpInput = 2 };
 
-struct TBuilder {
-  wc_unet_train* net;
-  Bump bump;
-  DeviceArena* arena;
-  cudaStream_t st;
-  bool dry;
-  int B;
-  int err = 0;
+struct TBuilder : PlanBuilder<wc_unet_train> {
+  using PlanBuilder::PlanBuilder;
   bool in_bwd = false;
   float* tproj = nullptr;
   float* dtproj = nullptr;
   int tproj_ld = 0, temb_off = 0;
   float* wg_partial = nullptr;
   void* red_ws = nullptr;
+  void* bw_scratch = nullptr;
+  float* w_in_t = nullptr;   // conv_in's weight, flipped and transposed: the input gradient's 64 -> 3 convolution
   std::vector<std::function<void()>> tape;
 
   // ---------------------------------------------------------------- gradient shadows
@@ -117,7 +117,7 @@ struct TBuilder {
   };
   std::vector<Alloc> allocs;
 
-  Act new_act(int H, int W, int C) {
+  Act act(int H, int W, int C) {   // every activation gets a gradient shadow record
     Act a = make_act(bump, B, H, W, C);
     allocs.push_back({a.ptr, C, a.pixels(), nullptr, {}});
     return a;
@@ -160,7 +160,6 @@ struct TBuilder {
   }
 
   // ---------------------------------------------------------------- helpers
-  const float* P(const std::string& n) { return dry ? nullptr : net->params.get(n, &err); }
   float* G(const std::string& n) {
     if (dry) return nullptr;
     auto it = net->grads.find(n);
@@ -238,20 +237,13 @@ struct TBuilder {
     const bool acc = written(x);
     mark(x);
     if (dry) return;
-    WeightSrc w; w.w = P(wname + ".weight"); w.d0 = cout; w.d1 = cin; w.KH = w.KW = K; w.transpose = 1;
+    WeightSrc w; w.w = P(wname + ".weight"); w.d0 = cout; w.d1 = cin; w.KH = w.KW = K;
     if (err) return;
+    ConvGeom g; g.K = K; g.stride = stride; g.pad = stride == 1 ? (K - 1) / 2 : 1; g.dil = 1;   // forward padding
     Epilogue ep; ep.res = acc ? &gx : nullptr;
     OutSpec os; os.mode = kOutNHWC; os.out = gx;
     auto op = std::make_shared<ConvOp>();
-    int e;
-    if (stride == 1) {
-      w.flip = 1;
-      ConvGeom g; g.K = K; g.stride = 1; g.dil = 1; g.pad = (K - 1) / 2;
-      e = build_conv(op.get(), arena, dy, w, g, cin, nullptr, nullptr, ep, os, st);
-    } else {
-      e = build_conv_transposed_s2(op.get(), arena, dy, w, K, 1, cin, ep, os, st);
-    }
-    if (e) { err = e; return; }
+    if (int e = build_conv_dgrad(op.get(), arena, dy, w, g, ep, os, st)) { err = e; return; }
     net->flops_bwd += op->flops;
     push([op](cudaStream_t s) { return op->run(s); });
   }
@@ -308,15 +300,15 @@ struct TBuilder {
   Act resnet(const Act& x, int cout, const std::string& p, int l, const Act* dest) {
     const std::string ls = std::to_string(l);
     const std::string n1 = p + ".resnet_conv_first." + ls, n2 = p + ".resnet_conv_second." + ls, nr = p + ".residual_input_conv." + ls;
-    Act a1 = new_act(x.H, x.W, x.C);
+    Act a1 = act(x.H, x.W, x.C);
     void* st1 = gn_fwd(x, a1, n1 + ".0", 1);
-    Act h = new_act(x.H, x.W, cout);
+    Act h = act(x.H, x.W, cout);
     const int toff = temb_off;
     temb_off += cout;
     conv_fwd(a1, n1 + ".2", cout, 3, 1, 1, P(n1 + ".2.bias"), dry ? nullptr : tproj + toff, tproj_ld, nullptr, nullptr, "", h);
-    Act a2 = new_act(x.H, x.W, cout);
+    Act a2 = act(x.H, x.W, cout);
     void* st2 = gn_fwd(h, a2, n2 + ".0", 1);
-    Act out = dest ? *dest : new_act(x.H, x.W, cout);
+    Act out = dest ? *dest : act(x.H, x.W, cout);
     float* bsum = nullptr;
     if (!dry) {
       bsum = static_cast<float*>(arena->alloc(cout * sizeof(float)));
@@ -345,12 +337,66 @@ struct TBuilder {
     return out;
   }
 
+  // ---------------------------------------------------------------- hooks of walk_unet (unet_plan.cuh)
+  void conv_in(const Act& skip0) {
+    const int B = skip0.B, H = skip0.H, W = skip0.W, c0 = skip0.C;
+    if (!dry) {
+      const float *w = P("conv_in.weight"), *bias = P("conv_in.bias");
+      if (err) return;
+      wc_unet_train* n = net;
+      const int cin = n->cfg.im_channels;
+      push([=](cudaStream_t s) {
+        return conv_small_cin(n->x_in, w, bias, nullptr, nullptr, skip0.ptr, B, cin, H, W, c0, 3, 1, 1, skip0.ld, 0, s);
+      });
+      net->flops_fwd += 2.0 * B * H * W * 9.0 * cin * c0;
+    }
+    tape.push_back([=]() {
+      Act d = grad_written(skip0);
+      if (dry) return;
+      const float* w = P("conv_in.weight");
+      float *dw = G("conv_in.weight"), *db = G("conv_in.bias");
+      if (err) return;
+      wc_unet_train* n = net;
+      const int cin = n->cfg.im_channels;
+      void* bws = bw_scratch;
+      float* wt = w_in_t;
+      push([=](cudaStream_t s) { return boundary_wgrad(d.ptr, d.ld, n->x_in, B, H, W, +1, dw, db, bws, s); }, kOpParam);
+      ready("conv_in.weight");
+      ready("conv_in.bias");
+      // dL/dx: the 64 -> 3 convolution of d(skip0) with the flipped, transposed conv_in weight (conv_out's forward kernel)
+      net->repack_ops.push_back([=](cudaStream_t s) { return flip_transpose_3x3(w, wt, c0, cin, s); });
+      push([=](cudaStream_t s) {
+        return n->dx_out ? conv_small_cout(d.ptr, wt, nullptr, n->dx_out, B, H, W, c0, cin, 3, d.ld, 0, s) : 0;
+      }, kOpInput);
+    });
+  }
+
+  void down_sample(const Act& xin, const std::string& p, int ch, const Act& out) {
+    conv_fwd(xin, p + ".down_sample_conv", ch, 4, 2, 1, P(p + ".down_sample_conv.bias"), nullptr, 0, nullptr, nullptr, "", out);
+    tape.push_back([=]() {
+      Act dout = grad_written(out);
+      dgrad(dout, p + ".down_sample_conv", ch, ch, 4, 2, xin);
+      wgrad(xin, dout, 4, 2, 1, p + ".down_sample_conv", nullptr, "");
+      bias_grad(dout, p + ".down_sample_conv.bias", "", nullptr, 0);
+    });
+  }
+
+  void up_sample(const Act& xin, const std::string& p, int ch, const Act& out) {
+    conv_fwd(xin, p + ".up_sample_conv", ch, 4, 2, 1, P(p + ".up_sample_conv.bias"), nullptr, 0, nullptr, nullptr, "", out, true);
+    tape.push_back([=]() {
+      Act dout = grad_written(out);
+      dgrad_convT(dout, p + ".up_sample_conv", ch, ch, xin);
+      wgrad(xin, dout, 4, 2, 1, p + ".up_sample_conv", nullptr, "", true);
+      bias_grad(dout, p + ".up_sample_conv.bias", "", nullptr, 0);
+    });
+  }
+
   // attention sub-layer (unet_base.py:153-161): out = x + out_proj(attn(in_proj(gn(x))))
   Act attention(const Act& x, const std::string& p, int l, int heads, const Act* dest) {
     const std::string ls = std::to_string(l);
     const std::string nn = p + ".attention_norms." + ls, ap = p + ".attentions." + ls;
     const int C = x.C, hd = C / heads, ntok = x.H * x.W;
-    Act a = new_act(x.H, x.W, C);
+    Act a = act(x.H, x.W, C);
     void* stn = gn_fwd(x, a, nn, 0);
     const size_t per = static_cast<size_t>(B) * ntok * C;
     auto* q = static_cast<__nv_bfloat16*>(bump.take(per * 2));
@@ -358,8 +404,8 @@ struct TBuilder {
     auto* vt = static_cast<__nv_bfloat16*>(bump.take(per * 2));
     auto* v = static_cast<__nv_bfloat16*>(bump.take(per * 2));
     float* lse = static_cast<float*>(bump.take(static_cast<size_t>(B) * heads * ntok * sizeof(float)));
-    Act o = new_act(x.H, x.W, C);
-    Act out = dest ? *dest : new_act(x.H, x.W, C);
+    Act o = act(x.H, x.W, C);
+    Act out = dest ? *dest : act(x.H, x.W, C);
     if (!dry) {
       WeightSrc w; w.w = P(ap + ".in_proj_weight"); w.d0 = 3 * C; w.d1 = C;
       ConvGeom g; g.K = 1; g.stride = 1; g.pad = 0; g.dil = 1;
@@ -381,7 +427,7 @@ struct TBuilder {
       wgrad(o, dout, 1, 1, 0, ap + ".out_proj", nullptr, "");
       bias_grad(dout, ap + ".out_proj.bias", "", nullptr, 0);
       Act d_o = grad(o);
-      Act dqkv = new_act(x.H, x.W, 3 * C);
+      Act dqkv = act(x.H, x.W, 3 * C);
       float* Dv = static_cast<float*>(bump.take(static_cast<size_t>(B) * heads * ntok * sizeof(float)));
       const int Bc = B;
       if (!dry) net->flops_bwd += attention_bwd_flops(B, heads, ntok, hd);
@@ -420,27 +466,16 @@ struct TBuilder {
   }
 };
 
-int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t st) {
-  const wc_unet_config& c = net->cfg;
-  const int B = net->B, H = net->H, W = net->W;
-  TBuilder b{net, dry ? Bump::dry() : Bump(ws, ws_bytes), net->arena.get(), st, dry, B};
-  const int nlev = c.n_down_channels - 1;
+int build(const wc_unet_train& cfg, const wc_unet_train::Geom& geo, wc_unet_train* net, cudaStream_t st, size_t* need) {
+  const wc_unet_config& c = cfg.cfg;
+  const int B = geo.B, H = geo.H, W = geo.W;
+  TBuilder b(net, B, st);
+  const bool dry = b.dry;
   const int* dc = c.down_channels;
   const int T = c.time_emb_dim;
 
   // ---- t-embedding layer table (execution order), concatenated projection
-  std::vector<std::pair<std::string, int>> tl;
-  for (int i = 0; i < nlev; ++i)
-    for (int l = 0; l < c.num_down_layers; ++l)
-      tl.push_back({"downs." + std::to_string(i) + ".t_emb_layers." + std::to_string(l) + ".1", dc[i + 1]});
-  for (int i = 0; i + 1 < c.n_mid_channels; ++i)
-    for (int l = 0; l < c.num_mid_layers + 1; ++l)
-      tl.push_back({"mids." + std::to_string(i) + ".t_emb_layers." + std::to_string(l) + ".1", c.mid_channels[i + 1]});
-  for (int j = 0; j < nlev; ++j) {
-    const int i = nlev - 1 - j;
-    for (int l = 0; l < c.num_up_layers; ++l)
-      tl.push_back({"ups." + std::to_string(j) + ".t_emb_layers." + std::to_string(l) + ".1", i != 0 ? dc[i - 1] : dc[0]});
-  }
+  const auto tl = temb_layers(c);
   int total = 0;
   for (auto& e : tl) total += e.second;
 
@@ -461,14 +496,15 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
   float* pred_ws = static_cast<float*>(b.bump.take(static_cast<size_t>(B) * c.im_channels * H * W * 4));
   void* mse_scratch = b.bump.take(8192);
   void* bw_scratch = b.bump.take(boundary_wgrad_scratch_bytes());
+  b.bw_scratch = bw_scratch;
 
-  float *wcat = nullptr, *bcat = nullptr, *w_out_t = nullptr, *w_in_t = nullptr;
+  float *wcat = nullptr, *bcat = nullptr, *w_out_t = nullptr;
   if (!dry) {
     wcat = static_cast<float*>(b.arena->alloc(static_cast<size_t>(total) * T * 4));
     bcat = static_cast<float*>(b.arena->alloc(static_cast<size_t>(total) * 4));
     w_out_t = static_cast<float*>(b.arena->alloc(static_cast<size_t>(dc[0]) * c.im_channels * 9 * 4));
-    w_in_t = static_cast<float*>(b.arena->alloc(static_cast<size_t>(dc[0]) * c.im_channels * 9 * 4));
-    if (!wcat || !bcat || !w_out_t || !w_in_t) return 1;
+    b.w_in_t = static_cast<float*>(b.arena->alloc(static_cast<size_t>(dc[0]) * c.im_channels * 9 * 4));
+    if (!wcat || !bcat || !w_out_t || !b.w_in_t) return 1;
     int off = 0;
     for (auto& e : tl) {
       const float *wsrc = b.P(e.first + ".weight"), *bsrc = b.P(e.first + ".bias");
@@ -491,132 +527,11 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
     });
   }
 
-  // ---- level geometry and concat buffers
-  std::vector<int> LH(nlev + 1), LW(nlev + 1);
-  LH[0] = H; LW[0] = W;
-  for (int i = 0; i < nlev; ++i) {
-    LH[i + 1] = c.down_sample[i] ? LH[i] / 2 : LH[i];
-    LW[i + 1] = c.down_sample[i] ? LW[i] / 2 : LW[i];
-  }
-  std::vector<Act> cat(nlev);
-  for (int i = 0; i < nlev; ++i) cat[i] = b.new_act(LH[i], LW[i], 2 * dc[i]);
-
-  // ---- conv_in
-  Act skip0 = slice_act(cat[0], dc[0], dc[0]);
-  if (!dry) {
-    const float *w = b.P("conv_in.weight"), *bias = b.P("conv_in.bias");
-    if (b.err) return b.err;
-    wc_unet_train* n = net;
-    const int cin = c.im_channels, c0 = dc[0];
-    b.push([=](cudaStream_t s) {
-      return conv_small_cin(n->x_in, w, bias, nullptr, nullptr, skip0.ptr, B, cin, H, W, c0, 3, 1, 1, skip0.ld, 0, s);
-    });
-    net->flops_fwd += 2.0 * B * H * W * 9.0 * cin * c0;
-  }
-  b.tape.push_back([&b, skip0, net, B, H, W, bw_scratch, w_in_t]() {
-    Act d = b.grad_written(skip0);
-    if (b.dry) return;
-    const float* w = b.P("conv_in.weight");
-    float *dw = b.G("conv_in.weight"), *db = b.G("conv_in.bias");
-    if (b.err) return;
-    wc_unet_train* n = net;
-    const int cin = net->cfg.im_channels, c0 = d.C;
-    b.push([=](cudaStream_t s) { return boundary_wgrad(d.ptr, d.ld, n->x_in, B, H, W, +1, dw, db, bw_scratch, s); }, kOpParam);
-    b.ready("conv_in.weight");
-    b.ready("conv_in.bias");
-    // dL/dx: the 64 -> 3 convolution of d(skip0) with the flipped, transposed conv_in weight (conv_out's forward kernel)
-    net->repack_ops.push_back([=](cudaStream_t s) { return flip_transpose_3x3(w, w_in_t, c0, cin, s); });
-    b.push([=](cudaStream_t s) {
-      return n->dx_out ? conv_small_cout(d.ptr, w_in_t, nullptr, n->dx_out, B, H, W, c0, cin, 3, d.ld, 0, s) : 0;
-    }, kOpInput);
-  });
-  Act cur = skip0;
-
-  auto use_attn = [&](int i) {
-    const int res = c.im_size >> i;
-    for (int k = 0; k < c.n_attn_resolutions; ++k)
-      if (c.attn_resolutions[k] == res) return true;
-    return false;
-  };
-
-  // ---- down path
-  for (int i = 0; i < nlev; ++i) {
-    const std::string p = "downs." + std::to_string(i);
-    const bool ua = use_attn(i);
-    const bool has_next_skip = (i + 1 != nlev);
-    Act next_skip;
-    if (has_next_skip) next_skip = slice_act(cat[i + 1], dc[i + 1], dc[i + 1]);
-    for (int l = 0; l < c.num_down_layers; ++l) {
-      const bool final_op = (l + 1 == c.num_down_layers) && !c.down_sample[i] && has_next_skip;
-      cur = b.resnet(cur, dc[i + 1], p, l, (final_op && !ua) ? &next_skip : nullptr);
-      if (ua) cur = b.attention(cur, p, l, c.num_heads, final_op ? &next_skip : nullptr);
-    }
-    if (c.down_sample[i]) {
-      Act out = has_next_skip ? next_skip : b.new_act(LH[i + 1], LW[i + 1], dc[i + 1]);
-      const Act xin = cur;
-      const int ch = dc[i + 1];
-      b.conv_fwd(xin, p + ".down_sample_conv", ch, 4, 2, 1, b.P(p + ".down_sample_conv.bias"), nullptr, 0, nullptr, nullptr, "", out);
-      b.tape.push_back([&b, xin, out, p, ch]() {
-        Act dout = b.grad_written(out);
-        b.dgrad(dout, p + ".down_sample_conv", ch, ch, 4, 2, xin);
-        b.wgrad(xin, dout, 4, 2, 1, p + ".down_sample_conv", nullptr, "");
-        b.bias_grad(dout, p + ".down_sample_conv.bias", "", nullptr, 0);
-      });
-      cur = out;
-    }
-    if (b.err) return b.err;
-  }
-
-  // ---- mid blocks
-  for (int i = 0; i + 1 < c.n_mid_channels; ++i) {
-    const std::string p = "mids." + std::to_string(i);
-    const int cout = c.mid_channels[i + 1];
-    const bool last_mid = (i + 2 == c.n_mid_channels);
-    const int top = nlev - 1;
-    const bool direct = last_mid && !c.down_sample[top];
-    Act dest = slice_act(cat[top], 0, dc[top]);
-    cur = b.resnet(cur, cout, p, 0, nullptr);
-    for (int l = 0; l < c.num_mid_layers; ++l) {
-      cur = b.attention(cur, p, l, c.num_heads, nullptr);
-      const bool final_op = direct && (l + 1 == c.num_mid_layers);
-      cur = b.resnet(cur, cout, p, l + 1, final_op ? &dest : nullptr);
-    }
-    if (b.err) return b.err;
-  }
-
-  // ---- up path
-  for (int j = 0; j < nlev; ++j) {
-    const int i = nlev - 1 - j;
-    const std::string p = "ups." + std::to_string(j);
-    const bool ua = use_attn(i);
-    const int cout = i != 0 ? dc[i - 1] : dc[0];
-    Act first_half = slice_act(cat[i], 0, dc[i]);
-    if (c.down_sample[i]) {
-      const Act xin = cur;
-      const int ch = dc[i];
-      b.conv_fwd(xin, p + ".up_sample_conv", ch, 4, 2, 1, b.P(p + ".up_sample_conv.bias"), nullptr, 0, nullptr, nullptr, "", first_half, true);
-      b.tape.push_back([&b, xin, first_half, p, ch]() {
-        Act dout = b.grad_written(first_half);
-        b.dgrad_convT(dout, p + ".up_sample_conv", ch, ch, xin);
-        b.wgrad(xin, dout, 4, 2, 1, p + ".up_sample_conv", nullptr, "", true);
-        b.bias_grad(dout, p + ".up_sample_conv.bias", "", nullptr, 0);
-      });
-    } else if (cur.ptr != first_half.ptr) {
-      return fail("internal: up block without up-sampling expects its input inside the concat buffer");
-    }
-    cur = cat[i];
-    const bool direct = (i > 0) && !c.down_sample[i - 1];
-    Act dest = direct ? slice_act(cat[i - 1], 0, dc[i - 1]) : Act();
-    for (int l = 0; l < c.num_up_layers; ++l) {
-      const bool final_op = direct && (l + 1 == c.num_up_layers);
-      cur = b.resnet(cur, cout, p, l, (final_op && !ua) ? &dest : nullptr);
-      if (ua) cur = b.attention(cur, p, l, c.num_heads, final_op ? &dest : nullptr);
-    }
-    if (b.err) return b.err;
-  }
+  Act cur = walk_unet(b, c, H, W);
+  if (b.err) return b.err;
 
   // ---- norm_out + SiLU + conv_out, MSE loss
-  Act fin = b.new_act(H, W, dc[0]);
+  Act fin = b.act(H, W, dc[0]);
   void* st_out = b.gn_fwd(cur, fin, "norm_out", 1);
   if (!dry) {
     const float *w = b.P("conv_out.weight"), *bias = b.P("conv_out.bias");
@@ -689,10 +604,7 @@ int build(wc_unet_train* net, bool dry, void* ws, size_t ws_bytes, cudaStream_t 
     for (auto& e : tl) { b.ready(e.first + ".weight"); b.ready(e.first + ".bias"); }
     b.ready("t_proj.0.weight"); b.ready("t_proj.0.bias"); b.ready("t_proj.2.weight"); b.ready("t_proj.2.bias");
   }
-  if (b.err) return b.err;
-  if (dry) net->ws_needed = b.bump.used() + 4096;
-  else if (b.bump.overflow()) return fail("UNet training workspace too small: need " + std::to_string(b.bump.used()) + " bytes");
-  return 0;
+  return b.finish("UNet training", need);
 }
 
 }  // namespace
@@ -705,11 +617,8 @@ extern "C" {
 int wc_unet_train_create(wc_unet_train** out, const wc_unet_config* cfg, int n_params, const char* const* names,
                          float* const* params, float* const* grads) {
   WC_REQUIRE(out && cfg && names && params && grads, "null argument");
-  WC_REQUIRE(cfg->im_channels == 3, "UNet boundary kernels support im_channels == 3");
-  WC_REQUIRE(cfg->n_down_channels >= 2 && cfg->n_down_channels <= 8 && cfg->n_mid_channels >= 2, "bad channel lists");
+  if (int e = check_unet_config(*cfg)) return e;
   WC_REQUIRE(cfg->down_channels[0] == 64, "the boundary weight-gradient kernels need down_channels[0] == 64");
-  for (int i = 0; i < cfg->n_down_channels; ++i) WC_REQUIRE(cfg->down_channels[i] % 64 == 0, "channels must be multiples of 64");
-  for (int i = 0; i < cfg->n_mid_channels; ++i) WC_REQUIRE(cfg->mid_channels[i] % 64 == 0, "channels must be multiples of 64");
   auto net = std::make_unique<wc_unet_train>();
   net->cfg = *cfg;
   for (int i = 0; i < n_params; ++i) {
@@ -723,49 +632,35 @@ int wc_unet_train_create(wc_unet_train** out, const wc_unet_config* cfg, int n_p
 void wc_unet_train_destroy(wc_unet_train* net) { delete net; }
 
 size_t wc_unet_train_workspace_bytes(wc_unet_train* net, int batch, int H, int W) {
-  const int sB = net->B, sH = net->H, sW = net->W;
-  net->B = batch; net->H = H; net->W = W;
-  size_t need = 0;
-  if (build(net, true, nullptr, 0, nullptr) == 0) need = net->ws_needed;
-  net->B = sB; net->H = sH; net->W = sW;
-  return need;
+  return plan_workspace_bytes(*net, {batch, H, W}, build);
 }
 
 int wc_unet_train_bind(wc_unet_train* net, int batch, int H, int W, void* workspace, size_t workspace_bytes, void* stream) {
   WC_REQUIRE(net && workspace, "null argument");
-  int div = 1;
-  for (int i = 0; i + 1 < net->cfg.n_down_channels; ++i) if (net->cfg.down_sample[i]) div *= 2;
-  WC_REQUIRE(H % div == 0 && W % div == 0, "H and W must be divisible by the total down-sampling factor");
-  net->repack_ops.clear(); net->fwd_ops.clear(); net->bwd_ops.clear(); net->bwd_kind.clear(); net->ready.clear();
-  net->arena = std::make_unique<DeviceArena>();
-  net->B = batch; net->H = H; net->W = W; net->ws = workspace; net->ws_bytes = workspace_bytes;
-  net->flops_fwd = net->flops_bwd = 0;
+  if (int e = check_unet_hw(net->cfg, H, W)) return e;
+  // always rebuilt: the weight-packing launches of the new plan are recorded into repack_ops
   set_pack_recorder(&net->repack_ops);
-  const int e = build(net, false, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+  const int e = bind(net, {batch, H, W}, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), build, true);
   set_pack_recorder(nullptr);
-  if (e) { net->B = 0; net->fwd_ops.clear(); net->bwd_ops.clear(); net->bwd_kind.clear(); net->repack_ops.clear(); }
   return e;
 }
 
 int wc_unet_train_forward(wc_unet_train* net, const float* x, const int64_t* t, const float* target, float* pred_out,
                           float* loss_out, float grad_scale, int repack, void* stream) {
-  WC_REQUIRE(net && net->B > 0, "wc_unet_train_forward: not bound");
+  WC_REQUIRE(net && net->geom.B > 0, "wc_unet_train_forward: not bound");
   WC_REQUIRE(x && t && (target ? loss_out != nullptr : pred_out != nullptr), "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   net->x_in = x; net->t_in = reinterpret_cast<const long long*>(t); net->target = target; net->pred_out = pred_out;
   net->loss_out = loss_out; net->grad_scale = grad_scale;
   if (repack)
-    for (auto& op : net->repack_ops)
-      if (int e = op(st)) return e;
-  for (auto& op : net->fwd_ops)
-    if (int e = op(st)) return e;
-  return 0;
+    if (int e = run_ops(net->repack_ops, st)) return e;
+  return run_ops(net->fwd_ops, st);
 }
 
 int wc_unet_train_num_backward_ops(const wc_unet_train* net) { return net ? static_cast<int>(net->bwd_ops.size()) : 0; }
 
 int wc_unet_train_backward(wc_unet_train* net, int op_begin, int op_end, void* stream) {
-  WC_REQUIRE(net && net->B > 0, "wc_unet_train_backward: not bound");
+  WC_REQUIRE(net && net->geom.B > 0, "wc_unet_train_backward: not bound");
   WC_REQUIRE(op_begin >= 0 && op_end <= static_cast<int>(net->bwd_ops.size()) && op_begin <= op_end, "bad op range");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   net->dpred_seed = nullptr;
@@ -776,7 +671,7 @@ int wc_unet_train_backward(wc_unet_train* net, int op_begin, int op_end, void* s
 }
 
 int wc_unet_train_backward_seeded(wc_unet_train* net, const float* dpred, float* dx, int param_grads, void* stream) {
-  WC_REQUIRE(net && net->B > 0, "wc_unet_train_backward_seeded: not bound");
+  WC_REQUIRE(net && net->geom.B > 0, "wc_unet_train_backward_seeded: not bound");
   WC_REQUIRE(dpred, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   net->dpred_seed = dpred;

@@ -200,20 +200,13 @@ int wc_conv2d_dgrad(const wc_bf16* dz, int batch, int Ho, int Wo, int Cout, cons
   Act out; out.ptr = BF(dx); out.B = batch; out.H = H; out.W = W; out.C = Cin; out.ld = Cin;
   Act res = out; res.ptr = const_cast<__nv_bfloat16*>(BF(residual));
   Act msk = out; msk.ptr = const_cast<__nv_bfloat16*>(BF(mask));
-  WeightSrc w; w.w = weight; w.d0 = Cout; w.d1 = Cin; w.KH = w.KW = K; w.transpose = 1;
+  WeightSrc w; w.w = weight; w.d0 = Cout; w.d1 = Cin; w.KH = w.KW = K;
+  ConvGeom gg; gg.K = K; gg.stride = stride; gg.dil = dil; gg.pad = stride == 1 ? dil * (K - 1) / 2 : (K == 3 ? 1 : 0);
   Epilogue ep; ep.res = residual ? &res : nullptr; ep.mask = mask ? &msk : nullptr;
   OutSpec os; os.mode = kOutNHWC; os.out = out;
-  int e;
-  if (stride == 1) {
-    w.flip = 1;
-    ConvGeom gg; gg.K = K; gg.stride = 1; gg.dil = dil; gg.pad = dil * (K - 1) / 2;
-    e = build_conv(&op, &arena, g, w, gg, Cin, nullptr, nullptr, ep, os, st);
-  } else {
-    if (!residual) WC_CHECK_CUDA(cudaMemsetAsync(out.ptr, 0, out.pixels() * Cin * 2, st));
-    e = build_conv_transposed_s2(&op, &arena, g, w, K, K == 3 ? 1 : 0, Cin, ep, os, st);
-  }
-  if (e) return e;
-  if ((e = op.run(st))) return e;
+  if (stride != 1 && !residual) WC_CHECK_CUDA(cudaMemsetAsync(out.ptr, 0, out.pixels() * Cin * 2, st));
+  if (int e = build_conv_dgrad(&op, &arena, g, w, gg, ep, os, st)) return e;
+  if (int e = op.run(st)) return e;
   WC_CHECK_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
