@@ -10,7 +10,7 @@
 //               the other group, so MUFU and tcgen05 overlap.
 // S, O and P live in TMEM (per query tile: BKV + hd fp32 columns, then BKV / 2 columns of bf16 pairs): the softmax threads write P
 // with tcgen05.st (lane = query row) and the PV tcgen05.mma reads it as its A operand; V is consumed as V^T[hd][keys] (K-major B
-// operand), which the QKV projection epilogue writes directly.  Head_dim 16 / 32 run on attention_small*.cu instead.  Online softmax with lazy rescaling (only when the running max grows
+// operand), which the QKV projection epilogue writes directly.  Head_dim 16 / 32 run on attention_small.cu instead.  Online softmax with lazy rescaling (only when the running max grows
 // by more than 2^8), accumulation in fp32.
 #include "wc_host.h"
 #include "wc_ptx.cuh"
@@ -26,10 +26,6 @@ struct AttnArgs {
   float scale_log2;  // log2(e) / sqrt(hd)
   __nv_bfloat16* out;
   float* lse;  // optional [B*heads][ntok]: log2-domain log-sum-exp of every row (saved for the backward pass)
-};
-
-struct AttnMaps {
-  CUtensorMap q, k, vt;
 };
 
 template <int HD, int BKV, int NQ>
@@ -346,23 +342,9 @@ template <int HD, int BKV, int NQ>
 int launch_attention(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
                      int heads, int ntok, int ldo, cudaStream_t st, float* lse, float scale) {
   using Cfg = AttnCfg<HD, BKV, NQ>;
-  AttnMaps maps;
   const int BH = B * heads;
-  const uint32_t inner = HD >= 64 ? 64 : HD;
-  {
-    uint64_t dims[3] = {static_cast<uint64_t>(HD), static_cast<uint64_t>(ntok), static_cast<uint64_t>(BH)};
-    uint64_t strides[3] = {1, static_cast<uint64_t>(HD), static_cast<uint64_t>(HD) * ntok};
-    uint32_t boxq[3] = {inner, 128, 1};
-    uint32_t boxk[3] = {inner, static_cast<uint32_t>(BKV), 1};
-    if (int e = encode_tmap_bf16(&maps.q, q, 3, dims, strides, boxq, Cfg::kSwz)) return e;
-    if (int e = encode_tmap_bf16(&maps.k, k, 3, dims, strides, boxk, Cfg::kSwz)) return e;
-  }
-  {
-    uint64_t dims[3] = {static_cast<uint64_t>(ntok), static_cast<uint64_t>(HD), static_cast<uint64_t>(BH)};
-    uint64_t strides[3] = {1, static_cast<uint64_t>(ntok), static_cast<uint64_t>(HD) * ntok};
-    uint32_t box[3] = {64, static_cast<uint32_t>(HD), 1};
-    if (int e = encode_tmap_bf16(&maps.vt, vt, 3, dims, strides, box, 128)) return e;
-  }
+  AttnMaps maps;
+  if (int e = encode_attn_maps(&maps, q, k, vt, BH, ntok, HD, BKV)) return e;
   AttnArgs args;
   args.ntok = ntok; args.heads = heads; args.ldo = ldo; args.out = out; args.lse = lse;
   args.scale_log2 = attn_scale_log2(scale, HD);
@@ -384,20 +366,30 @@ int launch_attention(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_
 
 int attention_small_forward(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
                             int heads, int ntok, int hd, int ldo, cudaStream_t st, float* lse, float scale);
-int attention_small4_forward(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
-                             int heads, int ntok, int hd, int ldo, cudaStream_t st, float* lse, float scale);
+
+int encode_attn_maps(AttnMaps* maps, const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, int BH, int ntok,
+                     int hd, int bkv) {
+  const uint32_t inner = hd >= 64 ? 64 : hd;
+  {
+    uint64_t dims[3] = {static_cast<uint64_t>(hd), static_cast<uint64_t>(ntok), static_cast<uint64_t>(BH)};
+    uint64_t strides[3] = {1, static_cast<uint64_t>(hd), static_cast<uint64_t>(hd) * ntok};
+    uint32_t boxq[3] = {inner, 128, 1};
+    uint32_t boxk[3] = {inner, static_cast<uint32_t>(bkv), 1};
+    if (int e = encode_tmap_bf16(&maps->q, q, 3, dims, strides, boxq, 2 * inner)) return e;
+    if (int e = encode_tmap_bf16(&maps->k, k, 3, dims, strides, boxk, 2 * inner)) return e;
+  }
+  uint64_t dims[3] = {static_cast<uint64_t>(ntok), static_cast<uint64_t>(hd), static_cast<uint64_t>(BH)};
+  uint64_t strides[3] = {1, static_cast<uint64_t>(ntok), static_cast<uint64_t>(hd) * ntok};
+  uint32_t box[3] = {64, static_cast<uint32_t>(hd), 1};
+  return encode_tmap_bf16(&maps->vt, vt, 3, dims, strides, box, 128);
+}
 
 // q,k [B,heads,ntok,hd]; vt [B,heads,hd,ntok]; out [B,ntok,ldo] (columns head*hd .. head*hd+hd).
 int attention_forward(const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, __nv_bfloat16* out, int B,
                       int heads, int ntok, int hd, int ldo, cudaStream_t st, float* lse, float scale) {
   WC_REQUIRE(ntok % 8 == 0, "token count must be a multiple of 8");
   WC_REQUIRE(ldo % 8 == 0, "output row stride must be a multiple of 8");
-  // Measured on B200 (batch 32, N 8192): head_dim 16 2.42 -> 2.24 ms with four softmax groups per CTA (attention_small4.cu) instead of
-  // three with a double-buffered S (attention_small.cu).  Four groups cover 512 queries: shorter sequences keep the 3-group kernel.
-  if (hd == 16 || hd == 32) {
-    if (ntok >= 2048) return attention_small4_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
-    return attention_small_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
-  }
+  if (hd == 16 || hd == 32) return attention_small_forward(q, k, vt, out, B, heads, ntok, hd, ldo, st, lse, scale);
   switch (hd) {
     case 64: return launch_attention<64, 128, 2>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);
     case 128: return launch_attention<128, 64, 2>(q, k, vt, out, B, heads, ntok, ldo, st, lse, scale);

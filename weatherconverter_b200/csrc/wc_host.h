@@ -124,4 +124,12 @@ struct Act {
 int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_elems,
                      const uint32_t* box, uint32_t swizzle_bytes);
 
+// Tensor maps of the attention forward kernels' operands: q, k [BH][ntok][hd] in boxes of 128 query / bkv key rows of
+// min(hd, 64) elements (swizzle span = one box row); vt [BH][hd][ntok] in boxes of 64 keys x hd, 128-byte swizzle.
+struct AttnMaps {
+  CUtensorMap q, k, vt;
+};
+int encode_attn_maps(AttnMaps* maps, const __nv_bfloat16* q, const __nv_bfloat16* k, const __nv_bfloat16* vt, int BH, int ntok,
+                     int hd, int bkv);
+
 }  // namespace wc
