@@ -31,41 +31,6 @@ void set_pack_recorder(std::vector<std::function<int(cudaStream_t)>>* recorder) 
 
 namespace {
 
-// Residual stream epilogue (igemm.cu, LEAN == 3) for layers with a residual input and a short main loop: K <= 768, plain mode, no
-// ReLU mask, no PReLU / GELU, full N tiles that are multiples of 64.  Layers with a ReLU-mask input (segmentor data gradients) stream
-// the mask rows the same way.
-constexpr int kStreamLoadSlots = 3;   // load buffers per epilogue warp (fewer when the ring would get too short)
-constexpr int kStreamMaxKb = 12;      // longest main loop (in 64-channel blocks) that still takes the stream epilogue (12 / 16 / 40 /
-                                      // unlimited measured equal on C3: 21.30 - 21.32 ms)
-constexpr int kStreamMinStages = 2;   // these layers are epilogue-bound: a short ring suffices
-void apply_res_deep(IgemmPlan* plan, int N, bool res_candidate) {
-  IgemmArgs& a = plan->args;
-  a.res_deep = 0;
-  const bool mask_candidate = a.stream_mask == 2;
-  a.stream_mask = 0;
-  a.stream_res = 0;
-  if (!a.tma_store || a.row3 || a.prelu || a.act == 3 || a.phase_n || a.total_kb > kStreamMaxKb || a.BN % 64 != 0 ||
-      N % a.BN != 0 || a.out_mode != kOutNHWC)
-    return;
-  if (a.res && !res_candidate) return;             // a residual that cannot go through TMA
-  if (a.mask && !mask_candidate) return;
-  const int nbox = (a.res ? 1 : 0) + (a.mask ? 1 : 0);
-  if (nbox == 0) return;
-  for (int nl = kStreamLoadSlots; nl >= 2; --nl) {
-    const int ns = igemm_res_deep_stages(a.BN, nl * nbox);
-    if (ns >= 2 && ns >= (a.total_kb < kStreamMinStages ? a.total_kb + 1 : kStreamMinStages)) {
-      a.res_deep = nl;
-      a.stream_res = a.res ? 1 : 0;
-      a.stream_mask = a.mask ? 1 : 0;
-      a.nstages = ns;
-      a.tma_res = a.res ? 1 : 0;
-      a.stage2 = 1;
-      a.lean = 3;
-      return;
-    }
-  }
-}
-
 struct TapDef {
   int map, dy, dx;
   const WeightSrc* w;
@@ -76,14 +41,16 @@ struct TapDef {
 int out_channels_of(const WeightSrc& w) { return w.transpose ? w.d1 : w.d0; }
 int in_channels_of(const WeightSrc& w) { return w.transpose ? w.d0 : w.d1; }
 
-// Pack weights for a tap list and fill everything of the plan except the A tensor maps.
+// Pack weights for a tap list and fill everything of the plan except the A tensor maps and what igemm_select decides.
+// *res_map / *mask_map: the residual / ReLU-mask maps were encoded for the TMA epilogue.
 int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& taps, int B, int H, int W, int tb,
                 int th, int tw, int N, const Epilogue& ep, const OutSpec& out, int sy, int sx, int py, int px,
-                cudaStream_t st) {
+                cudaStream_t st, bool* res_map, bool* mask_map) {
   WC_REQUIRE(N % 16 == 0, "igemm needs N % 16 == 0 (pad the output channels)");
   WC_REQUIRE(static_cast<int>(taps.size()) <= kMaxTaps && !taps.empty(), "tap count out of range");
   IgemmArgs& a = plan->args;
   a = IgemmArgs{};
+  *res_map = *mask_map = false;
   a.B = B; a.H = H; a.W = W; a.tb = tb; a.th = th; a.tw = tw;
   a.N = N;
   int total_kb = 0;
@@ -190,11 +157,11 @@ int finish_plan(IgemmPlan* plan, DeviceArena* arena, const std::vector<TapDef>& 
         a.tma_store = 1;
         if (ep.res && ep.res->ld % 8 == 0) {
           if (int e = igemm_make_cmap(&plan->maps.r, *ep.res, N, nc, a.qw, a.qh, a.qb, sy, sx, py, px)) return e;
-          a.tma_res = 2;   // candidate: confirmed by the caller once the ring depth is known
+          *res_map = true;
         }
         if (ep.mask && ep.mask->ld % 8 == 0) {
           if (int e = igemm_make_cmap(&plan->maps.m, *ep.mask, N, nc, a.qw, a.qh, a.qb, sy, sx, py, px)) return e;
-          a.stream_mask = 2;   // candidate for the stream epilogue
+          *mask_map = true;
         }
       }
     }
@@ -254,7 +221,7 @@ int build_conv(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w,
   op->plans.emplace_back();
   IgemmPlan& plan = op->plans.back();
   std::vector<TapDef> taps;
-  bool want_row3 = false;
+  int window = 0;
   int B = x.B, H, W, tb, th, tw;
   if (g.stride == 1) {
     WC_REQUIRE(2 * g.pad == g.dil * (g.K - 1), "stride-1 convolutions must be 'same' sized");
@@ -275,7 +242,7 @@ int build_conv(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w,
     // Row-segment mode: 3x3 / dilation 1 on maps at least 128 pixels wide with narrow N (the L2->SM bound layers)
     if (g.K == 3 && g.dil == 1 && tw == 128 && th == 1 && tb == 1 && (N <= 128 || (out.bn_max > 0 && out.bn_max <= 128))) {
       if (int e = igemm_make_rowseg_map(&plan.maps.a[2], x)) return e;
-      want_row3 = true;
+      window = 3;
     }
   } else {
     WC_REQUIRE(g.stride == 2 && g.dil == 1 && !x2, "only stride 1 or 2 (undilated, unfused) supported");
@@ -293,17 +260,12 @@ int build_conv(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSrc& w,
         taps.push_back({py * 2 + px, (oy - py) / 2, (ox - px) / 2, &w, ky, kx, x.C});
       }
   }
-  if (int e = finish_plan(&plan, arena, taps, B, H, W, tb, th, tw, N, ep, out, out.up, out.up, out.py, out.px, st)) return e;
-  plan.args.row3 = (want_row3 && plan.args.BN <= 128) ? 1 : 0;
-  plan.args.row_nky = plan.args.row_nkx = 3;
+  bool res_map, mask_map;
+  if (int e = finish_plan(&plan, arena, taps, B, H, W, tb, th, tw, N, ep, out, out.up, out.up, out.py, out.px, st, &res_map, &mask_map))
+    return e;
   // (resident weights do not pay here: measured on B200 (batch 32, 64 x 128) 3x3 64->64 in row-segment mode 34.7 -> 40.9 us, 1x1
   // 256->64 37.2 -> 35.9 us, 1x1 64->256 unchanged, although they cut the L2->SM traffic of the 3x3 layer 2.4x)
-  plan.args.nstages = igemm_stages_for(plan.args.BN, plan.args.row3);
-  plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, plan.args.row3, plan.args.nstages) ? 1 : 0;
-  const bool res_candidate = plan.args.tma_res == 2;
-  plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-  plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
-  apply_res_deep(&plan, N, res_candidate);
+  igemm_select(&plan, window, 0, res_map, mask_map, true);
   op->flops = plan.flops;
   return 0;
 }
@@ -336,12 +298,9 @@ int build_conv_stem7s2(ConvOp* op, DeviceArena* arena, const __nv_bfloat16* xp, 
     const int o = ky - 3, dy = (o >= 0) ? o / 2 : -((-o + 1) / 2), ph = o - 2 * dy;   // o = 2 dy + ph, ph in {0, 1}
     taps.push_back({ph, dy, 0, &w, ky, 0, 64});
   }
-  if (int e = finish_plan(&plan, arena, taps, B, Ho, Wo, tb, th, tw, N, ep, out, 1, 1, 0, 0, st)) return e;
-  plan.args.row3 = 0;
-  plan.args.nstages = igemm_stages_for(plan.args.BN, 0);
-  plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, 0, plan.args.nstages) ? 1 : 0;
-  plan.args.tma_res = 0;
-  plan.args.lean = (plan.args.tma_store && !plan.args.mask && !plan.args.res) ? 1 : 0;
+  bool res_map, mask_map;
+  if (int e = finish_plan(&plan, arena, taps, B, Ho, Wo, tb, th, tw, N, ep, out, 1, 1, 0, 0, st, &res_map, &mask_map)) return e;
+  igemm_select(&plan, 0, 0, res_map, mask_map, false);
   plan.flops = 2.0 * 147.0 * N * static_cast<double>(B) * Ho * Wo;   // algorithmic (the reference's 7x7x3 taps), not the padded K
   op->flops = plan.flops;
   return 0;
@@ -364,30 +323,20 @@ int build_conv_hrow(ConvOp* op, DeviceArena* arena, const Act& x, const WeightSr
   for (int i = 1; i < kMaxMaps; ++i) plan.maps.a[i] = plan.maps.a[0];
   std::vector<TapDef> taps;
   for (int kx = 0; kx < w.KW; ++kx) taps.push_back({0, 0, kx - w.KW / 2, &w, 0, kx, x.C});
-  if (int e = finish_plan(&plan, arena, taps, x.B, x.H, x.W, tb, th, tw, N, ep, out, 1, 1, 0, 0, st)) return e;
+  bool res_map, mask_map;
+  if (int e = finish_plan(&plan, arena, taps, x.B, x.H, x.W, tb, th, tw, N, ep, out, 1, 1, 0, 0, st, &res_map, &mask_map)) return e;
   // Row-segment mode with all KW taps in one stage: one box of 128 + KW - 1 pixels per tile instead of KW boxes of 128, one barrier
   // hand-over per tile instead of KW
-  plan.args.row3 = 0;
-  plan.args.row_nky = 1; plan.args.row_nkx = w.KW;
   // (the kernel is instantiated for 3 x 3 and 1 x 9 windows: other widths keep one stage per tap)
-  if (w.KW == 9 && tw == 128 && th == 1 && tb == 1 && plan.args.BN <= 128 && igemm_stages_for(plan.args.BN, 1, 0, w.KW) >= 2) {
+  int window = 0;
+  if (w.KW == 9 && tw == 128 && th == 1 && tb == 1) {
     if (int e = igemm_make_rowseg_map(&plan.maps.a[2], x, w.KW)) return e;
-    plan.args.row3 = 1;
+    window = 9;
   }
-  // the packed weights of all taps (KW x BN x 64 bf16) are the same for every tile: keep them resident (one load per CTA) when this
-  // is a single N tile - the ring then carries activations only
-  int wres_bytes = 0;
-  {
-    const long wb = static_cast<long>(plan.args.BN) * plan.args.total_kb * kIgemmBK * 2;
-    if (plan.args.row3 && plan.args.BN >= N && wb <= kIgemmWresMaxBytes) {
-      plan.args.wres = 1;
-      wres_bytes = static_cast<int>(wb);
-    }
-  }
-  plan.args.nstages = igemm_stages_for(plan.args.BN, plan.args.row3, wres_bytes, w.KW);
-  plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, plan.args.row3, plan.args.nstages, wres_bytes, w.KW) ? 1 : 0;
-  plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-  plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
+  // the packed weights of all taps (KW x BN x 64 bf16) are the same for every tile: keep them resident in row-segment mode (one load
+  // per CTA) when this is a single N tile - the ring then carries activations only
+  const long wb = static_cast<long>(plan.args.BN) * plan.args.total_kb * kIgemmBK * 2;
+  igemm_select(&plan, window, plan.args.BN >= N && wb <= kIgemmWresMaxBytes ? static_cast<int>(wb) : 0, res_map, mask_map, false);
   op->flops = plan.flops;
   return 0;
 }
@@ -411,11 +360,9 @@ int build_conv_transposed_s2(ConvOp* op, DeviceArena* arena, const Act& x, const
       IgemmPlan& plan = op->plans.back();
       if (int e = igemm_make_amap(&plan.maps.a[0], x, tb, th, tw)) return e;
       for (int i = 1; i < kMaxMaps; ++i) plan.maps.a[i] = plan.maps.a[0];
-      if (int e = finish_plan(&plan, arena, taps, x.B, x.H, x.W, tb, th, tw, N, ep, out, 2, 2, qy, qx, st)) return e;
-      plan.args.nstages = igemm_stages_for(plan.args.BN, 0);
-      plan.args.stage2 = igemm_res_staging_fits(plan.args.BN, 0, plan.args.nstages) ? 1 : 0;
-      plan.args.tma_res = (plan.args.tma_res == 2 && plan.args.stage2) ? 1 : 0;
-      plan.args.lean = (plan.args.tma_store && !plan.args.mask && (!plan.args.res || plan.args.tma_res)) ? 1 : 0;
+      bool res_map, mask_map;
+      if (int e = finish_plan(&plan, arena, taps, x.B, x.H, x.W, tb, th, tw, N, ep, out, 2, 2, qy, qx, st, &res_map, &mask_map)) return e;
+      igemm_select(&plan, 0, 0, res_map, mask_map, false);
       op->flops += plan.flops;
     }
   return 0;

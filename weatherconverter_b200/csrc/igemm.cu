@@ -10,7 +10,7 @@ namespace {
 constexpr int kThreads = 320;  // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue (two groups of 4, one per TMEM lane quadrant)
 constexpr uint32_t kABytes = kIgemmBM * kIgemmBK * 2;  // 16 KiB
 constexpr uint32_t kPipeBytes = 212992;  // shared-memory budget of the TMA ring (both modes), multiple of 1024; its last 16 KiB double as
-                                         // the residual staging of the TMA epilogue when the ring leaves them free (igemm_res_staging_fits)
+                                         // the residual staging of the TMA epilogue when the ring leaves them free (res_staging_fits)
 constexpr int kMaxStages = 8;
 // bias / PReLU vectors up to this many channels are staged in shared memory (wider layers: L1-cached broadcast loads); the two
 // limits are what is left of the 227 KiB after the ring, the output staging, the barriers and the alignment slack
@@ -34,6 +34,113 @@ template <int NC>
 __device__ __forceinline__ void tmem_ld_n(uint32_t taddr, uint32_t (&r)[NC]) {
   if constexpr (NC == 32) tmem_ld32(taddr, r);
   else tmem_ld16(taddr, r);
+}
+
+// ---- per-chunk epilogue steps: one thread holds v[NC], the NC channels of its pixel row in the current chunk
+
+// Row `lane` of a staged box keeps 16-byte chunk j at j ^ swizzle(row): 64-byte rows -> XOR with bits 1..2 of the row (SWIZZLE_64B),
+// 32-byte rows -> XOR with bit 2 (SWIZZLE_32B); conflict-free per quarter warp
+template <int NC>
+__device__ __forceinline__ uint32_t chunk_swizzle(int lane) { return NC == 32 ? ((lane >> 1) & 3) : ((lane >> 2) & 1); }
+
+// v as bf16 into the swizzled row at shared address `row`
+template <int NV>
+__device__ __forceinline__ void st_row_swz(uint32_t row, uint32_t sw, const float* v) {
+#pragma unroll
+  for (int j = 0; j < NV; ++j)
+    asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(row + ((static_cast<uint32_t>(j) ^ sw) << 4)),
+                 "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
+                 "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
+}
+
+// the swizzled bf16 row at shared address `row` (a residual or ReLU-mask box landed by TMA)
+template <int NV>
+__device__ __forceinline__ void ld_row_swz(uint32_t row, uint32_t sw, uint4 (&u)[NV]) {
+#pragma unroll
+  for (int j = 0; j < NV; ++j)
+    asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(u[j].x), "=r"(u[j].y), "=r"(u[j].z), "=r"(u[j].w)
+                 : "r"(row + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
+}
+
+// v += a bf16 row (residual)
+template <int NV>
+__device__ __forceinline__ void add_bf16_row(float* v, const uint4 (&u)[NV]) {
+#pragma unroll
+  for (int j = 0; j < NV; ++j) {
+    const float2 f0 = unpack_bf16(u[j].x), f1 = unpack_bf16(u[j].y), f2 = unpack_bf16(u[j].z), f3 = unpack_bf16(u[j].w);
+    v[8 * j + 0] += f0.x; v[8 * j + 1] += f0.y; v[8 * j + 2] += f1.x; v[8 * j + 3] += f1.y;
+    v[8 * j + 4] += f2.x; v[8 * j + 5] += f2.y; v[8 * j + 6] += f3.x; v[8 * j + 7] += f3.y;
+  }
+}
+
+// v := 0 where the bf16 row (the forward activation) is <= 0: the ReLU derivative of the data gradients
+template <int NV>
+__device__ __forceinline__ void mask_bf16_row(float* v, const uint4 (&u)[NV]) {
+#pragma unroll
+  for (int j = 0; j < NV; ++j) {
+    const float2 f0 = unpack_bf16(u[j].x), f1 = unpack_bf16(u[j].y), f2 = unpack_bf16(u[j].z), f3 = unpack_bf16(u[j].w);
+    if (!(f0.x > 0.f)) v[8 * j + 0] = 0.f;
+    if (!(f0.y > 0.f)) v[8 * j + 1] = 0.f;
+    if (!(f1.x > 0.f)) v[8 * j + 2] = 0.f;
+    if (!(f1.y > 0.f)) v[8 * j + 3] = 0.f;
+    if (!(f2.x > 0.f)) v[8 * j + 4] = 0.f;
+    if (!(f2.y > 0.f)) v[8 * j + 5] = 0.f;
+    if (!(f3.x > 0.f)) v[8 * j + 6] = 0.f;
+    if (!(f3.y > 0.f)) v[8 * j + 7] = 0.f;
+  }
+}
+
+// ReLU, then SiLU (act 2) or GELU (act 3)
+template <int NC>
+__device__ __forceinline__ void relu_act(float* v, int relu, int act) {
+  if (relu) {
+#pragma unroll
+    for (int j = 0; j < NC; ++j) v[j] = fmaxf(v[j], 0.f);
+  }
+  if (act == 2) {
+#pragma unroll
+    for (int j = 0; j < NC; ++j) v[j] = __fdividef(v[j], 1.f + __expf(-v[j]));
+  } else if (act == 3) {
+#pragma unroll
+    for (int j = 0; j < NC; ++j) v[j] = 0.5f * v[j] * (1.f + erff(v[j] * 0.70710678118654752f));
+  }
+}
+
+// v += bias (from shared memory when staged there, else global) + row bias (rb: this sample's t-embedding row, or nullptr).
+// This and prelu read the global vector from p inside the branch: passing the pointer in hoists its load and changes the code.
+template <int NC>
+__device__ __forceinline__ void add_bias(float* v, const float* s_bias, const IgemmArgs& p, const float* rb, int nb) {
+  if (s_bias) {
+#pragma unroll
+    for (int j = 0; j < NC; j += 4) {
+      const float4 bv = *reinterpret_cast<const float4*>(s_bias + nb + j);
+      v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
+    }
+  } else if (p.bias) {
+#pragma unroll
+    for (int j = 0; j < NC; j += 4) {
+      const float4 bv = __ldg(reinterpret_cast<const float4*>(p.bias + nb + j));
+      v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
+    }
+  }
+  if (rb) {
+#pragma unroll
+    for (int j = 0; j < NC; j += 4) {
+      const float4 bv = __ldg(reinterpret_cast<const float4*>(rb + nb + j));
+      v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
+    }
+  }
+}
+
+// PReLU with per-channel slopes (from shared memory when staged there, else global)
+template <int NC>
+__device__ __forceinline__ void prelu(float* v, const float* s_prelu, const IgemmArgs& p, int nb) {
+#pragma unroll
+  for (int j = 0; j < NC; j += 4) {
+    const float4 sv = s_prelu ? *reinterpret_cast<const float4*>(s_prelu + nb + j) : __ldg(reinterpret_cast<const float4*>(p.prelu + nb + j));
+    v[j] = v[j] > 0.f ? v[j] : v[j] * sv.x; v[j + 1] = v[j + 1] > 0.f ? v[j + 1] : v[j + 1] * sv.y;
+    v[j + 2] = v[j + 2] > 0.f ? v[j + 2] : v[j + 2] * sv.z; v[j + 3] = v[j + 3] > 0.f ? v[j + 3] : v[j + 3] * sv.w;
+  }
 }
 
 // Epilogue of one accumulator tile for one thread (= one output pixel row of the tile).  `grp` in {0,1}: the two
@@ -83,12 +190,7 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
     if (tma_res) {
       mbar_wait(res_bar, res_phase);
       res_phase ^= 1u;
-      const uint32_t mine = res_stage + lane * (NC * 2);
-      const uint32_t sw = NC == 32 ? ((lane >> 1) & 3) : ((lane >> 2) & 1);
-#pragma unroll
-      for (int j = 0; j < NV; ++j)
-        asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(res_cur[j].x), "=r"(res_cur[j].y), "=r"(res_cur[j].z), "=r"(res_cur[j].w)
-                     : "r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
+      ld_row_swz<NV>(res_stage + lane * (NC * 2), chunk_swizzle<NC>(lane), res_cur);
       // Cross-proxy WAR: the lanes read the staging buffer through the generic proxy and the NEXT residual box is written
       // into the same bytes by the TMA (async proxy).  Without this fence the two are unordered, and on B200 the next box
       // did overtake the reads whenever the epilogue was the bottleneck (1x1 convolutions with several tiles per CTA: a
@@ -103,6 +205,7 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
     float v[NC];
 #pragma unroll
     for (int j = 0; j < NC; ++j) v[j] = __uint_as_float(r[j]);
+    // bias and row bias stay written out here: add_bias<NC> changes the code of six generic instantiations (and the spills of one)
     if (p.bias) {
 #pragma unroll
       for (int j = 0; j < NC; j += 4) {
@@ -119,63 +222,15 @@ __device__ __forceinline__ void epilogue_tile(const IgemmArgs& p, uint32_t tacc,
         v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
       }
     }
-    if (p.res) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) {
-        const uint4 u = res_cur[j];
-        float2 f0 = unpack_bf16(u.x), f1 = unpack_bf16(u.y), f2 = unpack_bf16(u.z), f3 = unpack_bf16(u.w);
-        v[8 * j + 0] += f0.x; v[8 * j + 1] += f0.y; v[8 * j + 2] += f1.x; v[8 * j + 3] += f1.y;
-        v[8 * j + 4] += f2.x; v[8 * j + 5] += f2.y; v[8 * j + 6] += f3.x; v[8 * j + 7] += f3.y;
-      }
-    }
-    if (p.relu) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = fmaxf(v[j], 0.f);
-    }
-    if (p.act == 2) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = __fdividef(v[j], 1.f + __expf(-v[j]));
-    } else if (p.act == 3) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = 0.5f * v[j] * (1.f + erff(v[j] * 0.70710678118654752f));
-    }
-    if (p.prelu) {
-#pragma unroll
-      for (int j = 0; j < NC; j += 4) {
-        const float4 sv = s_prelu ? *reinterpret_cast<const float4*>(s_prelu + nb + j)
-                                  : __ldg(reinterpret_cast<const float4*>(p.prelu + nb + j));
-        v[j] = v[j] > 0.f ? v[j] : v[j] * sv.x; v[j + 1] = v[j + 1] > 0.f ? v[j + 1] : v[j + 1] * sv.y;
-        v[j + 2] = v[j + 2] > 0.f ? v[j + 2] : v[j + 2] * sv.z; v[j + 3] = v[j + 3] > 0.f ? v[j + 3] : v[j + 3] * sv.w;
-      }
-    }
-    if (p.mask) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) {
-        const uint4 u = mask_cur[j];
-        float2 f0 = unpack_bf16(u.x), f1 = unpack_bf16(u.y), f2 = unpack_bf16(u.z), f3 = unpack_bf16(u.w);
-        if (!(f0.x > 0.f)) v[8 * j + 0] = 0.f;
-        if (!(f0.y > 0.f)) v[8 * j + 1] = 0.f;
-        if (!(f1.x > 0.f)) v[8 * j + 2] = 0.f;
-        if (!(f1.y > 0.f)) v[8 * j + 3] = 0.f;
-        if (!(f2.x > 0.f)) v[8 * j + 4] = 0.f;
-        if (!(f2.y > 0.f)) v[8 * j + 5] = 0.f;
-        if (!(f3.x > 0.f)) v[8 * j + 6] = 0.f;
-        if (!(f3.y > 0.f)) v[8 * j + 7] = 0.f;
-      }
-    }
+    if (p.res) add_bf16_row<NV>(v, res_cur);
+    relu_act<NC>(v, p.relu, p.act);
+    if (p.prelu) prelu<NC>(v, s_prelu, p, nb);
+    if (p.mask) mask_bf16_row<NV>(v, mask_cur);
     if constexpr (tma_out) {
       // the previous chunk's store must have finished READING the staging buffer
-      if (lane == 0) tma_store_wait_read0();
+      if (lane == 0) tma_store_wait_read<0>();
       __syncwarp();
-      // row `lane` of the box, 16-byte chunk j at j ^ swizzle(row): 64-byte rows -> XOR with bits 1..2 of the row (SWIZZLE_64B),
-      // 32-byte rows -> XOR with bit 2 (SWIZZLE_32B); conflict-free per quarter warp
-      const uint32_t mine = out_stage + lane * (NC * 2);
-      const uint32_t sw = NC == 32 ? ((lane >> 1) & 3) : ((lane >> 2) & 1);
-#pragma unroll
-      for (int j = 0; j < NV; ++j)
-        asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)),
-                     "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
-                     "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
+      st_row_swz<NV>(out_stage + lane * (NC * 2), chunk_swizzle<NC>(lane), v);
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
@@ -259,7 +314,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
                                                    uint32_t& ectr, const CUtensorMap* qkv_maps = nullptr) {
   constexpr int NV = NC / 8;
   const int lane = threadIdx.x & 31;
-  const uint32_t sw = NC == 32 ? ((lane >> 1) & 3) : ((lane >> 2) & 1);
+  const uint32_t sw = chunk_swizzle<NC>(lane);
   const uint32_t row_off = static_cast<uint32_t>(lane) * (NC * 2);
   auto buf_of = [&](uint32_t i) { return ((i & 1u) && nbuf == 2) ? buf1 : buf0; };
   auto request = [&](uint32_t i, int nb) {   // residual box of chunk i (channels nb ..) -> its staging buffer
@@ -284,10 +339,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
     if (RES) {
       mbar_wait(res_bar, res_phase);
       res_phase ^= 1u;
-#pragma unroll
-      for (int j = 0; j < NV; ++j)
-        asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(rr[j].x), "=r"(rr[j].y), "=r"(rr[j].z), "=r"(rr[j].w)
-                     : "r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
+      ld_row_swz<NV>(mine, sw, rr);
       // the next box goes into the OTHER buffer (last touched, through the generic proxy, one chunk ago and fenced then)
       if (c0 + 2 * NC < p.BN && nb + 2 * NC < p.N) request(ectr + 1, nb + 2 * NC);
     }
@@ -295,54 +347,10 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
     float v[NC];
 #pragma unroll
     for (int j = 0; j < NC; ++j) v[j] = __uint_as_float(r[j]);
-    if (s_bias) {
-#pragma unroll
-      for (int j = 0; j < NC; j += 4) {
-        const float4 bv = *reinterpret_cast<const float4*>(s_bias + nb + j);
-        v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-      }
-    } else if (p.bias) {
-#pragma unroll
-      for (int j = 0; j < NC; j += 4) {
-        const float4 bv = __ldg(reinterpret_cast<const float4*>(p.bias + nb + j));
-        v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-      }
-    }
-    if (rb) {
-#pragma unroll
-      for (int j = 0; j < NC; j += 4) {
-        const float4 bv = __ldg(reinterpret_cast<const float4*>(rb + nb + j));
-        v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-      }
-    }
-    if (RES) {
-#pragma unroll
-      for (int j = 0; j < NV; ++j) {
-        const float2 f0 = unpack_bf16(rr[j].x), f1 = unpack_bf16(rr[j].y), f2 = unpack_bf16(rr[j].z), f3 = unpack_bf16(rr[j].w);
-        v[8 * j + 0] += f0.x; v[8 * j + 1] += f0.y; v[8 * j + 2] += f1.x; v[8 * j + 3] += f1.y;
-        v[8 * j + 4] += f2.x; v[8 * j + 5] += f2.y; v[8 * j + 6] += f3.x; v[8 * j + 7] += f3.y;
-      }
-    }
-    if (p.relu) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = fmaxf(v[j], 0.f);
-    }
-    if (p.act == 2) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = __fdividef(v[j], 1.f + __expf(-v[j]));
-    } else if (p.act == 3) {
-#pragma unroll
-      for (int j = 0; j < NC; ++j) v[j] = 0.5f * v[j] * (1.f + erff(v[j] * 0.70710678118654752f));
-    }
-    if (p.prelu) {
-#pragma unroll
-      for (int j = 0; j < NC; j += 4) {
-        const float4 sv = s_prelu ? *reinterpret_cast<const float4*>(s_prelu + nb + j)
-                                  : __ldg(reinterpret_cast<const float4*>(p.prelu + nb + j));
-        v[j] = v[j] > 0.f ? v[j] : v[j] * sv.x; v[j + 1] = v[j + 1] > 0.f ? v[j + 1] : v[j + 1] * sv.y;
-        v[j + 2] = v[j + 2] > 0.f ? v[j + 2] : v[j + 2] * sv.z; v[j + 3] = v[j + 3] > 0.f ? v[j + 3] : v[j + 3] * sv.w;
-      }
-    }
+    add_bias<NC>(v, s_bias, p, rb, nb);
+    if (RES) add_bf16_row<NV>(v, rr);
+    relu_act<NC>(v, p.relu, p.act);
+    if (p.prelu) prelu<NC>(v, s_prelu, p, nb);
     if (!RES) {   // the store that last read this buffer (two chunks ago with two buffers, the previous one otherwise)
       if (lane == 0) {
         if (nbuf == 2) tma_store_wait_read<1>();
@@ -388,11 +396,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
                          "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
                          "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
         } else {
-#pragma unroll
-          for (int j = 0; j < NV; ++j)
-            asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)),
-                         "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
-                         "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
+          st_row_swz<NV>(mine, sw, v);
         }
       } else {
 #pragma unroll
@@ -424,11 +428,7 @@ __device__ __forceinline__ void epilogue_tile_lean(const IgemmArgs& p, uint32_t 
       ++ectr;
       continue;
     }
-#pragma unroll
-    for (int j = 0; j < NV; ++j)
-      asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(mine + ((static_cast<uint32_t>(j) ^ sw) << 4)),
-                   "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
-                   "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
+    st_row_swz<NV>(mine, sw, v);
     fence_proxy_async_smem();
     __syncwarp();
     if (lane == 0) {
@@ -738,9 +738,10 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
       const uint32_t tacc = tmem_base + static_cast<uint32_t>(a) * 256u + (static_cast<uint32_t>(quad * 32) << 16);
       if (LEAN == 3) {
         // ---- residual stream: chunks grp*32 + k*64 of this tile; residual rows come from the load ring, results go out through two
-        // alternating store buffers
+        // alternating store buffers.  (Written here, not as a function beside the other two epilogues, with ResStream's steps as
+        // lambdas: every such move tried changed the generated code of this and of the generic TMA-store instantiations.)
         constexpr int NC = 32, NV = 4;
-        const uint32_t sw = (lane >> 1) & 3;
+        const uint32_t sw = chunk_swizzle<NC>(lane);
         const uint32_t row_off = static_cast<uint32_t>(lane) * (NC * 2);
         mbar_wait(tfull_bar(a), aphase);
         tc_fence_after();
@@ -755,51 +756,18 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
           {
             uint32_t src = lbuf0 + slot * static_cast<uint32_t>(nbox) * kOutStageBytes + row_off;
             if (p.stream_res) {
-#pragma unroll
-              for (int j = 0; j < NV; ++j)
-                asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(rr[j].x), "=r"(rr[j].y), "=r"(rr[j].z), "=r"(rr[j].w)
-                             : "r"(src + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
+              ld_row_swz<NV>(src, sw, rr);
               src += kOutStageBytes;
             }
-            if (p.stream_mask) {
-#pragma unroll
-              for (int j = 0; j < NV; ++j)
-                asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(mm[j].x), "=r"(mm[j].y), "=r"(mm[j].z), "=r"(mm[j].w)
-                             : "r"(src + ((static_cast<uint32_t>(j) ^ sw) << 4)) : "memory");
-            }
+            if (p.stream_mask) ld_row_swz<NV>(src, sw, mm);
           }
           tmem_wait_ld();
           float v[NC];
 #pragma unroll
           for (int j = 0; j < NC; ++j) v[j] = __uint_as_float(r[j]);
-          if (s_bias) {
-#pragma unroll
-            for (int j = 0; j < NC; j += 4) {
-              const float4 bv = *reinterpret_cast<const float4*>(s_bias + nb + j);
-              v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-            }
-          } else if (p.bias) {
-#pragma unroll
-            for (int j = 0; j < NC; j += 4) {
-              const float4 bv = __ldg(reinterpret_cast<const float4*>(p.bias + nb + j));
-              v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-            }
-          }
-          if (rb) {
-#pragma unroll
-            for (int j = 0; j < NC; j += 4) {
-              const float4 bv = __ldg(reinterpret_cast<const float4*>(rb + nb + j));
-              v[j] += bv.x; v[j + 1] += bv.y; v[j + 2] += bv.z; v[j + 3] += bv.w;
-            }
-          }
-          if (p.stream_res) {
-#pragma unroll
-            for (int j = 0; j < NV; ++j) {
-              const float2 f0 = unpack_bf16(rr[j].x), f1 = unpack_bf16(rr[j].y), f2 = unpack_bf16(rr[j].z), f3 = unpack_bf16(rr[j].w);
-              v[8 * j + 0] += f0.x; v[8 * j + 1] += f0.y; v[8 * j + 2] += f1.x; v[8 * j + 3] += f1.y;
-              v[8 * j + 4] += f2.x; v[8 * j + 5] += f2.y; v[8 * j + 6] += f3.x; v[8 * j + 7] += f3.y;
-            }
-          }
+          add_bias<NC>(v, s_bias, p, rb, nb);
+          if (p.stream_res) add_bf16_row<NV>(v, rr);
+          // ReLU / SiLU written out (no GELU layer takes the stream): relu_act<NC> here reorders two instructions of this kernel
           if (p.relu) {
 #pragma unroll
             for (int j = 0; j < NC; ++j) v[j] = fmaxf(v[j], 0.f);
@@ -808,28 +776,11 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
 #pragma unroll
             for (int j = 0; j < NC; ++j) v[j] = __fdividef(v[j], 1.f + __expf(-v[j]));
           }
-          if (p.stream_mask) {   // ReLU derivative of the forward activation (segmentor data gradients)
-#pragma unroll
-            for (int j = 0; j < NV; ++j) {
-              const float2 f0 = unpack_bf16(mm[j].x), f1 = unpack_bf16(mm[j].y), f2 = unpack_bf16(mm[j].z), f3 = unpack_bf16(mm[j].w);
-              if (!(f0.x > 0.f)) v[8 * j + 0] = 0.f;
-              if (!(f0.y > 0.f)) v[8 * j + 1] = 0.f;
-              if (!(f1.x > 0.f)) v[8 * j + 2] = 0.f;
-              if (!(f1.y > 0.f)) v[8 * j + 3] = 0.f;
-              if (!(f2.x > 0.f)) v[8 * j + 4] = 0.f;
-              if (!(f2.y > 0.f)) v[8 * j + 5] = 0.f;
-              if (!(f3.x > 0.f)) v[8 * j + 6] = 0.f;
-              if (!(f3.y > 0.f)) v[8 * j + 7] = 0.f;
-            }
-          }
+          if (p.stream_mask) mask_bf16_row<NV>(v, mm);   // ReLU derivative of the forward activation (segmentor data gradients)
           if (lane == 0) tma_store_wait_read<1>();   // the store that read this store buffer two chunks ago is done with it
           __syncwarp();
           const uint32_t dst = deep_base + rs.sbuf * kOutStageBytes;
-#pragma unroll
-          for (int j = 0; j < NV; ++j)
-            asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(dst + row_off + ((static_cast<uint32_t>(j) ^ sw) << 4)),
-                         "r"(pack_bf16(v[8 * j + 0], v[8 * j + 1])), "r"(pack_bf16(v[8 * j + 2], v[8 * j + 3])),
-                         "r"(pack_bf16(v[8 * j + 4], v[8 * j + 5])), "r"(pack_bf16(v[8 * j + 6], v[8 * j + 7])) : "memory");
+          st_row_swz<NV>(dst + row_off, sw, v);
           fence_proxy_async_smem();   // orders this lane's st.shared AND its earlier ld.shared of the load buffer before the async proxy
           __syncwarp();
           if (lane == 0) {
@@ -857,7 +808,7 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
       tc_fence_before();
       mbar_arrive(tempty_bar(a));
     }
-    if (TMA_OUT && lane == 0) tma_store_wait_read0();   // shared memory must outlive the last bulk store's read
+    if (TMA_OUT && lane == 0) tma_store_wait_read<0>();   // shared memory must outlive the last bulk store's read
   }
   tc_fence_before();
   __syncthreads();
@@ -867,36 +818,67 @@ igemm_kernel(const __grid_constant__ IgemmMaps maps, const __grid_constant__ Ige
   }
 }
 
-}  // namespace
+// ---- plan selection: row-segment mode, ring depth, residual staging and epilogue, all bound by the shared-memory layout above
+
+// One ring stage: the A box (a row segment for the row-segment window rowk = 3 / 9) and, unless the weights are resident, the B tiles
+// of its taps.  Stages stay 1024-byte aligned: BN is a multiple of 16 -> BN*128 is a multiple of 2048.
+uint32_t stage_bytes(int BN, int rowk, bool wres) {
+  return (rowk ? kRowABytes : kABytes) + (wres ? 0u : static_cast<uint32_t>(rowk ? rowk : 1) * static_cast<uint32_t>(BN) * kIgemmBK * 2);
+}
 
 // wres_bytes > 0: resident weights (that many bytes behind the ring), stages carry activations only; 16 KiB are then always
 // left for the second staging buffer of the lean epilogue
-int igemm_stages_for(int BN, int row3, int wres_bytes, int row_nkx) {
-  if (wres_bytes > 0) {
-    const uint32_t stage = row3 ? kRowABytes : kABytes;
-    int n = static_cast<int>((kPipeBytes - kOutStageBytes - static_cast<uint32_t>(wres_bytes)) / stage);
-    return n > kMaxStages ? kMaxStages : n;
-  }
-  const uint32_t stage = (row3 ? kRowABytes : kABytes) + (row3 ? static_cast<uint32_t>(row_nkx) : 1u) * static_cast<uint32_t>(BN) * kIgemmBK * 2;
-  // stages must stay 1024-byte aligned: BN is a multiple of 16 -> BN*128 is a multiple of 2048
-  int n = static_cast<int>(kPipeBytes / stage);
+int ring_stages(int BN, int rowk, int wres_bytes) {
+  const uint32_t room = wres_bytes > 0 ? kPipeBytes - kOutStageBytes - static_cast<uint32_t>(wres_bytes) : kPipeBytes;
+  const int n = static_cast<int>(room / stage_bytes(BN, rowk, wres_bytes > 0));
   return n > kMaxStages ? kMaxStages : n;
 }
 
-int igemm_res_deep_stages(int BN, int nl) {
-  const uint32_t stage = kABytes + static_cast<uint32_t>(BN) * kIgemmBK * 2;
+// true if 16 KiB stay free behind `nstages` stages of the TMA ring (room for the residual staging of the TMA epilogue)
+bool res_staging_fits(int BN, int rowk, int nstages, int wres_bytes) {
+  return static_cast<uint32_t>(nstages) * stage_bytes(BN, rowk, wres_bytes > 0) + static_cast<uint32_t>(wres_bytes) + kOutStageBytes <= kPipeBytes;
+}
+
+// ring depth left (plain mode) when the residual stream epilogue takes 2 store + nl load blocks of 16 KiB from the tail of the ring
+int res_deep_stages(int BN, int nl) {
   const uint32_t cap = kPipeBytes + kOutStageBytes - static_cast<uint32_t>(2 + nl) * kOutStageBytes;
-  int n = static_cast<int>(cap / stage);
+  const int n = static_cast<int>(cap / stage_bytes(BN, 0, false));
   return n > kMaxStages ? kMaxStages : n;
 }
 
-bool igemm_res_staging_fits(int BN, int row3, int nstages, int wres_bytes, int row_nkx) {
-  const uint32_t stage = (row3 ? kRowABytes : kABytes) + (wres_bytes > 0 ? 0u : (row3 ? static_cast<uint32_t>(row_nkx) : 1u) * static_cast<uint32_t>(BN) * kIgemmBK * 2);
-  return static_cast<uint32_t>(nstages) * stage + static_cast<uint32_t>(wres_bytes > 0 ? wres_bytes : 0) + kOutStageBytes <= kPipeBytes;
+// Residual stream epilogue (LEAN == 3) for layers with a residual input and a short main loop: K <= 768, plain mode, no ReLU mask,
+// no PReLU / GELU, full N tiles that are multiples of 64.  Layers with a ReLU-mask input (segmentor data gradients) stream the mask
+// rows the same way.
+constexpr int kStreamLoadSlots = 3;   // load buffers per epilogue warp (fewer when the ring would get too short)
+constexpr int kStreamMaxKb = 12;      // longest main loop (in 64-channel blocks) that still takes the stream epilogue (12 / 16 / 40 /
+                                      // unlimited measured equal on C3: 21.30 - 21.32 ms)
+constexpr int kStreamMinStages = 2;   // these layers are epilogue-bound: a short ring suffices
+bool apply_res_deep(IgemmArgs& a, bool res_map, bool mask_map) {
+  if (!a.tma_store || a.row3 || a.prelu || a.act == 3 || a.phase_n || a.total_kb > kStreamMaxKb || a.BN % 64 != 0 ||
+      a.N % a.BN != 0 || a.out_mode != kOutNHWC)
+    return false;
+  if (a.res && !res_map) return false;             // a residual that cannot go through TMA
+  if (a.mask && !mask_map) return false;
+  const int nbox = (a.res ? 1 : 0) + (a.mask ? 1 : 0);
+  if (nbox == 0) return false;
+  for (int nl = kStreamLoadSlots; nl >= 2; --nl) {
+    const int ns = res_deep_stages(a.BN, nl * nbox);
+    if (ns >= 2 && ns >= (a.total_kb < kStreamMinStages ? a.total_kb + 1 : kStreamMinStages)) {
+      a.res_deep = nl;
+      a.stream_res = a.res ? 1 : 0;
+      a.stream_mask = a.mask ? 1 : 0;
+      a.nstages = ns;
+      a.tma_res = a.res ? 1 : 0;
+      a.stage2 = 1;
+      a.lean = 3;
+      return true;
+    }
+  }
+  return false;
 }
 
 template <int ROWK, bool TMA_OUT, bool TMA_RES, int LEAN = 0>
-static int launch_variant(const IgemmPlan& plan, cudaStream_t stream) {
+int launch_variant(const IgemmPlan& plan, cudaStream_t stream) {
   static bool attr_set = false;
   if (!attr_set) {
     WC_CHECK_CUDA(cudaFuncSetAttribute(igemm_kernel<ROWK, TMA_OUT, TMA_RES, LEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
@@ -906,22 +888,41 @@ static int launch_variant(const IgemmPlan& plan, cudaStream_t stream) {
   return 0;
 }
 
+// The instantiation for a plain or 3 x 3 row-segment plan: lean (TMA residual or none), else generic with per-lane stores / TMA
+// store / TMA store + TMA residual
+template <int ROWK>
+IgemmLaunchFn pick_variant(const IgemmArgs& a) {
+  if (a.lean) return a.tma_res ? launch_variant<ROWK, true, true, 1> : launch_variant<ROWK, true, false, 1>;
+  if (!a.tma_store) return launch_variant<ROWK, false, false>;
+  return a.tma_res ? launch_variant<ROWK, true, true> : launch_variant<ROWK, true, false>;
+}
+
+}  // namespace
+
+void igemm_select(IgemmPlan* plan, int window, int wres_bytes, bool res_map, bool mask_map, bool stream) {
+  IgemmArgs& a = plan->args;
+  // (for a 3 x 3 window BN <= 128 always leaves at least three stages; the 1 x 9 window needs BN <= 64 for two)
+  a.row3 = window != 0 && a.BN <= 128 && ring_stages(a.BN, window, 0) >= 2 ? 1 : 0;
+  const int rowk = a.row3 ? window : 0;
+  a.row_nkx = rowk;
+  a.wres = a.row3 && wres_bytes > 0 ? 1 : 0;
+  if (!a.wres) wres_bytes = 0;
+  a.nstages = ring_stages(a.BN, rowk, wres_bytes);
+  a.stage2 = res_staging_fits(a.BN, rowk, a.nstages, wres_bytes) ? 1 : 0;
+  a.tma_res = res_map && a.stage2 ? 1 : 0;
+  a.lean = (a.tma_store && !a.mask && (!a.res || a.tma_res)) ? 1 : 0;
+  if (stream && apply_res_deep(a, res_map, mask_map)) plan->launch = launch_variant<0, true, true, 3>;
+  else if (rowk == 9) plan->launch = a.lean ? launch_variant<9, true, false, 1> : launch_variant<9, false, false>;
+  else if (rowk == 3) plan->launch = pick_variant<3>(a);
+  else plan->launch = pick_variant<0>(a);
+}
+
 int igemm_launch(const IgemmPlan& plan, cudaStream_t stream) {
   ProfScope prof(kProfIgemm, stream, plan.flops);
   prof.note(plan.args.B * plan.args.H * plan.args.W, plan.args.N, plan.args.total_kb * kIgemmBK, plan.args.BN, plan.args.ntaps + 100 * plan.args.row3 + 1000 * (plan.args.lean != 0) + 32000 * (plan.args.lean == 3) + 2000 * (plan.args.mask != nullptr) + 4000 * (plan.args.res != nullptr) +
                 8000 * (plan.args.out_mode != kOutNHWC) + 16000 * (plan.args.tma_store == 0), plan.grid);
-  const int variant = plan.args.tma_store ? (plan.args.tma_res ? 2 : 1) : 0;   // epilogue: per-lane stores / TMA store / TMA store + TMA residual
-  int e = 0;
-  if (plan.args.row3 && plan.args.row_nkx == 9) {   // 1 x 9 row-segment mode (build_conv_hrow): fp32 planes, lean or generic epilogue
-    e = plan.args.lean ? launch_variant<9, true, false, 1>(plan, stream) : launch_variant<9, false, false>(plan, stream);
-  } else if (plan.args.lean == 3) {
-    e = launch_variant<0, true, true, 3>(plan, stream);
-  } else if (plan.args.lean) {
-    if (plan.args.row3) e = plan.args.tma_res ? launch_variant<3, true, true, 1>(plan, stream) : launch_variant<3, true, false, 1>(plan, stream);
-    else e = plan.args.tma_res ? launch_variant<0, true, true, 1>(plan, stream) : launch_variant<0, true, false, 1>(plan, stream);
-  } else if (plan.args.row3) e = variant == 2 ? launch_variant<3, true, true>(plan, stream) : variant == 1 ? launch_variant<3, true, false>(plan, stream) : launch_variant<3, false, false>(plan, stream);
-  else e = variant == 2 ? launch_variant<0, true, true>(plan, stream) : variant == 1 ? launch_variant<0, true, false>(plan, stream) : launch_variant<0, false, false>(plan, stream);
-  if (e) return e;
+  WC_REQUIRE(plan.launch, "igemm plan without a kernel: igemm_select was not run");
+  if (int e = plan.launch(plan, stream)) return e;
   WC_LAUNCH_CHECK();
   return 0;
 }

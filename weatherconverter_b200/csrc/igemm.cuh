@@ -9,7 +9,7 @@
 //   a ResNet sub-layer is simply one more tap reading a different tensor.
 // * B (weights) are pre-packed bf16 [Npad][Ktotal] K-major, loaded with a 2-D tensor map (box 64 x BN).
 // * tcgen05.mma 128 x BN x 16 (cta_group::1), fp32 accumulators double-buffered in TMEM (2 x 256 columns).
-// * Persistent CTAs, 6 warps: warp 0 TMA producer, warp 1 MMA issuer (+TMEM alloc), warps 2-5 epilogue
+// * Persistent CTAs, 10 warps: warp 0 TMA producer, warp 1 MMA issuer (+TMEM alloc), warps 2-9 epilogue
 //   (TMEM -> registers -> bias / t-emb / residual / ReLU -> bf16 stores), so the epilogue of tile i overlaps
 //   the main loop of tile i+1.
 #pragma once
@@ -17,7 +17,6 @@
 
 namespace wc {
 
-constexpr int kIgemmStages = 4;
 constexpr int kIgemmBM = 128;
 constexpr int kIgemmBK = 64;
 constexpr int kMaxTaps = 20;
@@ -37,7 +36,7 @@ struct IgemmArgs {
   int tb, th, tw;  // tile shape, tb*th*tw == 128
   int N, BN;       // true output channels (multiple of 16) and N tile
   int ntaps, total_kb;
-  int nstages;  // depth of the TMA ring (set by igemm_stages_for)
+  int nstages;  // depth of the TMA ring (set by igemm_select)
   int row3;  // 1: taps 0..8 form a 3x3 stride-1 window executed in row-segment mode (see igemm.cu)
   IgemmTap taps[kMaxTaps];
   // epilogue
@@ -59,7 +58,7 @@ struct IgemmArgs {
   __nv_bfloat16 *q, *k, *vt;  // kOutQKV: Q,K [B,heads,ntok,hd]; V^T [B,heads,hd,ntok]
   __nv_bfloat16* v;           // kOutQKV, optional: V [B,heads,ntok,hd] as well (the attention backward reads it)
   int heads, hd, C;
-  int row_nky, row_nkx;        // row-segment mode: the window is row_nky x row_nkx taps (3 x 3, or 1 x 9 for build_conv_hrow)
+  int row_nkx;                 // row-segment mode: width of the window (3: 3 x 3, 9: 1 x 9 for build_conv_hrow)
   int phase_n;                 // > 0: kOutNHWC through the lean epilogue with four phase blocks of phase_n channels (maps c, qkv[0..2])
   int res_deep;                // LEAN == 3: load slots per epilogue warp of the residual / mask stream (igemm.cu)
   int stream_res, stream_mask; // LEAN == 3: which boxes a slot carries (residual rows, ReLU-mask rows)
@@ -88,19 +87,26 @@ struct IgemmMaps {
   CUtensorMap qkv[3];   // kOutQKV through the lean epilogue: Q, K as (hd, N, heads, B), V^T as (N, hd, heads, B)
 };
 
+struct IgemmPlan;
+using IgemmLaunchFn = int (*)(const IgemmPlan&, cudaStream_t);
+
 struct IgemmPlan {
   IgemmMaps maps;
   IgemmArgs args;
   int grid = 0;
   double flops = 0;  // algorithmic FLOPs (2*MAC) of the convolution this plan implements
+  IgemmLaunchFn launch = nullptr;  // the igemm_kernel instantiation igemm_select chose
 };
 
+// Completes a plan whose taps, tile, BN, epilogue inputs and output maps are set: row-segment mode, ring depth, residual staging,
+// epilogue (generic, lean or residual stream) and the kernel instantiation igemm_launch runs.
+//   window:     the row-segment window the builder encoded IgemmMaps::a[2] for: 0 none, 3 (3 x 3) or 9 (1 x 9); taken when
+//               BN <= 128 and two ring stages fit
+//   wres_bytes: > 0: keep that many bytes of packed weights resident in shared memory if the window is taken
+//   res_map / mask_map: IgemmMaps::r / ::m were encoded (residual / ReLU-mask rows can be loaded through TMA)
+//   stream:     the residual stream epilogue may be chosen
+void igemm_select(IgemmPlan* plan, int window, int wres_bytes, bool res_map, bool mask_map, bool stream);
 int igemm_launch(const IgemmPlan& plan, cudaStream_t stream);
-int igemm_stages_for(int BN, int row3, int wres_bytes = 0, int row_nkx = 3);
-// true if 16 KiB stay free behind `nstages` stages of the TMA ring (room for the residual staging of the TMA epilogue)
-bool igemm_res_staging_fits(int BN, int row3, int nstages, int wres_bytes = 0, int row_nkx = 3);
-// ring depth left (plain mode) when the residual stream epilogue takes 2 store + nl load blocks of 16 KiB from the tail of the ring
-int igemm_res_deep_stages(int BN, int nl);
 
 // Choose the M-tile shape for a (B,H,W) grid: widest power-of-two span of x, then y, then b.
 void igemm_pick_tile(int B, int H, int W, int* tb, int* th, int* tw);
