@@ -191,13 +191,18 @@ int wc_attention_bwd(const wc_bf16* q, const wc_bf16* k, const wc_bf16* v, const
  * nn.ConvTranspose2d (transposed != 0, stride 2: dw [Cin,Cout,K,K]); x [B,H,W,Cin], dy on the output grid. */
 int wc_conv2d_wgrad(const wc_bf16* x, const wc_bf16* dy, int batch, int H, int W, int Cin, int Cout, int K, int stride, int pad,
                     int dil, int transposed, const wc_bf16* x2, int Cin2, float* dw, float* dw2, void* stream);
-/* Backward of wc_groupnorm_silu: fwd_workspace is the workspace the forward call filled; dx = dGN(dy) (+add1) (+add2). */
+/* Backward of wc_groupnorm_silu: fwd_workspace is the workspace the forward call filled; dx = dGN(dy) (+add1) (+add2).
+ * ldx, ldd, ldo, lda1, lda2: pixel strides (elements, multiples of 8) of x, dy, dx, add1, add2; add2 may alias dx (in-place
+ * accumulation, lda2 == ldo).  dgamma, dbeta fp32 [C] are overwritten. */
 size_t wc_groupnorm_bwd_workspace_bytes(int batch, int channels);
-int wc_groupnorm_silu_bwd(const wc_bf16* x, const wc_bf16* dy, wc_bf16* dx, int batch, int hw, int channels, const float* gamma,
-                          const float* beta, float eps, int silu, const void* fwd_workspace, const wc_bf16* add1,
-                          const wc_bf16* add2, float* dgamma, float* dbeta, void* workspace, void* stream);
-/* Column sums of x [B,hw,C]: out_rows [B,C] (may be NULL), out_total [C] (may be NULL): bias / t-embedding gradients. */
-int wc_colsum(const wc_bf16* x, int batch, int hw, int channels, float* out_rows, float* out_total, void* workspace, void* stream);
+int wc_groupnorm_silu_bwd(const wc_bf16* x, const wc_bf16* dy, wc_bf16* dx, int batch, int hw, int channels, int ldx, int ldd,
+                          int ldo, const float* gamma, const float* beta, float eps, int silu, const void* fwd_workspace,
+                          const wc_bf16* add1, int lda1, const wc_bf16* add2, int lda2, float* dgamma, float* dbeta,
+                          void* workspace, void* stream);
+/* Column sums of x [B,hw,C] (pixel stride ldx, a multiple of 8): out_rows[b*ldo + c] (may be NULL), out_total [C] (may be
+ * NULL): bias / t-embedding gradients.  workspace >= wc_groupnorm_bwd_workspace_bytes(batch, channels). */
+int wc_colsum(const wc_bf16* x, int batch, int hw, int channels, int ldx, float* out_rows, int ldo, float* out_total,
+              void* workspace, void* stream);
 /* nn.MSELoss (train_ddpm.py:107): loss = mean((pred-target)^2), dpred = grad_scale * 2 (pred-target)/n. scratch: 8 KiB. */
 int wc_mse_loss_grad(const float* pred, const float* target, float* dpred, size_t n, float grad_scale, float* loss, void* scratch,
                      void* stream);

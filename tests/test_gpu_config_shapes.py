@@ -153,8 +153,10 @@ def test_c3_geometry_a_two_guided_steps_and_batch_invariance():
 
 
 def test_c5_training_step_128x256():
-    """Loss and gradients of the training step at the C5 geometry (batch 2 instead of 64: same kernels and tile shapes per
-    image; the fp32 oracle's autograd pass over 2 images takes tens of seconds on the host)."""
+    """Loss and gradients of the training step at the C5 geometry, at batch 2 instead of 64 (the fp32 oracle's autograd pass over
+    2 images takes tens of seconds on the host).  The kernels and tile shapes per image are those of batch 64 except the
+    GroupNorm backward and the column sums, whose split counts depend on the batch (32 blocks per sample at batch 2, 19 at
+    batch 64 for 128x256 maps); tests/test_gpu_groupnorm.py checks those at batch 64 against float64."""
     from oracle.scheduler import OracleScheduler
     from oracle.train import train_step
     from oracle.unet import DEFAULT_MODEL_CONFIG

@@ -65,34 +65,10 @@ def test_conv2d_wgrad(Cin, Cout, H, W, K, stride, dil, transposed, B, Cin2):
     assert _rel(got, w.grad) < 1e-4, _rel(got, w.grad)     # same bf16 inputs, fp32 accumulation on both sides
 
 
-@pytest.mark.parametrize("C,H,W,silu,B", [(64, 16, 16, True, 2), (128, 8, 32, False, 3), (768, 4, 8, True, 2), (1024, 16, 32, True, 1)])
-def test_groupnorm_silu_bwd(C, H, W, silu, B):
-    from weatherconverter_b200 import ops
-    dev = _dev()
-    g = torch.Generator(device="cpu").manual_seed(C + H)
-    x = _bf(torch.randn(B, C, H, W, generator=g) * 1.5 + 0.3).to(dev).requires_grad_(True)
-    gamma = (1 + 0.2 * torch.randn(C, generator=g)).to(dev).requires_grad_(True)
-    beta = (0.2 * torch.randn(C, generator=g)).to(dev).requires_grad_(True)
-    dy = _bf(torch.randn(B, C, H, W, generator=g)).to(dev)
-    a1 = _bf(torch.randn(B, C, H, W, generator=g)).to(dev)
-    y = F.group_norm(x, 8, gamma, beta, 1e-5)
-    if silu:
-        y = F.silu(y)
-    y.backward(dy)
-    _, dx, dg, db = ops.groupnorm_silu_fwd_bwd(ops.to_nhwc_bf16(x.detach()), gamma.detach(), beta.detach(), ops.to_nhwc_bf16(dy),
-                                               silu=silu, add1=ops.to_nhwc_bf16(a1))
-    assert _rel(ops.to_nchw_f32(dx), x.grad + a1) < 6e-3
-    assert _rel(dg, gamma.grad) < 2e-3, _rel(dg, gamma.grad)
-    assert _rel(db, beta.grad) < 2e-3, _rel(db, beta.grad)
-
-
-def test_colsum_mse_boundary_adam():
+def test_mse_boundary_adam():
     from weatherconverter_b200 import ops
     dev = _dev()
     g = torch.Generator(device="cpu").manual_seed(5)
-    x = _bf(torch.randn(3, 2304, 8, 16, generator=g)).to(dev)
-    rows, tot = ops.colsum(ops.to_nhwc_bf16(x))
-    assert _rel(rows, x.sum((2, 3))) < 1e-5 and _rel(tot, x.sum((0, 2, 3))) < 1e-5
     # MSE
     pred, tgt = torch.randn(2, 3, 32, 64, generator=g).to(dev), torch.randn(2, 3, 32, 64, generator=g).to(dev)
     pr = pred.clone().requires_grad_(True)

@@ -74,8 +74,9 @@ _SIGS = {
     "wc_attention_bwd": (C.c_int, [c_ptr] * 8 + [C.c_int] * 4 + [c_ptr]),
     "wc_conv2d_wgrad": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 10 + [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr]),
     "wc_groupnorm_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
-    "wc_groupnorm_silu_bwd": (C.c_int, [c_ptr] * 3 + [C.c_int] * 3 + [c_ptr, c_ptr, C.c_float, C.c_int] + [c_ptr] * 7),
-    "wc_colsum": (C.c_int, [c_ptr] + [C.c_int] * 3 + [c_ptr] * 4),
+    "wc_groupnorm_silu_bwd": (C.c_int, [c_ptr] * 3 + [C.c_int] * 6 + [c_ptr, c_ptr, C.c_float, C.c_int, c_ptr, c_ptr, C.c_int,
+                                                                           c_ptr, C.c_int] + [c_ptr] * 4),
+    "wc_colsum": (C.c_int, [c_ptr] + [C.c_int] * 4 + [c_ptr, C.c_int] + [c_ptr] * 3),
     "wc_mse_loss_grad": (C.c_int, [c_ptr] * 3 + [C.c_size_t, C.c_float, c_ptr, c_ptr, c_ptr]),
     "wc_boundary_wgrad_scratch_bytes": (C.c_size_t, []),
     "wc_boundary_wgrad": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 4 + [c_ptr] * 4),

@@ -432,6 +432,7 @@ int groupnorm_silu(const __nv_bfloat16* x, __nv_bfloat16* y, int B, int HW, int 
   launch_k(gn_apply_kernel, dim3(asplit, B), threads, 0, st, x, y, HW, C, ld, ldy, nsplit, asplit, partial, gamma, beta, eps,
                                                        silu);
   WC_LAUNCH_CHECK();
+  prof.note(HW, C, ld, ldy, nsplit, asplit);
   return 0;
 }
 
@@ -488,6 +489,8 @@ int groupnorm_silu_bwd(const __nv_bfloat16* x, const __nv_bfloat16* dy, __nv_bfl
   launch_k(gn_bwd_apply_kernel, dim3(asplit, B), threads, 0, st, x, dy, dx, HW, C, ld, ldd, ldo, ns_stats, asplit, partial, gs, gamma,
                                                            beta, eps, silu, add1, lda1, add2, lda2);
   WC_LAUNCH_CHECK();
+  // strides < 2^16 (C <= 2048 and concat buffers of at most 2C); a missing add term notes stride 0
+  prof.note(HW, C, ld | ldd << 16, ldo | (add1 ? lda1 : 0) << 16, add2 ? lda2 : 0, nsplit | asplit << 16);
   return 0;
 }
 
@@ -508,6 +511,8 @@ int colsum(const __nv_bfloat16* x, int B, int HW, int C, int ld, float* out_rows
   WC_LAUNCH_CHECK();
   launch_k(colsum_finish_kernel, (C + 63) / 64, 512, 0, st, part, B, C, nsplit, out_rows, ldo, out_total);
   WC_LAUNCH_CHECK();
+  // the last field tags the record (class kProfOther is shared): 1 + which outputs are written (2: rows, 4: total)
+  prof.note(HW, C, ld, out_rows ? ldo : 0, nsplit, 1 + (out_rows ? 2 : 0) + (out_total ? 4 : 0));
   return 0;
 }
 

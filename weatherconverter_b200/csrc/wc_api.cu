@@ -91,7 +91,7 @@ static inline const __nv_bfloat16* BF(const wc_bf16* p) { return reinterpret_cas
 extern "C" {
 
 const char* wc_last_error(void) { return last_error_cstr(); }
-int wc_abi_version(void) { return 6; }
+int wc_abi_version(void) { return 7; }
 long long wc_launch_count(void) { return launch_count(); }
 void wc_profile_begin(void) { prof_start(); }
 int wc_profile_detail(int cap, int* cls, double* ms, double* work, int* info) { return prof_detail(cap, cls, ms, work, info); }
@@ -300,14 +300,16 @@ int wc_conv2d_wgrad(const wc_bf16* x, const wc_bf16* dy, int batch, int H, int W
 }
 
 size_t wc_groupnorm_bwd_workspace_bytes(int batch, int channels) { return groupnorm_bwd_workspace_bytes(batch, channels); }
-int wc_groupnorm_silu_bwd(const wc_bf16* x, const wc_bf16* dy, wc_bf16* dx, int batch, int hw, int channels, const float* gamma,
-                          const float* beta, float eps, int silu, const void* fwd_workspace, const wc_bf16* add1,
-                          const wc_bf16* add2, float* dgamma, float* dbeta, void* workspace, void* stream) {
-  return groupnorm_silu_bwd(BF(x), BF(dy), BF(dx), batch, hw, channels, channels, channels, channels, gamma, beta, eps, silu,
-                            fwd_workspace, BF(add1), channels, BF(add2), channels, dgamma, dbeta, workspace, S(stream));
+int wc_groupnorm_silu_bwd(const wc_bf16* x, const wc_bf16* dy, wc_bf16* dx, int batch, int hw, int channels, int ldx, int ldd,
+                          int ldo, const float* gamma, const float* beta, float eps, int silu, const void* fwd_workspace,
+                          const wc_bf16* add1, int lda1, const wc_bf16* add2, int lda2, float* dgamma, float* dbeta,
+                          void* workspace, void* stream) {
+  return groupnorm_silu_bwd(BF(x), BF(dy), BF(dx), batch, hw, channels, ldx, ldd, ldo, gamma, beta, eps, silu, fwd_workspace,
+                            BF(add1), lda1, BF(add2), lda2, dgamma, dbeta, workspace, S(stream));
 }
-int wc_colsum(const wc_bf16* x, int batch, int hw, int channels, float* out_rows, float* out_total, void* workspace, void* stream) {
-  return colsum(BF(x), batch, hw, channels, channels, out_rows, channels, out_total, workspace, S(stream));
+int wc_colsum(const wc_bf16* x, int batch, int hw, int channels, int ldx, float* out_rows, int ldo, float* out_total,
+              void* workspace, void* stream) {
+  return colsum(BF(x), batch, hw, channels, ldx, out_rows, ldo, out_total, workspace, S(stream));
 }
 int wc_mse_loss_grad(const float* pred, const float* target, float* dpred, size_t n, float grad_scale, float* loss, void* scratch,
                      void* stream) {

@@ -34,7 +34,7 @@ def groupnorm_silu(x, gamma, beta, silu=True, eps=1e-5):
     B, H, W, Cc = x.shape
     y = torch.empty(B, H, W, Cc, device=x.device, dtype=torch.bfloat16)
     ws = torch.empty(lib().wc_groupnorm_workspace_bytes(B), device=x.device, dtype=torch.uint8)
-    check(lib().wc_groupnorm_silu(ptr(x), ptr(y), B, H * W, Cc, x.stride(2), Cc, ptr(gamma), ptr(beta), eps,
+    check(lib().wc_groupnorm_silu(ptr(x), ptr(y), B, H * W, Cc, pixel_stride(x), Cc, ptr(gamma), ptr(beta), eps,
                                   1 if silu else 0, ptr(ws), stream_ptr()))
     return y
 
@@ -166,35 +166,42 @@ def conv2d_wgrad(x, dy, K, stride=1, pad=None, dil=1, transposed=False, x2=None)
     return (dw, dw2) if x2 is not None else dw
 
 
+def pixel_stride(x):
+    """Pixel stride (elements) of an NHWC view [B,H,W,C] whose pixels are evenly spaced: a contiguous tensor or a channel slice
+    of a wider one."""
+    B, H, W, Cc = x.shape
+    assert x.stride(3) == 1 and x.stride(1) == W * x.stride(2) and x.stride(0) == H * x.stride(1), x.stride()
+    return x.stride(2)
+
+
 def groupnorm_silu_fwd_bwd(x, gamma, beta, dy, silu=True, eps=1e-5, add1=None, add2=None):
-    """Forward + backward of GroupNorm(8)[+SiLU]; returns (y, dx, dgamma, dbeta)."""
+    """Forward + backward of GroupNorm(8)[+SiLU]; returns (y, dx, dgamma, dbeta).  x, dy, add1, add2 may be channel slices."""
     require_cuda(x, gamma, beta, dy)
     B, H, W, Cc = x.shape
-    x, dy = x.contiguous(), dy.contiguous()
-    y = torch.empty_like(x)
+    y = torch.empty(B, H, W, Cc, device=x.device, dtype=torch.bfloat16)
     ws = torch.empty(lib().wc_groupnorm_workspace_bytes(B), device=x.device, dtype=torch.uint8)
-    check(lib().wc_groupnorm_silu(ptr(x), ptr(y), B, H * W, Cc, Cc, Cc, ptr(gamma), ptr(beta), eps, 1 if silu else 0,
+    check(lib().wc_groupnorm_silu(ptr(x), ptr(y), B, H * W, Cc, pixel_stride(x), Cc, ptr(gamma), ptr(beta), eps, 1 if silu else 0,
                                   ptr(ws), stream_ptr()))
-    dx = torch.empty_like(x)
+    dx = torch.empty_like(y)
     dg = torch.empty(Cc, device=x.device, dtype=torch.float32)
     db = torch.empty(Cc, device=x.device, dtype=torch.float32)
     ws2 = torch.empty(lib().wc_groupnorm_bwd_workspace_bytes(B, Cc), device=x.device, dtype=torch.uint8)
-    add1 = add1.contiguous() if add1 is not None else None
-    add2 = add2.contiguous() if add2 is not None else None
-    check(lib().wc_groupnorm_silu_bwd(ptr(x), ptr(dy), ptr(dx), B, H * W, Cc, ptr(gamma), ptr(beta), eps, 1 if silu else 0,
-                                      ptr(ws), ptr(add1), ptr(add2), ptr(dg), ptr(db), ptr(ws2), stream_ptr()))
+    lda1 = pixel_stride(add1) if add1 is not None else 8
+    lda2 = pixel_stride(add2) if add2 is not None else 8
+    check(lib().wc_groupnorm_silu_bwd(ptr(x), ptr(dy), ptr(dx), B, H * W, Cc, pixel_stride(x), pixel_stride(dy), Cc, ptr(gamma),
+                                      ptr(beta), eps, 1 if silu else 0, ptr(ws), ptr(add1), lda1, ptr(add2), lda2, ptr(dg), ptr(db),
+                                      ptr(ws2), stream_ptr()))
     return y, dx, dg, db
 
 
 def colsum(x):
-    """x [B,H,W,C] bf16 -> (per-sample sums [B,C] fp32, total [C] fp32)."""
+    """x [B,H,W,C] bf16 (may be a channel slice) -> (per-sample sums [B,C] fp32, total [C] fp32)."""
     require_cuda(x)
     B, H, W, Cc = x.shape
-    x = x.contiguous()
     rows = torch.empty(B, Cc, device=x.device, dtype=torch.float32)
     tot = torch.empty(Cc, device=x.device, dtype=torch.float32)
     ws = torch.empty(lib().wc_groupnorm_bwd_workspace_bytes(B, Cc), device=x.device, dtype=torch.uint8)
-    check(lib().wc_colsum(ptr(x), B, H * W, Cc, ptr(rows), ptr(tot), ptr(ws), stream_ptr()))
+    check(lib().wc_colsum(ptr(x), B, H * W, Cc, pixel_stride(x), ptr(rows), Cc, ptr(tot), ptr(ws), stream_ptr()))
     return rows, tot
 
 
